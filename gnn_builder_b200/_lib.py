@@ -52,6 +52,7 @@ EXPORTS = [
     "gnnb_pool_partial",
     "gnnb_halo_pack", "gnnb_halo_pack_ranges", "gnnb_halo_signal", "gnnb_halo_wait", "gnnb_ipc_alloc", "gnnb_ipc_open",
     "gnnb_ipc_close", "gnnb_ipc_free", "gnnb_mark_hub_sources", "gnnb_gcn_conv_halo",
+    "gnnb_gin_conv_halo", "gnnb_sage_conv_halo", "gnnb_pna_conv_halo",
 ]
 # include/gnnb_b200_debug.h: tcgen05 probes in libgnnb_b200_debug.so (tests / tools only)
 DEBUG_LIB_PATH = PKG / "libgnnb_b200_debug.so"
@@ -130,6 +131,12 @@ def load(build_if_missing: bool = True) -> C.CDLL:
     lib.gnnb_mark_hub_sources.argtypes = [vp, ci, ci, ci, C.c_int64, C.POINTER(ci), vp]
     lib.gnnb_gcn_conv_halo.argtypes = [ci, ci, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, ci, ci,
                                        ci, ci, ci, ci, ci, vp]
+    lib.gnnb_gin_conv_halo.argtypes = [ci, ci, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, cf, vp,
+                                       ci, ci, ci, ci, ci, ci, vp]
+    lib.gnnb_sage_conv_halo.argtypes = [ci, ci, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, ci,
+                                        ci, ci, ci, ci, vp]
+    lib.gnnb_pna_conv_halo.argtypes = [ci, ci, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp,
+                                       vp, vp, cf, vp, ci, ci, ci, ci, vp]
     lib.gnnb_partition_tables.argtypes = [vp, ci, ci, ci, vp, vp, vp, vp]
     lib.gnnb_degree_inv_sqrt.argtypes = [vp, vp, ci, vp]
     lib.gnnb_pool_partial.argtypes = [vp, C.c_int64, ci, vp, vp]

@@ -537,6 +537,146 @@ int launch_pna_agg(const PnaAggArgs &a, cudaStream_t s, int *launches)
     return GNNB_OK;
 }
 
+// ------------------------------------------------------------------------------ PNA, split CSR
+//
+// The row-partitioned form of pna_agg_kernel: the in-edges of an owned row come in two parts, the
+// owned-source edges and then the halo-source edges, and A_u is read from ext space (owned rows,
+// then the A rows the owners sent).  One running sample count spans both parts, so max/min take
+// the first sample of the combined order (lib:748-752, 784-788) and the Welford update (lib:693-695)
+// runs over it as if the row's neighbor list were the concatenation; mean, std and the degree
+// scalers use the row's full in-degree (= own + halo count), and in-degree 0 gives std = NaN like
+// lib:702.
+namespace {
+
+template <int VEC>
+__device__ __forceinline__ void store_scaled(const Vec<VEC> &x, float scale, float *p)
+{
+    Vec<VEC> o;
+#pragma unroll
+    for (int i = 0; i < VEC; i++) o.v[i] = __fmul_rn(scale, x.v[i]);
+    o.store(p);
+}
+
+template <int VEC>
+__device__ __forceinline__ void pna_halo_part(const PnaHaloArgs &a, const int32_t *nbr, int off, int len,
+                                              int c, const Vec<VEC> &b, int &cnt, Vec<VEC> &vmax,
+                                              Vec<VEC> &vmin, Vec<VEC> &vsum, Vec<VEC> &wmean,
+                                              Vec<VEC> &wm2)
+{
+    for (int k = 0; k < len; k++) {
+        const int u = __ldg(nbr + off + k) & 0x7fffffff;   // hub marks carry no index bits
+        Vec<VEC> t;
+        t.load(a.a_ext + (size_t)u * a.F + c);
+        const bool first = cnt == 0;
+        cnt++;
+        const float fc = (float)cnt;
+#pragma unroll
+        for (int i = 0; i < VEC; i++) {
+            const float tv = __fadd_rn(t.v[i], b.v[i]);
+            vmax.v[i] = (first || tv > vmax.v[i]) ? tv : vmax.v[i];
+            vmin.v[i] = (first || tv < vmin.v[i]) ? tv : vmin.v[i];
+            vsum.v[i] = __fadd_rn(vsum.v[i], tv);
+            const float d = __fsub_rn(tv, wmean.v[i]);
+            wmean.v[i] = __fadd_rn(wmean.v[i], __fdiv_rn(d, fc));
+            wm2.v[i] = __fadd_rn(wm2.v[i], __fmul_rn(d, __fsub_rn(tv, wmean.v[i])));
+        }
+    }
+}
+
+template <int VEC, int LPR>
+__global__ void __launch_bounds__(256) pna_halo_stats_kernel(const PnaHaloArgs a)
+{
+    constexpr int ROWS_PER_WARP = 32 / LPR;
+    const int lane = threadIdx.x & 31;
+    const int lg = lane % LPR, sub = lane / LPR;
+    const int warps_per_block = blockDim.x >> 5;
+    const int64_t warp_global = (int64_t)blockIdx.x * warps_per_block + (threadIdx.x >> 5);
+    const int64_t warp_stride = (int64_t)gridDim.x * warps_per_block;
+    const int F = a.F;
+    for (int64_t row0 = warp_global * ROWS_PER_WARP; row0 < a.n; row0 += warp_stride * ROWS_PER_WARP) {
+        const int v = (int)row0 + sub;
+        if (v >= a.n) continue;
+        const int deg = __ldg(a.in_deg + v);
+        const int own_off = __ldg(a.own_off + v), own_len = __ldg(a.own_cnt + v);
+        const int halo_off = a.halo_cnt != nullptr ? __ldg(a.halo_off + v) : 0;
+        const int halo_len = a.halo_cnt != nullptr ? __ldg(a.halo_cnt + v) : 0;
+        const int clamped = deg < 1 ? 1 : deg;
+        const float lg1 = logf((float)(clamped + 1));
+        const float amp = __fdiv_rn(lg1, a.delta), att = __fdiv_rn(a.delta, lg1);
+        for (int c = lg * VEC; c < F; c += LPR * VEC) {
+            Vec<VEC> b, vmax, vmin, vsum, wmean, wm2;
+            b.load(a.b + (size_t)v * F + c);
+#pragma unroll
+            for (int i = 0; i < VEC; i++) {
+                vmax.v[i] = 0.0f; vmin.v[i] = 0.0f; vsum.v[i] = 0.0f;
+                wmean.v[i] = 0.0f; wm2.v[i] = 0.0f;
+            }
+            int cnt = 0;
+            pna_halo_part<VEC>(a, a.own_nbr, own_off, own_len, c, b, cnt, vmax, vmin, vsum, wmean, wm2);
+            pna_halo_part<VEC>(a, a.halo_nbr, halo_off, halo_len, c, b, cnt, vmax, vmin, vsum, wmean, wm2);
+            Vec<VEC> mean, sd;
+#pragma unroll
+            for (int i = 0; i < VEC; i++) {
+                mean.v[i] = deg > 0 ? __fdiv_rn(vsum.v[i], (float)deg) : 0.0f;
+                const float var = __fdiv_rn(wm2.v[i], (float)deg);                 // lib:702
+                sd.v[i] = __fsqrt_rn(__fadd_rn(var, 1e-5f));                       // lib:703
+            }
+            float *dst = a.cat12 + (size_t)v * (a.compact ? 4 : 12) * F + c;
+            vmax.store(dst);
+            vmin.store(dst + F);
+            mean.store(dst + 2 * (size_t)F);
+            sd.store(dst + 3 * (size_t)F);
+            if (!a.compact) {   // [stats | amp stats | att stats], lib:1857-1875
+                store_scaled(vmax, amp, dst + 4 * (size_t)F);
+                store_scaled(vmin, amp, dst + 5 * (size_t)F);
+                store_scaled(mean, amp, dst + 6 * (size_t)F);
+                store_scaled(sd, amp, dst + 7 * (size_t)F);
+                store_scaled(vmax, att, dst + 8 * (size_t)F);
+                store_scaled(vmin, att, dst + 9 * (size_t)F);
+                store_scaled(mean, att, dst + 10 * (size_t)F);
+                store_scaled(sd, att, dst + 11 * (size_t)F);
+            }
+        }
+    }
+}
+
+template <int VEC>
+void launch_pna_halo_lpr(const PnaHaloArgs &a, int lpr, int grid, cudaStream_t s)
+{
+    switch (lpr) {
+    case 1: pna_halo_stats_kernel<VEC, 1><<<grid, 256, 0, s>>>(a); break;
+    case 2: pna_halo_stats_kernel<VEC, 2><<<grid, 256, 0, s>>>(a); break;
+    case 4: pna_halo_stats_kernel<VEC, 4><<<grid, 256, 0, s>>>(a); break;
+    case 8: pna_halo_stats_kernel<VEC, 8><<<grid, 256, 0, s>>>(a); break;
+    case 16: pna_halo_stats_kernel<VEC, 16><<<grid, 256, 0, s>>>(a); break;
+    default: pna_halo_stats_kernel<VEC, 32><<<grid, 256, 0, s>>>(a); break;
+    }
+}
+
+}  // namespace
+
+int launch_pna_halo_stats(const PnaHaloArgs &a, cudaStream_t s, int *launches)
+{
+    if (a.n <= 0) return GNNB_OK;
+    GNNB_REQUIRE(a.F > 0 && a.a_ext != nullptr && a.b != nullptr && a.cat12 != nullptr,
+                 "pna halo statistics: bad arguments");
+    const bool v4 = (a.F % 4 == 0) && aligned16(a.a_ext) && aligned16(a.b) && aligned16(a.cat12);
+    const int vec = v4 ? 4 : 1;
+    int lpr = 1;
+    while (lpr < 32 && lpr * vec < a.F) lpr *= 2;
+    const int rows_per_block = 8 * (32 / lpr);
+    int64_t grid64 = ceil_div64(a.n, rows_per_block);
+    const int64_t cap = (int64_t)kNumSMs * 8 * 4;
+    const int grid = (int)(grid64 < cap ? grid64 : cap);
+    if (vec == 4)
+        launch_pna_halo_lpr<4>(a, lpr, grid, s);
+    else
+        launch_pna_halo_lpr<1>(a, lpr, grid, s);
+    GNNB_CUDA(cudaGetLastError());
+    if (launches) ++*launches;
+    return GNNB_OK;
+}
+
 // ------------------------------------------------------------------------------------ GINE
 //
 // lib:1555-1623 gine_conv_agg: agg_v = sum_k relu(x[u_k] + proj[eid_k]) over the in-edges of v in

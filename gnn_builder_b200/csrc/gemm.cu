@@ -246,13 +246,13 @@ __global__ void __launch_bounds__(256) gemm_strict_kernel(const GemmArgs g, int 
 }
 
 __global__ void transpose_weight_kernel(const float *__restrict__ W, float *__restrict__ Wt,
-                                        int out_size, int in_size, int ldw)
+                                        int out_size, int in_size, int ldw, int ld_src)
 {
     const int64_t total = (int64_t)in_size * ldw;
     for (int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
          idx += (int64_t)gridDim.x * blockDim.x) {
         const int k = (int)(idx / ldw), n = (int)(idx % ldw);
-        Wt[idx] = (n < out_size) ? __ldg(W + (size_t)n * in_size + k) : 0.0f;
+        Wt[idx] = (n < out_size) ? __ldg(W + (size_t)n * ld_src + k) : 0.0f;
     }
 }
 
@@ -292,13 +292,14 @@ int launch_gemm(const GemmArgs &g, bool strict, cudaStream_t s, int *launches)
 }
 
 int launch_transpose_weight(const float *W, float *Wt, int out_size, int in_size, int ldw,
-                            cudaStream_t s, int *launches)
+                            cudaStream_t s, int *launches, int ld_src)
 {
     const int64_t total = (int64_t)in_size * ldw;
     if (total <= 0) return GNNB_OK;
     int64_t grid = ceil_div64(total, 256);
     if (grid > kNumSMs * 8) grid = kNumSMs * 8;
-    transpose_weight_kernel<<<(int)grid, 256, 0, s>>>(W, Wt, out_size, in_size, ldw);
+    transpose_weight_kernel<<<(int)grid, 256, 0, s>>>(W, Wt, out_size, in_size, ldw,
+                                                  ld_src > 0 ? ld_src : in_size);
     GNNB_CUDA(cudaGetLastError());
     if (launches) ++*launches;
     return GNNB_OK;

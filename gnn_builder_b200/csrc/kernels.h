@@ -158,6 +158,23 @@ struct PnaAggArgs {
 };
 int launch_pna_agg(const PnaAggArgs &a, cudaStream_t s, int *launches);
 
+// PNA statistics of the owned rows of a row-partitioned graph whose CSR is split by source
+// (owned-source part, then halo-source part; neighbor entries are ext indices, bit 31 ignored).
+// The message of edge u -> v is t = A_u + B_v with A in ext space: the owned rows' A and the A rows
+// the owners sent for the halo.  in_deg is the FULL in-degree of every owned row (mean, std and
+// the degree scalers).  Output as PnaAggArgs::cat12 / compact.
+struct PnaHaloArgs {
+    const float *a_ext;    // [n_ext][F]  A = x.W_nbr^T
+    const float *b;        // [n][F]      B = x.W_self^T + b_pre (owned rows)
+    int F;
+    float *cat12;          // [n][12F], or [n][4F] when compact
+    const int32_t *own_off, *own_cnt, *own_nbr, *halo_off, *halo_cnt, *halo_nbr, *in_deg;
+    int n;
+    float delta;
+    int compact;
+};
+int launch_pna_halo_stats(const PnaHaloArgs &a, cudaStream_t s, int *launches);
+
 // ---------------------------------------------------------------- GEMM (gemm.cu)
 // C[M][N] = act( A1[M][K1].W1t[K1][N] (+ A2[M][K2].W2t[K2][N]) + bias (+ skip) )
 // weights are pre-transposed: Wt[k][n], row stride ldw (multiple of 4, zero padded)
@@ -182,9 +199,10 @@ size_t gemm_tc_image_floats(int K, int N);
 int gemm_tc_build_image(const float *Wt, int ldw, int K, int N, float *img, cudaStream_t s);
 bool gemm_tc_supported(const GemmArgs &g);
 int launch_gemm_tc(const GemmArgs &g, cudaStream_t s, int *launches);
-// Wt[k][n] (ld = ldw) from W[n][k] (reference layout); pads columns n..ldw with zeros
+// Wt[k][n] (ld = ldw) from W[n][k] (reference layout); pads columns n..ldw with zeros.
+// ld_src: row stride of W when it is a column block of a wider matrix (0: in_size)
 int launch_transpose_weight(const float *W, float *Wt, int out_size, int in_size, int ldw,
-                            cudaStream_t s, int *launches);
+                            cudaStream_t s, int *launches, int ld_src = 0);
 
 // ---------------------------------------------------------------- pooling / misc (pool.cu)
 // pooled[g][p*F + f] for pools[p] over rows node_ptr[g]..node_ptr[g+1]

@@ -545,9 +545,16 @@ struct HeavyCache {
     int n = 0;
     HeavyList list;
 };
+// a weight in the reference layout, transposed for the GEMM on every call (so the caller may
+// change it between calls) plus its tensor-core image
+struct DevWeight {
+    DeviceBuf wt, img;
+    int ldw = 4;
+};
 struct PartitionCache {
     TableWorkspace ws;
-    DeviceBuf wt, img, agg, pool_tmp, pool_ptr;
+    DeviceBuf agg, hid, pna_b, pna_stats, pool_tmp, pool_ptr;
+    DevWeight w[5];       // the weights of the layer being computed
     int64_t pool_n = -1;
     HeavyCache whole;     // gnnb_gcn_conv_partition (one CSR)
     HeavyCache part[32];  // owned-source / halo-source parts of a split CSR, per row block
@@ -561,6 +568,62 @@ int heavy_rows_of(HeavyCache &hc, const int32_t *lengths, int n, cudaStream_t s)
     GNNB_TRY(find_heavy_rows(lengths, n, heavy_threshold(), g_part.ws, hc.list, s, nullptr));
     hc.key = lengths;
     hc.n = n;
+    return GNNB_OK;
+}
+
+// W[out][in] (device, row stride ld_src, 0 = in) -> dw.wt [in][ldw] and its tensor-core image
+int dev_weight(DevWeight &dw, const float *W, int out, int in, int ld_src, cudaStream_t s)
+{
+    dw.ldw = round_up(out, 4);
+    GNNB_TRY(dw.wt.ensure(sizeof(float) * (size_t)in * dw.ldw));
+    GNNB_TRY(launch_transpose_weight(W, dw.wt.as<float>(), out, in, dw.ldw, s, nullptr, ld_src));
+    GNNB_TRY(dw.img.ensure(sizeof(float) * gemm_tc_image_floats(in, out)));
+    GNNB_TRY(gemm_tc_build_image(dw.wt.as<float>(), dw.ldw, in, out, dw.img.as<float>(), s));
+    return GNNB_OK;
+}
+
+// heavy-row list of one part of a split CSR, cached by its row-length table and row count
+HeavyCache &part_cache(const int32_t *lengths, int n)
+{
+    for (HeavyCache &hc : g_part.part)
+        if (hc.key == lengths && hc.n == n) return hc;
+    HeavyCache &hc = g_part.part[g_part.part_next];
+    g_part.part_next = (g_part.part_next + 1) % 32;
+    hc.key = nullptr;
+    return hc;
+}
+
+// One part (owned-source or halo-source edges) of a split CSR through the aggregation kernels
+// for rows [row_begin, row_begin + row_count) of `a` (whose out / n / row_base address that
+// block), with the heavy rows of the part bucketed.  in_deg: the full in-degree of the owned
+// rows, for the modes that read it (mean); null passes the part's lengths as the degree, which
+// is all GCN (full degree through dinv) and GIN read.
+int halo_agg_part(const AggArgs &a, const int32_t *off, const int32_t *cnt, const int32_t *nbr,
+                  const int32_t *in_deg, bool accumulate, bool finish, int row_begin, int row_count,
+                  cudaStream_t s)
+{
+    HeavyCache &hc = part_cache(cnt + row_begin, row_count);
+    GNNB_TRY(heavy_rows_of(hc, cnt + row_begin, row_count, s));
+    GNNB_TRY(heavy_setup(g_part.ws, hc.list.n_chunks, a.F));
+    AggArgs b = a;
+    b.offsets = off + row_begin; b.nbr = nbr;
+    if (in_deg != nullptr) {
+        b.in_deg = in_deg + row_begin;
+        b.counts = cnt + row_begin;
+    } else {
+        b.in_deg = cnt + row_begin;
+    }
+    b.set_heavy(hc.list, g_part.ws.heavy_partial.as<float>());
+    b.accumulate = accumulate ? 1 : 0; b.no_finish = finish ? 0 : 1;
+    return launch_agg(b, false, s, nullptr);
+}
+
+// argument checks shared by the split-CSR layer entry points (before any device work)
+int check_halo_args(int n_local, int n_ext, int emb_in, int emb_out, int act, int phase)
+{
+    GNNB_REQUIRE(n_local >= 0 && n_ext >= n_local, "bad row counts");
+    GNNB_REQUIRE(emb_in > 0 && emb_out > 0 && act >= 0 && act <= GNNB_ACT_COS, "bad dims");
+    GNNB_REQUIRE(phase >= 1 && phase <= 3, "phase: 1 owned-source edges, 2 halo edges + transform, 3 both");
     return GNNB_OK;
 }
 }  // namespace
@@ -705,13 +768,11 @@ extern "C" int gnnb_gcn_conv_partition(int n_local, int row_begin, int n_total, 
     GNNB_REQUIRE(is_device_pointer(x_full) && is_device_pointer(y_local),
                  "gnnb_gcn_conv_partition takes device pointers");
     cudaStream_t s = (cudaStream_t)stream;
-    const int ldw = round_up(emb_out, 4), lda = round_up(emb_in, 4);
-    GNNB_TRY(g_part.wt.ensure(sizeof(float) * (size_t)emb_in * ldw));
+    const int lda = round_up(emb_in, 4);
     GNNB_TRY(g_part.agg.ensure(sizeof(float) * (size_t)n_local * lda));
-    GNNB_TRY(launch_transpose_weight(weight, g_part.wt.as<float>(), emb_out, emb_in, ldw, s, nullptr));
-    // tensor-core image of the same weight (two tiny kernels per call; the GEMM then runs on tcgen05)
-    GNNB_TRY(g_part.img.ensure(sizeof(float) * gemm_tc_image_floats(emb_in, emb_out)));
-    GNNB_TRY(gemm_tc_build_image(g_part.wt.as<float>(), ldw, emb_in, emb_out, g_part.img.as<float>(), s));
+    // transposed weight + its tensor-core image (two tiny kernels per call; the GEMM then runs on tcgen05)
+    DevWeight &dw = g_part.w[0];
+    GNNB_TRY(dev_weight(dw, weight, emb_out, emb_in, 0, s));
     // the row list is cached across layers; the partial-sum scratch is sized for THIS layer's
     // emb_in on every call (ensure() only grows)
     GNNB_TRY(heavy_rows_of(g_part.whole, in_degree_local, n_local, s));
@@ -723,10 +784,10 @@ extern "C" int gnnb_gcn_conv_partition(int n_local, int row_begin, int n_total, 
     a.heavy_threshold = heavy_threshold();
     a.set_heavy(g_part.whole.list, g_part.ws.heavy_partial.as<float>());
     GNNB_TRY(launch_agg(a, false, s, nullptr));
-    GemmArgs g = simple_gemm(a.out, lda, emb_in, g_part.wt.as<float>(), ldw, bias, y_local, emb_out,
+    GemmArgs g = simple_gemm(a.out, lda, emb_in, dw.wt.as<float>(), dw.ldw, bias, y_local, emb_out,
                              n_local, emb_out, act);
     g.skip = skip_local; g.ldskip = emb_out;
-    g.img1 = g_part.img.as<float>();
+    g.img1 = dw.img.as<float>();
     GNNB_TRY(launch_gemm(g, false, s, nullptr));
     return GNNB_OK;
 }
@@ -884,16 +945,14 @@ extern "C" int gnnb_gcn_conv_halo(int n_local, int n_ext, const float *x_ext, fl
                                   const float *skip_local, int emb_in, int emb_out, int act, int phase,
                                   int hub_bit, int row_begin, int row_count, void *stream)
 {
-    GNNB_REQUIRE(n_local >= 0 && n_ext >= n_local, "bad row counts");
-    GNNB_REQUIRE(emb_in > 0 && emb_out > 0 && act >= 0 && act <= GNNB_ACT_COS, "bad dims");
-    GNNB_REQUIRE(phase >= 1 && phase <= 3, "phase: 1 owned-source edges, 2 halo edges + transform, 3 both");
+    GNNB_TRY(check_halo_args(n_local, n_ext, emb_in, emb_out, act, phase));
     if (row_count <= 0) { row_begin = 0; row_count = n_local; }
     GNNB_REQUIRE(row_begin >= 0 && row_begin + row_count <= n_local, "row block outside the owned rows");
     if (n_local == 0) return GNNB_OK;
     GNNB_REQUIRE(is_device_pointer(x_ext) && is_device_pointer(y_local), "gnnb_gcn_conv_halo takes device pointers");
     const bool has_halo = halo_counts != nullptr && n_ext > n_local;
     cudaStream_t s = (cudaStream_t)stream;
-    const int ldw = round_up(emb_out, 4), lda = round_up(emb_in, 4);
+    const int lda = round_up(emb_in, 4);
     GNNB_TRY(g_part.agg.ensure(sizeof(float) * (size_t)n_local * lda));
     AggArgs a{};
     a.mode = AGG_GCN; a.x = x_ext; a.ldx = emb_in; a.F = emb_in;
@@ -903,38 +962,182 @@ extern "C" int gnnb_gcn_conv_halo(int n_local, int n_ext, const float *x_ext, fl
     a.heavy_threshold = heavy_threshold(); a.hub_bit = hub_bit ? 1 : 0;
     // block mode (opt-in): the halo pack of the previous row block runs beside these kernels
     a.short_ctas = row_count < n_local ? 1 : 0;
-    auto cache_of = [&](const int32_t *lengths) -> HeavyCache & {
-        for (HeavyCache &hc : g_part.part)
-            if (hc.key == lengths && hc.n == row_count) return hc;
-        HeavyCache &hc = g_part.part[g_part.part_next];
-        g_part.part_next = (g_part.part_next + 1) % 32;
-        hc.key = nullptr;
-        return hc;
-    };
-    auto run_part = [&](const int32_t *off, const int32_t *cnt, const int32_t *nbr, bool accumulate,
-                        bool finish) -> int {
-        HeavyCache &hc = cache_of(cnt + row_begin);
-        GNNB_TRY(heavy_rows_of(hc, cnt + row_begin, row_count, s));
-        GNNB_TRY(heavy_setup(g_part.ws, hc.list.n_chunks, emb_in));
-        AggArgs b = a;
-        b.offsets = off + row_begin; b.nbr = nbr;
-        b.in_deg = cnt + row_begin;   // GCN fast mode reads the full degree from dinv only
-        b.set_heavy(hc.list, g_part.ws.heavy_partial.as<float>());
-        b.accumulate = accumulate ? 1 : 0; b.no_finish = finish ? 0 : 1;
-        return launch_agg(b, false, s, nullptr);
-    };
-    if (phase & 1) GNNB_TRY(run_part(own_offsets, own_counts, own_nbr, false, !has_halo));
+    if (phase & 1)
+        GNNB_TRY(halo_agg_part(a, own_offsets, own_counts, own_nbr, nullptr, false, !has_halo,
+                               row_begin, row_count, s));
     if (!(phase & 2)) return GNNB_OK;
-    if (has_halo) GNNB_TRY(run_part(halo_offsets, halo_counts, halo_nbr, true, true));
-    GNNB_TRY(g_part.wt.ensure(sizeof(float) * (size_t)emb_in * ldw));
-    GNNB_TRY(launch_transpose_weight(weight, g_part.wt.as<float>(), emb_out, emb_in, ldw, s, nullptr));
-    GNNB_TRY(g_part.img.ensure(sizeof(float) * gemm_tc_image_floats(emb_in, emb_out)));
-    GNNB_TRY(gemm_tc_build_image(g_part.wt.as<float>(), ldw, emb_in, emb_out, g_part.img.as<float>(), s));
-    GemmArgs g = simple_gemm(a.out, lda, emb_in, g_part.wt.as<float>(), ldw, bias,
+    if (has_halo)
+        GNNB_TRY(halo_agg_part(a, halo_offsets, halo_counts, halo_nbr, nullptr, true, true,
+                               row_begin, row_count, s));
+    DevWeight &dw = g_part.w[0];
+    GNNB_TRY(dev_weight(dw, weight, emb_out, emb_in, 0, s));
+    GemmArgs g = simple_gemm(a.out, lda, emb_in, dw.wt.as<float>(), dw.ldw, bias,
                              y_local + (size_t)row_begin * emb_out, emb_out, row_count, emb_out, act);
     g.skip = skip_local != nullptr ? skip_local + (size_t)row_begin * emb_in : nullptr;
     g.ldskip = emb_in;
-    g.img1 = g_part.img.as<float>();
+    g.img1 = dw.img.as<float>();
     GNNB_TRY(launch_gemm(g, false, s, nullptr));
+    return GNNB_OK;
+}
+
+// ---- the other convs on the split CSR (same ext-space arguments as gnnb_gcn_conv_halo) -------
+extern "C" int gnnb_gin_conv_halo(int n_local, int n_ext, const float *x_ext, float *y_local,
+                                  const int32_t *own_offsets, const int32_t *own_counts,
+                                  const int32_t *own_nbr, const int32_t *halo_offsets,
+                                  const int32_t *halo_counts, const int32_t *halo_nbr,
+                                  const float *mlp_0_weight, const float *mlp_0_bias,
+                                  const float *mlp_1_weight, const float *mlp_1_bias, float gin_eps,
+                                  const float *skip_local, int emb_in, int hidden, int emb_out, int act,
+                                  int phase, int hub_bit, void *stream)
+{
+    GNNB_TRY(check_halo_args(n_local, n_ext, emb_in, emb_out, act, phase));
+    GNNB_REQUIRE(hidden > 0, "bad hidden size");
+    GNNB_REQUIRE(skip_local == nullptr || emb_in == emb_out, "a skip connection needs emb_in == emb_out");
+    if (n_local == 0) return GNNB_OK;
+    GNNB_REQUIRE(is_device_pointer(x_ext) && is_device_pointer(y_local), "gnnb_gin_conv_halo takes device pointers");
+    const bool has_halo = halo_counts != nullptr && n_ext > n_local;
+    cudaStream_t s = (cudaStream_t)stream;
+    const int lda = round_up(emb_in, 4);
+    GNNB_TRY(g_part.agg.ensure(sizeof(float) * (size_t)n_local * lda));
+    AggArgs a{};
+    a.mode = AGG_GIN; a.x = x_ext; a.ldx = emb_in; a.F = emb_in; a.out = g_part.agg.as<float>();
+    a.ldo = lda; a.n = n_local; a.eps = gin_eps;   // (1 + eps) x_v with ext row v = owned row v
+    a.heavy_threshold = heavy_threshold(); a.hub_bit = hub_bit ? 1 : 0;
+    if (phase & 1)
+        GNNB_TRY(halo_agg_part(a, own_offsets, own_counts, own_nbr, nullptr, false, !has_halo, 0,
+                               n_local, s));
+    if (!(phase & 2)) return GNNB_OK;
+    if (has_halo)
+        GNNB_TRY(halo_agg_part(a, halo_offsets, halo_counts, halo_nbr, nullptr, true, true, 0, n_local, s));
+    // the MLP (lib:1537-1541): linear_0 + ReLU into the hidden scratch, linear_1 (+ skip) + act
+    const int ldh = round_up(hidden, 4);
+    GNNB_TRY(g_part.hid.ensure(sizeof(float) * (size_t)n_local * ldh));
+    DevWeight &w0 = g_part.w[0], &w1 = g_part.w[1];
+    GNNB_TRY(dev_weight(w0, mlp_0_weight, hidden, emb_in, 0, s));
+    GNNB_TRY(dev_weight(w1, mlp_1_weight, emb_out, hidden, 0, s));
+    float *hid = g_part.hid.as<float>();
+    GemmArgs g0 = simple_gemm(a.out, lda, emb_in, w0.wt.as<float>(), w0.ldw, mlp_0_bias, hid, ldh,
+                              n_local, hidden, GNNB_ACT_RELU);
+    g0.img1 = w0.img.as<float>();
+    GNNB_TRY(launch_gemm(g0, false, s, nullptr));
+    GemmArgs g1 = simple_gemm(hid, ldh, hidden, w1.wt.as<float>(), w1.ldw, mlp_1_bias, y_local,
+                              emb_out, n_local, emb_out, act);
+    g1.skip = skip_local; g1.ldskip = emb_in;
+    g1.img1 = w1.img.as<float>();
+    GNNB_TRY(launch_gemm(g1, false, s, nullptr));
+    return GNNB_OK;
+}
+
+extern "C" int gnnb_sage_conv_halo(int n_local, int n_ext, const float *x_ext, float *y_local,
+                                   const int32_t *own_offsets, const int32_t *own_counts,
+                                   const int32_t *own_nbr, const int32_t *halo_offsets,
+                                   const int32_t *halo_counts, const int32_t *halo_nbr,
+                                   const int32_t *in_degree_local, const float *neighbor_lin_weight,
+                                   const float *neighbor_lin_bias, const float *self_lin_weight,
+                                   const float *skip_local, int emb_in, int emb_out, int act, int phase,
+                                   int hub_bit, void *stream)
+{
+    GNNB_TRY(check_halo_args(n_local, n_ext, emb_in, emb_out, act, phase));
+    GNNB_REQUIRE(skip_local == nullptr || emb_in == emb_out, "a skip connection needs emb_in == emb_out");
+    if (n_local == 0) return GNNB_OK;
+    GNNB_REQUIRE(is_device_pointer(x_ext) && is_device_pointer(y_local) && is_device_pointer(in_degree_local),
+                 "gnnb_sage_conv_halo takes device pointers");
+    const bool has_halo = halo_counts != nullptr && n_ext > n_local;
+    cudaStream_t s = (cudaStream_t)stream;
+    const int lda = round_up(emb_in, 4);
+    GNNB_TRY(g_part.agg.ensure(sizeof(float) * (size_t)n_local * lda));
+    AggArgs a{};
+    a.mode = AGG_MEAN; a.x = x_ext; a.ldx = emb_in; a.F = emb_in; a.out = g_part.agg.as<float>();
+    a.ldo = lda; a.n = n_local;
+    a.heavy_threshold = heavy_threshold(); a.hub_bit = hub_bit ? 1 : 0;
+    // the parts' lengths walk the edges, the full in-degree divides (in-degree 0 gives 0, lib:2180-2207)
+    if (phase & 1)
+        GNNB_TRY(halo_agg_part(a, own_offsets, own_counts, own_nbr, in_degree_local, false, !has_halo,
+                               0, n_local, s));
+    if (!(phase & 2)) return GNNB_OK;
+    if (has_halo)
+        GNNB_TRY(halo_agg_part(a, halo_offsets, halo_counts, halo_nbr, in_degree_local, true, true, 0,
+                               n_local, s));
+    // mean.W_l^T + b_l + x_v.W_r^T (lib:2316-2332) (+ skip) + act: one GEMM with two operands
+    DevWeight &wl = g_part.w[0], &wr = g_part.w[1];
+    GNNB_TRY(dev_weight(wl, neighbor_lin_weight, emb_out, emb_in, 0, s));
+    GNNB_TRY(dev_weight(wr, self_lin_weight, emb_out, emb_in, 0, s));
+    GemmArgs g = simple_gemm(a.out, lda, emb_in, wl.wt.as<float>(), wl.ldw, neighbor_lin_bias, y_local,
+                             emb_out, n_local, emb_out, act);
+    g.A2 = x_ext; g.lda2 = emb_in; g.K2 = emb_in; g.W2t = wr.wt.as<float>(); g.ldw2 = wr.ldw;
+    g.img1 = wl.img.as<float>(); g.img2 = wr.img.as<float>();
+    g.second_separate = 1;
+    g.skip = skip_local; g.ldskip = emb_in;
+    GNNB_TRY(launch_gemm(g, false, s, nullptr));
+    return GNNB_OK;
+}
+
+extern "C" int gnnb_pna_conv_halo(int n_local, int n_ext, const float *x_local, float *a_ext,
+                                  float *y_local, const int32_t *own_offsets, const int32_t *own_counts,
+                                  const int32_t *own_nbr, const int32_t *halo_offsets,
+                                  const int32_t *halo_counts, const int32_t *halo_nbr,
+                                  const int32_t *in_degree_local, const float *transform_lin_weight,
+                                  const float *transform_lin_bias, const float *apply_lin_weight,
+                                  const float *apply_lin_bias, const float *final_lin_weight,
+                                  const float *final_lin_bias, float pna_avg_degree_log,
+                                  const float *skip_local, int emb_in, int emb_out, int act, int phase,
+                                  void *stream)
+{
+    GNNB_TRY(check_halo_args(n_local, n_ext, emb_in, emb_out, act, phase));
+    GNNB_REQUIRE(skip_local == nullptr || emb_in == emb_out, "a skip connection needs emb_in == emb_out");
+    if (n_local == 0) return GNNB_OK;
+    GNNB_REQUIRE(is_device_pointer(x_local) && is_device_pointer(a_ext) && is_device_pointer(y_local) &&
+                     is_device_pointer(in_degree_local),
+                 "gnnb_pna_conv_halo takes device pointers");
+    const bool has_halo = halo_counts != nullptr && n_ext > n_local;
+    cudaStream_t s = (cudaStream_t)stream;
+    const int F = emb_in;
+    GNNB_TRY(g_part.pna_b.ensure(sizeof(float) * (size_t)n_local * F));
+    float *bself = g_part.pna_b.as<float>();
+    if (phase & 1) {
+        // W_pre = [W_self | W_nbr] (lib:1801-1807): A = x.W_nbr^T goes to the peers, B stays
+        DevWeight &wn = g_part.w[0], &ws = g_part.w[1];
+        GNNB_TRY(dev_weight(wn, transform_lin_weight + F, F, F, 2 * F, s));
+        GNNB_TRY(dev_weight(ws, transform_lin_weight, F, F, 2 * F, s));
+        GemmArgs ga = simple_gemm(x_local, F, F, wn.wt.as<float>(), wn.ldw, nullptr, a_ext, F, n_local, F,
+                                  GNNB_ACT_IDENTITY);
+        ga.img1 = wn.img.as<float>();
+        GNNB_TRY(launch_gemm(ga, false, s, nullptr));
+        GemmArgs gb = simple_gemm(x_local, F, F, ws.wt.as<float>(), ws.ldw, transform_lin_bias, bself, F,
+                                  n_local, F, GNNB_ACT_IDENTITY);
+        gb.img1 = ws.img.as<float>();
+        GNNB_TRY(launch_gemm(gb, false, s, nullptr));
+    }
+    if (!(phase & 2)) return GNNB_OK;
+    // post_nn = [W_post_self | W_post_agg] over [x | 12F statistics], then the final linear
+    const int ld_o = round_up(emb_out, 4);
+    DevWeight &wp = g_part.w[2], &wa = g_part.w[3], &wf = g_part.w[4];
+    GNNB_TRY(dev_weight(wp, apply_lin_weight, emb_out, F, 13 * F, s));
+    GNNB_TRY(dev_weight(wa, apply_lin_weight + F, emb_out, 12 * F, 13 * F, s));
+    GNNB_TRY(dev_weight(wf, final_lin_weight, emb_out, emb_out, 0, s));
+    GNNB_TRY(g_part.hid.ensure(sizeof(float) * (size_t)n_local * ld_o));
+    GNNB_TRY(g_part.pna_stats.ensure(sizeof(float) * (size_t)n_local * 12 * F));
+    float *hid = g_part.hid.as<float>(), *stats = g_part.pna_stats.as<float>();
+    GemmArgs g1 = simple_gemm(x_local, F, F, wp.wt.as<float>(), wp.ldw, apply_lin_bias, hid, ld_o, n_local,
+                              emb_out, GNNB_ACT_IDENTITY);
+    g1.img1 = wp.img.as<float>();
+    g1.A2 = stats; g1.K2 = 12 * F; g1.W2t = wa.wt.as<float>(); g1.ldw2 = wa.ldw; g1.img2 = wa.img.as<float>();
+    // tensor-core path: only the [n][4F] statistics are written and the GEMM expands them with the
+    // degree scalers, as the layerwise path does
+    g1.lda2 = 4 * F; g1.expand_deg = in_degree_local; g1.expand_delta = pna_avg_degree_log;
+    const bool expand = gemm_tc_supported(g1);
+    if (!expand) { g1.lda2 = 12 * F; g1.expand_deg = nullptr; }
+    PnaHaloArgs pa{};
+    pa.a_ext = a_ext; pa.b = bself; pa.F = F; pa.cat12 = stats;
+    pa.own_off = own_offsets; pa.own_cnt = own_counts; pa.own_nbr = own_nbr;
+    if (has_halo) { pa.halo_off = halo_offsets; pa.halo_cnt = halo_counts; pa.halo_nbr = halo_nbr; }
+    pa.in_deg = in_degree_local; pa.n = n_local; pa.delta = pna_avg_degree_log; pa.compact = expand ? 1 : 0;
+    GNNB_TRY(launch_pna_halo_stats(pa, s, nullptr));
+    GNNB_TRY(launch_gemm(g1, false, s, nullptr));
+    GemmArgs g2 = simple_gemm(hid, ld_o, emb_out, wf.wt.as<float>(), wf.ldw, final_lin_bias, y_local,
+                              emb_out, n_local, emb_out, act);
+    g2.skip = skip_local; g2.ldskip = emb_in;
+    g2.img1 = wf.img.as<float>();
+    GNNB_TRY(launch_gemm(g2, false, s, nullptr));
     return GNNB_OK;
 }

@@ -5,7 +5,8 @@ Two ways the hot path shards (SURVEY 8e):
 * **independent graphs** (BASELINE configs 1-4): a batch is cut into contiguous ranges of graphs
   balanced by node count; every rank runs its shard through its own ``Engine``; there is NO
   data-path collective (``run_sharded`` optionally gathers the per-graph outputs at the end).
-* **one large graph** (BASELINE config 5, GCN): 1D partition by destination row.  Rank g owns
+* **one large graph** (BASELINE config 5 is GCN; GIN, SAGE and PNA run the same way, PNA
+  exchanging its pre-transformed rows instead of the input): 1D partition by destination row.  Rank g owns
   rows ``[g*n/W, (g+1)*n/W)``, their CSR slice (in-edges) and the matching feature rows, plus a
   **halo**: ONE copy of every remote row its in-edges reference (on the 2M-node power-law graph
   that is 84 % / 65 % / 45 % of the remote rows at W = 2 / 4 / 8).  Sources are renumbered into
@@ -268,6 +269,32 @@ class CudaBackend:
             self._p(b), self._p(skip), emb_in, emb_out, act, phase, 1 if plan.hub_rows else 0,
             int(row_begin), int(row_count), self._stream()))
 
+    def _split_csr(self, plan: HaloPlan):
+        return (self._p(plan.own_off), self._p(plan.own_cnt), self._p(plan.own_nbr),
+                self._p(plan.halo_off), self._p(plan.halo_cnt), self._p(plan.halo_nbr))
+
+    def gin_layer_halo(self, x_ext, y_local, plan: HaloPlan, W0, b0, W1, b1, eps, skip, act, phase,
+                       emb_in, emb_out):
+        self._lib.check(self.lib.gnnb_gin_conv_halo(
+            plan.n_local, plan.n_ext, self._p(x_ext), self._p(y_local), *self._split_csr(plan),
+            self._p(W0), self._p(b0), self._p(W1), self._p(b1), float(eps), self._p(skip), emb_in,
+            int(W0.shape[0]), emb_out, act, phase, 1 if plan.hub_rows else 0, self._stream()))
+
+    def sage_layer_halo(self, x_ext, y_local, plan: HaloPlan, in_deg, Wl, bl, Wr, skip, act, phase,
+                        emb_in, emb_out):
+        self._lib.check(self.lib.gnnb_sage_conv_halo(
+            plan.n_local, plan.n_ext, self._p(x_ext), self._p(y_local), *self._split_csr(plan),
+            self._p(in_deg), self._p(Wl), self._p(bl), self._p(Wr), self._p(skip), emb_in, emb_out,
+            act, phase, 1 if plan.hub_rows else 0, self._stream()))
+
+    def pna_layer_halo(self, x_local, a_ext, y_local, plan: HaloPlan, in_deg, Wpre, bpre, Wpost,
+                       bpost, Wlin, blin, delta, skip, act, phase, emb_in, emb_out):
+        self._lib.check(self.lib.gnnb_pna_conv_halo(
+            plan.n_local, plan.n_ext, self._p(x_local), self._p(a_ext), self._p(y_local),
+            *self._split_csr(plan), self._p(in_deg), self._p(Wpre), self._p(bpre), self._p(Wpost),
+            self._p(bpost), self._p(Wlin), self._p(blin), float(delta), self._p(skip), emb_in,
+            emb_out, act, phase, self._stream()))
+
     def halo_pack(self, x_own, F: int, plan: HaloPlan, dst_ptrs, max_ctas: int = 0):
         """dst_ptrs: one raw device address per peer (0 where nothing is sent)"""
         W = len(dst_ptrs)
@@ -352,9 +379,22 @@ class CudaBackend:
         return t
 
 
-class LargeGraphGCN:
-    """GCN GNNModel over one large row-partitioned graph (BASELINE config 5) with a per-layer halo
-    exchange overlapped with the aggregation of the owned-source edges.
+# per conv: the flat reference names (after "gnn_convs_<k>_") of one layer's parameters, in the
+# order the backend's <conv>_layer_halo takes them
+_LAYER_PARAMS = {
+    "gcn": ("conv_lin_weight", "conv_bias"),
+    "gin": ("mlp_linear_0_weight", "mlp_linear_0_bias", "mlp_linear_1_weight", "mlp_linear_1_bias"),
+    "sage": ("conv_lin_l_weight", "conv_lin_l_bias", "conv_lin_r_weight"),
+    "pna": ("conv_pre_nns_0_0_weight", "conv_pre_nns_0_0_bias", "conv_post_nns_0_0_weight",
+            "conv_post_nns_0_0_bias", "conv_lin_weight", "conv_lin_bias"),
+}
+
+
+class LargeGraphModel:
+    """GNNModel (GCN, GIN, SAGE or PNA) over one large row-partitioned graph with a per-layer halo
+    exchange.  GCN, GIN and SAGE exchange the layer input and overlap it with the aggregation of
+    the owned-source edges; PNA computes its pre-transform A = x.W_nbr^T of the owned rows first
+    and exchanges A (as many floats per halo row as the input), so no GEMM runs on halo rows.
 
     transport: "p2p" (owners store the halo rows straight into the peers' buffers over NVLink
     through CUDA-IPC mappings; flag hand-off on the device), "nccl" (pack + all_to_all_single) or
@@ -363,8 +403,7 @@ class LargeGraphGCN:
     def __init__(self, model, n_total: int, rank: int, world: int, dist=None, backend=None,
                  transport: str = "auto", hub_l2_mb: Optional[int] = None):
         d = model.describe()
-        if d["conv_type"] != 0:
-            raise NotImplementedError("the row-partitioned path implements GCN (BASELINE config 5)")
+        self.conv = ("gcn", "gin", "sage", "pna")[d["conv_type"]]
         self.model, self.desc = model, d
         self.part = RowPartition(n_total, world)
         self.rank, self.world, self.dist = rank, world, dist
@@ -381,19 +420,22 @@ class LargeGraphGCN:
         # below, at 8 GPUs blocks 2 / 4 give 3.01 / 3.08 ms against 2.85 ms -- smaller kernels, and
         # the pack's CTAs queue behind the aggregation's -- so the default keeps one exchange per
         # layer, overlapped with the aggregation of the owned-source edges.
-        self.n_blocks = max(0, min(16, int(os.environ.get("GNNB_HALO_BLOCKS", 0))))
+        # (GCN only; the other convs run one exchange per layer)
+        self.n_blocks = (max(0, min(16, int(os.environ.get("GNNB_HALO_BLOCKS", 0))))
+                         if self.conv == "gcn" else 0)
         params = model.named_parameter_arrays()
-        names = list(params)
-        nh = d["mlp_num_linear"]
         B = self.backend
-        self.head = [(B.to_device(params[names[2 * j]]), B.to_device(params[names[2 * j + 1]]))
-                     for j in range(nh)]
-        self.layers = []
-        for k in range(d["num_layers"]):  # [conv_bias, conv_lin_weight] per layer
-            b, W = params[names[2 * nh + 2 * k]], params[names[2 * nh + 2 * k + 1]]
-            self.layers.append((B.to_device(W), B.to_device(b)))
-        self.dims = [int(W.shape[1]) for W, _ in self.layers] + [int(self.layers[-1][0].shape[0])]
+        self.head = [(B.to_device(params[f"mlp_head_linear_layers_{j}_weight"]),
+                      B.to_device(params[f"mlp_head_linear_layers_{j}_bias"]))
+                     for j in range(d["mlp_num_linear"])]
+        self.layers = [tuple(B.to_device(params[f"gnn_convs_{k}_{name}"])
+                             for name in _LAYER_PARAMS[self.conv])
+                       for k in range(d["num_layers"])]
+        # layer k maps dims[k] -> dims[k + 1]
+        L = d["num_layers"]
+        self.dims = [d["in_dim"]] + [d["hidden_dim"]] * (L - 1) + [d["out_dim"]]
         self.tables = None
+        self.in_deg = None
         self.plan: Optional[HaloPlan] = None
         self.dinv_ext = None
         self.transport = "none"
@@ -409,16 +451,21 @@ class LargeGraphGCN:
         n_local = self.part.n_local
         self.tables = B.partition_tables(B.to_device(coo_local.astype(np.int32)), r0, n_local)
         ind_local, _, nbr_global = self.tables
-        if W > 1:
-            ind_full = B.all_gather_rows(self.dist, ind_local.view(-1, 1), self.part.n_total).view(-1)
-        else:
-            ind_full = ind_local
-        dinv_full = B.dinv(ind_full)
+        self.in_deg = ind_local
+        if self.conv == "gcn":   # GCN normalises by the in-degree of both endpoints: all-gather it
+            if W > 1:
+                ind_full = B.all_gather_rows(self.dist, ind_local.view(-1, 1), self.part.n_total).view(-1)
+            else:
+                ind_full = ind_local
+            dinv_full = B.dinv(ind_full)
         self.plan = plan = HaloPlan(ind_local, nbr_global, self.rank, self.part,
                                     self.dist if W > 1 else None)
-        self.dinv_ext = dinv_full[plan.ext_ids(self.rank)].contiguous()
+        if self.conv == "gcn":
+            self.dinv_ext = dinv_full[plan.ext_ids(self.rank)].contiguous()
         fmax = max(self.dims)
-        if self.hub_l2_mb > 0 and hasattr(B, "mark_hubs") and plan.n_ext * fmax * 4 > (96 << 20):
+        # (PNA gathers A rows through its own statistics kernel, which takes no cache hints)
+        if self.conv != "pna" and self.hub_l2_mb > 0 and hasattr(B, "mark_hubs") and \
+                plan.n_ext * fmax * 4 > (96 << 20):
             plan.hub_rows = B.mark_hubs(plan.nbr_all, plan.n_ext, fmax * 4, self.hub_l2_mb << 20)
         self._setup_buffers(fmax)
         self._blocks = (plan.block_ranges(self.n_blocks)
@@ -450,7 +497,7 @@ class LargeGraphGCN:
                                        + getattr(self, "_p2p_error", "(another rank)"))
                 self.ext = None
         if self.ext is None:
-            self.ext = [B.empty((plan.n_ext * fmax,)) for _ in range(3)]
+            self.ext = [B.empty((plan.n_ext * fmax,)) for _ in range(self._n_bufs())]
             self.transport = "nccl" if W > 1 else "none"
         else:
             self.transport = "p2p"
@@ -493,15 +540,17 @@ class LargeGraphGCN:
 
         B, W, plan, dist = self.backend, self.world, self.plan, self.dist
         nbytes = max(plan.n_ext * fmax * 4, 256)
-        bufs = [B.ipc_alloc(nbytes) for _ in range(3)]
+        nb = self._n_bufs()
+        bufs = [B.ipc_alloc(nbytes) for _ in range(nb)]
         flags_t, flags_ptr, flags_h = B.ipc_alloc(8 * 32)
         self.ext = [t.view(torch.float32) for t, _, _ in bufs]
         self._ext_ptr = [p for _, p, _ in bufs]
         self._flags, self._flags_ptr = flags_t.view(torch.int64), flags_ptr
         self._timed_out = torch.zeros(1, dtype=torch.int32, device=flags_t.device)
-        mine = torch.frombuffer(bytearray(bufs[0][2] + bufs[1][2] + bufs[2][2] + flags_h),
+        mine = torch.frombuffer(bytearray(b"".join(h for _, _, h in bufs) + flags_h),
                                 dtype=torch.uint8).to(flags_t.device)
-        allh = torch.empty(W * 256, dtype=torch.uint8, device=flags_t.device)
+        hb = 64 * (nb + 1)       # handle bytes per rank: the buffers', then the flags'
+        allh = torch.empty(W * hb, dtype=torch.uint8, device=flags_t.device)
         dist.all_gather_into_tensor(allh, mine)
         allh = allh.cpu().numpy().tobytes()
         # where do MY rows start inside peer p's halo region?  p's recv_off[my rank], in rows
@@ -509,15 +558,15 @@ class LargeGraphGCN:
         at_peer = torch.empty(W, dtype=torch.int64, device=flags_t.device)
         dist.all_to_all_single(at_peer, recv_off)
         self._row_at_peer = [int(v) for v in at_peer.cpu().tolist()]
-        self._peer_ext = [[0] * W, [0] * W, [0] * W]
+        self._peer_ext = [[0] * W for _ in range(nb)]
         self._peer_flag = [0] * W
         for p in range(W):
             if p == self.rank:
                 continue
-            h = allh[256 * p: 256 * (p + 1)]
-            for i in range(3):
+            h = allh[hb * p: hb * (p + 1)]
+            for i in range(nb):
                 self._peer_ext[i][p] = B.ipc_open(h[64 * i: 64 * (i + 1)])
-            self._peer_flag[p] = B.ipc_open(h[192:256]) + 8 * self.rank
+            self._peer_flag[p] = B.ipc_open(h[64 * nb: hb]) + 8 * self.rank
         self._peer_flag[self.rank] = flags_ptr + 8 * self.rank
 
     def close(self):
@@ -534,14 +583,24 @@ class LargeGraphGCN:
         input has a buffer of its own, so a forward never overwrites it; the others alternate"""
         return 2 if k == 0 else (k & 1)
 
+    def _n_bufs(self) -> int:
+        """three layer-input buffers; PNA adds two for the exchanged A rows (layer parity: a peer
+        may push layer k+1's rows while this rank still reads layer k's)"""
+        return 5 if self.conv == "pna" else 3
+
+    def _xbuf(self, k: int) -> int:
+        """ext buffer whose halo region layer k's exchange fills"""
+        return 3 + (k & 1) if self.conv == "pna" else self._buf(k)
+
     def input_view(self):
         """where the layer-0 input of this rank lives: [n_local][in_dim] (write here to skip a copy)"""
         return self.ext[2][: self.part.n_local * self.dims[0]].view(self.part.n_local, self.dims[0])
 
     def _exchange(self, k: int, F: int):
-        """fills the halo region of layer k's input buffer with the peers' rows (comm stream)"""
+        """fills the halo region of layer k's input buffer (PNA: A buffer) with the peers' rows
+        (comm stream)"""
         B, W, plan = self.backend, self.world, self.plan
-        cur = self.ext[self._buf(k)]
+        cur = self.ext[self._xbuf(k)]
         x_own = cur[: plan.n_local * F]
         self.epoch += 1
         B.fork()
@@ -549,7 +608,7 @@ class LargeGraphGCN:
             if self.transport == "p2p":
                 n_local = plan.n_local
                 dst = [0 if p == self.rank or plan.send_counts[p] == 0 else
-                       self._peer_ext[self._buf(k)][p] + 4 * F * (n_local + self._row_at_peer[p])
+                       self._peer_ext[self._xbuf(k)][p] + 4 * F * (n_local + self._row_at_peer[p])
                        for p in range(W)]
                 B.halo_pack(x_own, F, plan, dst)
                 B.halo_signal(self._peer_flag, self.epoch)
@@ -581,15 +640,17 @@ class LargeGraphGCN:
         L = d["num_layers"]
         pipelined = self.world > 1 and self.transport == "p2p" and self._blocks is not None
         pushed = False    # layer k's halo is already on its way (pushed block by block during layer k-1)
-        for k, (W, b) in enumerate(self.layers):
+        for k in range(L):
             fi, fo = self.dims[k], self.dims[k + 1]
             cur, nxt = self.ext[self._buf(k)], self.ext[self._buf(k + 1)]
             x_ext = cur[: plan.n_ext * fi]
             y_local = nxt[: n_local * fo]
             do_skip = bool(d["skip"]) and k != 0 and k != L - 1
             skip = cur[: n_local * fi] if do_skip else None
-            args = (x_ext, y_local, plan, self.dinv_ext, W, b, skip, d["gnn_act"])
-            if self.world == 1:
+            args = (x_ext, y_local, plan, self.dinv_ext, *self.layers[k], skip, d["gnn_act"])
+            if self.conv != "gcn":
+                self._conv_layer(k, x_ext, y_local, skip)
+            elif self.world == 1:
                 B.gcn_layer_halo(*args, 3, fi, fo)
             else:   # (every rank takes part in the exchange, even with an empty halo)
                 if pushed:
@@ -639,10 +700,50 @@ class LargeGraphGCN:
         out = B.head(pooled, self.head, d["mlp_act"], d["out_act"])
         return (out, emb.clone()) if return_embeddings else out
 
+    def _conv_layer(self, k: int, x_ext, y_local, skip):
+        """layer k of a GIN, SAGE or PNA model: one exchange, then the layer in two phases"""
+        B, d, plan = self.backend, self.desc, self.plan
+        fi, fo = self.dims[k], self.dims[k + 1]
+        p, act = self.layers[k], d["gnn_act"]
+
+        def call(phase):
+            if self.conv == "gin":
+                B.gin_layer_halo(x_ext, y_local, plan, *p, d["gin_eps"], skip, act, phase, fi, fo)
+            elif self.conv == "sage":
+                B.sage_layer_halo(x_ext, y_local, plan, self.in_deg, *p, skip, act, phase, fi, fo)
+            else:
+                B.pna_layer_halo(x_ext[: plan.n_local * fi], self.ext[self._xbuf(k)][: plan.n_ext * fi],
+                                 y_local, plan, self.in_deg, *p, d["pna_delta"], skip, act, phase,
+                                 fi, fo)
+
+        if self.world == 1:
+            call(3)
+        elif self.conv == "pna":   # A of the owned rows first: it is what the peers receive
+            call(1)
+            self._exchange(k, fi)
+            self._arrived()
+            call(2)
+        else:   # (every rank takes part in the exchange, even with an empty halo)
+            self._exchange(k, fi)
+            call(1)                # owned-source edges: overlaps the exchange
+            self._arrived()
+            call(2)                # halo-source edges, finish, transform
+
     def check_transport(self):
         """after a synchronisation: raises if a device-side halo wait gave up (p2p transport)"""
         if self.transport == "p2p" and int(self._timed_out.item()) != 0:
             raise RuntimeError("halo exchange: a peer's rows did not arrive within the wait limit")
+
+
+class LargeGraphGCN(LargeGraphModel):
+    """LargeGraphModel restricted to GCN models (BASELINE config 5)."""
+
+    def __init__(self, model, n_total: int, rank: int, world: int, dist=None, backend=None,
+                 transport: str = "auto", hub_l2_mb: Optional[int] = None):
+        if model.describe()["conv_type"] != 0:
+            raise NotImplementedError("LargeGraphGCN runs GCN models; LargeGraphModel runs every conv")
+        super().__init__(model, n_total, rank, world, dist=dist, backend=backend,
+                         transport=transport, hub_l2_mb=hub_l2_mb)
 
 
 def _cat(ts):

@@ -293,6 +293,47 @@ int gnnb_gcn_conv_halo(int n_local, int n_ext, const float *x_ext, float *y_loca
                        const int32_t *halo_nbr, const float *dinv_ext, const float *weight,
                        const float *bias, const float *skip_local, int emb_in, int emb_out, int act,
                        int phase, int hub_bit, int row_begin, int row_count, void *stream);
+/* The same for the other convs, FAST math, whole layers (no row blocks).  phase 1 aggregates the
+ * owned-source edges (PNA: computes the pre-transform instead, see below), phase 2 the halo-source
+ * edges and the transform, phase 3 both; y_local[n_local][emb_out] = act(conv (+ skip_local)).
+ * Weights in the reference layout as for gnnb_gin_conv / gnnb_sage_conv / gnnb_pna_conv.
+ * hub_bit: the neighbor tables carry the marks of gnnb_mark_hub_sources.
+ *
+ * GIN (lib:1440-1549): sum over both parts + (1 + gin_eps) x_v, then linear_0 + ReLU and
+ * linear_1. */
+int gnnb_gin_conv_halo(int n_local, int n_ext, const float *x_ext, float *y_local,
+                       const int32_t *own_offsets, const int32_t *own_counts, const int32_t *own_nbr,
+                       const int32_t *halo_offsets, const int32_t *halo_counts,
+                       const int32_t *halo_nbr, const float *mlp_0_weight, const float *mlp_0_bias,
+                       const float *mlp_1_weight, const float *mlp_1_bias, float gin_eps,
+                       const float *skip_local, int emb_in, int hidden, int emb_out, int act,
+                       int phase, int hub_bit, void *stream);
+/* SAGE, mean aggregation (lib:2211-2341): the parts' counts walk the edges and in_degree_local
+ * (the FULL in-degree of every owned row) divides; in-degree 0 gives a zero mean. */
+int gnnb_sage_conv_halo(int n_local, int n_ext, const float *x_ext, float *y_local,
+                        const int32_t *own_offsets, const int32_t *own_counts, const int32_t *own_nbr,
+                        const int32_t *halo_offsets, const int32_t *halo_counts,
+                        const int32_t *halo_nbr, const int32_t *in_degree_local,
+                        const float *neighbor_lin_weight, const float *neighbor_lin_bias,
+                        const float *self_lin_weight, const float *skip_local, int emb_in,
+                        int emb_out, int act, int phase, int hub_bit, void *stream);
+/* PNA (lib:1891-2157).  What crosses ranks is A = x.W_nbr^T rather than x (W_pre = [W_self |
+ * W_nbr]): phase 1 writes A of the owned rows to a_ext[0 .. n_local) and keeps B = x.W_self^T +
+ * b_pre in library scratch (the caller then sends the A rows, e.g. with gnnb_halo_pack, into the
+ * peers' a_ext halo regions); phase 2, once this rank's halo rows of A have arrived in
+ * a_ext[n_local .. n_ext), reduces t = A_u + B_v over both parts in order (max, min, mean, std with
+ * the full in_degree_local; in-degree 0 gives std = NaN as in gnnb_pna_conv) and applies the
+ * apply and final linears.  x_local[n_local][emb_in] are the owned input rows; a_ext is
+ * [n_ext][emb_in].  Hub marks in the neighbor tables are ignored. */
+int gnnb_pna_conv_halo(int n_local, int n_ext, const float *x_local, float *a_ext, float *y_local,
+                       const int32_t *own_offsets, const int32_t *own_counts, const int32_t *own_nbr,
+                       const int32_t *halo_offsets, const int32_t *halo_counts,
+                       const int32_t *halo_nbr, const int32_t *in_degree_local,
+                       const float *transform_lin_weight, const float *transform_lin_bias,
+                       const float *apply_lin_weight, const float *apply_lin_bias,
+                       const float *final_lin_weight, const float *final_lin_bias,
+                       float pna_avg_degree_log, const float *skip_local, int emb_in, int emb_out,
+                       int act, int phase, void *stream);
 
 #ifdef __cplusplus
 }
