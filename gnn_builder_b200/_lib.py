@@ -26,6 +26,7 @@ class ModelDesc(C.Structure):
         ("num_pools", C.c_int32), ("pools", C.c_int32 * 4), ("mlp_num_linear", C.c_int32),
         ("mlp_hidden", C.c_int32), ("mlp_out", C.c_int32), ("mlp_act", C.c_int32),
         ("out_act", C.c_int32), ("max_nodes", C.c_int32), ("max_edges", C.c_int32),
+        ("edge_dim", C.c_int32),
     ]
 
 
@@ -40,6 +41,7 @@ EXPORTS = [
     "gnnb_model_create", "gnnb_model_destroy", "gnnb_model_num_params", "gnnb_model_param_info",
     "gnnb_model_set_param", "gnnb_model_finalize", "gnnb_model_set_path", "gnnb_model_set_math",
     "gnnb_model_run_graph", "gnnb_model_run_batch", "gnnb_model_run_batch_async",
+    "gnnb_model_run_batch_edges", "gnnb_model_run_batch_edges_async",
     "gnnb_model_get_node_embeddings", "gnnb_model_last_launches", "gnnb_model_last_path", "gnnb_model_last_kernel",
     "gnnb_model_stream", "gnnb_model_synchronize", "gnnb_model_set_profile",
     "gnnb_model_profile_read",
@@ -95,6 +97,11 @@ def load(build_if_missing: bool = True) -> C.CDLL:
     lib.gnnb_model_run_batch_async.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                                C.c_void_p, C.c_int, C.c_int64, C.c_int64,
                                                C.c_void_p, C.c_void_p]
+    lib.gnnb_model_run_batch_edges.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
+    lib.gnnb_model_run_batch_edges_async.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                      C.c_void_p, C.c_void_p, C.c_int, C.c_int64,
+                                                      C.c_int64, C.c_void_p, C.c_void_p]
     lib.gnnb_model_get_node_embeddings.argtypes = [C.c_void_p, C.c_void_p, C.c_int64]
     lib.gnnb_model_last_launches.argtypes = [C.c_void_p]
     lib.gnnb_model_last_path.argtypes = [C.c_void_p]

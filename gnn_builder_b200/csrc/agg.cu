@@ -759,4 +759,168 @@ int launch_gine_agg(const GineAggArgs &a, cudaStream_t s, int *launches)
     return GNNB_OK;
 }
 
+// ------------------------------------------------------------------------- GINE, model path
+//
+// gine_agg_kernel reads a materialised projection proj[E][F] (4F bytes per edge, written by a GEMM
+// and read back, every layer).  Here each edge's projection is computed where it is consumed:
+// W_e^T [edge_dim][F] and b_e sit in shared memory, the edge's edge_dim features are one broadcast
+// load per (sub-)warp, and the lanes of the row's (sub-)warp compute their columns of
+// b_e + sum_j W_e[c][j] ef[j] (separately rounded, ascending j: the reference's linear, lib:852-903
+// with BLOCK_SIZE_IN = 1), add x_u, apply ReLU and accumulate in neighbor-table order.  Per edge the
+// kernel reads 4 edge_dim bytes of features instead of 4F of projection.  No heavy-row bucketing:
+// a hub row is one (sub-)warp's serial work.
+namespace {
+
+template <int VEC, int LPR, bool SMEM>
+__global__ void __launch_bounds__(256) gine_agg_proj_kernel(const GineProjAggArgs a)
+{
+    extern __shared__ float4 gine_smem4[];
+    float *const smem = reinterpret_cast<float *>(gine_smem4);
+    const float *Wt = a.We_t;
+    const float *be = a.be;
+    if (SMEM) {   // [edge_dim][ldw] W_e^T, then [F] b_e
+        const int nw = a.edge_dim * a.ldw;
+        for (int i = threadIdx.x; i < nw; i += blockDim.x) smem[i] = __ldg(a.We_t + i);
+        for (int i = threadIdx.x; i < a.F; i += blockDim.x) smem[nw + i] = __ldg(a.be + i);
+        __syncthreads();
+        Wt = smem;
+        be = smem + nw;
+    }
+    constexpr int ROWS_PER_WARP = 32 / LPR;
+    const int lane = threadIdx.x & 31;
+    const int lg = lane % LPR, sub = lane / LPR;
+    const int warps_per_block = blockDim.x >> 5;
+    const int64_t warp_global = (int64_t)blockIdx.x * warps_per_block + (threadIdx.x >> 5);
+    const int64_t warp_stride = (int64_t)gridDim.x * warps_per_block;
+    const float self_scale = __fadd_rn(1.0f, a.eps);   // lib:1522
+    const int ed = a.edge_dim;
+    for (int64_t row0 = warp_global * ROWS_PER_WARP; row0 < a.n; row0 += warp_stride * ROWS_PER_WARP) {
+        const int v = (int)row0 + sub;
+        if (v >= a.n) continue;
+        const int deg = __ldg(a.in_deg + v);
+        const int off = __ldg(a.offsets + v);
+        for (int c = lg * VEC; c < a.F; c += LPR * VEC) {
+            float bias[VEC];
+#pragma unroll
+            for (int i = 0; i < VEC; i++) bias[i] = be[c + i];
+            Vec<VEC> acc;
+#pragma unroll
+            for (int i = 0; i < VEC; i++) acc.v[i] = 0.0f;
+#pragma unroll 2
+            for (int k = 0; k < deg; k++) {
+                const int u = __ldg(a.nbr + off + k);
+                Vec<VEC> xu;
+                xu.load(a.x + (size_t)u * a.ldx + c);
+                const float *ef = a.ef_sorted + (size_t)(off + k) * a.lde;
+                float p[VEC];
+#pragma unroll
+                for (int i = 0; i < VEC; i++) p[i] = bias[i];   // lib:852-864
+                for (int j0 = 0; j0 < ed; j0 += 4) {
+                    const float4 e4 = __ldg(reinterpret_cast<const float4 *>(ef + j0));
+#pragma unroll
+                    for (int jj = 0; jj < 4; jj++) {
+                        if (j0 + jj < ed) {
+                            const float ej = jj == 0 ? e4.x : jj == 1 ? e4.y : jj == 2 ? e4.z : e4.w;
+                            Vec<VEC> w;
+                            if (SMEM) w.load_rw(Wt + (size_t)(j0 + jj) * a.ldw + c);
+                            else w.load(Wt + (size_t)(j0 + jj) * a.ldw + c);
+#pragma unroll
+                            for (int i = 0; i < VEC; i++)
+                                p[i] = __fadd_rn(p[i], __fmul_rn(w.v[i], ej));   // lib:891, 901
+                        }
+                    }
+                }
+#pragma unroll
+                for (int i = 0; i < VEC; i++) {
+                    const float m = __fadd_rn(xu.v[i], p[i]);                     // lib:1603
+                    acc.v[i] = __fadd_rn(acc.v[i], m > 0.0f ? m : 0.0f);         // lib:1606-1610
+                }
+            }
+            Vec<VEC> xs;
+            xs.load(a.x + (size_t)v * a.ldx + c);
+#pragma unroll
+            for (int i = 0; i < VEC; i++) acc.v[i] = __fadd_rn(acc.v[i], __fmul_rn(xs.v[i], self_scale));
+            acc.store(a.out + (size_t)v * a.ldo + c);
+        }
+    }
+}
+
+template <int VEC, bool SMEM>
+int launch_gine_proj_lpr(const GineProjAggArgs &a, int lpr, int grid, size_t smem, cudaStream_t s)
+{
+    void (*k)(const GineProjAggArgs);
+    switch (lpr) {
+    case 1: k = gine_agg_proj_kernel<VEC, 1, SMEM>; break;
+    case 2: k = gine_agg_proj_kernel<VEC, 2, SMEM>; break;
+    case 4: k = gine_agg_proj_kernel<VEC, 4, SMEM>; break;
+    case 8: k = gine_agg_proj_kernel<VEC, 8, SMEM>; break;
+    case 16: k = gine_agg_proj_kernel<VEC, 16, SMEM>; break;
+    default: k = gine_agg_proj_kernel<VEC, 32, SMEM>; break;
+    }
+    if (smem > 48 * 1024) GNNB_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k<<<grid, 256, smem, s>>>(a);
+    return GNNB_OK;
+}
+
+__global__ void permute_edge_rows_kernel(const float *__restrict__ src, int dim,
+                                         const int32_t *__restrict__ idx, int64_t e,
+                                         float *__restrict__ dst, int ldd)
+{
+    const int64_t total = e * ldd;
+    for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < total;
+         t += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t k = t / ldd;
+        const int j = (int)(t - k * ldd);
+        dst[t] = j < dim ? __ldg(src + (size_t)__ldg(idx + k) * dim + j) : 0.0f;
+    }
+}
+
+}  // namespace
+
+int launch_gine_agg_proj(const GineProjAggArgs &a, cudaStream_t s, int *launches)
+{
+    if (a.n <= 0) return GNNB_OK;
+    GNNB_REQUIRE(a.F > 0 && a.edge_dim >= 1 && a.edge_dim <= kGineMaxEdgeDim && a.lde % 4 == 0 &&
+                     a.lde >= a.edge_dim && a.ldw % 4 == 0 && a.ldw >= a.F && aligned16(a.ef_sorted),
+                 "gine aggregation: bad arguments");
+    const bool v4 = (a.F % 4 == 0) && (a.ldx % 4 == 0) && (a.ldo % 4 == 0) && aligned16(a.x) &&
+                    aligned16(a.out) && aligned16(a.We_t);
+    const int vec = v4 ? 4 : 1;
+    int lpr = 1;
+    while (lpr < 32 && lpr * vec < a.F) lpr *= 2;
+    const int rows_per_block = 8 * (32 / lpr);
+    int64_t grid64 = ceil_div64(a.n, rows_per_block);
+    const int64_t cap = (int64_t)kNumSMs * 8 * 4;
+    const int grid = (int)(grid64 < cap ? grid64 : cap);
+    // W_e^T + b_e in shared memory when they fit (edge_dim 64 at F = 512: 130 KB); wider layers
+    // read them through the read-only cache
+    const size_t smem = sizeof(float) * ((size_t)a.edge_dim * a.ldw + a.F);
+    const bool in_smem = smem <= 200 * 1024;
+    int rc;
+    if (in_smem)
+        rc = vec == 4 ? launch_gine_proj_lpr<4, true>(a, lpr, grid, smem, s)
+                      : launch_gine_proj_lpr<1, true>(a, lpr, grid, smem, s);
+    else
+        rc = vec == 4 ? launch_gine_proj_lpr<4, false>(a, lpr, grid, 0, s)
+                      : launch_gine_proj_lpr<1, false>(a, lpr, grid, 0, s);
+    GNNB_TRY(rc);
+    GNNB_CUDA(cudaGetLastError());
+    if (launches) ++*launches;
+    return GNNB_OK;
+}
+
+int launch_permute_edge_rows(const float *src, int dim, const int32_t *idx, int e, float *dst,
+                             int ldd, cudaStream_t s, int *launches)
+{
+    if (e <= 0) return GNNB_OK;
+    const int64_t total = (int64_t)e * ldd;
+    int64_t grid64 = ceil_div64(total, 256);
+    const int64_t cap = (int64_t)kNumSMs * 16;
+    permute_edge_rows_kernel<<<(int)(grid64 < cap ? grid64 : cap), 256, 0, s>>>(src, dim, idx, e,
+                                                                                 dst, ldd);
+    GNNB_CUDA(cudaGetLastError());
+    if (launches) ++*launches;
+    return GNNB_OK;
+}
+
 }  // namespace gnnb

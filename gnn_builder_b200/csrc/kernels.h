@@ -20,7 +20,8 @@ struct TableWorkspace {
 
 // edge_list [E][2] local ids; node_ptr/edge_ptr (device int64, G+1 entries) translate them to
 // ids in the batch union (pass nullptr for a single graph).  Writes in/out degree, offsets
-// (n entries), neighbor_table (e entries) and, when non-null, edge_index_table.
+// (n entries), neighbor_table (e entries) and, when non-null, edge_index_table (edge ids relative
+// to edge_list, i.e. to edge_base).
 // node_base/edge_base: values of node_ptr[0]/edge_ptr[0] when the pointers address a sub-range
 // (chunk) of a larger batch whose x / edge_list pointers were advanced accordingly.
 int build_tables(const int32_t *edge_list, const int64_t *node_ptr, const int64_t *edge_ptr,
@@ -145,6 +146,30 @@ struct GineAggArgs {
     float eps;
 };
 int launch_gine_agg(const GineAggArgs &a, cudaStream_t s, int *launches);
+
+// GINE aggregation of the model path: the same sum with the edge projection computed on the fly,
+// proj_e = b_e + sum_j W_e[.][j] ef[e][j], so the [E][F] projection is never materialised.  The edge
+// features are read in CSR slot order (ef_sorted[k] belongs to neighbor slot k, see
+// launch_permute_edge_rows).  Every operation is separately rounded in the reference's order.
+constexpr int kGineMaxEdgeDim = 64;
+struct GineProjAggArgs {
+    const float *x;          // [n][ldx]
+    int ldx, F;
+    const float *ef_sorted;  // [E][lde] edge features in neighbor-slot order (lde = round_up(edge_dim, 4))
+    int lde, edge_dim;
+    const float *We_t;       // [edge_dim][ldw] W_e^T (ldw multiple of 4, zero padded)
+    int ldw;
+    const float *be;         // [F] b_e
+    float *out;              // [n][ldo]
+    int ldo;
+    const int32_t *offsets, *nbr, *in_deg;
+    int n;
+    float eps;
+};
+int launch_gine_agg_proj(const GineProjAggArgs &a, cudaStream_t s, int *launches);
+// dst[k][0..dim) = src[idx[k]][0..dim) for k < e (dst row stride ldd, src row stride dim)
+int launch_permute_edge_rows(const float *src, int dim, const int32_t *idx, int e, float *dst,
+                             int ldd, cudaStream_t s, int *launches);
 
 struct PnaAggArgs {
     const float *ab;       // [n][2F]: cols [0,F) = x.W_nbr^T, cols [F,2F) = x.W_self^T + b_pre

@@ -7,6 +7,7 @@
 #include "model.h"
 
 #include <algorithm>
+#include <cstddef>
 #include <cstring>
 #include <mutex>
 
@@ -91,10 +92,15 @@ void enumerate_params(gnnb_model *m)
             add_param(m, base + "_conv_lin_weight", {fo, fi});
             break;
         case GNNB_CONV_GIN:
+        case GNNB_CONV_GINE:
             add_param(m, base + "_mlp_linear_0_weight", {fo, fi});
             add_param(m, base + "_mlp_linear_0_bias", {fo});
             add_param(m, base + "_mlp_linear_1_weight", {fo, fo});
             add_param(m, base + "_mlp_linear_1_bias", {fo});
+            if (d.conv_type == GNNB_CONV_GINE) {   // PyG GINEConv's edge linear: lin [F_in][edge_dim]
+                add_param(m, base + "_conv_lin_weight", {fi, d.edge_dim});
+                add_param(m, base + "_conv_lin_bias", {fi});
+            }
             break;
         case GNNB_CONV_SAGE:
             add_param(m, base + "_conv_lin_l_weight", {fo, fi});
@@ -206,10 +212,19 @@ extern "C" int gnnb_host_unregister(void *ptr)
 extern "C" int gnnb_model_create(const gnnb_model_desc *desc, int device, gnnb_model_t **out)
 {
     GNNB_REQUIRE(desc != nullptr && out != nullptr, "null argument");
-    const gnnb_model_desc &d = *desc;
-    GNNB_REQUIRE(d.conv_type >= GNNB_CONV_GCN && d.conv_type <= GNNB_CONV_PNA,
-                 "conv_type must be GCN, GIN, SAGE or PNA (models.py:453-459; GAT has no kernel "
-                 "in the reference either)");
+    // edge_dim is the last field and only GINE callers are required to have it: copy the fields
+    // before it, then read it for GINE only (a caller built against the older, shorter struct
+    // never has bytes read past its end)
+    gnnb_model_desc d{};
+    std::memcpy(&d, desc, offsetof(gnnb_model_desc, edge_dim));
+    GNNB_REQUIRE(d.conv_type >= GNNB_CONV_GCN && d.conv_type <= GNNB_CONV_GINE,
+                 "conv_type must be GCN, GIN, SAGE, PNA or GINE (models.py:453-459; GAT has no "
+                 "kernel in the reference either)");
+    if (d.conv_type == GNNB_CONV_GINE) {
+        d.edge_dim = desc->edge_dim;
+        GNNB_REQUIRE(d.edge_dim >= 1 && d.edge_dim <= kGineMaxEdgeDim,
+                     "GINE edge_dim must be 1.." + std::to_string(kGineMaxEdgeDim));
+    }
     GNNB_REQUIRE(d.num_layers >= 0 && d.num_layers <= 64, "num_layers out of range");
     GNNB_REQUIRE(d.in_dim > 0 && d.hidden_dim > 0 && d.out_dim > 0, "dimensions must be positive");
     GNNB_REQUIRE(d.num_layers > 0 || d.in_dim == d.out_dim,
@@ -258,8 +273,9 @@ extern "C" int gnnb_model_destroy(gnnb_model_t *m)
     fused_release(m);
     fused_tc_release(m);
     m->prof.release();
-    DeviceBuf *bufs[] = {&m->weights, &m->weight_images, &m->st_x, &m->st_coo, &m->st_nptr, &m->st_eptr, &m->st_out,
+    DeviceBuf *bufs[] = {&m->weights, &m->weight_images, &m->st_x, &m->st_coo, &m->st_ef, &m->st_nptr, &m->st_eptr, &m->st_out,
                          &m->in_deg, &m->out_deg, &m->offsets, &m->nbr, &m->nbr_hub, &m->dinv,
+                         &m->edge_index, &m->ef_sorted,
                          &m->feat[0], &m->feat[1], &m->agg, &m->hid, &m->wide, &m->pooled,
                          &m->hbuf[0], &m->hbuf[1], &m->pool_tmp, &m->ptr_tmp, &m->edge_flag};
     for (DeviceBuf *b : bufs) b->release();
@@ -327,7 +343,7 @@ extern "C" int gnnb_model_finalize(gnnb_model_t *m)
     const gnnb_model_desc &d = m->d;
     Packer pk;
     std::vector<PendingLinear> head_p;
-    struct PendingLayer { int fi, fo; PendingLinear a, b, c, d; };
+    struct PendingLayer { int fi, fo; PendingLinear a, b, c, d, e; };
     std::vector<PendingLayer> layer_p;
     size_t idx = 0;
     {
@@ -352,6 +368,12 @@ extern "C" int gnnb_model_finalize(gnnb_model_t *m)
             L.a = pack_linear(pk, param(m, idx), param(m, idx + 1), fo, fi);
             L.b = pack_linear(pk, param(m, idx + 2), param(m, idx + 3), fo, fo);
             idx += 4;
+            break;
+        case GNNB_CONV_GINE:  // a, b: the GIN MLP; e: the edge linear (read by the aggregation)
+            L.a = pack_linear(pk, param(m, idx), param(m, idx + 1), fo, fi);
+            L.b = pack_linear(pk, param(m, idx + 2), param(m, idx + 3), fo, fo);
+            L.e = pack_linear(pk, param(m, idx + 4), param(m, idx + 5), fi, d.edge_dim);
+            idx += 6;
             break;
         case GNNB_CONV_SAGE:  // a = lin_l (bias), b = lin_r (no bias)
             L.a = pack_linear(pk, param(m, idx), param(m, idx + 1), fo, fi);
@@ -390,7 +412,7 @@ extern "C" int gnnb_model_finalize(gnnb_model_t *m)
         LayerPack lp;
         lp.fi = L.fi; lp.fo = L.fo;
         lp.a = resolve(L.a, base); lp.b = resolve(L.b, base);
-        lp.c = resolve(L.c, base); lp.d = resolve(L.d, base);
+        lp.c = resolve(L.c, base); lp.d = resolve(L.d, base); lp.e = resolve(L.e, base);
         m->layers.push_back(lp);
     }
     {   // tensor-core weight images for the layerwise GEMMs (one allocation, built on the device)
@@ -413,6 +435,7 @@ extern "C" int gnnb_model_finalize(gnnb_model_t *m)
     }
     fused_release(m);
     fused_tc_release(m);
+    // neither fused kernel takes GINE (they leave m->fused / m->fused_tc null): it runs layerwise
     GNNB_TRY(fused_prepare(m));
     GNNB_TRY(fused_tc_prepare(m));
     m->finalized = true;
@@ -484,9 +507,11 @@ static GemmArgs gemm_args(const float *A, int lda, const PackedLinear &L, float 
     return g;
 }
 
-// x/coo/node_ptr/edge_ptr/out are DEVICE pointers; node_ptr/edge_ptr address graph 0 of this
-// chunk and hold absolute offsets (node_base/edge_base = their first values).
-static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, const int64_t *node_ptr,
+// x/coo/ef/node_ptr/edge_ptr/out are DEVICE pointers; node_ptr/edge_ptr address graph 0 of this
+// chunk and hold absolute offsets (node_base/edge_base = their first values).  ef: the chunk's edge
+// features [E][edge_dim] (GINE only).
+static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, const float *ef,
+                         const int64_t *node_ptr,
                          const int64_t *edge_ptr, int64_t node_base, int64_t edge_base,
                          int n_graphs, int64_t T64, int64_t E64, float *out, cudaStream_t s,
                          int *launches)
@@ -505,14 +530,30 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
     GNNB_TRY(m->nbr.ensure(sizeof(int32_t) * (size_t)En));
     int32_t *in_deg = m->in_deg.as<int32_t>(), *offsets = m->offsets.as<int32_t>();
     int32_t *nbr = m->nbr.as<int32_t>();
+    const bool gine = d.conv_type == GNNB_CONV_GINE;
+    // GINE has no heavy-row bucketing or hub hints, as PNA
+    const bool bucketed = d.conv_type != GNNB_CONV_PNA && !gine;
+    const int lde = round_up(std::max(d.edge_dim, 1), 4);
     if (d.num_layers > 0) {
         ProfScope ps(m->prof, PROF_TABLES, s);
         // the out-degree table (lib:1051-1083) is only read by the optional hub-row hints
-        const bool want_out_deg = !strict && hub_l2_budget() > 0 && d.conv_type != GNNB_CONV_PNA &&
-                                  n_graphs > 0 && T64 / n_graphs > 50000;
-        GNNB_TRY(build_tables(coo, n_graphs > 1 ? node_ptr : nullptr, edge_ptr, node_base, edge_base,
-                              n_graphs, T, E, in_deg, want_out_deg ? m->out_deg.as<int32_t>() : nullptr,
-                              offsets, nbr, nullptr, m->tws, s, launches, m->edge_flag.as<int>()));
+        const bool want_out_deg = !strict && hub_l2_budget() > 0 && bucketed && n_graphs > 0 &&
+                                  T64 / n_graphs > 50000;
+        int32_t *eidx = nullptr;
+        if (gine) {
+            GNNB_TRY(m->edge_index.ensure(sizeof(int32_t) * (size_t)En));
+            eidx = m->edge_index.as<int32_t>();
+        }
+        // GINE always passes the offsets: its slot -> source gather then checks every endpoint
+        GNNB_TRY(build_tables(coo, n_graphs > 1 || gine ? node_ptr : nullptr, edge_ptr, node_base,
+                              edge_base, n_graphs, T, E, in_deg,
+                              want_out_deg ? m->out_deg.as<int32_t>() : nullptr, offsets, nbr, eidx,
+                              m->tws, s, launches, m->edge_flag.as<int>()));
+        if (gine) {   // edge features in neighbor-slot order, once per run; every layer reads them in order
+            GNNB_TRY(m->ef_sorted.ensure(sizeof(float) * (size_t)En * lde));
+            GNNB_TRY(launch_permute_edge_rows(ef, d.edge_dim, eidx, E, m->ef_sorted.as<float>(), lde, s,
+                                              launches));
+        }
     }
     const float *dinv = nullptr;
     if (d.conv_type == GNNB_CONV_GCN && !strict && d.num_layers > 0) {
@@ -525,8 +566,7 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
     m->heavy.n_heavy = m->heavy.n_chunks = 0;
     const int heavy_thr = heavy_threshold();
     m->last_hub_rows = 0;
-    if (!strict && d.num_layers > 0 && d.conv_type != GNNB_CONV_PNA && n_graphs > 0 &&
-        T64 / n_graphs > 50000) {
+    if (!strict && d.num_layers > 0 && bucketed && n_graphs > 0 && T64 / n_graphs > 50000) {
         GNNB_TRY(find_heavy_rows(in_deg, T, heavy_thr, m->tws, m->heavy, s, launches));
         GNNB_TRY(heavy_setup(m->tws, m->heavy.n_chunks, maxf));
         // a feature matrix larger than L2: keep the rows of the most-referenced sources resident
@@ -548,7 +588,7 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
     GNNB_TRY(m->feat[0].ensure(sizeof(float) * (size_t)Tn * ldf));
     GNNB_TRY(m->feat[1].ensure(sizeof(float) * (size_t)Tn * ldf));
     GNNB_TRY(m->agg.ensure(sizeof(float) * (size_t)Tn * ldf));
-    if (d.conv_type == GNNB_CONV_GIN || d.conv_type == GNNB_CONV_PNA)
+    if (d.conv_type == GNNB_CONV_GIN || d.conv_type == GNNB_CONV_PNA || gine)
         GNNB_TRY(m->hid.ensure(sizeof(float) * (size_t)Tn * ldf));
     if (d.conv_type == GNNB_CONV_PNA)
         GNNB_TRY(m->wide.ensure(sizeof(float) * (size_t)Tn * 14 * (size_t)ldf));
@@ -580,6 +620,20 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
         case GNNB_CONV_GIN: {
             a.mode = AGG_GIN;
             { ProfScope ps(m->prof, PROF_AGG, s); GNNB_TRY(launch_agg(a, strict, s, launches)); }
+            float *hid = m->hid.as<float>();
+            GemmArgs g0 = gemm_args(a.out, a.ldo, L.a, hid, ld_out, T, GNNB_ACT_RELU);  // lib:1537-1541
+            { ProfScope ps(m->prof, PROF_GEMM, s); GNNB_TRY(launch_gemm(g0, strict, s, launches)); }
+            GemmArgs g1 = gemm_args(hid, ld_out, L.b, dst, ld_out, T, d.gnn_act, skip, cur_ld);
+            { ProfScope ps(m->prof, PROF_GEMM, s); GNNB_TRY(launch_gemm(g1, strict, s, launches)); }
+            break;
+        }
+        case GNNB_CONV_GINE: {
+            GineProjAggArgs ga{};
+            ga.x = cur; ga.ldx = cur_ld; ga.F = fi; ga.ef_sorted = m->ef_sorted.as<float>();
+            ga.lde = lde; ga.edge_dim = d.edge_dim; ga.We_t = L.e.Wt; ga.ldw = L.e.ldw; ga.be = L.e.bias;
+            ga.out = a.out; ga.ldo = a.ldo; ga.offsets = offsets; ga.nbr = nbr; ga.in_deg = in_deg;
+            ga.n = T; ga.eps = d.gin_eps;
+            { ProfScope ps(m->prof, PROF_AGG, s); GNNB_TRY(launch_gine_agg_proj(ga, s, launches)); }
             float *hid = m->hid.as<float>();
             GemmArgs g0 = gemm_args(a.out, a.ldo, L.a, hid, ld_out, T, GNNB_ACT_RELU);  // lib:1537-1541
             { ProfScope ps(m->prof, PROF_GEMM, s); GNNB_TRY(launch_gemm(g0, strict, s, launches)); }
@@ -733,17 +787,37 @@ static int fused_any_status(gnnb_model_t *m, int *status)
     return m->last_kernel == 3 ? fused_tc_status(m, status) : fused_status(m, status);
 }
 
-extern "C" int gnnb_model_run_batch_async(gnnb_model_t *m, const float *x, const int32_t *edge_list,
-                                          const int64_t *node_ptr, const int64_t *edge_ptr,
-                                          int n_graphs, int64_t total_nodes, int64_t total_edges,
-                                          float *out, void *stream)
+// a GINE handle takes its edge features through the *_edges entry points, every other handle
+// through the plain ones
+static int check_edges_entry(gnnb_model_t *m, bool edges_entry)
 {
     GNNB_TRY(check_ready(m));
+    const bool gine = m->d.conv_type == GNNB_CONV_GINE;
+    if (gine && !edges_entry) {
+        set_error("a GINE model needs its edge features: run it with gnnb_model_run_batch_edges or "
+                  "gnnb_model_run_batch_edges_async");
+        return GNNB_ERR_INVALID;
+    }
+    if (!gine && edges_entry) {
+        set_error("the *_edges entry points run GINE models only; this model has no edge features");
+        return GNNB_ERR_INVALID;
+    }
+    return GNNB_OK;
+}
+
+static int run_batch_async(gnnb_model_t *m, const float *x, const int32_t *edge_list,
+                           const float *edge_attr, const int64_t *node_ptr, const int64_t *edge_ptr,
+                           int n_graphs, int64_t total_nodes, int64_t total_edges, float *out,
+                           void *stream)
+{
     DeviceScope on_device(m->device);
     GNNB_REQUIRE(n_graphs >= 0 && total_nodes >= 0 && total_edges >= 0, "negative size");
     GNNB_REQUIRE(node_ptr != nullptr && edge_ptr != nullptr && out != nullptr, "null argument");
     if (n_graphs == 0) return GNNB_OK;
     GNNB_REQUIRE(is_device_pointer(x) || total_nodes == 0, "run_batch_async needs device pointers");
+    if (m->d.conv_type == GNNB_CONV_GINE)
+        GNNB_REQUIRE(total_edges == 0 || is_device_pointer(edge_attr),
+                     "edge_attr must be a device pointer (null with edges present)");
     cudaStream_t s = stream ? (cudaStream_t)stream : m->stream;
     m->last_launches = 0;
     int path, kernel;
@@ -757,15 +831,35 @@ extern "C" int gnnb_model_run_batch_async(gnnb_model_t *m, const float *x, const
         return run_fused(m, kernel, x, edge_list, node_ptr, edge_ptr, n_graphs, total_nodes, hint_n,
                          out, s);
     GNNB_TRY(edge_flag_reset(m, s));
-    return run_layerwise(m, x, edge_list, node_ptr, edge_ptr, 0, 0, n_graphs, total_nodes,
+    return run_layerwise(m, x, edge_list, edge_attr, node_ptr, edge_ptr, 0, 0, n_graphs, total_nodes,
                          total_edges, out, s, &m->last_launches);
 }
 
-extern "C" int gnnb_model_run_batch(gnnb_model_t *m, const float *x, const int32_t *edge_list,
-                                    const int64_t *node_ptr, const int64_t *edge_ptr, int n_graphs,
-                                    float *out)
+extern "C" int gnnb_model_run_batch_async(gnnb_model_t *m, const float *x, const int32_t *edge_list,
+                                          const int64_t *node_ptr, const int64_t *edge_ptr,
+                                          int n_graphs, int64_t total_nodes, int64_t total_edges,
+                                          float *out, void *stream)
 {
-    GNNB_TRY(check_ready(m));
+    GNNB_TRY(check_edges_entry(m, false));
+    return run_batch_async(m, x, edge_list, nullptr, node_ptr, edge_ptr, n_graphs, total_nodes,
+                           total_edges, out, stream);
+}
+
+extern "C" int gnnb_model_run_batch_edges_async(gnnb_model_t *m, const float *x,
+                                                const int32_t *edge_list, const float *edge_attr,
+                                                const int64_t *node_ptr, const int64_t *edge_ptr,
+                                                int n_graphs, int64_t total_nodes,
+                                                int64_t total_edges, float *out, void *stream)
+{
+    GNNB_TRY(check_edges_entry(m, true));
+    return run_batch_async(m, x, edge_list, edge_attr, node_ptr, edge_ptr, n_graphs, total_nodes,
+                           total_edges, out, stream);
+}
+
+static int run_batch(gnnb_model_t *m, const float *x, const int32_t *edge_list,
+                     const float *edge_attr, const int64_t *node_ptr, const int64_t *edge_ptr,
+                     int n_graphs, float *out)
+{
     DeviceScope on_device(m->device);
     GNNB_REQUIRE(n_graphs >= 0, "negative n_graphs");
     if (n_graphs == 0) return GNNB_OK;
@@ -789,6 +883,12 @@ extern "C" int gnnb_model_run_batch(gnnb_model_t *m, const float *x, const int32
     GNNB_REQUIRE(T >= 0 && E >= 0 && T < (1ll << 40) && E < (1ll << 40), "bad node_ptr/edge_ptr totals");
     GNNB_REQUIRE(T == 0 || x != nullptr, "x is null");
     GNNB_REQUIRE(E == 0 || edge_list != nullptr, "edge_list is null");
+    const bool gine = d.conv_type == GNNB_CONV_GINE;
+    if (gine) {
+        GNNB_REQUIRE(E == 0 || edge_attr != nullptr, "edge_attr is null");
+        GNNB_REQUIRE(E == 0 || is_device_pointer(edge_attr) == dev,
+                     "edge_attr must live in the same memory space as node_ptr");
+    }
     // validation of graphs [a, b): offsets non-decreasing, capacities respected; updates the maxima
     int64_t max_n = 0, max_e = 0;
     auto scan = [&](int a, int b) -> int {
@@ -914,7 +1014,7 @@ extern "C" int gnnb_model_run_batch(gnnb_model_t *m, const float *x, const int32
             if (!too_big) {
                 // capacity overflow or non-finite activations: redo the batch on the layerwise path
                 m->path = GNNB_PATH_LAYERWISE;
-                const int rc2 = gnnb_model_run_batch(m, x, edge_list, node_ptr, edge_ptr, n_graphs, out);
+                const int rc2 = run_batch(m, x, edge_list, edge_attr, node_ptr, edge_ptr, n_graphs, out);
                 m->path = GNNB_PATH_AUTO;
                 return rc2;
             }
@@ -927,7 +1027,7 @@ extern "C" int gnnb_model_run_batch(gnnb_model_t *m, const float *x, const int32
         GNNB_TRY(scan(0, n_graphs));
     }
 
-    const float *dx = x;
+    const float *dx = x, *def = edge_attr;
     const int32_t *dcoo = edge_list;
     const int64_t *dnp = node_ptr, *dep = edge_ptr;
     float *dout = out;
@@ -943,6 +1043,13 @@ extern "C" int gnnb_model_run_batch(gnnb_model_t *m, const float *x, const int32
         if (E > 0)
             GNNB_CUDA(cudaMemcpyAsync(m->st_coo.ptr, edge_list, sizeof(int32_t) * 2 * (size_t)E,
                                       cudaMemcpyHostToDevice, s));
+        if (gine) {
+            GNNB_TRY(m->st_ef.ensure(sizeof(float) * (size_t)std::max<int64_t>(E, 1) * d.edge_dim));
+            if (E > 0)
+                GNNB_CUDA(cudaMemcpyAsync(m->st_ef.ptr, edge_attr, sizeof(float) * (size_t)E * d.edge_dim,
+                                          cudaMemcpyHostToDevice, s));
+            def = m->st_ef.as<float>();
+        }
         GNNB_CUDA(cudaMemcpyAsync(m->st_nptr.ptr, node_ptr, 8 * ((size_t)n_graphs + 1), cudaMemcpyHostToDevice, s));
         GNNB_CUDA(cudaMemcpyAsync(m->st_eptr.ptr, edge_ptr, 8 * ((size_t)n_graphs + 1), cudaMemcpyHostToDevice, s));
         dx = m->st_x.as<float>();
@@ -967,7 +1074,7 @@ extern "C" int gnnb_model_run_batch(gnnb_model_t *m, const float *x, const int32
             int g1 = g0 + 1;
             while (g1 < n_graphs && hn[g1 + 1] - hn[g0] <= kChunkNodes) g1++;
             GNNB_TRY(run_layerwise(m, dx + (size_t)hn[g0] * d.in_dim, dcoo + 2 * (size_t)he[g0],
-                                   dnp + g0, dep + g0, hn[g0], he[g0], g1 - g0, hn[g1] - hn[g0],
+                                   gine ? def + (size_t)he[g0] * d.edge_dim : nullptr, dnp + g0, dep + g0, hn[g0], he[g0], g1 - g0, hn[g1] - hn[g0],
                                    he[g1] - he[g0], dout + (size_t)g0 * d.mlp_out, s,
                                    &m->last_launches));
             g0 = g1;
@@ -1004,6 +1111,22 @@ extern "C" int gnnb_model_run_batch(gnnb_model_t *m, const float *x, const int32
     GNNB_CUDA(cudaStreamSynchronize(s));
     if (ran_layerwise) GNNB_TRY(edge_flag_check(m));
     return GNNB_OK;
+}
+
+extern "C" int gnnb_model_run_batch(gnnb_model_t *m, const float *x, const int32_t *edge_list,
+                                    const int64_t *node_ptr, const int64_t *edge_ptr, int n_graphs,
+                                    float *out)
+{
+    GNNB_TRY(check_edges_entry(m, false));
+    return run_batch(m, x, edge_list, nullptr, node_ptr, edge_ptr, n_graphs, out);
+}
+
+extern "C" int gnnb_model_run_batch_edges(gnnb_model_t *m, const float *x, const int32_t *edge_list,
+                                          const float *edge_attr, const int64_t *node_ptr,
+                                          const int64_t *edge_ptr, int n_graphs, float *out)
+{
+    GNNB_TRY(check_edges_entry(m, true));
+    return run_batch(m, x, edge_list, edge_attr, node_ptr, edge_ptr, n_graphs, out);
 }
 
 extern "C" int gnnb_model_run_graph(gnnb_model_t *m, const float *node_features,

@@ -27,6 +27,7 @@ struct PackedLinear {
 struct LayerPack {
     int fi = 0, fo = 0;
     PackedLinear a, b, c, d;  // meaning depends on the conv type (see model.cu pack_layer)
+    PackedLinear e;           // GINE: the edge linear W_e^T [edge_dim][ldw], b_e
 };
 
 // fused-kernel plans (fused.cu, fused_tc.cu)
@@ -92,7 +93,7 @@ struct gnnb_model {
     gnnb::TcPlan *fused_tc = nullptr;
 
     // staging for host-pointer calls
-    gnnb::DeviceBuf st_x, st_coo, st_nptr, st_eptr, st_out;
+    gnnb::DeviceBuf st_x, st_coo, st_ef, st_nptr, st_eptr, st_out;
     // chunked ingest pipeline (host buffers -> fused kernel): double-buffered chunk staging, a
     // copy-in and a copy-out stream beside the compute stream, events for the hand-offs
     gnnb::DeviceBuf ch_x[2], ch_coo[2], ch_nptr[2], ch_eptr[2];
@@ -101,6 +102,7 @@ struct gnnb_model {
     // layerwise workspaces
     gnnb::DeviceBuf in_deg, out_deg, offsets, nbr, nbr_hub, dinv, feat[2], agg, hid, wide, pooled,
         hbuf[2], pool_tmp, ptr_tmp;
+    gnnb::DeviceBuf edge_index, ef_sorted;   // GINE: edge id and edge features per neighbor slot
     int last_hub_rows = 0;   // sources whose feature rows the last large-graph run kept L2-resident
     gnnb::TableWorkspace tws;
     gnnb::HeavyList heavy;       // rows above the heavy threshold of the current layerwise run

@@ -96,6 +96,26 @@ __global__ void gather_sources_kernel(const int32_t *__restrict__ edge_list,
         nbr[i] = __ldg(edge_list + 2 * (size_t)__ldg(edge_index + i));
 }
 
+// the same for a batch of graphs: local source ids are translated to union ids.  A slot whose edge
+// has an endpoint outside its graph (flagged by edge_prepare_kernel, parked on edge 0) reads
+// source 0, so the tables stay memory-safe until the caller reports the error.
+__global__ void gather_sources_batch_kernel(const int32_t *__restrict__ edge_list,
+                                            const int32_t *__restrict__ edge_index,
+                                            const int64_t *__restrict__ node_ptr,
+                                            const int64_t *__restrict__ edge_ptr, int64_t node_base,
+                                            int64_t edge_base, int n_graphs, int e,
+                                            int32_t *__restrict__ nbr)
+{
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < e; i += gridDim.x * blockDim.x) {
+        const int eid = __ldg(edge_index + i);
+        const int g = find_segment(edge_ptr, n_graphs, (int64_t)eid + edge_base);
+        const int64_t b0 = __ldg(node_ptr + g);
+        const int limit = (int)(__ldg(node_ptr + g + 1) - b0);
+        const int src = __ldg(edge_list + 2 * (size_t)eid);
+        nbr[i] = (unsigned)src < (unsigned)limit ? src + (int)(b0 - node_base) : 0;
+    }
+}
+
 // row-partitioned graph: this rank owns destination rows [row_begin, row_begin + n_local); sources
 // keep their global ids
 __global__ void edge_prepare_partition_kernel(const int32_t *__restrict__ edge_list, int e,
@@ -274,6 +294,21 @@ int build_neighbor_tables(const int32_t *edge_list, const int32_t *in_deg, int n
     return GNNB_OK;
 }
 
+// neighbor table from the sorted edge-index table (sources as union ids for a batch of graphs)
+static int gather_sources(const int32_t *edge_list, const int32_t *edge_index, const int64_t *node_ptr,
+                          const int64_t *edge_ptr, int64_t node_base, int64_t edge_base, int n_graphs,
+                          int e, int32_t *nbr, cudaStream_t s, int *launches)
+{
+    if (node_ptr != nullptr)
+        gather_sources_batch_kernel<<<grid_for(e, 256), 256, 0, s>>>(
+            edge_list, edge_index, node_ptr, edge_ptr, node_base, edge_base, n_graphs, e, nbr);
+    else
+        gather_sources_kernel<<<grid_for(e, 256), 256, 0, s>>>(edge_list, edge_index, e, nbr);
+    GNNB_CUDA(cudaGetLastError());
+    if (launches) ++*launches;
+    return GNNB_OK;
+}
+
 int build_tables(const int32_t *edge_list, const int64_t *node_ptr, const int64_t *edge_ptr,
                  int64_t node_base, int64_t edge_base, int n_graphs, int n, int e, int32_t *in_deg, int32_t *out_deg, int32_t *offsets,
                  int32_t *nbr, int32_t *edge_index, TableWorkspace &ws, cudaStream_t s,
@@ -283,17 +318,17 @@ int build_tables(const int32_t *edge_list, const int64_t *node_ptr, const int64_
     // large edge lists: in-degrees as run lengths of the sorted destination keys (no atomics);
     // out_deg == nullptr: the caller does not need the out-degree table (nothing in the model path
     // reads it unless the hub-row hints are on -- the reference never reads it at all)
-    const bool sorted_degrees = e >= (1 << 20) && edge_index == nullptr;
+    const bool sorted_degrees = e >= (1 << 20);
     GNNB_CUDA(cudaMemsetAsync(in_deg, 0, sizeof(int32_t) * (size_t)n, s));
     if (out_deg != nullptr) GNNB_CUDA(cudaMemsetAsync(out_deg, 0, sizeof(int32_t) * (size_t)n, s));
     if (e > 0) {
         GNNB_TRY(ws.keys_in.ensure(sizeof(uint32_t) * (size_t)e));
         GNNB_TRY(ws.vals_in.ensure(sizeof(int32_t) * (size_t)e));
         if (edge_index) {
-            GNNB_REQUIRE(node_ptr == nullptr, "edge-index tables are single-graph only");
             edge_prepare_kernel<true, true><<<grid_for(e, 256), 256, 0, s>>>(
-                edge_list, nullptr, nullptr, 0, 0, 0, n, e, ws.keys_in.as<uint32_t>(),
-                ws.vals_in.as<int32_t>(), in_deg, out_deg, bad);
+                edge_list, node_ptr, edge_ptr, node_base, edge_base, n_graphs, n, e,
+                ws.keys_in.as<uint32_t>(), ws.vals_in.as<int32_t>(),
+                sorted_degrees ? nullptr : in_deg, out_deg, bad);
         } else {
             edge_prepare_kernel<true, false><<<grid_for(e, 256), 256, 0, s>>>(
                 edge_list, node_ptr, edge_ptr, node_base, edge_base, n_graphs, n, e,
@@ -304,21 +339,23 @@ int build_tables(const int32_t *edge_list, const int64_t *node_ptr, const int64_
         if (launches) ++*launches;
     }
     if (sorted_degrees) {
-        GNNB_TRY(sort_pairs(ws, e, n, nbr, s, launches));
+        GNNB_TRY(sort_pairs(ws, e, n, edge_index ? edge_index : nbr, s, launches));
         GNNB_CUDA(cudaMemsetAsync(offsets, 0, sizeof(int32_t) * (size_t)n, s));   // run starts (scratch)
         run_bounds_kernel<<<grid_for(e, 256), 256, 0, s>>>(ws.keys_out.as<uint32_t>(), e, offsets, in_deg);
         run_length_kernel<<<grid_for(n, 256), 256, 0, s>>>(in_deg, offsets, n);
         GNNB_CUDA(cudaGetLastError());
         if (launches) *launches += 2;
-        return scan_offsets(in_deg, offsets, n, ws, s, launches);
+        GNNB_TRY(scan_offsets(in_deg, offsets, n, ws, s, launches));
+        if (edge_index) GNNB_TRY(gather_sources(edge_list, edge_index, node_ptr, edge_ptr, node_base,
+                                                edge_base, n_graphs, e, nbr, s, launches));
+        return GNNB_OK;
     }
     GNNB_TRY(scan_offsets(in_deg, offsets, n, ws, s, launches));
     if (e > 0) {
         if (edge_index) {
             GNNB_TRY(sort_pairs(ws, e, n, edge_index, s, launches));
-            gather_sources_kernel<<<grid_for(e, 256), 256, 0, s>>>(edge_list, edge_index, e, nbr);
-            GNNB_CUDA(cudaGetLastError());
-            if (launches) ++*launches;
+            GNNB_TRY(gather_sources(edge_list, edge_index, node_ptr, edge_ptr, node_base, edge_base,
+                                    n_graphs, e, nbr, s, launches));
         } else {
             GNNB_TRY(sort_pairs(ws, e, n, nbr, s, launches));
         }

@@ -24,6 +24,7 @@ class GraphBatch:
     coo: np.ndarray        # int32   [total_edges, 2]  (src, dst), node ids local to the graph
     node_ptr: np.ndarray   # int64   [n_graphs + 1]
     edge_ptr: np.ndarray   # int64   [n_graphs + 1]
+    edge_attr: Optional[np.ndarray] = None   # float32 [total_edges, edge_dim], row i = COO edge i
 
     @property
     def n_graphs(self) -> int:
@@ -46,12 +47,19 @@ class GraphBatch:
         e0, e1 = int(self.edge_ptr[g]), int(self.edge_ptr[g + 1])
         return self.x[n0:n1], self.coo[e0:e1]
 
+    def graph_edge_attr(self, g: int) -> Optional[np.ndarray]:
+        """edge features of graph ``g`` (None when the batch has none)"""
+        if self.edge_attr is None:
+            return None
+        return self.edge_attr[int(self.edge_ptr[g]):int(self.edge_ptr[g + 1])]
+
     def slice(self, g0: int, g1: int) -> "GraphBatch":
         """Contiguous sub-batch [g0, g1) (views, re-based offsets)."""
         n0, n1 = int(self.node_ptr[g0]), int(self.node_ptr[g1])
         e0, e1 = int(self.edge_ptr[g0]), int(self.edge_ptr[g1])
+        ea = None if self.edge_attr is None else self.edge_attr[e0:e1]
         return GraphBatch(self.x[n0:n1], self.coo[e0:e1],
-                          self.node_ptr[g0:g1 + 1] - n0, self.edge_ptr[g0:g1 + 1] - e0)
+                          self.node_ptr[g0:g1 + 1] - n0, self.edge_ptr[g0:g1 + 1] - e0, ea)
 
     def algorithmic_bytes(self, out_dim: int) -> int:
         """SURVEY 8(d): 4*n*F + 8*e + 8 read and 4*out_dim written, per graph."""
@@ -60,23 +68,39 @@ class GraphBatch:
 
     @staticmethod
     def from_graphs(graphs: Sequence) -> "GraphBatch":
-        xs, coos, nptr, eptr = [], [], [0], [0]
-        for x, coo in graphs:
+        """``graphs``: ``(x, coo)`` items, or ``(x, coo, edge_attr)`` items (all of one kind)."""
+        xs, coos, eas, nptr, eptr = [], [], [], [0], [0]
+        kinds = set()
+        for item in graphs:
+            kinds.add(len(item))
+            x, coo = item[0], item[1]
             x = np.ascontiguousarray(x, dtype=np.float32)
             coo = np.ascontiguousarray(coo, dtype=np.int32).reshape(-1, 2)
+            if len(item) == 3:
+                ea = np.ascontiguousarray(item[2], dtype=np.float32)
+                if ea.ndim != 2 or ea.shape[0] != coo.shape[0]:
+                    raise ValueError(f"edge_attr must be [num_edges={coo.shape[0]}, edge_dim], got "
+                                     f"shape {ea.shape}")
+                if eas and ea.shape[1] != eas[0].shape[1]:
+                    raise ValueError(f"every graph's edge_attr needs the same edge_dim "
+                                     f"({eas[0].shape[1]}), got {ea.shape[1]}")
+                eas.append(ea)
             xs.append(x)
             coos.append(coo)
             nptr.append(nptr[-1] + x.shape[0])
             eptr.append(eptr[-1] + coo.shape[0])
+        if len(kinds) > 1:
+            raise ValueError("either every graph has edge features or none has")
         f = xs[0].shape[1] if xs else 0
         x = np.concatenate(xs, 0) if xs else np.zeros((0, f), np.float32)
         coo = np.concatenate(coos, 0) if coos else np.zeros((0, 2), np.int32)
-        return GraphBatch(x, coo, np.asarray(nptr, np.int64), np.asarray(eptr, np.int64))
+        ea = np.concatenate(eas, 0) if eas else None
+        return GraphBatch(x, coo, np.asarray(nptr, np.int64), np.asarray(eptr, np.int64), ea)
 
 
 def make_molecular_batch(n_graphs: int, mu_nodes: float, mu_edges: float, in_dim: int,
-                         seed: int, max_nodes: int = 600, shuffle_edges: bool = True
-                         ) -> GraphBatch:
+                         seed: int, max_nodes: int = 600, shuffle_edges: bool = True,
+                         edge_dim: int = 0) -> GraphBatch:
     """Vectorised molecular-shaped generator.
 
     n ~ clip(round(Normal(mu_N, 0.25 mu_N)), 2, max_nodes); a random tree whose node i attaches
@@ -84,6 +108,10 @@ def make_molecular_batch(n_graphs: int, mu_nodes: float, mu_edges: float, in_dim
     ring-closure edges so that undirected bonds ~= mu_E / 2; both directions are stored (PyG
     convention) so every node has in-degree >= 1; COO order is shuffled per graph; features
     U(-1, 1) float32 (as gen_test_data.py:90-93).
+
+    ``edge_dim > 0`` adds U(-1, 1) bond features, one row per bond shared by both stored
+    directions, from a generator of their own (seeded from ``seed``): ``x``, ``coo`` and the offsets
+    are the same as with ``edge_dim=0``.
     """
     rng = np.random.default_rng(seed)
     n = np.clip(np.rint(rng.normal(mu_nodes, 0.25 * mu_nodes, n_graphs)), 2, max_nodes)
@@ -130,7 +158,14 @@ def make_molecular_batch(n_graphs: int, mu_nodes: float, mu_edges: float, in_dim
     coo[:, 0] = src
     coo[:, 1] = dst
     x = (rng.random((total, in_dim), dtype=np.float32) * 2.0 - 1.0).astype(np.float32)
-    return GraphBatch(x, coo, node_ptr, edge_ptr)
+    edge_attr = None
+    if edge_dim > 0:
+        n_und = und_g.shape[0]
+        erng = np.random.default_rng([seed, 0x6564676500])   # independent of `rng`'s stream
+        bond = (erng.random((n_und, edge_dim), dtype=np.float32) * 2.0 - 1.0).astype(np.float32)
+        # stored edge k (before the shuffle) is bond k % n_und in either direction
+        edge_attr = bond[order % n_und]
+    return GraphBatch(x, coo, node_ptr, edge_ptr, edge_attr)
 
 
 def make_powerlaw_graph(num_nodes: int, avg_degree: int, in_dim: int, seed: int,

@@ -403,6 +403,9 @@ class LargeGraphModel:
     def __init__(self, model, n_total: int, rank: int, world: int, dist=None, backend=None,
                  transport: str = "auto", hub_l2_mb: Optional[int] = None):
         d = model.describe()
+        if d["conv_type"] not in (0, 1, 2, 3):
+            raise NotImplementedError("row-partitioned inference runs GCN, GIN, SAGE and PNA models "
+                                      "(GINE has no edge-feature halo exchange)")
         self.conv = ("gcn", "gin", "sage", "pna")[d["conv_type"]]
         self.model, self.desc = model, d
         self.part = RowPartition(n_total, world)

@@ -27,6 +27,7 @@ def _desc_struct(d: dict, max_nodes: int, max_edges: int) -> _lib.ModelDesc:
         s.pools[i] = int(p)
     s.max_nodes = int(max_nodes)
     s.max_edges = int(max_edges)
+    s.edge_dim = int(d.get("edge_dim", 0))
     return s
 
 
@@ -45,6 +46,8 @@ class Engine:
         self.desc = dict(desc)
         self.out_dim = int(desc["mlp_out"])
         self.in_dim = int(desc["in_dim"])
+        # GINE models take edge features and run through the *_edges entry points
+        self.edge_dim = int(desc.get("edge_dim", 0)) if int(desc["conv_type"]) == 4 else 0
         self._h = C.c_void_p()
         self._pinned = {}
         s = _desc_struct(desc, max_nodes, max_edges)
@@ -112,6 +115,14 @@ class Engine:
                 for i, k in enumerate(self.PROFILE_CLASSES)}
 
     # ------------------------------------------------------------------ running
+    def _host_edge_attr(self, edge_attr, n_edges: int):
+        if edge_attr is None:
+            raise _lib.GnnbError("this GINE model needs edge_attr")
+        ea = np.ascontiguousarray(edge_attr, np.float32)
+        if ea.shape != (n_edges, self.edge_dim):
+            raise _lib.GnnbError(f"edge_attr must be [{n_edges}, {self.edge_dim}], got {ea.shape}")
+        return ea
+
     def run(self, batch: GraphBatch, out: Optional[np.ndarray] = None) -> np.ndarray:
         """Host buffers in, host buffer out (H2D + kernels + D2H inside the call)."""
         x = np.ascontiguousarray(batch.x, np.float32)
@@ -122,6 +133,13 @@ class Engine:
         g = batch.n_graphs
         if out is None:
             out = np.empty((g, self.out_dim), np.float32)
+        if self.edge_dim:
+            ea = self._host_edge_attr(batch.edge_attr, coo.shape[0])
+            _lib.check(self.lib.gnnb_model_run_batch_edges(
+                self._h, C.c_void_p(x.ctypes.data), C.c_void_p(coo.ctypes.data),
+                C.c_void_p(ea.ctypes.data), C.c_void_p(nptr.ctypes.data),
+                C.c_void_p(eptr.ctypes.data), g, C.c_void_p(out.ctypes.data)))
+            return out
         _lib.check(self.lib.gnnb_model_run_batch(
             self._h, C.c_void_p(x.ctypes.data), C.c_void_p(coo.ctypes.data),
             C.c_void_p(nptr.ctypes.data), C.c_void_p(eptr.ctypes.data), g,
@@ -140,41 +158,65 @@ class Engine:
             self._pinned[a.ctypes.data] = a
 
     def pin_batch(self, batch: GraphBatch):
-        self.pin(batch.x, batch.coo, batch.node_ptr, batch.edge_ptr)
+        self.pin(batch.x, batch.coo, batch.node_ptr, batch.edge_ptr, batch.edge_attr)
 
     def unpin(self):
         for ptr in list(self._pinned):
             self.lib.gnnb_host_unregister(C.c_void_p(ptr))
         self._pinned.clear()
 
-    def run_graph(self, x: np.ndarray, coo: np.ndarray) -> np.ndarray:
-        """One graph, the exact data ``<name>_top`` receives."""
+    def run_graph(self, x: np.ndarray, coo: np.ndarray,
+                  edge_attr: Optional[np.ndarray] = None) -> np.ndarray:
+        """One graph, the exact data ``<name>_top`` receives (plus its edge features for GINE)."""
         x = np.ascontiguousarray(x, np.float32)
         coo = np.ascontiguousarray(coo, np.int32).reshape(-1, 2)
         out = np.empty(self.out_dim, np.float32)
+        if self.edge_dim:
+            ea = self._host_edge_attr(edge_attr, coo.shape[0])
+            nptr = np.array([0, x.shape[0]], np.int64)
+            eptr = np.array([0, coo.shape[0]], np.int64)
+            _lib.check(self.lib.gnnb_model_run_batch_edges(
+                self._h, C.c_void_p(x.ctypes.data), C.c_void_p(coo.ctypes.data),
+                C.c_void_p(ea.ctypes.data), C.c_void_p(nptr.ctypes.data),
+                C.c_void_p(eptr.ctypes.data), 1, C.c_void_p(out.ctypes.data)))
+            return out
         _lib.check(self.lib.gnnb_model_run_graph(
             self._h, C.c_void_p(x.ctypes.data), C.c_void_p(coo.ctypes.data), x.shape[0],
             coo.shape[0], C.c_void_p(out.ctypes.data)))
         return out
 
     def run_device(self, x, coo, node_ptr, edge_ptr, out, n_graphs: int, total_nodes: int,
-                   total_edges: int, stream: Optional[int] = None, sync: bool = False):
-        """torch CUDA tensors (or raw device pointers as ints); enqueues without synchronising."""
+                   total_edges: int, stream: Optional[int] = None, sync: bool = False,
+                   edge_attr=None):
+        """torch CUDA tensors (or raw device pointers as ints); enqueues without synchronising.
+        GINE models take ``edge_attr`` [total_edges][edge_dim] on the device as well."""
         def p(a):
+            if a is None:
+                return None
             return C.c_void_p(a.data_ptr() if hasattr(a, "data_ptr") else int(a))
 
-        _lib.check(self.lib.gnnb_model_run_batch_async(
-            self._h, p(x), p(coo), p(node_ptr), p(edge_ptr), n_graphs, total_nodes, total_edges,
-            p(out), C.c_void_p(stream) if stream else None))
+        st = C.c_void_p(stream) if stream else None
+        if self.edge_dim:
+            _lib.check(self.lib.gnnb_model_run_batch_edges_async(
+                self._h, p(x), p(coo), p(edge_attr), p(node_ptr), p(edge_ptr), n_graphs,
+                total_nodes, total_edges, p(out), st))
+        else:
+            _lib.check(self.lib.gnnb_model_run_batch_async(
+                self._h, p(x), p(coo), p(node_ptr), p(edge_ptr), n_graphs, total_nodes,
+                total_edges, p(out), st))
         if sync:
             self.synchronize()
         return out
 
-    def run_device_sync(self, x, coo, node_ptr, edge_ptr, out, n_graphs: int):
+    def run_device_sync(self, x, coo, node_ptr, edge_ptr, out, n_graphs: int, edge_attr=None):
         """Device tensors through the synchronous entry point (path chosen from real sizes)."""
         def p(a):
-            return C.c_void_p(a.data_ptr())
+            return None if a is None else C.c_void_p(a.data_ptr())
 
+        if self.edge_dim:
+            _lib.check(self.lib.gnnb_model_run_batch_edges(
+                self._h, p(x), p(coo), p(edge_attr), p(node_ptr), p(edge_ptr), n_graphs, p(out)))
+            return out
         _lib.check(self.lib.gnnb_model_run_batch(self._h, p(x), p(coo), p(node_ptr), p(edge_ptr),
                                                  n_graphs, p(out)))
         return out

@@ -79,6 +79,21 @@ class _GINConv(nn.Module):
         return self.nn(agg + (1.0 + self.eps) * x)
 
 
+class _GINEConv(nn.Module):
+    """PyG GINEConv with ``edge_dim``: ``lin`` projects the edge features to ``in_channels``."""
+
+    def __init__(self, mlp: nn.Module, eps: float = 0.0, edge_dim: int = 1, in_channels: int = 1):
+        super().__init__()
+        self.nn = mlp
+        self.register_buffer("eps", torch.tensor([float(eps)]))
+        self.lin = nn.Linear(edge_dim, in_channels)
+
+    def forward(self, x: Tensor, edge_index: Tensor, edge_attr: Tensor) -> Tensor:
+        msg = (x[edge_index[0]] + self.lin(edge_attr)).relu()
+        agg = _scatter_sum(msg, edge_index[1], x.shape[0])
+        return self.nn(agg + (1.0 + self.eps) * x)
+
+
 class _SAGEConv(nn.Module):
     def __init__(self, in_channels: int, out_channels: int):
         super().__init__()
@@ -180,6 +195,31 @@ class GINConv_GNNB(nn.Module):
 
     def forward(self, x: Tensor, edge_index: Tensor) -> Tensor:
         return self.conv(x, edge_index)
+
+
+class GINEConv_GNNB(nn.Module):
+    """GIN with edge features (PyG ``GINEConv`` with ``edge_dim``; the reference lib's gine_conv,
+    lib:1555-1742): y_v = MLP((1 + eps) x_v + sum_{u->v} ReLU(x_u + e_uv W_e^T + b_e)).  Built like
+    ``GINConv_GNNB``; each layer has its own edge linear ``conv.lin`` [in_channels][edge_dim] over
+    the same raw edge features."""
+
+    def __init__(self, in_channels: int, out_channels: int, edge_dim: int,
+                 hidden_dim: Optional[int] = None, eps: float = 0.0, p_in: int = 1, p_out: int = 1):
+        super().__init__()
+        if not isinstance(edge_dim, int) or isinstance(edge_dim, bool) or edge_dim < 1:
+            raise ValueError(f"edge_dim must be a positive int, got {edge_dim!r}")
+        self.in_channels = in_channels
+        self.out_channels = out_channels
+        self.edge_dim = edge_dim
+        self.hidden_dim = hidden_dim
+        self.eps = eps
+        self.p_in = p_in
+        self.p_out = p_out
+        self.mlp = GIN_MLP(in_channels, out_channels, None)
+        self.conv = _GINEConv(self.mlp, eps=eps, edge_dim=edge_dim, in_channels=in_channels)
+
+    def forward(self, x: Tensor, edge_index: Tensor, edge_attr: Tensor) -> Tensor:
+        return self.conv(x, edge_index, edge_attr)
 
 
 class PNAConv_GNNB(nn.Module):
@@ -323,9 +363,10 @@ class MLP(nn.Module):
         return len(self.linear_layers)
 
 
-SUPPORTED_GNN_CONVS = [GCNConv_GNNB, GINConv_GNNB, PNAConv_GNNB, SAGEConv_GNNB]
+SUPPORTED_GNN_CONVS = [GCNConv_GNNB, GINConv_GNNB, PNAConv_GNNB, SAGEConv_GNNB, GINEConv_GNNB]
 
-CONV_TYPE_IDS = {"GCNConv_GNNB": 0, "GINConv_GNNB": 1, "SAGEConv_GNNB": 2, "PNAConv_GNNB": 3}
+CONV_TYPE_IDS = {"GCNConv_GNNB": 0, "GINConv_GNNB": 1, "SAGEConv_GNNB": 2, "PNAConv_GNNB": 3,
+                 "GINEConv_GNNB": 4}
 ACTIVATION_IDS = {None: 0, "ReLU": 1, "GELU": 2, "Sigmoid": 3, "Tanh": 4}
 POOL_IDS = {"add": 0, "mean": 1, "max": 2}
 
@@ -349,6 +390,14 @@ class GNNModel(nn.Module):
         conv_cls = getattr(gnn_conv, "func", gnn_conv)  # allow functools.partial(delta=..)
         if conv_cls not in SUPPORTED_GNN_CONVS:
             raise ValueError(f"gnn_conv must be one of {SUPPORTED_GNN_CONVS}")
+        self.uses_edge_features = conv_cls is GINEConv_GNNB
+        conv_kwargs = {}
+        if self.uses_edge_features:
+            e = graph_input_edge_dim
+            if not isinstance(e, int) or isinstance(e, bool) or e < 1:
+                raise ValueError("GINEConv_GNNB needs graph_input_edge_dim to be a positive int, "
+                                 f"got {e!r}")
+            conv_kwargs["edge_dim"] = e
         self.gnn_activation = gnn_activation
         if self.gnn_activation not in SUPPORTED_ACTIVATIONS:
             raise ValueError(f"gnn_activation must be one of {SUPPORTED_ACTIVATIONS}")
@@ -379,7 +428,8 @@ class GNNModel(nn.Module):
             out_dim = self.gnn_output_dim if i == L - 1 else self.gnn_hidden_dim
             p_in = self.gnn_p_in if i == 0 else self.gnn_p_hidden
             p_out = self.gnn_p_out if i == L - 1 else self.gnn_p_hidden
-            self.gnn_convs.append(self.gnn_conv(in_dim, out_dim, p_in=p_in, p_out=p_out))
+            self.gnn_convs.append(self.gnn_conv(in_dim, out_dim, p_in=p_in, p_out=p_out,
+                                                **conv_kwargs))
             self.gnn_activations.append(self.gnn_activation())
         if self.gnn_skip_connection:
             for i in range(1, L - 1):
@@ -387,11 +437,17 @@ class GNNModel(nn.Module):
                 if c.in_channels != c.out_channels:
                     raise ValueError("skip connections need in_channels == out_channels")
 
-    def forward(self, x: Tensor, edge_index: Tensor, batch: Optional[Tensor] = None) -> Tensor:
+    def forward(self, x: Tensor, edge_index: Tensor, batch: Optional[Tensor] = None,
+                edge_attr: Optional[Tensor] = None) -> Tensor:
+        if self.uses_edge_features and self.gnn_num_layers > 0 and edge_attr is None:
+            raise ValueError("a GINEConv_GNNB model needs edge_attr")
         x_gnn = x
         for i, (conv, act) in enumerate(zip(self.gnn_convs, self.gnn_activations)):
             x_in = x_gnn
-            x_gnn = conv(x_gnn, edge_index)
+            if self.uses_edge_features:
+                x_gnn = conv(x_gnn, edge_index, edge_attr)
+            else:
+                x_gnn = conv(x_gnn, edge_index)
             if self.gnn_skip_connection and i != 0 and i != self.gnn_num_layers - 1:
                 x_gnn = x_gnn + x_in
             x_gnn = act(x_gnn)
@@ -461,7 +517,9 @@ class GNNModel(nn.Module):
         """Plain description consumed by the C-ABI (gnnb_model_desc, include/gnnb_b200.h)."""
         conv0 = self.gnn_convs[0] if self.gnn_num_layers > 0 else None
         conv_name = conv0.__class__.__name__ if conv0 is not None else "GCNConv_GNNB"
-        return dict(
+        if self.uses_edge_features:
+            conv_name = "GINEConv_GNNB"
+        d = dict(
             conv_type=CONV_TYPE_IDS[conv_name],
             num_layers=self.gnn_num_layers,
             in_dim=self.graph_input_feature_dim,
@@ -479,6 +537,9 @@ class GNNModel(nn.Module):
             out_act=ACTIVATION_IDS[self.output_activation.__name__
                                    if self.output_activation is not None else None],
         )
+        if self.uses_edge_features:
+            d["edge_dim"] = int(self.graph_input_edge_dim)
+        return d
 
 
 def build_model(workload, pna_delta: float = 1.0, seed: int = 0) -> GNNModel:

@@ -41,7 +41,11 @@ enum {
     GNNB_ACT_GELU_ERF = 8, GNNB_ACT_SILU = 9, GNNB_ACT_SOFTSIGN = 10, GNNB_ACT_SIN = 11,
     GNNB_ACT_COS = 12
 };
-enum { GNNB_CONV_GCN = 0, GNNB_CONV_GIN = 1, GNNB_CONV_SAGE = 2, GNNB_CONV_PNA = 3 };
+/* GINE (GIN with an edge linear, PyG GINEConv with edge_dim; lib:1555-1742) runs on the layerwise
+ * path only and takes its edge features through the gnnb_model_run_batch_edges* entry points */
+enum { GNNB_CONV_GCN = 0, GNNB_CONV_GIN = 1, GNNB_CONV_SAGE = 2, GNNB_CONV_PNA = 3, GNNB_CONV_GINE = 4 };
+/* edge feature widths a GINE model handle accepts */
+#define GNNB_GINE_MAX_EDGE_DIM 64
 enum { GNNB_POOL_ADD = 0, GNNB_POOL_MEAN = 1, GNNB_POOL_MAX = 2 };
 
 /* execution path of gnnb_model_run_batch */
@@ -78,6 +82,9 @@ typedef struct gnnb_model_desc {
     int32_t out_act;        /* output_activation, 0 = None */
     int32_t max_nodes;      /* capacity hints (Project.max_nodes/max_edges, code_gen.py:71-72); */
     int32_t max_edges;      /* 0 = unbounded.  A graph larger than a non-zero hint is an error. */
+    int32_t edge_dim;       /* GINE only: edge feature width, 1..GNNB_GINE_MAX_EDGE_DIM.  Last field,
+                               read only when conv_type == GNNB_CONV_GINE, so a caller built
+                               against a header without it keeps working for the other convs. */
 } gnnb_model_desc;
 
 typedef struct gnnb_model gnnb_model_t;
@@ -129,6 +136,18 @@ int gnnb_model_run_batch(gnnb_model_t *m, const float *x, const int32_t *edge_li
 int gnnb_model_run_batch_async(gnnb_model_t *m, const float *x, const int32_t *edge_list,
                                const int64_t *node_ptr, const int64_t *edge_ptr, int n_graphs,
                                int64_t total_nodes, int64_t total_edges, float *out, void *stream);
+/* GINE models: the same contracts as gnnb_model_run_batch / gnnb_model_run_batch_async, plus
+ * edge_attr float [edge_ptr[G]][edge_dim] in the memory space of the other buffers, row i the
+ * features of COO edge i (one row per stored direction).  A GINE handle must be run through these
+ * two; a handle of another conv type is rejected by them (GNNB_ERR_INVALID), and so is a null
+ * edge_attr with edges present. */
+int gnnb_model_run_batch_edges(gnnb_model_t *m, const float *x, const int32_t *edge_list,
+                               const float *edge_attr, const int64_t *node_ptr,
+                               const int64_t *edge_ptr, int n_graphs, float *out);
+int gnnb_model_run_batch_edges_async(gnnb_model_t *m, const float *x, const int32_t *edge_list,
+                                     const float *edge_attr, const int64_t *node_ptr,
+                                     const int64_t *edge_ptr, int n_graphs, int64_t total_nodes,
+                                     int64_t total_edges, float *out, void *stream);
 /* node embeddings after the last conv (node_emb_out, cpp:22,349-354) of the most recent
  * LAYERWISE run: copies [total_nodes][out_dim] floats to `dst` (host or device) */
 int gnnb_model_get_node_embeddings(gnnb_model_t *m, float *dst, int64_t total_nodes);
