@@ -26,7 +26,7 @@ class ModelDesc(C.Structure):
         ("num_pools", C.c_int32), ("pools", C.c_int32 * 4), ("mlp_num_linear", C.c_int32),
         ("mlp_hidden", C.c_int32), ("mlp_out", C.c_int32), ("mlp_act", C.c_int32),
         ("out_act", C.c_int32), ("max_nodes", C.c_int32), ("max_edges", C.c_int32),
-        ("edge_dim", C.c_int32),
+        ("edge_dim", C.c_int32), ("gat_heads", C.c_int32), ("gat_negative_slope", C.c_float),
     ]
 
 

@@ -106,7 +106,7 @@ class Project:
     # ------------------------------------------------------------------ generation
     def gen_hw_model(self):
         """Bind the model to the GPU (the analogue of rendering model.h/model.cpp)."""
-        self._no_edge_features("gen_hw_model")
+        self._check_top_renderable("gen_hw_model")
         if self.float_or_fixed == "fixed":
             raise NotImplementedError(
                 "ap_fixed mode needs Xilinx's ap_fixed.h/hls_math.h to pin results against; "
@@ -131,7 +131,7 @@ class Project:
         ``layer_parameter_names_flat`` order) forwarding to the C-ABI model handle -- what a
         maintainer renders instead of model.cpp.jinja:686-766.  The reference's own ``model.h``
         and ``model_tb.cpp`` compile and link against it unchanged (float build)."""
-        self._no_edge_features("render_top")
+        self._check_top_renderable("render_top")
         d = self.model.describe()
         names = self.model.layer_parameter_names_flat
         shapes = self.model.layer_parameter_shapes_flat
@@ -206,11 +206,16 @@ extern "C" void {self.name}_top(
 }}
 """
 
-    def _no_edge_features(self, what):
+    def _check_top_renderable(self, what):
         if getattr(self.model, "uses_edge_features", False):
             raise NotImplementedError(
                 f"{what}: the reference's <name>_top signature has no edge-feature argument, so a "
                 "GINEConv_GNNB model cannot be rendered; run it through Engine instead")
+        if self.model is not None and self.model.describe()["conv_type"] == 5:
+            raise NotImplementedError(
+                f"{what}: the reference has no GAT kernel and its <name>_top no attention-head "
+                "arguments, so a GATConv_GNNB model cannot be rendered; run it through Engine "
+                "instead")
 
     def build_top(self, testbench: Optional[Path] = None) -> Path:
         """Compile the generated ``model.cpp`` into ``lib<name>.so`` (exports ``<name>_top``).

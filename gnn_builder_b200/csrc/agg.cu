@@ -923,4 +923,285 @@ int launch_permute_edge_rows(const float *src, int dim, const int32_t *idx, int 
     return GNNB_OK;
 }
 
+// ------------------------------------------------------------------------------------- GAT
+//
+// PyG GATConv (concat heads, self loops replaced by one per node, inference).  The layer's one GEMM
+// wrote [h (H*C) | a_src (H) | a_dst (H)] per row (the logit vectors are folded into the weights at
+// finalize), so this is a pure gather.  A (sub-)warp per destination row with the LPR/VEC scheme of
+// agg_rows_kernel; each lane owns VEC columns of one head (VEC = 4 needs C % 4 == 0).  Every lane
+// runs one online softmax over the row in neighbor-table order: it starts from the self term
+// (logit e_vv, weight 1, h_v), skips neighbor entries equal to v (the input's self loops are
+// replaced by that one term; duplicate edges count once per entry), and for each other entry keeps
+// the running max m, the sum s of exp(e - m) and the accumulator of exp(e - m) h_u, rescaling both
+// when the max grows.  Every exponent is <= 0, so logits of any size neither overflow nor give NaN,
+// and s >= 1.  The epilogue writes act(acc / s + bias (+ skip)): the bias, skip and activation the
+// other convs apply in their GEMM epilogue.
+//
+// Heavy rows (the same bucketing as launch_agg): each kHeavyChunk-neighbor chunk is one warp's work
+// and stores its per-head (m, s) and its accumulator (relative to its own m) in the partial scratch.
+// One CTA per row then merges the chunks -- 8 warps over contiguous chunk ranges, then the self term
+// and the 8 range results in warp order -- a fixed order, so the result does not depend on
+// scheduling.  Algorithmic bytes per layer: E (4 + 4H + 4HC) + N (8 + 4H + 4HC [+ 4HC skip]).
+namespace {
+
+__device__ __forceinline__ float leaky_relu(float x, float slope) { return x > 0.0f ? x : x * slope; }
+
+template <int VEC>
+struct OnlineSoftmax {
+    float m, s;
+    Vec<VEC> acc;
+    __device__ __forceinline__ void reset()
+    {
+        m = -INFINITY;
+        s = 0.0f;
+#pragma unroll
+        for (int i = 0; i < VEC; i++) acc.v[i] = 0.0f;
+    }
+    // adds a part with max m2, sum s2 and accumulator acc2 (one edge: e, 1, h_u); an empty part
+    // (m2 = -inf, from a chunk of self loops only) changes nothing
+    __device__ __forceinline__ void merge(float m2, float s2, const Vec<VEC> &acc2)
+    {
+        if (m2 == -INFINITY) return;
+        const float mn = fmaxf(m, m2);
+        const float r = expf(m - mn), p = expf(m2 - mn);
+        s = fmaf(s, r, s2 * p);
+#pragma unroll
+        for (int i = 0; i < VEC; i++) acc.v[i] = fmaf(acc.v[i], r, acc2.v[i] * p);
+        m = mn;
+    }
+};
+
+// the self term of row v for the lane's columns [c, c + VEC) of head hd; returns a_dst[v][hd]
+template <int VEC>
+__device__ __forceinline__ float gat_self(const GatAggArgs &a, int v, int c, int hd, OnlineSoftmax<VEC> &st)
+{
+    const int HC = a.H * a.C;
+    const float *row = a.hg + (size_t)v * a.ldg;
+    const float adst = __ldg(row + HC + a.H + hd);
+    st.m = leaky_relu(__ldg(row + HC + hd) + adst, a.slope);
+    st.s = 1.0f;
+    st.acc.load(row + c);
+    return adst;
+}
+
+// neighbor entries [k0, k1) of row v (entries equal to v skipped), four gathers in flight
+template <int VEC>
+__device__ __forceinline__ void gat_gather(const GatAggArgs &a, int v, int off, int k0, int k1, int c,
+                                           int hd, float adst, OnlineSoftmax<VEC> &st)
+{
+    const int HC = a.H * a.C;
+    int k = k0;
+    for (; k + 4 <= k1; k += 4) {
+        int u[4];
+        float as[4];
+        Vec<VEC> x[4];
+#pragma unroll
+        for (int j = 0; j < 4; j++) u[j] = __ldg(a.nbr + off + k + j);
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            const float *row = a.hg + (size_t)u[j] * a.ldg;
+            as[j] = __ldg(row + HC + hd);
+            x[j].load(row + c);
+        }
+#pragma unroll
+        for (int j = 0; j < 4; j++)
+            if (u[j] != v) st.merge(leaky_relu(as[j] + adst, a.slope), 1.0f, x[j]);
+    }
+    for (; k < k1; k++) {
+        const int u = __ldg(a.nbr + off + k);
+        if (u == v) continue;
+        const float *row = a.hg + (size_t)u * a.ldg;
+        Vec<VEC> x;
+        x.load(row + c);
+        st.merge(leaky_relu(__ldg(row + HC + hd) + adst, a.slope), 1.0f, x);
+    }
+}
+
+template <int VEC>
+__device__ __forceinline__ void gat_finish(const GatAggArgs &a, int v, int c, const OnlineSoftmax<VEC> &st)
+{
+    Vec<VEC> b, sk, y;
+    b.load(a.bias + c);
+    if (a.skip != nullptr) sk.load(a.skip + (size_t)v * a.ldskip + c);
+#pragma unroll
+    for (int i = 0; i < VEC; i++) {
+        float t = st.acc.v[i] / st.s + b.v[i];
+        if (a.skip != nullptr) t += sk.v[i];
+        y.v[i] = act_apply_compact(a.act, t);
+    }
+    y.store(a.out + (size_t)v * a.ldo + c);
+}
+
+template <int VEC, int LPR>
+__global__ void __launch_bounds__(256) gat_agg_kernel(const GatAggArgs a)
+{
+    constexpr int ROWS_PER_WARP = 32 / LPR;
+    const int lane = threadIdx.x & 31;
+    const int lg = lane % LPR, sub = lane / LPR;
+    const int warps_per_block = blockDim.x >> 5;
+    const int64_t warp_global = (int64_t)blockIdx.x * warps_per_block + (threadIdx.x >> 5);
+    const int64_t warp_stride = (int64_t)gridDim.x * warps_per_block;
+    const int HC = a.H * a.C;
+    for (int64_t row0 = warp_global * ROWS_PER_WARP; row0 < a.n; row0 += warp_stride * ROWS_PER_WARP) {
+        const int v = (int)row0 + sub;
+        if (v >= a.n) continue;
+        const int deg = __ldg(a.in_deg + v);
+        if (a.n_heavy > 0 && deg > a.heavy_threshold) continue;  // the heavy-row kernels do these
+        const int off = __ldg(a.offsets + v);
+        for (int c = lg * VEC; c < HC; c += LPR * VEC) {
+            const int hd = c / a.C;
+            OnlineSoftmax<VEC> st;
+            const float adst = gat_self(a, v, c, hd, st);
+            gat_gather(a, v, off, 0, deg, c, hd, adst, st);
+            gat_finish(a, v, c, st);
+        }
+    }
+}
+
+template <int VEC>
+__global__ void __launch_bounds__(256) gat_heavy_chunk_kernel(const GatAggArgs a)
+{
+    const int lane = threadIdx.x & 31;
+    const int warps_per_block = blockDim.x >> 5;
+    const int warp_global = blockIdx.x * warps_per_block + (threadIdx.x >> 5);
+    const int warp_stride = gridDim.x * warps_per_block;
+    const int HC = a.H * a.C;
+    for (int chunk = warp_global; chunk < a.heavy_chunks; chunk += warp_stride) {
+        const int h = __ldg(a.heavy_chunk_row + chunk);
+        const int v = __ldg(a.heavy_rows + h);
+        const int j = chunk - __ldg(a.heavy_chunk_base + h);
+        const int deg = __ldg(a.in_deg + v);
+        const int off = __ldg(a.offsets + v);
+        const int k0 = j * kHeavyChunk, k1 = min(deg, k0 + kHeavyChunk);
+        const float *rowv = a.hg + (size_t)v * a.ldg;
+        float *dst = a.heavy_partial + (size_t)chunk * a.ldp;
+        for (int c = lane * VEC; c < HC; c += 32 * VEC) {
+            const int hd = c / a.C;
+            OnlineSoftmax<VEC> st;
+            st.reset();
+            gat_gather(a, v, off, k0, k1, c, hd, __ldg(rowv + HC + a.H + hd), st);
+            st.acc.store(dst + c);
+            if (c % a.C == 0) {   // one lane per head
+                dst[HC + hd] = st.m;
+                dst[HC + a.H + hd] = st.s;
+            }
+        }
+    }
+}
+
+template <int VEC>
+__global__ void __launch_bounds__(256) gat_heavy_combine_kernel(const GatAggArgs a)
+{
+    extern __shared__ float4 gat_smem4[];
+    float *const ranges = reinterpret_cast<float *>(gat_smem4);   // [8][ldp], laid out as the partials
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int HC = a.H * a.C;
+    for (int h = blockIdx.x; h < a.n_heavy; h += gridDim.x) {
+        const int v = __ldg(a.heavy_rows + h);
+        const int deg = __ldg(a.in_deg + v);
+        const int nch = (deg + kHeavyChunk - 1) / kHeavyChunk;
+        const float *src = a.heavy_partial + (size_t)__ldg(a.heavy_chunk_base + h) * a.ldp;
+        const int per = (nch + 7) / 8;
+        const int j0 = min(nch, warp * per), j1 = min(nch, j0 + per);
+        float *mine = ranges + warp * a.ldp;
+        for (int c = lane * VEC; c < HC; c += 32 * VEC) {
+            const int hd = c / a.C;
+            OnlineSoftmax<VEC> st;
+            st.reset();
+            for (int j = j0; j < j1; j++) {
+                const float *p = src + (size_t)j * a.ldp;
+                Vec<VEC> t;
+                t.load_rw(p + c);
+                st.merge(p[HC + hd], p[HC + a.H + hd], t);
+            }
+            st.acc.store(mine + c);
+            if (c % a.C == 0) {
+                mine[HC + hd] = st.m;
+                mine[HC + a.H + hd] = st.s;
+            }
+        }
+        __syncthreads();
+        if (warp == 0) {
+            for (int c = lane * VEC; c < HC; c += 32 * VEC) {
+                const int hd = c / a.C;
+                OnlineSoftmax<VEC> st;
+                gat_self(a, v, c, hd, st);
+#pragma unroll 1
+                for (int w = 0; w < 8; w++) {
+                    const float *r = ranges + w * a.ldp;
+                    Vec<VEC> t;
+                    t.load_rw(r + c);
+                    st.merge(r[HC + hd], r[HC + a.H + hd], t);
+                }
+                gat_finish(a, v, c, st);
+            }
+        }
+        __syncthreads();
+    }
+}
+
+template <int VEC>
+void launch_gat_lpr(const GatAggArgs &a, int lpr, int grid, cudaStream_t s)
+{
+    switch (lpr) {
+    case 1: gat_agg_kernel<VEC, 1><<<grid, 256, 0, s>>>(a); break;
+    case 2: gat_agg_kernel<VEC, 2><<<grid, 256, 0, s>>>(a); break;
+    case 4: gat_agg_kernel<VEC, 4><<<grid, 256, 0, s>>>(a); break;
+    case 8: gat_agg_kernel<VEC, 8><<<grid, 256, 0, s>>>(a); break;
+    case 16: gat_agg_kernel<VEC, 16><<<grid, 256, 0, s>>>(a); break;
+    default: gat_agg_kernel<VEC, 32><<<grid, 256, 0, s>>>(a); break;
+    }
+}
+
+template <int VEC>
+int launch_gat_heavy(const GatAggArgs &a, cudaStream_t s)
+{
+    const int cap = kNumSMs * 8;   // 8 resident CTAs per SM, grid-stride beyond
+    const int g1 = min((a.heavy_chunks + 7) / 8, cap), g2 = min(a.n_heavy, cap);
+    gat_heavy_chunk_kernel<VEC><<<g1, 256, 0, s>>>(a);
+    const size_t smem = sizeof(float) * 8 * (size_t)a.ldp;
+    if (smem > 48 * 1024)
+        GNNB_CUDA(cudaFuncSetAttribute(gat_heavy_combine_kernel<VEC>,
+                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    gat_heavy_combine_kernel<VEC><<<g2, 256, smem, s>>>(a);
+    return GNNB_OK;
+}
+
+}  // namespace
+
+int launch_gat_agg(const GatAggArgs &a, cudaStream_t s, int *launches)
+{
+    if (a.n <= 0) return GNNB_OK;
+    const int HC = a.H * a.C;
+    GNNB_REQUIRE(a.H >= 1 && a.C >= 1 && a.ldg >= HC + 2 * a.H && a.ldo >= HC && a.bias != nullptr &&
+                     (a.skip == nullptr || a.ldskip >= HC),
+                 "gat aggregation: bad arguments");
+    const bool v4 = (a.C % 4 == 0) && (a.ldg % 4 == 0) && (a.ldo % 4 == 0) && aligned16(a.hg) &&
+                    aligned16(a.out) && aligned16(a.bias) &&
+                    (a.skip == nullptr || ((a.ldskip % 4 == 0) && aligned16(a.skip)));
+    const int vec = v4 ? 4 : 1;
+    int lpr = 1;
+    while (lpr < 32 && lpr * vec < HC) lpr *= 2;
+    const int rows_per_block = 8 * (32 / lpr);
+    int64_t grid64 = ceil_div64(a.n, rows_per_block);
+    const int64_t cap = (int64_t)kNumSMs * 8 * 4;
+    const int grid = (int)(grid64 < cap ? grid64 : cap);
+    if (vec == 4)
+        launch_gat_lpr<4>(a, lpr, grid, s);
+    else
+        launch_gat_lpr<1>(a, lpr, grid, s);
+    GNNB_CUDA(cudaGetLastError());
+    if (launches) ++*launches;
+    if (a.n_heavy > 0) {
+        GNNB_REQUIRE(a.heavy_rows != nullptr && a.heavy_partial != nullptr && a.heavy_chunks > 0 &&
+                         a.heavy_chunk_base != nullptr && a.heavy_chunk_row != nullptr &&
+                         a.ldp >= HC + 2 * a.H && a.ldp % 4 == 0,
+                     "gat heavy rows: row list / partial buffer missing");
+        GNNB_TRY(vec == 4 ? launch_gat_heavy<4>(a, s) : launch_gat_heavy<1>(a, s));
+        GNNB_CUDA(cudaGetLastError());
+        if (launches) *launches += 2;
+    }
+    return GNNB_OK;
+}
+
 }  // namespace gnnb

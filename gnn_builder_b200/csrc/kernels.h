@@ -171,6 +171,41 @@ int launch_gine_agg_proj(const GineProjAggArgs &a, cudaStream_t s, int *launches
 int launch_permute_edge_rows(const float *src, int dim, const int32_t *idx, int e, float *dst,
                              int ldd, cudaStream_t s, int *launches);
 
+// GAT attention aggregation (PyG GATConv, concat heads, inference).  hg is the output of the layer's
+// one GEMM: per row h (H*C columns, head-major), then a_src [H] and a_dst [H].  Per destination v and
+// head: e_uv = LeakyReLU(a_src[u] + a_dst[v]) over the in-neighbours u != v plus one self term,
+// y_v = act(sum softmax_v(e) h_u + bias (+ skip_v)), written to out.  One gather pass with an online
+// softmax (running max, rescaled sum and accumulator).  Rows longer than heavy_threshold (when a
+// heavy list is given) are cut into kHeavyChunk-neighbour chunks whose (max, sum, accumulator)
+// partials are merged per row in a fixed order.
+struct GatAggArgs {
+    const float *hg;       // [n][ldg]
+    int ldg, H, C;
+    float slope;
+    const float *bias;     // [H*C]
+    const float *skip;     // [n][ldskip] or null
+    int ldskip;
+    int act;
+    float *out;            // [n][ldo]
+    int ldo;
+    const int32_t *offsets, *nbr, *in_deg;
+    int n;
+    const int32_t *heavy_rows;
+    int n_heavy;
+    int heavy_threshold;
+    float *heavy_partial;  // [heavy_chunks][ldp]: accumulator (H*C), then max [H], sum [H]
+    int ldp;               // round_up(H*C + 2H, 4)
+    const int32_t *heavy_chunk_base, *heavy_chunk_row;
+    int heavy_chunks;
+    void set_heavy(const HeavyList &hl, float *partial)
+    {
+        heavy_rows = hl.rows.as<int32_t>(); n_heavy = hl.n_heavy;
+        heavy_chunk_base = hl.chunk_base.as<int32_t>(); heavy_chunk_row = hl.chunk_row.as<int32_t>();
+        heavy_chunks = hl.n_chunks; heavy_partial = partial;
+    }
+};
+int launch_gat_agg(const GatAggArgs &a, cudaStream_t s, int *launches);
+
 struct PnaAggArgs {
     const float *ab;       // [n][2F]: cols [0,F) = x.W_nbr^T, cols [F,2F) = x.W_self^T + b_pre
     int F;

@@ -7,6 +7,7 @@
 #include "model.h"
 
 #include <algorithm>
+#include <cmath>
 #include <cstddef>
 #include <cstring>
 #include <mutex>
@@ -115,6 +116,12 @@ void enumerate_params(gnnb_model *m)
             add_param(m, base + "_conv_lin_weight", {fo, fo});
             add_param(m, base + "_conv_lin_bias", {fo});
             break;
+        case GNNB_CONV_GAT:   // PyG GATConv: its own parameters, then lin's
+            add_param(m, base + "_conv_att_src", {1, d.gat_heads, fo / d.gat_heads});
+            add_param(m, base + "_conv_att_dst", {1, d.gat_heads, fo / d.gat_heads});
+            add_param(m, base + "_conv_bias", {fo});
+            add_param(m, base + "_conv_lin_weight", {fo, fi});
+            break;
         }
     }
 }
@@ -217,9 +224,8 @@ extern "C" int gnnb_model_create(const gnnb_model_desc *desc, int device, gnnb_m
     // never has bytes read past its end)
     gnnb_model_desc d{};
     std::memcpy(&d, desc, offsetof(gnnb_model_desc, edge_dim));
-    GNNB_REQUIRE(d.conv_type >= GNNB_CONV_GCN && d.conv_type <= GNNB_CONV_GINE,
-                 "conv_type must be GCN, GIN, SAGE, PNA or GINE (models.py:453-459; GAT has no "
-                 "kernel in the reference either)");
+    GNNB_REQUIRE(d.conv_type >= GNNB_CONV_GCN && d.conv_type <= GNNB_CONV_GAT,
+                 "conv_type must be GCN, GIN, SAGE, PNA, GINE or GAT");
     if (d.conv_type == GNNB_CONV_GINE) {
         d.edge_dim = desc->edge_dim;
         GNNB_REQUIRE(d.edge_dim >= 1 && d.edge_dim <= kGineMaxEdgeDim,
@@ -227,6 +233,20 @@ extern "C" int gnnb_model_create(const gnnb_model_desc *desc, int device, gnnb_m
     }
     GNNB_REQUIRE(d.num_layers >= 0 && d.num_layers <= 64, "num_layers out of range");
     GNNB_REQUIRE(d.in_dim > 0 && d.hidden_dim > 0 && d.out_dim > 0, "dimensions must be positive");
+    if (d.conv_type == GNNB_CONV_GAT) {   // the GAT fields follow edge_dim; only GAT callers set them
+        d.gat_heads = desc->gat_heads;
+        d.gat_negative_slope = desc->gat_negative_slope;
+        GNNB_REQUIRE(d.gat_heads >= 1 && d.gat_heads <= GNNB_GAT_MAX_HEADS,
+                     "GAT gat_heads must be 1.." + std::to_string(GNNB_GAT_MAX_HEADS));
+        GNNB_REQUIRE(std::isfinite(d.gat_negative_slope), "GAT gat_negative_slope must be finite");
+        for (int k = 0; k < d.num_layers; k++) {
+            const int fo = k == d.num_layers - 1 ? d.out_dim : d.hidden_dim;
+            GNNB_REQUIRE(fo % d.gat_heads == 0,
+                         "GAT: every layer's output width (hidden_dim, out_dim) must be a multiple of "
+                         "gat_heads, got width " + std::to_string(fo) + " with " +
+                             std::to_string(d.gat_heads) + " heads");
+        }
+    }
     GNNB_REQUIRE(d.num_layers > 0 || d.in_dim == d.out_dim,
                  "gnn_num_layers=0 needs gnn_output_dim == graph_input_feature_dim (models.py:512)");
     GNNB_REQUIRE(d.num_pools >= 1 && d.num_pools <= 4, "1..4 global pooling aggregations");
@@ -397,6 +417,34 @@ extern "C" int gnnb_model_finalize(gnnb_model_t *m)
             idx += 6;
             break;
         }
+        case GNNB_CONV_GAT: {
+            // [att_src, att_dst, bias, lin_weight].  a: W with the per-head logit vectors
+            // w_src,h = W_h^T att_src,h and w_dst,h = W_h^T att_dst,h appended as 2H extra output
+            // rows (folded in double, rounded once), so one GEMM gives h, a_src and a_dst.
+            // b: the conv bias alone, added by the aggregation epilogue.
+            const int H = d.gat_heads, C = fo / H;
+            const float *att_src = param(m, idx), *att_dst = param(m, idx + 1);
+            const float *W = param(m, idx + 3);
+            std::vector<float> Wg((size_t)(fo + 2 * H) * fi);
+            std::copy(W, W + (size_t)fo * fi, Wg.begin());
+            for (int h = 0; h < H; h++)
+                for (int k = 0; k < fi; k++) {
+                    double ss = 0.0, sd = 0.0;
+                    for (int c = 0; c < C; c++) {
+                        const double w = W[(size_t)(h * C + c) * fi + k];
+                        ss += w * att_src[h * C + c];
+                        sd += w * att_dst[h * C + c];
+                    }
+                    Wg[(size_t)(fo + h) * fi + k] = (float)ss;
+                    Wg[(size_t)(fo + H + h) * fi + k] = (float)sd;
+                }
+            L.a = pack_linear(pk, Wg.data(), nullptr, fo + 2 * H, fi);
+            L.b.out = fo;
+            L.b.has_bias = true;
+            L.b.bias_off = pk.add_vector(param(m, idx + 2), fo);
+            idx += 4;
+            break;
+        }
         }
         layer_p.push_back(L);
     }
@@ -435,7 +483,8 @@ extern "C" int gnnb_model_finalize(gnnb_model_t *m)
     }
     fused_release(m);
     fused_tc_release(m);
-    // neither fused kernel takes GINE (they leave m->fused / m->fused_tc null): it runs layerwise
+    // neither fused kernel takes GINE or GAT (they leave m->fused / m->fused_tc null): those run
+    // layerwise
     GNNB_TRY(fused_prepare(m));
     GNNB_TRY(fused_tc_prepare(m));
     m->finalized = true;
@@ -531,13 +580,18 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
     int32_t *in_deg = m->in_deg.as<int32_t>(), *offsets = m->offsets.as<int32_t>();
     int32_t *nbr = m->nbr.as<int32_t>();
     const bool gine = d.conv_type == GNNB_CONV_GINE;
-    // GINE has no heavy-row bucketing or hub hints, as PNA
+    const bool gat = d.conv_type == GNNB_CONV_GAT;
+    // GINE has no heavy-row bucketing or hub hints, as PNA; GAT is bucketed but takes no hub hints
     const bool bucketed = d.conv_type != GNNB_CONV_PNA && !gine;
+    const bool hub_hints = bucketed && !gat;
     const int lde = round_up(std::max(d.edge_dim, 1), 4);
+    // GAT: the layer GEMM's output rows [h | a_src | a_dst], and the heavy-row partials, are
+    // H*C + 2H floats wide
+    const int ld_gat = gat ? round_up(std::max(d.hidden_dim, d.out_dim) + 2 * d.gat_heads, 4) : 0;
     if (d.num_layers > 0) {
         ProfScope ps(m->prof, PROF_TABLES, s);
         // the out-degree table (lib:1051-1083) is only read by the optional hub-row hints
-        const bool want_out_deg = !strict && hub_l2_budget() > 0 && bucketed && n_graphs > 0 &&
+        const bool want_out_deg = !strict && hub_l2_budget() > 0 && hub_hints && n_graphs > 0 &&
                                   T64 / n_graphs > 50000;
         int32_t *eidx = nullptr;
         if (gine) {
@@ -568,11 +622,11 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
     m->last_hub_rows = 0;
     if (!strict && d.num_layers > 0 && bucketed && n_graphs > 0 && T64 / n_graphs > 50000) {
         GNNB_TRY(find_heavy_rows(in_deg, T, heavy_thr, m->tws, m->heavy, s, launches));
-        GNNB_TRY(heavy_setup(m->tws, m->heavy.n_chunks, maxf));
+        GNNB_TRY(heavy_setup(m->tws, m->heavy.n_chunks, gat ? ld_gat : maxf));
         // a feature matrix larger than L2: keep the rows of the most-referenced sources resident
         // (the out-degree table, lib:1051-1083, is what ranks them)
         const size_t row_bytes = sizeof(float) * (size_t)std::max(d.in_dim, d.hidden_dim);
-        if (hub_l2_budget() > 0 && E > 0 && (size_t)T * row_bytes > (96u << 20)) {
+        if (hub_hints && hub_l2_budget() > 0 && E > 0 && (size_t)T * row_bytes > (96u << 20)) {
             ProfScope ps(m->prof, PROF_TABLES, s);
             GNNB_TRY(m->nbr_hub.ensure(sizeof(int32_t) * (size_t)En));
             GNNB_TRY(mark_hub_sources(nbr, m->nbr_hub.as<int32_t>(), E, m->out_deg.as<int32_t>(), T,
@@ -587,9 +641,10 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
 
     GNNB_TRY(m->feat[0].ensure(sizeof(float) * (size_t)Tn * ldf));
     GNNB_TRY(m->feat[1].ensure(sizeof(float) * (size_t)Tn * ldf));
-    GNNB_TRY(m->agg.ensure(sizeof(float) * (size_t)Tn * ldf));
+    if (!gat) GNNB_TRY(m->agg.ensure(sizeof(float) * (size_t)Tn * ldf));   // GAT aggregates into dst
     if (d.conv_type == GNNB_CONV_GIN || d.conv_type == GNNB_CONV_PNA || gine)
         GNNB_TRY(m->hid.ensure(sizeof(float) * (size_t)Tn * ldf));
+    if (gat) GNNB_TRY(m->hid.ensure(sizeof(float) * (size_t)Tn * ld_gat));
     if (d.conv_type == GNNB_CONV_PNA)
         GNNB_TRY(m->wide.ensure(sizeof(float) * (size_t)Tn * 14 * (size_t)ldf));
 
@@ -673,6 +728,24 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
             { ProfScope ps(m->prof, PROF_GEMM, s); GNNB_TRY(launch_gemm(g2, false, s, launches)); }   // lib:2150
             break;
         }
+        case GNNB_CONV_GAT: {
+            // one GEMM: [h | a_src | a_dst] = x.[W | w_src | w_dst]^T, no bias; then the attention
+            // aggregation, whose epilogue applies bias, skip and activation and writes the layer
+            const int H = d.gat_heads, ldg = round_up(fo + 2 * H, 4);
+            float *hg = m->hid.as<float>();
+            GemmArgs g = gemm_args(cur, cur_ld, L.a, hg, ldg, T, GNNB_ACT_IDENTITY);
+            { ProfScope ps(m->prof, PROF_GEMM, s); GNNB_TRY(launch_gemm(g, strict, s, launches)); }
+            GatAggArgs ga{};
+            ga.hg = hg; ga.ldg = ldg; ga.H = H; ga.C = fo / H; ga.slope = d.gat_negative_slope;
+            ga.bias = L.b.bias; ga.skip = skip; ga.ldskip = cur_ld; ga.act = d.gnn_act;
+            ga.out = dst; ga.ldo = ld_out;
+            ga.offsets = offsets; ga.nbr = nbr; ga.in_deg = in_deg; ga.n = T;
+            ga.heavy_threshold = heavy_thr;
+            ga.set_heavy(m->heavy, m->tws.heavy_partial.as<float>());
+            ga.ldp = ldg;
+            { ProfScope ps(m->prof, PROF_AGG, s); GNNB_TRY(launch_gat_agg(ga, s, launches)); }
+            break;
+        }
         }
         cur = dst;
         cur_ld = ld_out;
@@ -751,6 +824,11 @@ static int choose_path(gnnb_model_t *m, int max_n, int max_e, int *path, int *ke
     const bool can_tc = fast && fused_tc_supports(m, max_n, max_e);
     const bool can_fma = fast && fused_supports(m, max_n, max_e);
     if (m->path == GNNB_PATH_FUSED) {
+        if (m->d.conv_type == GNNB_CONV_GAT) {
+            set_error("fused path requested but the fused kernels have no GAT attention; GAT models "
+                      "run on the layerwise path");
+            return GNNB_ERR_INVALID;
+        }
         if (!can_tc && !can_fma) {
             set_error("fused path requested but unsupported for this model/batch (graph larger than "
                       "a CTA tile, strict math, or unsupported dims)");

@@ -29,6 +29,8 @@ struct LayerPack {
     PackedLinear a, b, c, d;  // meaning depends on the conv type (see model.cu pack_layer)
     PackedLinear e;           // GINE: the edge linear W_e^T [edge_dim][ldw], b_e
 };
+// GAT: a = [W | w_src | w_dst]^T, H*C + 2H columns and no bias (one GEMM gives h and both logits
+// of a row); b carries only the conv bias [H*C], which the aggregation epilogue adds
 
 // fused-kernel plans (fused.cu, fused_tc.cu)
 struct FusedPlan;

@@ -28,6 +28,8 @@ def _desc_struct(d: dict, max_nodes: int, max_edges: int) -> _lib.ModelDesc:
     s.max_nodes = int(max_nodes)
     s.max_edges = int(max_edges)
     s.edge_dim = int(d.get("edge_dim", 0))
+    s.gat_heads = int(d.get("gat_heads", 0))
+    s.gat_negative_slope = float(d.get("gat_negative_slope", 0.0))
     return s
 
 

@@ -94,6 +94,41 @@ class _GINEConv(nn.Module):
         return self.nn(agg + (1.0 + self.eps) * x)
 
 
+class _GATConv(nn.Module):
+    """PyG GATConv with an int ``in_channels``, concatenated heads and self loops, for inference.
+    Its own parameters come first in the flat order: ``att_src`` and ``att_dst`` [1][H][C], ``bias``
+    [H*C], then ``lin.weight`` [H*C][in] (no bias in ``lin``)."""
+
+    def __init__(self, in_channels: int, out_channels: int, heads: int, negative_slope: float):
+        super().__init__()
+        self.heads = heads
+        self.head_channels = out_channels // heads
+        self.negative_slope = negative_slope
+        self.lin = nn.Linear(in_channels, out_channels, bias=False)
+        self.att_src = nn.Parameter(torch.empty(1, heads, self.head_channels))
+        self.att_dst = nn.Parameter(torch.empty(1, heads, self.head_channels))
+        self.bias = nn.Parameter(torch.zeros(out_channels))
+        nn.init.xavier_uniform_(self.att_src)
+        nn.init.xavier_uniform_(self.att_dst)
+        nn.init.uniform_(self.bias, -0.1, 0.1)
+
+    def forward(self, x: Tensor, edge_index: Tensor) -> Tensor:
+        n, H, C = x.shape[0], self.heads, self.head_channels
+        # every self loop of the input is replaced by exactly one per node; duplicates stay
+        keep = edge_index[0] != edge_index[1]
+        loops = torch.arange(n, dtype=edge_index.dtype)
+        src = torch.cat([edge_index[0][keep], loops])
+        dst = torch.cat([edge_index[1][keep], loops])
+        h = self.lin(x).view(n, H, C)
+        a_src = (h * self.att_src).sum(-1)
+        a_dst = (h * self.att_dst).sum(-1)
+        e = torch.nn.functional.leaky_relu(a_src[src] + a_dst[dst], self.negative_slope)
+        p = (e - _scatter_minmax(e, dst, n, "amax")[dst]).exp()
+        alpha = p / _scatter_sum(p, dst, n)[dst]
+        msg = (h[src] * alpha.unsqueeze(-1)).reshape(-1, H * C)
+        return _scatter_sum(msg, dst, n) + self.bias
+
+
 class _SAGEConv(nn.Module):
     def __init__(self, in_channels: int, out_channels: int):
         super().__init__()
@@ -220,6 +255,33 @@ class GINEConv_GNNB(nn.Module):
 
     def forward(self, x: Tensor, edge_index: Tensor, edge_attr: Tensor) -> Tensor:
         return self.conv(x, edge_index, edge_attr)
+
+
+class GATConv_GNNB(nn.Module):
+    """Graph attention (PyG ``GATConv``, inference): per head, h = x W^T, logits
+    e_uv = LeakyReLU(<h_u, att_src> + <h_v, att_dst>) over the in-edges of v plus one self loop,
+    y_v = sum softmax_v(e) h_u + bias, heads concatenated.  ``out_channels`` is the concatenated
+    width and must be a multiple of ``heads``.  Pass ``heads`` with ``functools.partial``."""
+
+    def __init__(self, in_channels: int, out_channels: int, heads: int = 1,
+                 negative_slope: float = 0.2, p_in: int = 1, p_out: int = 1):
+        super().__init__()
+        if not isinstance(heads, int) or isinstance(heads, bool) or heads < 1:
+            raise ValueError(f"heads must be a positive int, got {heads!r}")
+        if out_channels % heads != 0:
+            raise ValueError(f"out_channels ({out_channels}) must be a multiple of heads ({heads})")
+        if not math.isfinite(negative_slope):
+            raise ValueError(f"negative_slope must be finite, got {negative_slope!r}")
+        self.in_channels = in_channels
+        self.out_channels = out_channels
+        self.heads = heads
+        self.negative_slope = float(negative_slope)
+        self.p_in = p_in
+        self.p_out = p_out
+        self.conv = _GATConv(in_channels, out_channels, heads, self.negative_slope)
+
+    def forward(self, x: Tensor, edge_index: Tensor) -> Tensor:
+        return self.conv(x, edge_index)
 
 
 class PNAConv_GNNB(nn.Module):
@@ -363,10 +425,11 @@ class MLP(nn.Module):
         return len(self.linear_layers)
 
 
-SUPPORTED_GNN_CONVS = [GCNConv_GNNB, GINConv_GNNB, PNAConv_GNNB, SAGEConv_GNNB, GINEConv_GNNB]
+SUPPORTED_GNN_CONVS = [GCNConv_GNNB, GINConv_GNNB, PNAConv_GNNB, SAGEConv_GNNB, GINEConv_GNNB,
+                       GATConv_GNNB]
 
 CONV_TYPE_IDS = {"GCNConv_GNNB": 0, "GINConv_GNNB": 1, "SAGEConv_GNNB": 2, "PNAConv_GNNB": 3,
-                 "GINEConv_GNNB": 4}
+                 "GINEConv_GNNB": 4, "GATConv_GNNB": 5}
 ACTIVATION_IDS = {None: 0, "ReLU": 1, "GELU": 2, "Sigmoid": 3, "Tanh": 4}
 POOL_IDS = {"add": 0, "mean": 1, "max": 2}
 
@@ -539,6 +602,9 @@ class GNNModel(nn.Module):
         )
         if self.uses_edge_features:
             d["edge_dim"] = int(self.graph_input_edge_dim)
+        if conv_name == "GATConv_GNNB":
+            d["gat_heads"] = int(conv0.heads)
+            d["gat_negative_slope"] = float(conv0.negative_slope)
         return d
 
 

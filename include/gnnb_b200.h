@@ -43,9 +43,18 @@ enum {
 };
 /* GINE (GIN with an edge linear, PyG GINEConv with edge_dim; lib:1555-1742) runs on the layerwise
  * path only and takes its edge features through the gnnb_model_run_batch_edges* entry points */
-enum { GNNB_CONV_GCN = 0, GNNB_CONV_GIN = 1, GNNB_CONV_SAGE = 2, GNNB_CONV_PNA = 3, GNNB_CONV_GINE = 4 };
+/* GAT (PyG GATConv for inference: concat heads, self loops replaced by one per node, no edge
+ * features) runs on the layerwise path only, through the plain run entry points.  It has no
+ * reference float build: GNNB_MATH_STRICT means deterministic fp32 without tensor cores for it,
+ * held to the same error bound as FAST. */
+enum {
+    GNNB_CONV_GCN = 0, GNNB_CONV_GIN = 1, GNNB_CONV_SAGE = 2, GNNB_CONV_PNA = 3, GNNB_CONV_GINE = 4,
+    GNNB_CONV_GAT = 5
+};
 /* edge feature widths a GINE model handle accepts */
 #define GNNB_GINE_MAX_EDGE_DIM 64
+/* attention head counts a GAT model handle accepts */
+#define GNNB_GAT_MAX_HEADS 16
 enum { GNNB_POOL_ADD = 0, GNNB_POOL_MEAN = 1, GNNB_POOL_MAX = 2 };
 
 /* execution path of gnnb_model_run_batch */
@@ -85,6 +94,10 @@ typedef struct gnnb_model_desc {
     int32_t edge_dim;       /* GINE only: edge feature width, 1..GNNB_GINE_MAX_EDGE_DIM.  Last field,
                                read only when conv_type == GNNB_CONV_GINE, so a caller built
                                against a header without it keeps working for the other convs. */
+    int32_t gat_heads;      /* GAT only: heads H, 1..GNNB_GAT_MAX_HEADS; every layer's output width
+                               must be a multiple of H (C = width / H channels per head) */
+    float gat_negative_slope;  /* GAT only: LeakyReLU slope of the attention logits (PyG: 0.2).
+                                  Both GAT fields are read only when conv_type == GNNB_CONV_GAT. */
 } gnnb_model_desc;
 
 typedef struct gnnb_model gnnb_model_t;
