@@ -207,15 +207,15 @@ extern "C" void {self.name}_top(
 """
 
     def _check_top_renderable(self, what):
-        if getattr(self.model, "uses_edge_features", False):
-            raise NotImplementedError(
-                f"{what}: the reference's <name>_top signature has no edge-feature argument, so a "
-                "GINEConv_GNNB model cannot be rendered; run it through Engine instead")
         if self.model is not None and self.model.describe()["conv_type"] == 5:
             raise NotImplementedError(
                 f"{what}: the reference has no GAT kernel and its <name>_top no attention-head "
                 "arguments, so a GATConv_GNNB model cannot be rendered; run it through Engine "
                 "instead")
+        if getattr(self.model, "uses_edge_features", False):
+            raise NotImplementedError(
+                f"{what}: the reference's <name>_top signature has no edge-feature argument, so a "
+                "GINEConv_GNNB model cannot be rendered; run it through Engine instead")
 
     def build_top(self, testbench: Optional[Path] = None) -> Path:
         """Compile the generated ``model.cpp`` into ``lib<name>.so`` (exports ``<name>_top``).

@@ -942,6 +942,11 @@ int launch_permute_edge_rows(const float *src, int dim, const int32_t *idx, int 
 // One CTA per row then merges the chunks -- 8 warps over contiguous chunk ranges, then the self term
 // and the 8 range results in warp order -- a fixed order, so the result does not depend on
 // scheduling.  Algorithmic bytes per layer: E (4 + 4H + 4HC) + N (8 + 4H + 4HC [+ 4HC skip]).
+//
+// Edge attention (GATConv with edge_dim; the EDGE instantiations): the logit of slot k adds the edge
+// term elog[k][hd] and the self term self_elog[v][hd], both computed once per run by
+// gat_edge_logits_kernel, so a layer reads H more floats per edge and per node: + E 4H + N 4H.
+// The plain instantiations are unchanged.
 namespace {
 
 __device__ __forceinline__ float leaky_relu(float x, float slope) { return x > 0.0f ? x : x * slope; }
@@ -972,20 +977,22 @@ struct OnlineSoftmax {
 };
 
 // the self term of row v for the lane's columns [c, c + VEC) of head hd; returns a_dst[v][hd]
-template <int VEC>
+template <int VEC, bool EDGE>
 __device__ __forceinline__ float gat_self(const GatAggArgs &a, int v, int c, int hd, OnlineSoftmax<VEC> &st)
 {
     const int HC = a.H * a.C;
     const float *row = a.hg + (size_t)v * a.ldg;
     const float adst = __ldg(row + HC + a.H + hd);
-    st.m = leaky_relu(__ldg(row + HC + hd) + adst, a.slope);
+    float e = __ldg(row + HC + hd) + adst;
+    if (EDGE) e += __ldg(a.self_elog + (size_t)v * a.ldl + hd);
+    st.m = leaky_relu(e, a.slope);
     st.s = 1.0f;
     st.acc.load(row + c);
     return adst;
 }
 
 // neighbor entries [k0, k1) of row v (entries equal to v skipped), four gathers in flight
-template <int VEC>
+template <int VEC, bool EDGE>
 __device__ __forceinline__ void gat_gather(const GatAggArgs &a, int v, int off, int k0, int k1, int c,
                                            int hd, float adst, OnlineSoftmax<VEC> &st)
 {
@@ -993,7 +1000,7 @@ __device__ __forceinline__ void gat_gather(const GatAggArgs &a, int v, int off, 
     int k = k0;
     for (; k + 4 <= k1; k += 4) {
         int u[4];
-        float as[4];
+        float as[4], el[4];
         Vec<VEC> x[4];
 #pragma unroll
         for (int j = 0; j < 4; j++) u[j] = __ldg(a.nbr + off + k + j);
@@ -1001,11 +1008,15 @@ __device__ __forceinline__ void gat_gather(const GatAggArgs &a, int v, int off, 
         for (int j = 0; j < 4; j++) {
             const float *row = a.hg + (size_t)u[j] * a.ldg;
             as[j] = __ldg(row + HC + hd);
+            if (EDGE) el[j] = __ldg(a.elog + (size_t)(off + k + j) * a.ldl + hd);
             x[j].load(row + c);
         }
 #pragma unroll
-        for (int j = 0; j < 4; j++)
-            if (u[j] != v) st.merge(leaky_relu(as[j] + adst, a.slope), 1.0f, x[j]);
+        for (int j = 0; j < 4; j++) {
+            float e = as[j] + adst;
+            if (EDGE) e += el[j];
+            if (u[j] != v) st.merge(leaky_relu(e, a.slope), 1.0f, x[j]);
+        }
     }
     for (; k < k1; k++) {
         const int u = __ldg(a.nbr + off + k);
@@ -1013,7 +1024,9 @@ __device__ __forceinline__ void gat_gather(const GatAggArgs &a, int v, int off, 
         const float *row = a.hg + (size_t)u * a.ldg;
         Vec<VEC> x;
         x.load(row + c);
-        st.merge(leaky_relu(__ldg(row + HC + hd) + adst, a.slope), 1.0f, x);
+        float e = __ldg(row + HC + hd) + adst;
+        if (EDGE) e += __ldg(a.elog + (size_t)(off + k) * a.ldl + hd);
+        st.merge(leaky_relu(e, a.slope), 1.0f, x);
     }
 }
 
@@ -1032,7 +1045,7 @@ __device__ __forceinline__ void gat_finish(const GatAggArgs &a, int v, int c, co
     y.store(a.out + (size_t)v * a.ldo + c);
 }
 
-template <int VEC, int LPR>
+template <int VEC, int LPR, bool EDGE>
 __global__ void __launch_bounds__(256) gat_agg_kernel(const GatAggArgs a)
 {
     constexpr int ROWS_PER_WARP = 32 / LPR;
@@ -1051,14 +1064,14 @@ __global__ void __launch_bounds__(256) gat_agg_kernel(const GatAggArgs a)
         for (int c = lg * VEC; c < HC; c += LPR * VEC) {
             const int hd = c / a.C;
             OnlineSoftmax<VEC> st;
-            const float adst = gat_self(a, v, c, hd, st);
-            gat_gather(a, v, off, 0, deg, c, hd, adst, st);
+            const float adst = gat_self<VEC, EDGE>(a, v, c, hd, st);
+            gat_gather<VEC, EDGE>(a, v, off, 0, deg, c, hd, adst, st);
             gat_finish(a, v, c, st);
         }
     }
 }
 
-template <int VEC>
+template <int VEC, bool EDGE>
 __global__ void __launch_bounds__(256) gat_heavy_chunk_kernel(const GatAggArgs a)
 {
     const int lane = threadIdx.x & 31;
@@ -1079,7 +1092,7 @@ __global__ void __launch_bounds__(256) gat_heavy_chunk_kernel(const GatAggArgs a
             const int hd = c / a.C;
             OnlineSoftmax<VEC> st;
             st.reset();
-            gat_gather(a, v, off, k0, k1, c, hd, __ldg(rowv + HC + a.H + hd), st);
+            gat_gather<VEC, EDGE>(a, v, off, k0, k1, c, hd, __ldg(rowv + HC + a.H + hd), st);
             st.acc.store(dst + c);
             if (c % a.C == 0) {   // one lane per head
                 dst[HC + hd] = st.m;
@@ -1089,8 +1102,8 @@ __global__ void __launch_bounds__(256) gat_heavy_chunk_kernel(const GatAggArgs a
     }
 }
 
-template <int VEC>
-__global__ void __launch_bounds__(256) gat_heavy_combine_kernel(const GatAggArgs a)
+template <int VEC, bool EDGE>
+__device__ __forceinline__ void gat_heavy_combine(const GatAggArgs &a)
 {
     extern __shared__ float4 gat_smem4[];
     float *const ranges = reinterpret_cast<float *>(gat_smem4);   // [8][ldp], laid out as the partials
@@ -1125,7 +1138,7 @@ __global__ void __launch_bounds__(256) gat_heavy_combine_kernel(const GatAggArgs
             for (int c = lane * VEC; c < HC; c += 32 * VEC) {
                 const int hd = c / a.C;
                 OnlineSoftmax<VEC> st;
-                gat_self(a, v, c, hd, st);
+                gat_self<VEC, EDGE>(a, v, c, hd, st);
 #pragma unroll 1
                 for (int w = 0; w < 8; w++) {
                     const float *r = ranges + w * a.ldp;
@@ -1140,30 +1153,45 @@ __global__ void __launch_bounds__(256) gat_heavy_combine_kernel(const GatAggArgs
     }
 }
 
+// plain GAT: the kernel as it always was
 template <int VEC>
+__global__ void __launch_bounds__(256) gat_heavy_combine_kernel(const GatAggArgs a)
+{
+    gat_heavy_combine<VEC, false>(a);
+}
+// edge attention: capped at 64 registers, where ptxas's own choice under __launch_bounds__(256)
+// spilled it (one CTA per heavy row, so occupancy does not matter here)
+template <int VEC>
+__global__ void __maxnreg__(64) gat_heavy_combine_edge_kernel(const GatAggArgs a)
+{
+    gat_heavy_combine<VEC, true>(a);
+}
+
+template <int VEC, bool EDGE>
 void launch_gat_lpr(const GatAggArgs &a, int lpr, int grid, cudaStream_t s)
 {
     switch (lpr) {
-    case 1: gat_agg_kernel<VEC, 1><<<grid, 256, 0, s>>>(a); break;
-    case 2: gat_agg_kernel<VEC, 2><<<grid, 256, 0, s>>>(a); break;
-    case 4: gat_agg_kernel<VEC, 4><<<grid, 256, 0, s>>>(a); break;
-    case 8: gat_agg_kernel<VEC, 8><<<grid, 256, 0, s>>>(a); break;
-    case 16: gat_agg_kernel<VEC, 16><<<grid, 256, 0, s>>>(a); break;
-    default: gat_agg_kernel<VEC, 32><<<grid, 256, 0, s>>>(a); break;
+    case 1: gat_agg_kernel<VEC, 1, EDGE><<<grid, 256, 0, s>>>(a); break;
+    case 2: gat_agg_kernel<VEC, 2, EDGE><<<grid, 256, 0, s>>>(a); break;
+    case 4: gat_agg_kernel<VEC, 4, EDGE><<<grid, 256, 0, s>>>(a); break;
+    case 8: gat_agg_kernel<VEC, 8, EDGE><<<grid, 256, 0, s>>>(a); break;
+    case 16: gat_agg_kernel<VEC, 16, EDGE><<<grid, 256, 0, s>>>(a); break;
+    default: gat_agg_kernel<VEC, 32, EDGE><<<grid, 256, 0, s>>>(a); break;
     }
 }
 
-template <int VEC>
+template <int VEC, bool EDGE>
 int launch_gat_heavy(const GatAggArgs &a, cudaStream_t s)
 {
     const int cap = kNumSMs * 8;   // 8 resident CTAs per SM, grid-stride beyond
     const int g1 = min((a.heavy_chunks + 7) / 8, cap), g2 = min(a.n_heavy, cap);
-    gat_heavy_chunk_kernel<VEC><<<g1, 256, 0, s>>>(a);
+    gat_heavy_chunk_kernel<VEC, EDGE><<<g1, 256, 0, s>>>(a);
     const size_t smem = sizeof(float) * 8 * (size_t)a.ldp;
+    void (*combine)(const GatAggArgs) =
+        EDGE ? gat_heavy_combine_edge_kernel<VEC> : gat_heavy_combine_kernel<VEC>;
     if (smem > 48 * 1024)
-        GNNB_CUDA(cudaFuncSetAttribute(gat_heavy_combine_kernel<VEC>,
-                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    gat_heavy_combine_kernel<VEC><<<g2, 256, smem, s>>>(a);
+        GNNB_CUDA(cudaFuncSetAttribute(combine, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    combine<<<g2, 256, smem, s>>>(a);
     return GNNB_OK;
 }
 
@@ -1186,10 +1214,12 @@ int launch_gat_agg(const GatAggArgs &a, cudaStream_t s, int *launches)
     int64_t grid64 = ceil_div64(a.n, rows_per_block);
     const int64_t cap = (int64_t)kNumSMs * 8 * 4;
     const int grid = (int)(grid64 < cap ? grid64 : cap);
+    const bool edge = a.elog != nullptr;
+    if (edge) GNNB_REQUIRE(a.self_elog != nullptr && a.ldl >= a.H, "gat aggregation: bad edge logits");
     if (vec == 4)
-        launch_gat_lpr<4>(a, lpr, grid, s);
+        edge ? launch_gat_lpr<4, true>(a, lpr, grid, s) : launch_gat_lpr<4, false>(a, lpr, grid, s);
     else
-        launch_gat_lpr<1>(a, lpr, grid, s);
+        edge ? launch_gat_lpr<1, true>(a, lpr, grid, s) : launch_gat_lpr<1, false>(a, lpr, grid, s);
     GNNB_CUDA(cudaGetLastError());
     if (launches) ++*launches;
     if (a.n_heavy > 0) {
@@ -1197,10 +1227,103 @@ int launch_gat_agg(const GatAggArgs &a, cudaStream_t s, int *launches)
                          a.heavy_chunk_base != nullptr && a.heavy_chunk_row != nullptr &&
                          a.ldp >= HC + 2 * a.H && a.ldp % 4 == 0,
                      "gat heavy rows: row list / partial buffer missing");
-        GNNB_TRY(vec == 4 ? launch_gat_heavy<4>(a, s) : launch_gat_heavy<1>(a, s));
+        GNNB_TRY(vec == 4 ? (edge ? launch_gat_heavy<4, true>(a, s) : launch_gat_heavy<4, false>(a, s))
+                          : (edge ? launch_gat_heavy<1, true>(a, s) : launch_gat_heavy<1, false>(a, s)));
         GNNB_CUDA(cudaGetLastError());
         if (launches) *launches += 2;
     }
+    return GNNB_OK;
+}
+
+// Edge logits of every layer and head, once per run (kernels.h).  LPR lanes per destination row; the
+// row's items i = k * LH + lh (slot k, layer-head lh) are spread over them, so each lane's elog
+// writes are contiguous with its neighbours'.  The LH lanes of one slot read the same edge_attr row
+// (L1 hits); w_edge is staged in shared memory when it fits.  Then, after the warp barrier, each
+// lane averages one lh column of the row's elog in slot order for self_elog.  Hub rows are one
+// sub-warp's serial work (no bucketing: the pass runs once per run, not once per layer).
+// Algorithmic bytes: E (4 + 4 + 4 edge_dim + 4 LH) + N (8 + 4 LH).
+namespace {
+
+template <int LPR>
+__global__ void __launch_bounds__(256) gat_edge_logits_kernel(const GatEdgeLogitsArgs a, bool w_smem)
+{
+    extern __shared__ float4 elog_smem4[];
+    const float *w = a.w_edge;
+    if (w_smem) {
+        float *sw = reinterpret_cast<float *>(elog_smem4);
+        for (int i = threadIdx.x; i < a.LH * a.edge_dim; i += blockDim.x) sw[i] = __ldg(a.w_edge + i);
+        __syncthreads();
+        w = sw;
+    }
+    constexpr int ROWS_PER_WARP = 32 / LPR;
+    const int lane = threadIdx.x & 31;
+    const int lg = lane % LPR, sub = lane / LPR;
+    const int warps_per_block = blockDim.x >> 5;
+    const int64_t warp_global = (int64_t)blockIdx.x * warps_per_block + (threadIdx.x >> 5);
+    const int64_t warp_stride = (int64_t)gridDim.x * warps_per_block;
+    const int LH = a.LH;
+    // row0 is warp-uniform, so every lane reaches the __syncwarp
+    for (int64_t row0 = warp_global * ROWS_PER_WARP; row0 < a.n; row0 += warp_stride * ROWS_PER_WARP) {
+        const int v = (int)row0 + sub;
+        const bool valid = v < a.n;
+        const int deg = valid ? __ldg(a.in_deg + v) : 0;
+        const int off = valid ? __ldg(a.offsets + v) : 0;
+        float *el = a.elog + (size_t)off * LH;
+        // int64 items: one hub row may hold deg * LH >= 2^31 of them
+        const int64_t items = (int64_t)deg * LH;
+        for (int64_t i = lg; i < items; i += LPR) {
+            const int k = (int)(i / LH), lh = (int)(i - (int64_t)k * LH);
+            float acc = 0.0f;   // self-loop slots hold 0: never read as logits, but defined
+            if (__ldg(a.nbr + off + k) != v) {
+                const float *ef = a.ef + (size_t)__ldg(a.edge_index + off + k) * a.edge_dim;
+                const float *wr = w + (size_t)lh * a.edge_dim;
+                for (int j = 0; j < a.edge_dim; j++) acc = fmaf(__ldg(ef + j), wr[j], acc);
+            }
+            el[i] = acc;
+        }
+        __syncwarp();
+        if (!valid) continue;
+        for (int lh = lg; lh < LH; lh += LPR) {
+            float sum = 0.0f;
+            int cnt = 0;
+            for (int k = 0; k < deg; k++) {
+                if (__ldg(a.nbr + off + k) == v) continue;
+                sum += el[(size_t)k * LH + lh];
+                cnt++;
+            }
+            a.self_elog[(size_t)v * LH + lh] = cnt > 0 ? sum / (float)cnt : 0.0f;
+        }
+    }
+}
+
+}  // namespace
+
+int launch_gat_edge_logits(const GatEdgeLogitsArgs &a, int avg_deg, cudaStream_t s, int *launches)
+{
+    if (a.n <= 0) return GNNB_OK;
+    GNNB_REQUIRE(a.edge_dim >= 1 && a.LH >= 1 && a.w_edge != nullptr && a.elog != nullptr &&
+                     a.self_elog != nullptr && a.edge_index != nullptr,
+                 "gat edge logits: bad arguments");
+    int lpr = 1;
+    const int64_t items = (int64_t)std::max(avg_deg, 1) * a.LH;
+    while (lpr < 32 && lpr < items) lpr *= 2;
+    const size_t smem_w = sizeof(float) * (size_t)a.LH * a.edge_dim;
+    const bool w_smem = smem_w <= 48 * 1024;
+    const size_t smem = w_smem ? smem_w : 0;
+    const int rows_per_block = 8 * (32 / lpr);
+    const int64_t grid64 = ceil_div64(a.n, rows_per_block);
+    const int64_t cap = (int64_t)kNumSMs * 8;
+    const int grid = (int)(grid64 < cap ? grid64 : cap);
+    switch (lpr) {
+    case 1: gat_edge_logits_kernel<1><<<grid, 256, smem, s>>>(a, w_smem); break;
+    case 2: gat_edge_logits_kernel<2><<<grid, 256, smem, s>>>(a, w_smem); break;
+    case 4: gat_edge_logits_kernel<4><<<grid, 256, smem, s>>>(a, w_smem); break;
+    case 8: gat_edge_logits_kernel<8><<<grid, 256, smem, s>>>(a, w_smem); break;
+    case 16: gat_edge_logits_kernel<16><<<grid, 256, smem, s>>>(a, w_smem); break;
+    default: gat_edge_logits_kernel<32><<<grid, 256, smem, s>>>(a, w_smem); break;
+    }
+    GNNB_CUDA(cudaGetLastError());
+    if (launches) ++*launches;
     return GNNB_OK;
 }
 

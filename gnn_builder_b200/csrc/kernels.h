@@ -197,6 +197,11 @@ struct GatAggArgs {
     int ldp;               // round_up(H*C + 2H, 4)
     const int32_t *heavy_chunk_base, *heavy_chunk_row;
     int heavy_chunks;
+    // edge attention (GATConv with edge_dim), else null: the logits of launch_gat_edge_logits
+    // advanced to this layer's H columns; the neighbor logit adds elog[slot][hd], the self term
+    // self_elog[v][hd]
+    const float *elog, *self_elog;   // [slots][ldl], [n][ldl]
+    int ldl;
     void set_heavy(const HeavyList &hl, float *partial)
     {
         heavy_rows = hl.rows.as<int32_t>(); n_heavy = hl.n_heavy;
@@ -205,6 +210,24 @@ struct GatAggArgs {
     }
 };
 int launch_gat_agg(const GatAggArgs &a, cudaStream_t s, int *launches);
+
+// Edge terms of GAT's attention logits for every layer and head at once (they do not depend on the
+// layer input), once per run.  w_edge [lh][edge_dim], lh = layer * H + head, is lin_edge folded with
+// att_edge.  A (sub-)warp per destination row v walks its neighbor slots: elog[slot][lh] =
+// sum_j ef[edge_index[slot]][j] w_edge[lh][j] (fp32, ascending j), and self_elog[v][lh] = the mean
+// of elog over the row's slots whose source is not v (0 when there is none).  Slots whose source is
+// v get 0 and are left out of the mean: the aggregation never uses them.
+struct GatEdgeLogitsArgs {
+    const float *ef;           // [E][edge_dim], COO edge order
+    int edge_dim;
+    const float *w_edge;       // [LH][edge_dim]
+    int LH;
+    const int32_t *offsets, *nbr, *in_deg, *edge_index;
+    int n;
+    float *elog;               // [E][LH], neighbor-slot order
+    float *self_elog;          // [n][LH]
+};
+int launch_gat_edge_logits(const GatEdgeLogitsArgs &a, int avg_deg, cudaStream_t s, int *launches);
 
 struct PnaAggArgs {
     const float *ab;       // [n][2F]: cols [0,F) = x.W_nbr^T, cols [F,2F) = x.W_self^T + b_pre

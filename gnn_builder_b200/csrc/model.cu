@@ -116,11 +116,14 @@ void enumerate_params(gnnb_model *m)
             add_param(m, base + "_conv_lin_weight", {fo, fo});
             add_param(m, base + "_conv_lin_bias", {fo});
             break;
-        case GNNB_CONV_GAT:   // PyG GATConv: its own parameters, then lin's
+        case GNNB_CONV_GAT:   // PyG GATConv: its own parameters, then lin's (and lin_edge's)
             add_param(m, base + "_conv_att_src", {1, d.gat_heads, fo / d.gat_heads});
             add_param(m, base + "_conv_att_dst", {1, d.gat_heads, fo / d.gat_heads});
+            if (m->has_edge_features())
+                add_param(m, base + "_conv_att_edge", {1, d.gat_heads, fo / d.gat_heads});
             add_param(m, base + "_conv_bias", {fo});
             add_param(m, base + "_conv_lin_weight", {fo, fi});
+            if (m->has_edge_features()) add_param(m, base + "_conv_lin_edge_weight", {fo, d.edge_dim});
             break;
         }
     }
@@ -219,9 +222,9 @@ extern "C" int gnnb_host_unregister(void *ptr)
 extern "C" int gnnb_model_create(const gnnb_model_desc *desc, int device, gnnb_model_t **out)
 {
     GNNB_REQUIRE(desc != nullptr && out != nullptr, "null argument");
-    // edge_dim is the last field and only GINE callers are required to have it: copy the fields
-    // before it, then read it for GINE only (a caller built against the older, shorter struct
-    // never has bytes read past its end)
+    // edge_dim and the GAT fields after it are only required of GINE and GAT callers: copy the
+    // fields before it, then read it for GINE and GAT only (a caller built against the older,
+    // shorter struct never has bytes read past its end; a GAT caller's struct always holds it)
     gnnb_model_desc d{};
     std::memcpy(&d, desc, offsetof(gnnb_model_desc, edge_dim));
     GNNB_REQUIRE(d.conv_type >= GNNB_CONV_GCN && d.conv_type <= GNNB_CONV_GAT,
@@ -234,6 +237,10 @@ extern "C" int gnnb_model_create(const gnnb_model_desc *desc, int device, gnnb_m
     GNNB_REQUIRE(d.num_layers >= 0 && d.num_layers <= 64, "num_layers out of range");
     GNNB_REQUIRE(d.in_dim > 0 && d.hidden_dim > 0 && d.out_dim > 0, "dimensions must be positive");
     if (d.conv_type == GNNB_CONV_GAT) {   // the GAT fields follow edge_dim; only GAT callers set them
+        d.edge_dim = desc->edge_dim;
+        GNNB_REQUIRE(d.edge_dim >= 0 && d.edge_dim <= kGineMaxEdgeDim,
+                     "GAT edge_dim must be 0 (no edge features) or 1.." +
+                         std::to_string(kGineMaxEdgeDim));
         d.gat_heads = desc->gat_heads;
         d.gat_negative_slope = desc->gat_negative_slope;
         GNNB_REQUIRE(d.gat_heads >= 1 && d.gat_heads <= GNNB_GAT_MAX_HEADS,
@@ -295,7 +302,7 @@ extern "C" int gnnb_model_destroy(gnnb_model_t *m)
     m->prof.release();
     DeviceBuf *bufs[] = {&m->weights, &m->weight_images, &m->st_x, &m->st_coo, &m->st_ef, &m->st_nptr, &m->st_eptr, &m->st_out,
                          &m->in_deg, &m->out_deg, &m->offsets, &m->nbr, &m->nbr_hub, &m->dinv,
-                         &m->edge_index, &m->ef_sorted,
+                         &m->edge_index, &m->ef_sorted, &m->elog, &m->self_elog,
                          &m->feat[0], &m->feat[1], &m->agg, &m->hid, &m->wide, &m->pooled,
                          &m->hbuf[0], &m->hbuf[1], &m->pool_tmp, &m->ptr_tmp, &m->edge_flag};
     for (DeviceBuf *b : bufs) b->release();
@@ -366,6 +373,9 @@ extern "C" int gnnb_model_finalize(gnnb_model_t *m)
     struct PendingLayer { int fi, fo; PendingLinear a, b, c, d, e; };
     std::vector<PendingLayer> layer_p;
     size_t idx = 0;
+    std::vector<float> gat_w_edge;   // GAT with edge_dim: [L][H][edge_dim]
+    if (d.conv_type == GNNB_CONV_GAT && m->has_edge_features())
+        gat_w_edge.resize((size_t)d.num_layers * d.gat_heads * d.edge_dim);
     {
         int in = m->emb_dim() * d.num_pools;
         for (int j = 0; j < d.mlp_num_linear; j++) {
@@ -418,13 +428,16 @@ extern "C" int gnnb_model_finalize(gnnb_model_t *m)
             break;
         }
         case GNNB_CONV_GAT: {
-            // [att_src, att_dst, bias, lin_weight].  a: W with the per-head logit vectors
+            // [att_src, att_dst, (att_edge,) bias, lin_weight (, lin_edge_weight)].  a: W with the
+            // per-head logit vectors
             // w_src,h = W_h^T att_src,h and w_dst,h = W_h^T att_dst,h appended as 2H extra output
             // rows (folded in double, rounded once), so one GEMM gives h, a_src and a_dst.
             // b: the conv bias alone, added by the aggregation epilogue.
             const int H = d.gat_heads, C = fo / H;
+            const bool edges = m->has_edge_features();
+            const size_t ib = idx + (edges ? 3 : 2), iw = ib + 1;   // bias, lin_weight
             const float *att_src = param(m, idx), *att_dst = param(m, idx + 1);
-            const float *W = param(m, idx + 3);
+            const float *W = param(m, iw);
             std::vector<float> Wg((size_t)(fo + 2 * H) * fi);
             std::copy(W, W + (size_t)fo * fi, Wg.begin());
             for (int h = 0; h < H; h++)
@@ -441,18 +454,33 @@ extern "C" int gnnb_model_finalize(gnnb_model_t *m)
             L.a = pack_linear(pk, Wg.data(), nullptr, fo + 2 * H, fi);
             L.b.out = fo;
             L.b.has_bias = true;
-            L.b.bias_off = pk.add_vector(param(m, idx + 2), fo);
-            idx += 4;
+            L.b.bias_off = pk.add_vector(param(m, ib), fo);
+            if (edges) {
+                // w_edge,h[j] = sum_c W_e[h*C + c][j] att_edge[h*C + c], folded in double and
+                // rounded once, as w_src / w_dst: lin_edge never runs as a GEMM
+                const int ed = d.edge_dim;
+                const float *att_edge = param(m, idx + 2), *We = param(m, iw + 1);
+                for (int h = 0; h < H; h++)
+                    for (int j = 0; j < ed; j++) {
+                        double se = 0.0;
+                        for (int c = 0; c < C; c++)
+                            se += (double)We[(size_t)(h * C + c) * ed + j] * att_edge[h * C + c];
+                        gat_w_edge[((size_t)k * H + h) * ed + j] = (float)se;
+                    }
+            }
+            idx += edges ? 6 : 4;
             break;
         }
         }
         layer_p.push_back(L);
     }
+    const size_t w_edge_off = gat_w_edge.empty() ? 0 : pk.add_vector(gat_w_edge.data(), (int)gat_w_edge.size());
     GNNB_TRY(m->weights.ensure(pk.data.size() * sizeof(float)));
     GNNB_CUDA(cudaMemcpyAsync(m->weights.ptr, pk.data.data(), pk.data.size() * sizeof(float),
                               cudaMemcpyHostToDevice, m->stream));
     GNNB_CUDA(cudaStreamSynchronize(m->stream));
     const float *base = m->weights.as<float>();
+    m->gat_w_edge = gat_w_edge.empty() ? nullptr : base + w_edge_off;
     m->head.clear();
     for (const PendingLinear &p : head_p) m->head.push_back(resolve(p, base));
     m->layers.clear();
@@ -558,7 +586,7 @@ static GemmArgs gemm_args(const float *A, int lda, const PackedLinear &L, float 
 
 // x/coo/ef/node_ptr/edge_ptr/out are DEVICE pointers; node_ptr/edge_ptr address graph 0 of this
 // chunk and hold absolute offsets (node_base/edge_base = their first values).  ef: the chunk's edge
-// features [E][edge_dim] (GINE only).
+// features [E][edge_dim] (models with edge features only).
 static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, const float *ef,
                          const int64_t *node_ptr,
                          const int64_t *edge_ptr, int64_t node_base, int64_t edge_base,
@@ -581,6 +609,8 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
     int32_t *nbr = m->nbr.as<int32_t>();
     const bool gine = d.conv_type == GNNB_CONV_GINE;
     const bool gat = d.conv_type == GNNB_CONV_GAT;
+    const bool gat_edges = gat && m->has_edge_features();
+    const int LH = gat_edges ? d.num_layers * d.gat_heads : 0;   // edge logit columns per slot / row
     // GINE has no heavy-row bucketing or hub hints, as PNA; GAT is bucketed but takes no hub hints
     const bool bucketed = d.conv_type != GNNB_CONV_PNA && !gine;
     const bool hub_hints = bucketed && !gat;
@@ -594,12 +624,13 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
         const bool want_out_deg = !strict && hub_l2_budget() > 0 && hub_hints && n_graphs > 0 &&
                                   T64 / n_graphs > 50000;
         int32_t *eidx = nullptr;
-        if (gine) {
+        if (m->has_edge_features()) {
             GNNB_TRY(m->edge_index.ensure(sizeof(int32_t) * (size_t)En));
             eidx = m->edge_index.as<int32_t>();
         }
-        // GINE always passes the offsets: its slot -> source gather then checks every endpoint
-        GNNB_TRY(build_tables(coo, n_graphs > 1 || gine ? node_ptr : nullptr, edge_ptr, node_base,
+        // with edge features the offsets are always passed: the slot -> source gather then checks
+        // every endpoint
+        GNNB_TRY(build_tables(coo, n_graphs > 1 || eidx ? node_ptr : nullptr, edge_ptr, node_base,
                               edge_base, n_graphs, T, E, in_deg,
                               want_out_deg ? m->out_deg.as<int32_t>() : nullptr, offsets, nbr, eidx,
                               m->tws, s, launches, m->edge_flag.as<int>()));
@@ -608,6 +639,16 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
             GNNB_TRY(launch_permute_edge_rows(ef, d.edge_dim, eidx, E, m->ef_sorted.as<float>(), lde, s,
                                               launches));
         }
+    }
+    if (gat_edges && d.num_layers > 0) {   // every layer's edge logits, once per run
+        ProfScope ps(m->prof, PROF_EDGE_LOGITS, s);
+        GNNB_TRY(m->elog.ensure(sizeof(float) * (size_t)En * LH));
+        GNNB_TRY(m->self_elog.ensure(sizeof(float) * (size_t)Tn * LH));
+        GatEdgeLogitsArgs la{};
+        la.ef = ef; la.edge_dim = d.edge_dim; la.w_edge = m->gat_w_edge; la.LH = LH;
+        la.offsets = offsets; la.nbr = nbr; la.in_deg = in_deg; la.edge_index = m->edge_index.as<int32_t>();
+        la.n = T; la.elog = m->elog.as<float>(); la.self_elog = m->self_elog.as<float>();
+        GNNB_TRY(launch_gat_edge_logits(la, (int)(((int64_t)E + Tn - 1) / Tn), s, launches));
     }
     const float *dinv = nullptr;
     if (d.conv_type == GNNB_CONV_GCN && !strict && d.num_layers > 0) {
@@ -743,6 +784,11 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
             ga.heavy_threshold = heavy_thr;
             ga.set_heavy(m->heavy, m->tws.heavy_partial.as<float>());
             ga.ldp = ldg;
+            if (gat_edges) {
+                ga.elog = m->elog.as<float>() + (size_t)k * H;
+                ga.self_elog = m->self_elog.as<float>() + (size_t)k * H;
+                ga.ldl = LH;
+            }
             { ProfScope ps(m->prof, PROF_AGG, s); GNNB_TRY(launch_gat_agg(ga, s, launches)); }
             break;
         }
@@ -865,19 +911,22 @@ static int fused_any_status(gnnb_model_t *m, int *status)
     return m->last_kernel == 3 ? fused_tc_status(m, status) : fused_status(m, status);
 }
 
-// a GINE handle takes its edge features through the *_edges entry points, every other handle
-// through the plain ones
+// a handle with edge features (GINE, GAT with edge_dim) takes them through the *_edges entry
+// points, every other handle runs through the plain ones
 static int check_edges_entry(gnnb_model_t *m, bool edges_entry)
 {
     GNNB_TRY(check_ready(m));
-    const bool gine = m->d.conv_type == GNNB_CONV_GINE;
-    if (gine && !edges_entry) {
-        set_error("a GINE model needs its edge features: run it with gnnb_model_run_batch_edges or "
+    const bool edges = m->has_edge_features();
+    if (edges && !edges_entry) {
+        set_error(std::string(m->d.conv_type == GNNB_CONV_GAT ? "a GAT model with edge_dim"
+                                                                : "a GINE model") +
+                  " needs its edge features: run it with gnnb_model_run_batch_edges or "
                   "gnnb_model_run_batch_edges_async");
         return GNNB_ERR_INVALID;
     }
-    if (!gine && edges_entry) {
-        set_error("the *_edges entry points run GINE models only; this model has no edge features");
+    if (!edges && edges_entry) {
+        set_error("the *_edges entry points run GINE models and GAT models with edge_dim only; this "
+                  "model has no edge features");
         return GNNB_ERR_INVALID;
     }
     return GNNB_OK;
@@ -893,7 +942,7 @@ static int run_batch_async(gnnb_model_t *m, const float *x, const int32_t *edge_
     GNNB_REQUIRE(node_ptr != nullptr && edge_ptr != nullptr && out != nullptr, "null argument");
     if (n_graphs == 0) return GNNB_OK;
     GNNB_REQUIRE(is_device_pointer(x) || total_nodes == 0, "run_batch_async needs device pointers");
-    if (m->d.conv_type == GNNB_CONV_GINE)
+    if (m->has_edge_features())
         GNNB_REQUIRE(total_edges == 0 || is_device_pointer(edge_attr),
                      "edge_attr must be a device pointer (null with edges present)");
     cudaStream_t s = stream ? (cudaStream_t)stream : m->stream;
@@ -961,8 +1010,8 @@ static int run_batch(gnnb_model_t *m, const float *x, const int32_t *edge_list,
     GNNB_REQUIRE(T >= 0 && E >= 0 && T < (1ll << 40) && E < (1ll << 40), "bad node_ptr/edge_ptr totals");
     GNNB_REQUIRE(T == 0 || x != nullptr, "x is null");
     GNNB_REQUIRE(E == 0 || edge_list != nullptr, "edge_list is null");
-    const bool gine = d.conv_type == GNNB_CONV_GINE;
-    if (gine) {
+    const bool edges = m->has_edge_features();
+    if (edges) {
         GNNB_REQUIRE(E == 0 || edge_attr != nullptr, "edge_attr is null");
         GNNB_REQUIRE(E == 0 || is_device_pointer(edge_attr) == dev,
                      "edge_attr must live in the same memory space as node_ptr");
@@ -1121,7 +1170,7 @@ static int run_batch(gnnb_model_t *m, const float *x, const int32_t *edge_list,
         if (E > 0)
             GNNB_CUDA(cudaMemcpyAsync(m->st_coo.ptr, edge_list, sizeof(int32_t) * 2 * (size_t)E,
                                       cudaMemcpyHostToDevice, s));
-        if (gine) {
+        if (edges) {
             GNNB_TRY(m->st_ef.ensure(sizeof(float) * (size_t)std::max<int64_t>(E, 1) * d.edge_dim));
             if (E > 0)
                 GNNB_CUDA(cudaMemcpyAsync(m->st_ef.ptr, edge_attr, sizeof(float) * (size_t)E * d.edge_dim,
@@ -1152,7 +1201,7 @@ static int run_batch(gnnb_model_t *m, const float *x, const int32_t *edge_list,
             int g1 = g0 + 1;
             while (g1 < n_graphs && hn[g1 + 1] - hn[g0] <= kChunkNodes) g1++;
             GNNB_TRY(run_layerwise(m, dx + (size_t)hn[g0] * d.in_dim, dcoo + 2 * (size_t)he[g0],
-                                   gine ? def + (size_t)he[g0] * d.edge_dim : nullptr, dnp + g0, dep + g0, hn[g0], he[g0], g1 - g0, hn[g1] - hn[g0],
+                                   edges ? def + (size_t)he[g0] * d.edge_dim : nullptr, dnp + g0, dep + g0, hn[g0], he[g0], g1 - g0, hn[g1] - hn[g0],
                                    he[g1] - he[g0], dout + (size_t)g0 * d.mlp_out, s,
                                    &m->last_launches));
             g0 = g1;
@@ -1246,7 +1295,8 @@ extern "C" int gnnb_model_set_profile(gnnb_model_t *m, int on)
 }
 
 // Sum of CUDA-event durations (ms) and launch-group counts per kernel class since the last
-// call: [0] tables, [1] aggregation, [2] GEMM, [3] pooling, [4] fused.  Synchronises the stream.
+// call: [0] tables, [1] aggregation, [2] GEMM, [3] pooling, [4] fused, [5] GAT edge logits.
+// Synchronises the stream.
 extern "C" int gnnb_model_profile_read(gnnb_model_t *m, float *ms, int *counts)
 {
     GNNB_REQUIRE(m != nullptr && ms != nullptr && counts != nullptr, "null argument");

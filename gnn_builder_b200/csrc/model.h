@@ -30,7 +30,8 @@ struct LayerPack {
     PackedLinear e;           // GINE: the edge linear W_e^T [edge_dim][ldw], b_e
 };
 // GAT: a = [W | w_src | w_dst]^T, H*C + 2H columns and no bias (one GEMM gives h and both logits
-// of a row); b carries only the conv bias [H*C], which the aggregation epilogue adds
+// of a row); b carries only the conv bias [H*C], which the aggregation epilogue adds.  With edge_dim,
+// the edge linear folded with att_edge is one [L*H][edge_dim] table for all layers (gat_w_edge).
 
 // fused-kernel plans (fused.cu, fused_tc.cu)
 struct FusedPlan;
@@ -39,7 +40,7 @@ struct TcPlan;
 // Optional per-kernel-class timing with CUDA events on the launching stream (bench.py uses it
 // for the live roofline numbers).  Off by default: no events are recorded.
 enum ProfCat { PROF_TABLES = 0, PROF_AGG = 1, PROF_GEMM = 2, PROF_POOL = 3, PROF_FUSED = 4,
-               PROF_NCAT = 8 };
+               PROF_EDGE_LOGITS = 5, PROF_NCAT = 8 };
 struct Profiler {
     bool on = false;
     struct Rec { int cat; cudaEvent_t a, b; };
@@ -105,6 +106,10 @@ struct gnnb_model {
     gnnb::DeviceBuf in_deg, out_deg, offsets, nbr, nbr_hub, dinv, feat[2], agg, hid, wide, pooled,
         hbuf[2], pool_tmp, ptr_tmp;
     gnnb::DeviceBuf edge_index, ef_sorted;   // GINE: edge id and edge features per neighbor slot
+    // GAT with edge_dim: the edge logits of every layer and head per neighbor slot and per row
+    // (gat_edge_logits_kernel), and the folded edge weights [L*H][edge_dim] inside `weights`
+    gnnb::DeviceBuf elog, self_elog;
+    const float *gat_w_edge = nullptr;
     int last_hub_rows = 0;   // sources whose feature rows the last large-graph run kept L2-resident
     gnnb::TableWorkspace tws;
     gnnb::HeavyList heavy;       // rows above the heavy threshold of the current layerwise run
@@ -119,6 +124,8 @@ struct gnnb_model {
     int64_t last_emb_rows = 0;
 
     int emb_dim() const { return d.num_layers == 0 ? d.in_dim : d.out_dim; }
+    // GINE, and GAT with edge_dim: edge features come through the *_edges entry points
+    bool has_edge_features() const { return d.edge_dim > 0; }
     void layer_dims(int layer, int *fi, int *fo) const
     {
         if (d.num_layers == 1) { *fi = d.in_dim; *fo = d.out_dim; return; }

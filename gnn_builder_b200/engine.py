@@ -48,8 +48,9 @@ class Engine:
         self.desc = dict(desc)
         self.out_dim = int(desc["mlp_out"])
         self.in_dim = int(desc["in_dim"])
-        # GINE models take edge features and run through the *_edges entry points
-        self.edge_dim = int(desc.get("edge_dim", 0)) if int(desc["conv_type"]) == 4 else 0
+        # GINE models, and GAT models with edge_dim, take edge features and run through the
+        # *_edges entry points
+        self.edge_dim = int(desc.get("edge_dim", 0)) if int(desc["conv_type"]) in (4, 5) else 0
         self._h = C.c_void_p()
         self._pinned = {}
         s = _desc_struct(desc, max_nodes, max_edges)
@@ -104,6 +105,8 @@ class Engine:
         _lib.check(self.lib.gnnb_model_synchronize(self._h))
 
     PROFILE_CLASSES = ("tables", "aggregate", "gemm", "pool", "fused")
+    # the once-per-run edge-logit pass of GAT models with edge_dim: reported when it ran
+    EDGE_LOGITS_CLASS = 5
 
     def set_profile(self, on: bool):
         """per-kernel-class CUDA-event timing on the launching stream (off by default)"""
@@ -113,13 +116,17 @@ class Engine:
         ms = (C.c_float * 8)()
         cnt = (C.c_int * 8)()
         _lib.check(self.lib.gnnb_model_profile_read(self._h, ms, cnt))
-        return {k: dict(ms=float(ms[i]), count=int(cnt[i]))
+        prof = {k: dict(ms=float(ms[i]), count=int(cnt[i]))
                 for i, k in enumerate(self.PROFILE_CLASSES)}
+        i = self.EDGE_LOGITS_CLASS
+        if cnt[i]:
+            prof["edge_logits"] = dict(ms=float(ms[i]), count=int(cnt[i]))
+        return prof
 
     # ------------------------------------------------------------------ running
     def _host_edge_attr(self, edge_attr, n_edges: int):
         if edge_attr is None:
-            raise _lib.GnnbError("this GINE model needs edge_attr")
+            raise _lib.GnnbError("this model has edge features and needs edge_attr")
         ea = np.ascontiguousarray(edge_attr, np.float32)
         if ea.shape != (n_edges, self.edge_dim):
             raise _lib.GnnbError(f"edge_attr must be [{n_edges}, {self.edge_dim}], got {ea.shape}")
@@ -169,7 +176,8 @@ class Engine:
 
     def run_graph(self, x: np.ndarray, coo: np.ndarray,
                   edge_attr: Optional[np.ndarray] = None) -> np.ndarray:
-        """One graph, the exact data ``<name>_top`` receives (plus its edge features for GINE)."""
+        """One graph, the exact data ``<name>_top`` receives (plus its edge features for models
+        that have them)."""
         x = np.ascontiguousarray(x, np.float32)
         coo = np.ascontiguousarray(coo, np.int32).reshape(-1, 2)
         out = np.empty(self.out_dim, np.float32)
@@ -191,7 +199,7 @@ class Engine:
                    total_edges: int, stream: Optional[int] = None, sync: bool = False,
                    edge_attr=None):
         """torch CUDA tensors (or raw device pointers as ints); enqueues without synchronising.
-        GINE models take ``edge_attr`` [total_edges][edge_dim] on the device as well."""
+        Models with edge features take ``edge_attr`` [total_edges][edge_dim] on the device as well."""
         def p(a):
             if a is None:
                 return None

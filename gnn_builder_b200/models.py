@@ -96,23 +96,32 @@ class _GINEConv(nn.Module):
 
 class _GATConv(nn.Module):
     """PyG GATConv with an int ``in_channels``, concatenated heads and self loops, for inference.
-    Its own parameters come first in the flat order: ``att_src`` and ``att_dst`` [1][H][C], ``bias``
-    [H*C], then ``lin.weight`` [H*C][in] (no bias in ``lin``)."""
+    Its own parameters come first in the flat order: ``att_src`` and ``att_dst`` [1][H][C], with
+    ``edge_dim`` ``att_edge`` [1][H][C], ``bias`` [H*C], then ``lin.weight`` [H*C][in] (no bias in
+    ``lin``) and with ``edge_dim`` ``lin_edge.weight`` [H*C][edge_dim] -- PyG's registration order.
+    With edge features each self loop's attribute is the mean of the node's other in-edge
+    attributes (PyG's ``fill_value="mean"``), the zero vector for a node without one."""
 
-    def __init__(self, in_channels: int, out_channels: int, heads: int, negative_slope: float):
+    def __init__(self, in_channels: int, out_channels: int, heads: int, negative_slope: float,
+                 edge_dim: Optional[int] = None):
         super().__init__()
         self.heads = heads
         self.head_channels = out_channels // heads
         self.negative_slope = negative_slope
+        self.edge_dim = edge_dim
         self.lin = nn.Linear(in_channels, out_channels, bias=False)
         self.att_src = nn.Parameter(torch.empty(1, heads, self.head_channels))
         self.att_dst = nn.Parameter(torch.empty(1, heads, self.head_channels))
+        if edge_dim is not None:
+            self.lin_edge = nn.Linear(edge_dim, out_channels, bias=False)
+            self.att_edge = nn.Parameter(torch.empty(1, heads, self.head_channels))
+            nn.init.xavier_uniform_(self.att_edge)
         self.bias = nn.Parameter(torch.zeros(out_channels))
         nn.init.xavier_uniform_(self.att_src)
         nn.init.xavier_uniform_(self.att_dst)
         nn.init.uniform_(self.bias, -0.1, 0.1)
 
-    def forward(self, x: Tensor, edge_index: Tensor) -> Tensor:
+    def forward(self, x: Tensor, edge_index: Tensor, edge_attr: Optional[Tensor] = None) -> Tensor:
         n, H, C = x.shape[0], self.heads, self.head_channels
         # every self loop of the input is replaced by exactly one per node; duplicates stay
         keep = edge_index[0] != edge_index[1]
@@ -122,7 +131,13 @@ class _GATConv(nn.Module):
         h = self.lin(x).view(n, H, C)
         a_src = (h * self.att_src).sum(-1)
         a_dst = (h * self.att_dst).sum(-1)
-        e = torch.nn.functional.leaky_relu(a_src[src] + a_dst[dst], self.negative_slope)
+        logit = a_src[src] + a_dst[dst]
+        if self.edge_dim is not None:
+            ea = edge_attr.reshape(-1, self.edge_dim)[keep]
+            cnt = _in_degree(edge_index[:, keep], n).clamp(min=1.0).view(-1, 1)
+            ea = torch.cat([ea, _scatter_sum(ea, edge_index[1][keep], n) / cnt])
+            logit = logit + (self.lin_edge(ea).view(-1, H, C) * self.att_edge).sum(-1)
+        e = torch.nn.functional.leaky_relu(logit, self.negative_slope)
         p = (e - _scatter_minmax(e, dst, n, "amax")[dst]).exp()
         alpha = p / _scatter_sum(p, dst, n)[dst]
         msg = (h[src] * alpha.unsqueeze(-1)).reshape(-1, H * C)
@@ -261,13 +276,21 @@ class GATConv_GNNB(nn.Module):
     """Graph attention (PyG ``GATConv``, inference): per head, h = x W^T, logits
     e_uv = LeakyReLU(<h_u, att_src> + <h_v, att_dst>) over the in-edges of v plus one self loop,
     y_v = sum softmax_v(e) h_u + bias, heads concatenated.  ``out_channels`` is the concatenated
-    width and must be a multiple of ``heads``.  Pass ``heads`` with ``functools.partial``."""
+    width and must be a multiple of ``heads``.  Pass ``heads`` with ``functools.partial``.
+
+    ``edge_dim`` (a positive int, also passed with ``functools.partial``) adds PyG's edge term to
+    every logit: + <(e_uv W_e^T)_h, att_edge_h>, where the self loop's e_vv is the mean of v's other
+    in-edge attributes.  The model's ``graph_input_edge_dim`` must then equal it."""
 
     def __init__(self, in_channels: int, out_channels: int, heads: int = 1,
-                 negative_slope: float = 0.2, p_in: int = 1, p_out: int = 1):
+                 negative_slope: float = 0.2, edge_dim: Optional[int] = None, p_in: int = 1,
+                 p_out: int = 1):
         super().__init__()
         if not isinstance(heads, int) or isinstance(heads, bool) or heads < 1:
             raise ValueError(f"heads must be a positive int, got {heads!r}")
+        if edge_dim is not None and (not isinstance(edge_dim, int) or isinstance(edge_dim, bool)
+                                     or edge_dim < 1):
+            raise ValueError(f"edge_dim must be None or a positive int, got {edge_dim!r}")
         if out_channels % heads != 0:
             raise ValueError(f"out_channels ({out_channels}) must be a multiple of heads ({heads})")
         if not math.isfinite(negative_slope):
@@ -276,12 +299,15 @@ class GATConv_GNNB(nn.Module):
         self.out_channels = out_channels
         self.heads = heads
         self.negative_slope = float(negative_slope)
+        self.edge_dim = edge_dim
         self.p_in = p_in
         self.p_out = p_out
-        self.conv = _GATConv(in_channels, out_channels, heads, self.negative_slope)
+        self.conv = _GATConv(in_channels, out_channels, heads, self.negative_slope, edge_dim)
 
-    def forward(self, x: Tensor, edge_index: Tensor) -> Tensor:
-        return self.conv(x, edge_index)
+    def forward(self, x: Tensor, edge_index: Tensor, edge_attr: Optional[Tensor] = None) -> Tensor:
+        if self.edge_dim is not None and edge_attr is None:
+            raise ValueError("a GATConv_GNNB with edge_dim needs edge_attr")
+        return self.conv(x, edge_index, edge_attr)
 
 
 class PNAConv_GNNB(nn.Module):
@@ -453,14 +479,24 @@ class GNNModel(nn.Module):
         conv_cls = getattr(gnn_conv, "func", gnn_conv)  # allow functools.partial(delta=..)
         if conv_cls not in SUPPORTED_GNN_CONVS:
             raise ValueError(f"gnn_conv must be one of {SUPPORTED_GNN_CONVS}")
-        self.uses_edge_features = conv_cls is GINEConv_GNNB
+        self._conv_cls = conv_cls
+        # GAT takes edge features only when its partial carries edge_dim
+        self._conv_kwargs = dict(getattr(gnn_conv, "keywords", None) or {})
+        gat_edge_dim = (self._conv_kwargs.get("edge_dim") if conv_cls is GATConv_GNNB else None)
+        self.uses_edge_features = conv_cls is GINEConv_GNNB or gat_edge_dim is not None
         conv_kwargs = {}
-        if self.uses_edge_features:
+        if conv_cls is GINEConv_GNNB:
             e = graph_input_edge_dim
             if not isinstance(e, int) or isinstance(e, bool) or e < 1:
                 raise ValueError("GINEConv_GNNB needs graph_input_edge_dim to be a positive int, "
                                  f"got {e!r}")
             conv_kwargs["edge_dim"] = e
+        elif gat_edge_dim is not None:
+            e = graph_input_edge_dim
+            for v in (gat_edge_dim, e):
+                if not isinstance(v, int) or isinstance(v, bool) or v < 1 or v != gat_edge_dim:
+                    raise ValueError(f"GATConv_GNNB with edge_dim={gat_edge_dim!r} needs a positive "
+                                     f"int edge_dim and graph_input_edge_dim equal to it, got {e!r}")
         self.gnn_activation = gnn_activation
         if self.gnn_activation not in SUPPORTED_ACTIVATIONS:
             raise ValueError(f"gnn_activation must be one of {SUPPORTED_ACTIVATIONS}")
@@ -503,7 +539,7 @@ class GNNModel(nn.Module):
     def forward(self, x: Tensor, edge_index: Tensor, batch: Optional[Tensor] = None,
                 edge_attr: Optional[Tensor] = None) -> Tensor:
         if self.uses_edge_features and self.gnn_num_layers > 0 and edge_attr is None:
-            raise ValueError("a GINEConv_GNNB model needs edge_attr")
+            raise ValueError(f"a {self._conv_cls.__name__} model with edge features needs edge_attr")
         x_gnn = x
         for i, (conv, act) in enumerate(zip(self.gnn_convs, self.gnn_activations)):
             x_in = x_gnn
@@ -581,7 +617,7 @@ class GNNModel(nn.Module):
         conv0 = self.gnn_convs[0] if self.gnn_num_layers > 0 else None
         conv_name = conv0.__class__.__name__ if conv0 is not None else "GCNConv_GNNB"
         if self.uses_edge_features:
-            conv_name = "GINEConv_GNNB"
+            conv_name = self._conv_cls.__name__
         d = dict(
             conv_type=CONV_TYPE_IDS[conv_name],
             num_layers=self.gnn_num_layers,
@@ -603,8 +639,10 @@ class GNNModel(nn.Module):
         if self.uses_edge_features:
             d["edge_dim"] = int(self.graph_input_edge_dim)
         if conv_name == "GATConv_GNNB":
-            d["gat_heads"] = int(conv0.heads)
-            d["gat_negative_slope"] = float(conv0.negative_slope)
+            kw = self._conv_kwargs   # a model without layers has no conv to ask
+            d["gat_heads"] = int(conv0.heads if conv0 is not None else kw.get("heads", 1))
+            d["gat_negative_slope"] = float(conv0.negative_slope if conv0 is not None
+                                            else kw.get("negative_slope", 0.2))
         return d
 
 

@@ -43,15 +43,18 @@ enum {
 };
 /* GINE (GIN with an edge linear, PyG GINEConv with edge_dim; lib:1555-1742) runs on the layerwise
  * path only and takes its edge features through the gnnb_model_run_batch_edges* entry points */
-/* GAT (PyG GATConv for inference: concat heads, self loops replaced by one per node, no edge
- * features) runs on the layerwise path only, through the plain run entry points.  It has no
- * reference float build: GNNB_MATH_STRICT means deterministic fp32 without tensor cores for it,
- * held to the same error bound as FAST. */
+/* GAT (PyG GATConv for inference: concat heads, self loops replaced by one per node) runs on the
+ * layerwise path only.  Without edge features (edge_dim = 0) it runs through the plain run entry
+ * points; with edge_dim > 0 (GATConv's edge_dim: lin_edge and att_edge add an edge term to every
+ * attention logit, and the self loop's attribute is the mean of the node's other in-edge
+ * attributes) through the gnnb_model_run_batch_edges* ones.  It has no reference float build:
+ * GNNB_MATH_STRICT means deterministic fp32 without tensor cores for it, held to the same error
+ * bound as FAST. */
 enum {
     GNNB_CONV_GCN = 0, GNNB_CONV_GIN = 1, GNNB_CONV_SAGE = 2, GNNB_CONV_PNA = 3, GNNB_CONV_GINE = 4,
     GNNB_CONV_GAT = 5
 };
-/* edge feature widths a GINE model handle accepts */
+/* edge feature widths a GINE or edge-attention GAT model handle accepts */
 #define GNNB_GINE_MAX_EDGE_DIM 64
 /* attention head counts a GAT model handle accepts */
 #define GNNB_GAT_MAX_HEADS 16
@@ -91,9 +94,12 @@ typedef struct gnnb_model_desc {
     int32_t out_act;        /* output_activation, 0 = None */
     int32_t max_nodes;      /* capacity hints (Project.max_nodes/max_edges, code_gen.py:71-72); */
     int32_t max_edges;      /* 0 = unbounded.  A graph larger than a non-zero hint is an error. */
-    int32_t edge_dim;       /* GINE only: edge feature width, 1..GNNB_GINE_MAX_EDGE_DIM.  Last field,
-                               read only when conv_type == GNNB_CONV_GINE, so a caller built
-                               against a header without it keeps working for the other convs. */
+    int32_t edge_dim;       /* GINE: edge feature width, 1..GNNB_GINE_MAX_EDGE_DIM.  GAT: 0 for no
+                               edge features, else 1..GNNB_GINE_MAX_EDGE_DIM (edge attention), so
+                               C callers of GAT must set it to 0 for plain GAT (zero-initialising
+                               the struct does).  Read only when conv_type is GNNB_CONV_GINE or
+                               GNNB_CONV_GAT, so a caller built against a header without it keeps
+                               working for the other convs. */
     int32_t gat_heads;      /* GAT only: heads H, 1..GNNB_GAT_MAX_HEADS; every layer's output width
                                must be a multiple of H (C = width / H channels per head) */
     float gat_negative_slope;  /* GAT only: LeakyReLU slope of the attention logits (PyG: 0.2).
@@ -149,11 +155,11 @@ int gnnb_model_run_batch(gnnb_model_t *m, const float *x, const int32_t *edge_li
 int gnnb_model_run_batch_async(gnnb_model_t *m, const float *x, const int32_t *edge_list,
                                const int64_t *node_ptr, const int64_t *edge_ptr, int n_graphs,
                                int64_t total_nodes, int64_t total_edges, float *out, void *stream);
-/* GINE models: the same contracts as gnnb_model_run_batch / gnnb_model_run_batch_async, plus
- * edge_attr float [edge_ptr[G]][edge_dim] in the memory space of the other buffers, row i the
- * features of COO edge i (one row per stored direction).  A GINE handle must be run through these
- * two; a handle of another conv type is rejected by them (GNNB_ERR_INVALID), and so is a null
- * edge_attr with edges present. */
+/* GINE models and GAT models with edge_dim > 0: the same contracts as gnnb_model_run_batch /
+ * gnnb_model_run_batch_async, plus edge_attr float [edge_ptr[G]][edge_dim] in the memory space of
+ * the other buffers, row i the features of COO edge i (one row per stored direction).  Such a handle
+ * must be run through these two; a handle without edge features is rejected by them
+ * (GNNB_ERR_INVALID), and so is a null edge_attr with edges present. */
 int gnnb_model_run_batch_edges(gnnb_model_t *m, const float *x, const int32_t *edge_list,
                                const float *edge_attr, const int64_t *node_ptr,
                                const int64_t *edge_ptr, int n_graphs, float *out);
@@ -170,7 +176,8 @@ int gnnb_model_last_path(const gnnb_model_t *m);
 /* which kernel family ran: 1 layerwise, 2 fused (fp32 FMA node transform), 3 fused (tcgen05) */
 int gnnb_model_last_kernel(const gnnb_model_t *m);
 /* optional per-kernel-class timing with CUDA events on the launching stream: ms[8]/counts[8]
- * indexed 0 tables, 1 aggregation, 2 GEMM, 3 pooling, 4 fused kernel; reading resets */
+ * indexed 0 tables, 1 aggregation, 2 GEMM, 3 pooling, 4 fused kernel, 5 GAT edge logits (the
+ * once-per-run pass of GAT models with edge_dim); reading resets */
 int gnnb_model_set_profile(gnnb_model_t *m, int on);
 int gnnb_model_profile_read(gnnb_model_t *m, float *ms, int *counts);
 void *gnnb_model_stream(gnnb_model_t *m);
