@@ -11,8 +11,9 @@ from .data import (GraphBatch, cached_powerlaw_graph, make_molecular_batch,  # n
                    make_powerlaw_graph)
 from .engine import (MATH_FAST, MATH_STRICT, PATH_AUTO, PATH_FUSED, PATH_LAYERWISE,  # noqa: F401
                      Engine)
-from .models import (MLP, GATConv_GNNB, GCNConv_GNNB, GINConv_GNNB, GINEConv_GNNB,  # noqa: F401
-                     GlobalPooling, GNNModel, PNAConv_GNNB, SAGEConv_GNNB, build_model)
+from .models import (MLP, GATConv_GNNB, GATv2Conv_GNNB, GCNConv_GNNB, GINConv_GNNB,  # noqa: F401
+                     GINEConv_GNNB, GlobalPooling, GNNModel, PNAConv_GNNB, SAGEConv_GNNB,
+                     build_model)
 from .utils import (compute_average_degree, compute_average_nodes_and_edges,  # noqa: F401
                     compute_in_deg_histogram, compute_max_nodes_and_edges,
                     compute_median_degree, compute_median_nodes_and_edges)

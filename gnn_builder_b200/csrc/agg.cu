@@ -1327,4 +1327,497 @@ int launch_gat_edge_logits(const GatEdgeLogitsArgs &a, int avg_deg, cudaStream_t
     return GNNB_OK;
 }
 
+// ----------------------------------------------------------------------------------- GATv2
+//
+// PyG GATv2Conv (concat heads, self loops replaced by one per node, inference).  The layer's two
+// GEMMs wrote [xl | xr] per row.  The logit e_uvh = <att_h, LeakyReLU(xl_u + xr_v (+ e_uv W_e^T))_h>
+// has its nonlinearity inside the dot product, so it is formed per edge from the gathered row: each
+// lane holds xr_v and att for its columns in registers, forms its partial dot product and the head's
+// lanes add the partials with an xor butterfly.  A butterfly gives every lane of the head the same
+// bits (each level adds the same two values, commutatively), so their online-softmax states stay
+// identical.
+//
+// Lane layout: a head's columns are spread over G lanes, G the smallest power of two >= C / VEC
+// (at most 32), each lane holding NJ <= 2 groups of VEC columns; the G-lane groups are aligned inside
+// the row's LPR-lane sub-warp and a sub-warp covers LPR / G heads per pass.  Lanes past C, and the
+// groups of a pass past the last head, contribute 0 but run the same shuffles: every shuffle's mask
+// is the row's sub-warp, whose lanes all reach it (rows of one warp differ in degree).
+//
+// The online softmax, the self term first and the skipping of entries equal to v are GAT's.  With
+// edge features each edge's projection is computed where it is consumed from ef_sorted[slot] and
+// W_e^T (staged in shared memory when it fits), never materialised.  Heavy rows are GAT's chunk /
+// fixed-order combine scheme.  The kernels declare one resident CTA per SM as their minimum: ptxas's
+// own register choice under __launch_bounds__(256) spilled them.  Algorithmic bytes per layer:
+// E (4 + 4HC [+ 4 lde]) + N (8 + 8HC + 4HC [+ 4HC skip] [+ 4 lde]).
+namespace {
+
+template <int VEC, int NJ>
+struct Gatv2State {
+    float m, s;
+    float acc[NJ][VEC];
+    __device__ __forceinline__ void reset()
+    {
+        m = -INFINITY;
+        s = 0.0f;
+#pragma unroll
+        for (int j = 0; j < NJ; j++)
+#pragma unroll
+            for (int i = 0; i < VEC; i++) acc[j][i] = 0.0f;
+    }
+    // OnlineSoftmax::merge over the lane's NJ column groups
+    __device__ __forceinline__ void merge(float m2, float s2, const float (&acc2)[NJ][VEC])
+    {
+        if (m2 == -INFINITY) return;
+        const float mn = fmaxf(m, m2);
+        const float r = expf(m - mn), p = expf(m2 - mn);
+        s = fmaf(s, r, s2 * p);
+#pragma unroll
+        for (int j = 0; j < NJ; j++)
+#pragma unroll
+            for (int i = 0; i < VEC; i++) acc[j][i] = fmaf(acc[j][i], r, acc2[j][i] * p);
+        m = mn;
+    }
+};
+
+// one lane's share of one head: columns col[j] .. col[j] + VEC of the head (valid[j]), xr_v and att
+template <int VEC, int NJ>
+struct Gatv2Lane {
+    int hd;
+    int col[NJ];
+    bool valid[NJ];
+    float xr[NJ][VEC], att[NJ][VEC];
+};
+
+template <int VEC, int NJ>
+__device__ __forceinline__ void gatv2_load(const float *row, const Gatv2Lane<VEC, NJ> &ln,
+                                           float (&x)[NJ][VEC])
+{
+#pragma unroll
+    for (int j = 0; j < NJ; j++) {
+        Vec<VEC> t;
+        if (ln.valid[j]) t.load(row + ln.col[j]);
+        else {
+#pragma unroll
+            for (int i = 0; i < VEC; i++) t.v[i] = 0.0f;
+        }
+#pragma unroll
+        for (int i = 0; i < VEC; i++) x[j][i] = t.v[i];
+    }
+}
+
+// head hd (>= H: an idle group), lane hl of its G lanes
+template <int VEC, int NJ>
+__device__ __forceinline__ Gatv2Lane<VEC, NJ> gatv2_lane(const Gatv2AggArgs &a, int v, int hd, int hl,
+                                                         int G)
+{
+    Gatv2Lane<VEC, NJ> ln;
+    ln.hd = hd;
+#pragma unroll
+    for (int j = 0; j < NJ; j++) {
+        const int cl = (hl + j * G) * VEC;
+        ln.valid[j] = hd < a.H && cl < a.C;
+        ln.col[j] = hd * a.C + cl;
+    }
+    const int HC = a.H * a.C;
+    Gatv2Lane<VEC, NJ> sh = ln;   // the same columns, shifted to xr
+#pragma unroll
+    for (int j = 0; j < NJ; j++) sh.col[j] += HC;
+    gatv2_load<VEC, NJ>(a.xlr + (size_t)v * a.ldg, sh, ln.xr);
+    gatv2_load<VEC, NJ>(a.att, ln, ln.att);
+    return ln;
+}
+
+// z += ef W_e^T for the lane's columns: ef one row of lde floats (edge_dim used), We [edge_dim][ldw]
+template <int VEC, int NJ>
+__device__ __forceinline__ void gatv2_edge_proj(const Gatv2AggArgs &a, const float *We, const float *ef,
+                                                const Gatv2Lane<VEC, NJ> &ln, float (&z)[NJ][VEC])
+{
+    for (int j0 = 0; j0 < a.edge_dim; j0 += 4) {
+        const float4 e4 = __ldg(reinterpret_cast<const float4 *>(ef + j0));
+#pragma unroll
+        for (int jj = 0; jj < 4; jj++) {
+            if (j0 + jj < a.edge_dim) {
+                const float ej = jj == 0 ? e4.x : jj == 1 ? e4.y : jj == 2 ? e4.z : e4.w;
+                const float *wr = We + (size_t)(j0 + jj) * a.ldw;
+#pragma unroll
+                for (int j = 0; j < NJ; j++) {
+                    if (!ln.valid[j]) continue;
+#pragma unroll
+                    for (int i = 0; i < VEC; i++) z[j][i] = fmaf(wr[ln.col[j] + i], ej, z[j][i]);
+                }
+            }
+        }
+    }
+}
+
+// the lane's partial dot product <att, LeakyReLU(xl + xr + ep)> (columns past C hold att = 0)
+template <int VEC, int NJ>
+__device__ __forceinline__ float gatv2_partial(const Gatv2AggArgs &a, const Gatv2Lane<VEC, NJ> &ln,
+                                               const float (&xl)[NJ][VEC], const float (&ep)[NJ][VEC])
+{
+    float part = 0.0f;
+#pragma unroll
+    for (int j = 0; j < NJ; j++)
+#pragma unroll
+        for (int i = 0; i < VEC; i++)
+            part = fmaf(ln.att[j][i], leaky_relu(xl[j][i] + ln.xr[j][i] + ep[j][i], a.slope), part);
+    return part;
+}
+
+__device__ __forceinline__ float gatv2_head_sum(float part, unsigned mask, int G)
+{
+    for (int o = G >> 1; o > 0; o >>= 1) part += __shfl_xor_sync(mask, part, o);
+    return part;
+}
+
+// the self term of row v: logit from xl_v + xr_v (+ self_attr_v W_e^T), weight 1, message xl_v
+template <int VEC, int NJ, bool EDGE>
+__device__ __forceinline__ void gatv2_self(const Gatv2AggArgs &a, const float *We, int v,
+                                           const Gatv2Lane<VEC, NJ> &ln, unsigned mask, int G,
+                                           Gatv2State<VEC, NJ> &st)
+{
+    float xl[NJ][VEC], ep[NJ][VEC];
+    gatv2_load<VEC, NJ>(a.xlr + (size_t)v * a.ldg, ln, xl);
+#pragma unroll
+    for (int j = 0; j < NJ; j++)
+#pragma unroll
+        for (int i = 0; i < VEC; i++) ep[j][i] = 0.0f;
+    if (EDGE) gatv2_edge_proj<VEC, NJ>(a, We, a.self_attr + (size_t)v * a.lde, ln, ep);
+    st.m = gatv2_head_sum(gatv2_partial<VEC, NJ>(a, ln, xl, ep), mask, G);
+    st.s = 1.0f;
+#pragma unroll
+    for (int j = 0; j < NJ; j++)
+#pragma unroll
+        for (int i = 0; i < VEC; i++) st.acc[j][i] = xl[j][i];
+}
+
+// neighbor slots [k0, k1) of row v (entries equal to v skipped, uniformly over the sub-warp), U
+// gathers in flight
+template <int VEC, int NJ, bool EDGE>
+__device__ __forceinline__ void gatv2_gather(const Gatv2AggArgs &a, const float *We, int v, int off,
+                                             int k0, int k1, const Gatv2Lane<VEC, NJ> &ln,
+                                             unsigned mask, int G, Gatv2State<VEC, NJ> &st)
+{
+    constexpr int U = NJ == 1 ? 4 : 2;
+    int k = k0;
+#pragma unroll 1
+    for (; k + U <= k1; k += U) {
+        int u[U];
+        float xl[U][NJ][VEC], ep[U][NJ][VEC], e[U];
+#pragma unroll
+        for (int q = 0; q < U; q++) u[q] = __ldg(a.nbr + off + k + q);
+#pragma unroll
+        for (int q = 0; q < U; q++) gatv2_load<VEC, NJ>(a.xlr + (size_t)u[q] * a.ldg, ln, xl[q]);
+#pragma unroll
+        for (int q = 0; q < U; q++) {
+#pragma unroll
+            for (int j = 0; j < NJ; j++)
+#pragma unroll
+                for (int i = 0; i < VEC; i++) ep[q][j][i] = 0.0f;
+            if (EDGE) gatv2_edge_proj<VEC, NJ>(a, We, a.ef_sorted + (size_t)(off + k + q) * a.lde, ln, ep[q]);
+            e[q] = gatv2_partial<VEC, NJ>(a, ln, xl[q], ep[q]);
+        }
+        for (int o = G >> 1; o > 0; o >>= 1)
+#pragma unroll
+            for (int q = 0; q < U; q++) e[q] += __shfl_xor_sync(mask, e[q], o);
+#pragma unroll
+        for (int q = 0; q < U; q++)
+            if (u[q] != v) st.merge(e[q], 1.0f, xl[q]);
+    }
+#pragma unroll 1
+    for (; k < k1; k++) {
+        const int u = __ldg(a.nbr + off + k);
+        if (u == v) continue;
+        float xl[NJ][VEC], ep[NJ][VEC];
+        gatv2_load<VEC, NJ>(a.xlr + (size_t)u * a.ldg, ln, xl);
+#pragma unroll
+        for (int j = 0; j < NJ; j++)
+#pragma unroll
+            for (int i = 0; i < VEC; i++) ep[j][i] = 0.0f;
+        if (EDGE) gatv2_edge_proj<VEC, NJ>(a, We, a.ef_sorted + (size_t)(off + k) * a.lde, ln, ep);
+        st.merge(gatv2_head_sum(gatv2_partial<VEC, NJ>(a, ln, xl, ep), mask, G), 1.0f, xl);
+    }
+}
+
+template <int VEC, int NJ>
+__device__ __forceinline__ void gatv2_finish(const Gatv2AggArgs &a, int v, const Gatv2Lane<VEC, NJ> &ln,
+                                             const Gatv2State<VEC, NJ> &st)
+{
+#pragma unroll
+    for (int j = 0; j < NJ; j++) {
+        if (!ln.valid[j]) continue;
+        const int c = ln.col[j];
+        Vec<VEC> b, sk, y;
+        b.load(a.bias + c);
+        if (a.skip != nullptr) sk.load(a.skip + (size_t)v * a.ldskip + c);
+#pragma unroll
+        for (int i = 0; i < VEC; i++) {
+            float t = st.acc[j][i] / st.s + b.v[i];
+            if (a.skip != nullptr) t += sk.v[i];
+            y.v[i] = act_apply_compact(a.act, t);
+        }
+        y.store(a.out + (size_t)v * a.ldo + c);
+    }
+}
+
+// W_e^T staged in shared memory (w_smem) or read in place
+__device__ __forceinline__ const float *gatv2_stage_we(const Gatv2AggArgs &a, bool w_smem)
+{
+    extern __shared__ float4 gatv2_smem4[];
+    if (!w_smem) return a.We_t;
+    float *sw = reinterpret_cast<float *>(gatv2_smem4);
+    const int nw = a.edge_dim * a.ldw;
+    for (int i = threadIdx.x; i < nw; i += blockDim.x) sw[i] = __ldg(a.We_t + i);
+    __syncthreads();
+    return sw;
+}
+
+// lpr lanes per destination row (a power of two, a multiple of G); G lanes per head
+template <int VEC, int NJ, bool EDGE>
+__global__ void __launch_bounds__(256, 1) gatv2_agg_kernel(const Gatv2AggArgs a, int lpr, int G, bool w_smem)
+{
+    const float *We = EDGE ? gatv2_stage_we(a, w_smem) : nullptr;
+    const int rows_per_warp = 32 / lpr;
+    const int lane = threadIdx.x & 31;
+    const int lg = lane % lpr, sub = lane / lpr;
+    const unsigned mask = lpr == 32 ? 0xffffffffu : ((1u << lpr) - 1u) << (sub * lpr);
+    const int grp = lg / G, hl = lg % G, heads_per_pass = lpr / G;
+    const int warps_per_block = blockDim.x >> 5;
+    const int64_t warp_global = (int64_t)blockIdx.x * warps_per_block + (threadIdx.x >> 5);
+    const int64_t warp_stride = (int64_t)gridDim.x * warps_per_block;
+    for (int64_t row0 = warp_global * rows_per_warp; row0 < a.n; row0 += warp_stride * rows_per_warp) {
+        // everything below is uniform over the row's sub-warp, so all its lanes reach every shuffle
+        const int v = (int)row0 + sub;
+        if (v >= a.n) continue;
+        const int deg = __ldg(a.in_deg + v);
+        if (a.n_heavy > 0 && deg > a.heavy_threshold) continue;  // the heavy-row kernels do these
+        const int off = __ldg(a.offsets + v);
+        for (int h0 = 0; h0 < a.H; h0 += heads_per_pass) {
+            const Gatv2Lane<VEC, NJ> ln = gatv2_lane<VEC, NJ>(a, v, h0 + grp, hl, G);
+            Gatv2State<VEC, NJ> st;
+            gatv2_self<VEC, NJ, EDGE>(a, We, v, ln, mask, G, st);
+            gatv2_gather<VEC, NJ, EDGE>(a, We, v, off, 0, deg, ln, mask, G, st);
+            if (ln.hd < a.H) gatv2_finish<VEC, NJ>(a, v, ln, st);
+        }
+    }
+}
+
+// one warp per kHeavyChunk-neighbor chunk of a heavy row: the chunk's per-head (m, s) and its
+// accumulator, as GAT's chunk kernel
+template <int VEC, int NJ, bool EDGE>
+__global__ void __launch_bounds__(256, 1) gatv2_heavy_chunk_kernel(const Gatv2AggArgs a, int G)
+{
+    const int lane = threadIdx.x & 31;
+    const int grp = lane / G, hl = lane % G, heads_per_pass = 32 / G;
+    const int warps_per_block = blockDim.x >> 5;
+    const int warp_global = blockIdx.x * warps_per_block + (threadIdx.x >> 5);
+    const int warp_stride = gridDim.x * warps_per_block;
+    const int HC = a.H * a.C;
+    for (int chunk = warp_global; chunk < a.heavy_chunks; chunk += warp_stride) {
+        const int h = __ldg(a.heavy_chunk_row + chunk);
+        const int v = __ldg(a.heavy_rows + h);
+        const int j = chunk - __ldg(a.heavy_chunk_base + h);
+        const int deg = __ldg(a.in_deg + v);
+        const int off = __ldg(a.offsets + v);
+        const int k0 = j * kHeavyChunk, k1 = min(deg, k0 + kHeavyChunk);
+        float *dst = a.heavy_partial + (size_t)chunk * a.ldp;
+        for (int h0 = 0; h0 < a.H; h0 += heads_per_pass) {
+            const Gatv2Lane<VEC, NJ> ln = gatv2_lane<VEC, NJ>(a, v, h0 + grp, hl, G);
+            Gatv2State<VEC, NJ> st;
+            st.reset();
+            gatv2_gather<VEC, NJ, EDGE>(a, a.We_t, v, off, k0, k1, ln, 0xffffffffu, G, st);
+#pragma unroll
+            for (int q = 0; q < NJ; q++) {
+                if (!ln.valid[q]) continue;
+#pragma unroll
+                for (int i = 0; i < VEC; i++) dst[ln.col[q] + i] = st.acc[q][i];
+            }
+            if (hl == 0 && ln.hd < a.H) {   // one lane per head
+                dst[HC + ln.hd] = st.m;
+                dst[HC + a.H + ln.hd] = st.s;
+            }
+        }
+    }
+}
+
+// one CTA per heavy row: 8 warps merge contiguous chunk ranges column by column, then warp 0 starts
+// from the self term and merges the 8 range results in warp order (a fixed order)
+template <int VEC, int NJ, bool EDGE>
+__global__ void __launch_bounds__(256, 1) gatv2_heavy_combine_kernel(const Gatv2AggArgs a, int G)
+{
+    extern __shared__ float4 gatv2_comb_smem4[];
+    float *const ranges = reinterpret_cast<float *>(gatv2_comb_smem4);   // [8][ldp], as the partials
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int HC = a.H * a.C;
+    const int grp = lane / G, hl = lane % G, heads_per_pass = 32 / G;
+    for (int h = blockIdx.x; h < a.n_heavy; h += gridDim.x) {
+        const int v = __ldg(a.heavy_rows + h);
+        const int deg = __ldg(a.in_deg + v);
+        const int nch = (deg + kHeavyChunk - 1) / kHeavyChunk;
+        const float *src = a.heavy_partial + (size_t)__ldg(a.heavy_chunk_base + h) * a.ldp;
+        const int per = (nch + 7) / 8;
+        const int j0 = min(nch, warp * per), j1 = min(nch, j0 + per);
+        float *mine = ranges + warp * a.ldp;
+        for (int c = lane * VEC; c < HC; c += 32 * VEC) {
+            const int hd = c / a.C;
+            Gatv2State<VEC, 1> st;
+            st.reset();
+            for (int j = j0; j < j1; j++) {
+                const float *p = src + (size_t)j * a.ldp;
+                Vec<VEC> t;
+                t.load_rw(p + c);
+                float t2[1][VEC];
+#pragma unroll
+                for (int i = 0; i < VEC; i++) t2[0][i] = t.v[i];
+                st.merge(p[HC + hd], p[HC + a.H + hd], t2);
+            }
+#pragma unroll
+            for (int i = 0; i < VEC; i++) mine[c + i] = st.acc[0][i];
+            if (c % a.C == 0) {
+                mine[HC + hd] = st.m;
+                mine[HC + a.H + hd] = st.s;
+            }
+        }
+        __syncthreads();
+        if (warp == 0) {
+            for (int h0 = 0; h0 < a.H; h0 += heads_per_pass) {
+                const Gatv2Lane<VEC, NJ> ln = gatv2_lane<VEC, NJ>(a, v, h0 + grp, hl, G);
+                Gatv2State<VEC, NJ> st;
+                gatv2_self<VEC, NJ, EDGE>(a, a.We_t, v, ln, 0xffffffffu, G, st);
+                const int hd = ln.hd < a.H ? ln.hd : 0;
+#pragma unroll 1
+                for (int w = 0; w < 8; w++) {
+                    const float *r = ranges + w * a.ldp;
+                    float t[NJ][VEC];
+#pragma unroll
+                    for (int q = 0; q < NJ; q++)
+#pragma unroll
+                        for (int i = 0; i < VEC; i++) t[q][i] = ln.valid[q] ? r[ln.col[q] + i] : 0.0f;
+                    st.merge(r[HC + hd], r[HC + a.H + hd], t);
+                }
+                if (ln.hd < a.H) gatv2_finish<VEC, NJ>(a, v, ln, st);
+            }
+        }
+        __syncthreads();
+    }
+}
+
+template <int VEC, int NJ, bool EDGE>
+int launch_gatv2_variant(const Gatv2AggArgs &a, int lpr, int G, int grid, size_t smem, cudaStream_t s,
+                         int *launches)
+{
+    auto k = gatv2_agg_kernel<VEC, NJ, EDGE>;
+    if (smem > 48 * 1024) GNNB_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k<<<grid, 256, smem, s>>>(a, lpr, G, smem > 0);
+    GNNB_CUDA(cudaGetLastError());
+    if (launches) ++*launches;
+    if (a.n_heavy > 0) {
+        const int cap = kNumSMs * 8;   // 8 resident CTAs per SM, grid-stride beyond
+        const int g1 = min((a.heavy_chunks + 7) / 8, cap), g2 = min(a.n_heavy, cap);
+        gatv2_heavy_chunk_kernel<VEC, NJ, EDGE><<<g1, 256, 0, s>>>(a, G);
+        const size_t csmem = sizeof(float) * 8 * (size_t)a.ldp;
+        auto combine = gatv2_heavy_combine_kernel<VEC, NJ, EDGE>;
+        if (csmem > 48 * 1024)
+            GNNB_CUDA(cudaFuncSetAttribute(combine, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)csmem));
+        combine<<<g2, 256, csmem, s>>>(a, G);
+        GNNB_CUDA(cudaGetLastError());
+        if (launches) *launches += 2;
+    }
+    return GNNB_OK;
+}
+
+__global__ void gatv2_self_attr_kernel(const float *__restrict__ ef, int lde, int edge_dim,
+                                       const int32_t *__restrict__ offsets,
+                                       const int32_t *__restrict__ nbr,
+                                       const int32_t *__restrict__ in_deg, int n,
+                                       float *__restrict__ self_attr)
+{
+    const int64_t total = (int64_t)n * lde;
+    for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < total;
+         t += (int64_t)gridDim.x * blockDim.x) {
+        const int v = (int)(t / lde), j = (int)(t - (int64_t)v * lde);
+        float sum = 0.0f;
+        int cnt = 0;
+        if (j < edge_dim) {
+            const int off = __ldg(offsets + v), deg = __ldg(in_deg + v);
+            for (int k = 0; k < deg; k++) {
+                if (__ldg(nbr + off + k) == v) continue;
+                sum += __ldg(ef + (size_t)(off + k) * lde + j);
+                cnt++;
+            }
+        }
+        self_attr[t] = cnt > 0 ? sum / (float)cnt : 0.0f;
+    }
+}
+
+}  // namespace
+
+int launch_gatv2_agg(const Gatv2AggArgs &a, cudaStream_t s, int *launches)
+{
+    if (a.n <= 0) return GNNB_OK;
+    const int HC = a.H * a.C;
+    GNNB_REQUIRE(a.H >= 1 && a.C >= 1 && a.ldg >= 2 * HC && a.ldo >= HC && a.bias != nullptr &&
+                     a.att != nullptr && (a.skip == nullptr || a.ldskip >= HC),
+                 "gatv2 aggregation: bad arguments");
+    const bool edge = a.ef_sorted != nullptr;
+    if (edge)
+        GNNB_REQUIRE(a.self_attr != nullptr && a.We_t != nullptr && a.edge_dim >= 1 &&
+                         a.edge_dim <= kGineMaxEdgeDim && a.lde % 4 == 0 && a.lde >= a.edge_dim &&
+                         a.ldw % 4 == 0 && a.ldw >= HC && aligned16(a.ef_sorted) && aligned16(a.self_attr),
+                     "gatv2 aggregation: bad edge features");
+    const bool v4 = (a.C % 4 == 0) && (a.ldg % 4 == 0) && (a.ldo % 4 == 0) && aligned16(a.xlr) &&
+                    aligned16(a.out) && aligned16(a.bias) && aligned16(a.att) &&
+                    (a.skip == nullptr || ((a.ldskip % 4 == 0) && aligned16(a.skip))) &&
+                    (!edge || aligned16(a.We_t));
+    const int vec = v4 ? 4 : 1;
+    const int cg = (a.C + vec - 1) / vec;   // VEC-column groups per head
+    int G = 1;
+    while (G < 32 && G < cg) G *= 2;
+    const int nj = (cg + G - 1) / G;
+    GNNB_REQUIRE(nj <= 2, "gatv2 aggregation: head width C = " + std::to_string(a.C) +
+                              " exceeds the lanes of a warp (at most " +
+                              std::to_string(kGatv2MaxHeadWidth) + " with C % 4 == 0, else " +
+                              std::to_string(kGatv2MaxHeadWidth1) + ")");
+    int lpr = G;
+    while (lpr < 32 && lpr < G * a.H) lpr *= 2;
+    const int rows_per_block = 8 * (32 / lpr);
+    const int64_t grid64 = ceil_div64(a.n, rows_per_block);
+    const int64_t cap = (int64_t)kNumSMs * 8 * 4;
+    const int grid = (int)(grid64 < cap ? grid64 : cap);
+    // W_e^T in shared memory when it fits (edge_dim 64 at H*C = 256: 64 KB), as the GINE aggregation
+    const size_t w_bytes = edge ? sizeof(float) * (size_t)a.edge_dim * a.ldw : 0;
+    const size_t smem = w_bytes <= 200 * 1024 ? w_bytes : 0;
+    if (a.n_heavy > 0)
+        GNNB_REQUIRE(a.heavy_rows != nullptr && a.heavy_partial != nullptr && a.heavy_chunks > 0 &&
+                         a.heavy_chunk_base != nullptr && a.heavy_chunk_row != nullptr &&
+                         a.ldp >= HC + 2 * a.H && a.ldp % 4 == 0,
+                     "gatv2 heavy rows: row list / partial buffer missing");
+    if (vec == 4) {
+        if (nj == 1)
+            return edge ? launch_gatv2_variant<4, 1, true>(a, lpr, G, grid, smem, s, launches)
+                        : launch_gatv2_variant<4, 1, false>(a, lpr, G, grid, 0, s, launches);
+        return edge ? launch_gatv2_variant<4, 2, true>(a, lpr, G, grid, smem, s, launches)
+                    : launch_gatv2_variant<4, 2, false>(a, lpr, G, grid, 0, s, launches);
+    }
+    if (nj == 1)
+        return edge ? launch_gatv2_variant<1, 1, true>(a, lpr, G, grid, smem, s, launches)
+                    : launch_gatv2_variant<1, 1, false>(a, lpr, G, grid, 0, s, launches);
+    return edge ? launch_gatv2_variant<1, 2, true>(a, lpr, G, grid, smem, s, launches)
+                : launch_gatv2_variant<1, 2, false>(a, lpr, G, grid, 0, s, launches);
+}
+
+int launch_gatv2_self_attr(const float *ef_sorted, int lde, int edge_dim, const int32_t *offsets,
+                           const int32_t *nbr, const int32_t *in_deg, int n, float *self_attr,
+                           cudaStream_t s, int *launches)
+{
+    if (n <= 0) return GNNB_OK;
+    const int64_t grid64 = ceil_div64((int64_t)n * lde, 256);
+    const int64_t cap = (int64_t)kNumSMs * 16;
+    gatv2_self_attr_kernel<<<(int)(grid64 < cap ? grid64 : cap), 256, 0, s>>>(
+        ef_sorted, lde, edge_dim, offsets, nbr, in_deg, n, self_attr);
+    GNNB_CUDA(cudaGetLastError());
+    if (launches) ++*launches;
+    return GNNB_OK;
+}
+
 }  // namespace gnnb

@@ -229,6 +229,56 @@ struct GatEdgeLogitsArgs {
 };
 int launch_gat_edge_logits(const GatEdgeLogitsArgs &a, int avg_deg, cudaStream_t s, int *launches);
 
+// GATv2 attention aggregation (PyG GATv2Conv, concat heads, inference).  xlr holds the layer's two
+// GEMM outputs per row: xl = x W_l^T + b_l in columns [0, H*C), xr = x W_r^T + b_r in [H*C, 2 H*C).
+// Per destination v and head h, over the in-neighbours u != v plus one self term (u = v):
+// z = xl_u + xr_v (+ e_uv W_e^T), e_uvh = sum_c att_hc LeakyReLU(z_hc), y_v = act(sum softmax_v(e)
+// xl_u + bias (+ skip_v)).  The logit is a dot product over each head's lanes, computed per edge; the
+// online softmax and the heavy-row partials [acc H*C | max H | sum H] are GAT's.
+// a head's columns are spread over at most 32 lanes, each holding at most two VEC-column groups
+constexpr int kGatv2MaxHeadWidth = 256;   // C % 4 == 0 (float4 lanes)
+constexpr int kGatv2MaxHeadWidth1 = 64;   // other C (scalar lanes)
+struct Gatv2AggArgs {
+    const float *xlr;      // [n][ldg]
+    int ldg, H, C;
+    float slope;
+    const float *att;      // [H*C]
+    const float *bias;     // [H*C]
+    const float *skip;     // [n][ldskip] or null
+    int ldskip;
+    int act;
+    float *out;            // [n][ldo]
+    int ldo;
+    const int32_t *offsets, *nbr, *in_deg;
+    int n;
+    // edge features (edge_dim > 0), else ef_sorted null: the edge term of slot k is
+    // ef_sorted[k] W_e^T, the self term's self_attr[v] W_e^T
+    const float *ef_sorted;  // [slots][lde], neighbor-slot order
+    const float *self_attr;  // [n][lde]
+    int lde, edge_dim;
+    const float *We_t;       // [edge_dim][ldw] (ldw multiple of 4, zero padded)
+    int ldw;
+    const int32_t *heavy_rows;
+    int n_heavy;
+    int heavy_threshold;
+    float *heavy_partial;  // [heavy_chunks][ldp]: accumulator (H*C), then max [H], sum [H]
+    int ldp;               // >= H*C + 2H, multiple of 4
+    const int32_t *heavy_chunk_base, *heavy_chunk_row;
+    int heavy_chunks;
+    void set_heavy(const HeavyList &hl, float *partial)
+    {
+        heavy_rows = hl.rows.as<int32_t>(); n_heavy = hl.n_heavy;
+        heavy_chunk_base = hl.chunk_base.as<int32_t>(); heavy_chunk_row = hl.chunk_row.as<int32_t>();
+        heavy_chunks = hl.n_chunks; heavy_partial = partial;
+    }
+};
+int launch_gatv2_agg(const Gatv2AggArgs &a, cudaStream_t s, int *launches);
+// self_attr[v][0..lde) = the mean of ef_sorted[k] over the slots k of row v whose source is not v, in
+// slot order (0 when there is none); columns past edge_dim are 0
+int launch_gatv2_self_attr(const float *ef_sorted, int lde, int edge_dim, const int32_t *offsets,
+                           const int32_t *nbr, const int32_t *in_deg, int n, float *self_attr,
+                           cudaStream_t s, int *launches);
+
 struct PnaAggArgs {
     const float *ab;       // [n][2F]: cols [0,F) = x.W_nbr^T, cols [F,2F) = x.W_self^T + b_pre
     int F;

@@ -125,6 +125,15 @@ void enumerate_params(gnnb_model *m)
             add_param(m, base + "_conv_lin_weight", {fo, fi});
             if (m->has_edge_features()) add_param(m, base + "_conv_lin_edge_weight", {fo, d.edge_dim});
             break;
+        case GNNB_CONV_GATV2:   // PyG GATv2Conv: its own parameters, then lin_l's, lin_r's, lin_edge's
+            add_param(m, base + "_conv_att", {1, d.gat_heads, fo / d.gat_heads});
+            add_param(m, base + "_conv_bias", {fo});
+            add_param(m, base + "_conv_lin_l_weight", {fo, fi});
+            add_param(m, base + "_conv_lin_l_bias", {fo});
+            add_param(m, base + "_conv_lin_r_weight", {fo, fi});
+            add_param(m, base + "_conv_lin_r_bias", {fo});
+            if (m->has_edge_features()) add_param(m, base + "_conv_lin_edge_weight", {fo, d.edge_dim});
+            break;
         }
     }
 }
@@ -227,8 +236,9 @@ extern "C" int gnnb_model_create(const gnnb_model_desc *desc, int device, gnnb_m
     // shorter struct never has bytes read past its end; a GAT caller's struct always holds it)
     gnnb_model_desc d{};
     std::memcpy(&d, desc, offsetof(gnnb_model_desc, edge_dim));
-    GNNB_REQUIRE(d.conv_type >= GNNB_CONV_GCN && d.conv_type <= GNNB_CONV_GAT,
-                 "conv_type must be GCN, GIN, SAGE, PNA, GINE or GAT");
+    GNNB_REQUIRE((d.conv_type >= GNNB_CONV_GCN && d.conv_type <= GNNB_CONV_GAT) ||
+                     d.conv_type == GNNB_CONV_GATV2,
+                 "conv_type must be GCN, GIN, SAGE, PNA, GINE, GAT or GATv2 (0..5 or 7)");
     if (d.conv_type == GNNB_CONV_GINE) {
         d.edge_dim = desc->edge_dim;
         GNNB_REQUIRE(d.edge_dim >= 1 && d.edge_dim <= kGineMaxEdgeDim,
@@ -236,22 +246,32 @@ extern "C" int gnnb_model_create(const gnnb_model_desc *desc, int device, gnnb_m
     }
     GNNB_REQUIRE(d.num_layers >= 0 && d.num_layers <= 64, "num_layers out of range");
     GNNB_REQUIRE(d.in_dim > 0 && d.hidden_dim > 0 && d.out_dim > 0, "dimensions must be positive");
-    if (d.conv_type == GNNB_CONV_GAT) {   // the GAT fields follow edge_dim; only GAT callers set them
+    if (d.conv_type == GNNB_CONV_GAT || d.conv_type == GNNB_CONV_GATV2) {
+        // the GAT fields follow edge_dim; only GAT and GATv2 callers set them
+        const std::string conv = d.conv_type == GNNB_CONV_GAT ? "GAT" : "GATv2";
         d.edge_dim = desc->edge_dim;
         GNNB_REQUIRE(d.edge_dim >= 0 && d.edge_dim <= kGineMaxEdgeDim,
-                     "GAT edge_dim must be 0 (no edge features) or 1.." +
+                     conv + " edge_dim must be 0 (no edge features) or 1.." +
                          std::to_string(kGineMaxEdgeDim));
         d.gat_heads = desc->gat_heads;
         d.gat_negative_slope = desc->gat_negative_slope;
         GNNB_REQUIRE(d.gat_heads >= 1 && d.gat_heads <= GNNB_GAT_MAX_HEADS,
-                     "GAT gat_heads must be 1.." + std::to_string(GNNB_GAT_MAX_HEADS));
-        GNNB_REQUIRE(std::isfinite(d.gat_negative_slope), "GAT gat_negative_slope must be finite");
+                     conv + " gat_heads must be 1.." + std::to_string(GNNB_GAT_MAX_HEADS));
+        GNNB_REQUIRE(std::isfinite(d.gat_negative_slope), conv + " gat_negative_slope must be finite");
         for (int k = 0; k < d.num_layers; k++) {
             const int fo = k == d.num_layers - 1 ? d.out_dim : d.hidden_dim;
             GNNB_REQUIRE(fo % d.gat_heads == 0,
-                         "GAT: every layer's output width (hidden_dim, out_dim) must be a multiple of "
-                         "gat_heads, got width " + std::to_string(fo) + " with " +
+                         conv + ": every layer's output width (hidden_dim, out_dim) must be a multiple "
+                         "of gat_heads, got width " + std::to_string(fo) + " with " +
                              std::to_string(d.gat_heads) + " heads");
+            // GATv2 spreads a head's columns over at most one warp (agg.cu)
+            const int C = fo / d.gat_heads;
+            GNNB_REQUIRE(d.conv_type == GNNB_CONV_GAT ||
+                             C <= (C % 4 == 0 ? kGatv2MaxHeadWidth : kGatv2MaxHeadWidth1),
+                         "GATv2: a head's width (layer width / gat_heads) must be at most " +
+                             std::to_string(kGatv2MaxHeadWidth) + " when a multiple of 4, else at "
+                             "most " + std::to_string(kGatv2MaxHeadWidth1) + ", got " +
+                             std::to_string(C));
         }
     }
     GNNB_REQUIRE(d.num_layers > 0 || d.in_dim == d.out_dim,
@@ -302,7 +322,7 @@ extern "C" int gnnb_model_destroy(gnnb_model_t *m)
     m->prof.release();
     DeviceBuf *bufs[] = {&m->weights, &m->weight_images, &m->st_x, &m->st_coo, &m->st_ef, &m->st_nptr, &m->st_eptr, &m->st_out,
                          &m->in_deg, &m->out_deg, &m->offsets, &m->nbr, &m->nbr_hub, &m->dinv,
-                         &m->edge_index, &m->ef_sorted, &m->elog, &m->self_elog,
+                         &m->edge_index, &m->ef_sorted, &m->self_attr, &m->elog, &m->self_elog,
                          &m->feat[0], &m->feat[1], &m->agg, &m->hid, &m->wide, &m->pooled,
                          &m->hbuf[0], &m->hbuf[1], &m->pool_tmp, &m->ptr_tmp, &m->edge_flag};
     for (DeviceBuf *b : bufs) b->release();
@@ -471,6 +491,21 @@ extern "C" int gnnb_model_finalize(gnnb_model_t *m)
             idx += edges ? 6 : 4;
             break;
         }
+        case GNNB_CONV_GATV2: {
+            // [att, bias, lin_l_weight, lin_l_bias, lin_r_weight, lin_r_bias (, lin_edge_weight)]:
+            // a = lin_l, b = lin_r, c = att and d = the conv bias as vectors, e = W_e^T (no bias)
+            L.a = pack_linear(pk, param(m, idx + 2), param(m, idx + 3), fo, fi);
+            L.b = pack_linear(pk, param(m, idx + 4), param(m, idx + 5), fo, fi);
+            L.c.out = fo;
+            L.c.has_bias = true;
+            L.c.bias_off = pk.add_vector(param(m, idx), fo);
+            L.d.out = fo;
+            L.d.has_bias = true;
+            L.d.bias_off = pk.add_vector(param(m, idx + 1), fo);
+            if (m->has_edge_features()) L.e = pack_linear(pk, param(m, idx + 6), nullptr, fo, d.edge_dim);
+            idx += m->has_edge_features() ? 7 : 6;
+            break;
+        }
         }
         layer_p.push_back(L);
     }
@@ -511,8 +546,8 @@ extern "C" int gnnb_model_finalize(gnnb_model_t *m)
     }
     fused_release(m);
     fused_tc_release(m);
-    // neither fused kernel takes GINE or GAT (they leave m->fused / m->fused_tc null): those run
-    // layerwise
+    // neither fused kernel takes GINE, GAT or GATv2 (they leave m->fused / m->fused_tc null): those
+    // run layerwise
     GNNB_TRY(fused_prepare(m));
     GNNB_TRY(fused_tc_prepare(m));
     m->finalized = true;
@@ -610,14 +645,19 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
     const bool gine = d.conv_type == GNNB_CONV_GINE;
     const bool gat = d.conv_type == GNNB_CONV_GAT;
     const bool gat_edges = gat && m->has_edge_features();
+    const bool gatv2 = d.conv_type == GNNB_CONV_GATV2;
+    const bool gatv2_edges = gatv2 && m->has_edge_features();
     const int LH = gat_edges ? d.num_layers * d.gat_heads : 0;   // edge logit columns per slot / row
-    // GINE has no heavy-row bucketing or hub hints, as PNA; GAT is bucketed but takes no hub hints
+    // GINE has no heavy-row bucketing or hub hints, as PNA; GAT and GATv2 are bucketed but take no
+    // hub hints
     const bool bucketed = d.conv_type != GNNB_CONV_PNA && !gine;
-    const bool hub_hints = bucketed && !gat;
+    const bool hub_hints = bucketed && !gat && !gatv2;
     const int lde = round_up(std::max(d.edge_dim, 1), 4);
     // GAT: the layer GEMM's output rows [h | a_src | a_dst], and the heavy-row partials, are
     // H*C + 2H floats wide
-    const int ld_gat = gat ? round_up(std::max(d.hidden_dim, d.out_dim) + 2 * d.gat_heads, 4) : 0;
+    const int ld_gat = gat || gatv2 ? round_up(std::max(d.hidden_dim, d.out_dim) + 2 * d.gat_heads, 4) : 0;
+    // GATv2: the layer GEMMs' output rows [xl | xr], 2 H*C floats wide
+    const int ld_xlr = gatv2 ? round_up(2 * std::max(d.hidden_dim, d.out_dim), 4) : 0;
     if (d.num_layers > 0) {
         ProfScope ps(m->prof, PROF_TABLES, s);
         // the out-degree table (lib:1051-1083) is only read by the optional hub-row hints
@@ -634,10 +674,16 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
                               edge_base, n_graphs, T, E, in_deg,
                               want_out_deg ? m->out_deg.as<int32_t>() : nullptr, offsets, nbr, eidx,
                               m->tws, s, launches, m->edge_flag.as<int>()));
-        if (gine) {   // edge features in neighbor-slot order, once per run; every layer reads them in order
+        // edge features in neighbor-slot order, once per run; every layer reads them in order
+        if (gine || gatv2_edges) {
             GNNB_TRY(m->ef_sorted.ensure(sizeof(float) * (size_t)En * lde));
             GNNB_TRY(launch_permute_edge_rows(ef, d.edge_dim, eidx, E, m->ef_sorted.as<float>(), lde, s,
                                               launches));
+        }
+        if (gatv2_edges) {   // each row's self-loop attribute: the mean of its other in-edge attributes
+            GNNB_TRY(m->self_attr.ensure(sizeof(float) * (size_t)Tn * lde));
+            GNNB_TRY(launch_gatv2_self_attr(m->ef_sorted.as<float>(), lde, d.edge_dim, offsets, nbr,
+                                            in_deg, T, m->self_attr.as<float>(), s, launches));
         }
     }
     if (gat_edges && d.num_layers > 0) {   // every layer's edge logits, once per run
@@ -663,7 +709,7 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
     m->last_hub_rows = 0;
     if (!strict && d.num_layers > 0 && bucketed && n_graphs > 0 && T64 / n_graphs > 50000) {
         GNNB_TRY(find_heavy_rows(in_deg, T, heavy_thr, m->tws, m->heavy, s, launches));
-        GNNB_TRY(heavy_setup(m->tws, m->heavy.n_chunks, gat ? ld_gat : maxf));
+        GNNB_TRY(heavy_setup(m->tws, m->heavy.n_chunks, gat || gatv2 ? ld_gat : maxf));
         // a feature matrix larger than L2: keep the rows of the most-referenced sources resident
         // (the out-degree table, lib:1051-1083, is what ranks them)
         const size_t row_bytes = sizeof(float) * (size_t)std::max(d.in_dim, d.hidden_dim);
@@ -682,10 +728,12 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
 
     GNNB_TRY(m->feat[0].ensure(sizeof(float) * (size_t)Tn * ldf));
     GNNB_TRY(m->feat[1].ensure(sizeof(float) * (size_t)Tn * ldf));
-    if (!gat) GNNB_TRY(m->agg.ensure(sizeof(float) * (size_t)Tn * ldf));   // GAT aggregates into dst
+    // GAT and GATv2 aggregate into dst
+    if (!gat && !gatv2) GNNB_TRY(m->agg.ensure(sizeof(float) * (size_t)Tn * ldf));
     if (d.conv_type == GNNB_CONV_GIN || d.conv_type == GNNB_CONV_PNA || gine)
         GNNB_TRY(m->hid.ensure(sizeof(float) * (size_t)Tn * ldf));
     if (gat) GNNB_TRY(m->hid.ensure(sizeof(float) * (size_t)Tn * ld_gat));
+    if (gatv2) GNNB_TRY(m->hid.ensure(sizeof(float) * (size_t)Tn * ld_xlr));
     if (d.conv_type == GNNB_CONV_PNA)
         GNNB_TRY(m->wide.ensure(sizeof(float) * (size_t)Tn * 14 * (size_t)ldf));
 
@@ -792,6 +840,31 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
             { ProfScope ps(m->prof, PROF_AGG, s); GNNB_TRY(launch_gat_agg(ga, s, launches)); }
             break;
         }
+        case GNNB_CONV_GATV2: {
+            // two GEMMs, xl = x.W_l^T + b_l and xr = x.W_r^T + b_r, side by side in one buffer (one GEMM
+            // of N = 2 H*C would not fit the tensor-core GEMM at H*C = 128); then the attention
+            // aggregation, whose epilogue applies bias, skip and activation and writes the layer
+            const int H = d.gat_heads, ldg = round_up(2 * fo, 4);
+            float *xlr = m->hid.as<float>();
+            GemmArgs gl = gemm_args(cur, cur_ld, L.a, xlr, ldg, T, GNNB_ACT_IDENTITY);
+            GemmArgs gr = gemm_args(cur, cur_ld, L.b, xlr + fo, ldg, T, GNNB_ACT_IDENTITY);
+            { ProfScope ps(m->prof, PROF_GEMM, s); GNNB_TRY(launch_gemm(gl, strict, s, launches)); }
+            { ProfScope ps(m->prof, PROF_GEMM, s); GNNB_TRY(launch_gemm(gr, strict, s, launches)); }
+            Gatv2AggArgs ga{};
+            ga.xlr = xlr; ga.ldg = ldg; ga.H = H; ga.C = fo / H; ga.slope = d.gat_negative_slope;
+            ga.att = L.c.bias; ga.bias = L.d.bias; ga.skip = skip; ga.ldskip = cur_ld; ga.act = d.gnn_act;
+            ga.out = dst; ga.ldo = ld_out;
+            ga.offsets = offsets; ga.nbr = nbr; ga.in_deg = in_deg; ga.n = T;
+            if (gatv2_edges) {
+                ga.ef_sorted = m->ef_sorted.as<float>(); ga.self_attr = m->self_attr.as<float>();
+                ga.lde = lde; ga.edge_dim = d.edge_dim; ga.We_t = L.e.Wt; ga.ldw = L.e.ldw;
+            }
+            ga.heavy_threshold = heavy_thr;
+            ga.set_heavy(m->heavy, m->tws.heavy_partial.as<float>());
+            ga.ldp = round_up(fo + 2 * H, 4);
+            { ProfScope ps(m->prof, PROF_AGG, s); GNNB_TRY(launch_gatv2_agg(ga, s, launches)); }
+            break;
+        }
         }
         cur = dst;
         cur_ld = ld_out;
@@ -875,6 +948,11 @@ static int choose_path(gnnb_model_t *m, int max_n, int max_e, int *path, int *ke
                       "run on the layerwise path");
             return GNNB_ERR_INVALID;
         }
+        if (m->d.conv_type == GNNB_CONV_GATV2) {
+            set_error("fused path requested but the fused kernels have no GATv2 attention; GATv2 "
+                      "models run on the layerwise path");
+            return GNNB_ERR_INVALID;
+        }
         if (!can_tc && !can_fma) {
             set_error("fused path requested but unsupported for this model/batch (graph larger than "
                       "a CTA tile, strict math, or unsupported dims)");
@@ -918,15 +996,16 @@ static int check_edges_entry(gnnb_model_t *m, bool edges_entry)
     GNNB_TRY(check_ready(m));
     const bool edges = m->has_edge_features();
     if (edges && !edges_entry) {
-        set_error(std::string(m->d.conv_type == GNNB_CONV_GAT ? "a GAT model with edge_dim"
-                                                                : "a GINE model") +
+        set_error(std::string(m->d.conv_type == GNNB_CONV_GAT     ? "a GAT model with edge_dim"
+                              : m->d.conv_type == GNNB_CONV_GATV2 ? "a GATv2 model with edge_dim"
+                                                                  : "a GINE model") +
                   " needs its edge features: run it with gnnb_model_run_batch_edges or "
                   "gnnb_model_run_batch_edges_async");
         return GNNB_ERR_INVALID;
     }
     if (!edges && edges_entry) {
-        set_error("the *_edges entry points run GINE models and GAT models with edge_dim only; this "
-                  "model has no edge features");
+        set_error("the *_edges entry points run GINE models and GAT and GATv2 models with edge_dim "
+                  "only; this model has no edge features");
         return GNNB_ERR_INVALID;
     }
     return GNNB_OK;

@@ -32,6 +32,9 @@ struct LayerPack {
 // GAT: a = [W | w_src | w_dst]^T, H*C + 2H columns and no bias (one GEMM gives h and both logits
 // of a row); b carries only the conv bias [H*C], which the aggregation epilogue adds.  With edge_dim,
 // the edge linear folded with att_edge is one [L*H][edge_dim] table for all layers (gat_w_edge).
+// GATv2: a = lin_l and b = lin_r (weights and biases, two GEMMs into one [T][round_up(2 H*C, 4)]
+// buffer); c carries att [H*C] and d the conv bias [H*C] as vectors; e = lin_edge's W_e^T
+// [edge_dim][ldw] without a bias (edge_dim > 0 only), applied per edge by the aggregation.
 
 // fused-kernel plans (fused.cu, fused_tc.cu)
 struct FusedPlan;
@@ -105,7 +108,8 @@ struct gnnb_model {
     // layerwise workspaces
     gnnb::DeviceBuf in_deg, out_deg, offsets, nbr, nbr_hub, dinv, feat[2], agg, hid, wide, pooled,
         hbuf[2], pool_tmp, ptr_tmp;
-    gnnb::DeviceBuf edge_index, ef_sorted;   // GINE: edge id and edge features per neighbor slot
+    gnnb::DeviceBuf edge_index, ef_sorted;   // GINE, GATv2: edge id and edge features per neighbor slot
+    gnnb::DeviceBuf self_attr;   // GATv2 with edge_dim: each row's self-loop attribute [n][lde]
     // GAT with edge_dim: the edge logits of every layer and head per neighbor slot and per row
     // (gat_edge_logits_kernel), and the folded edge weights [L*H][edge_dim] inside `weights`
     gnnb::DeviceBuf elog, self_elog;
@@ -124,7 +128,7 @@ struct gnnb_model {
     int64_t last_emb_rows = 0;
 
     int emb_dim() const { return d.num_layers == 0 ? d.in_dim : d.out_dim; }
-    // GINE, and GAT with edge_dim: edge features come through the *_edges entry points
+    // GINE, and GAT and GATv2 with edge_dim: edge features come through the *_edges entry points
     bool has_edge_features() const { return d.edge_dim > 0; }
     void layer_dims(int layer, int *fi, int *fo) const
     {

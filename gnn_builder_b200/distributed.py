@@ -405,8 +405,8 @@ class LargeGraphModel:
         d = model.describe()
         if d["conv_type"] not in (0, 1, 2, 3):
             raise NotImplementedError("row-partitioned inference runs GCN, GIN, SAGE and PNA models "
-                                      "(GINE has no edge-feature halo exchange, GAT no split-CSR "
-                                      "attention kernel)")
+                                      "(GINE has no edge-feature halo exchange, GAT and GATv2 no "
+                                      "split-CSR attention kernel)")
         self.conv = ("gcn", "gin", "sage", "pna")[d["conv_type"]]
         self.model, self.desc = model, d
         self.part = RowPartition(n_total, world)

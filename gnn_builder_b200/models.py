@@ -144,6 +144,54 @@ class _GATConv(nn.Module):
         return _scatter_sum(msg, dst, n) + self.bias
 
 
+class _GATv2Conv(nn.Module):
+    """PyG GATv2Conv with an int ``in_channels``, concatenated heads, self loops and
+    ``share_weights=False``, for inference.  Its own parameters come first in the flat order:
+    ``att`` [1][H][C], ``bias`` [H*C], then ``lin_l`` and ``lin_r`` (weight [H*C][in] and bias each)
+    and with ``edge_dim`` ``lin_edge.weight`` [H*C][edge_dim] (no bias) -- PyG's order.  With edge
+    features each self loop's attribute is the mean of the node's other in-edge attributes (PyG's
+    ``fill_value="mean"``), the zero vector for a node without one."""
+
+    def __init__(self, in_channels: int, out_channels: int, heads: int, negative_slope: float,
+                 edge_dim: Optional[int] = None):
+        super().__init__()
+        self.heads = heads
+        self.head_channels = out_channels // heads
+        self.negative_slope = negative_slope
+        self.edge_dim = edge_dim
+        self.att = nn.Parameter(torch.empty(1, heads, self.head_channels))
+        self.bias = nn.Parameter(torch.zeros(out_channels))
+        self.lin_l = nn.Linear(in_channels, out_channels, bias=True)
+        self.lin_r = nn.Linear(in_channels, out_channels, bias=True)
+        if edge_dim is not None:
+            self.lin_edge = nn.Linear(edge_dim, out_channels, bias=False)
+        nn.init.xavier_uniform_(self.att)
+        nn.init.uniform_(self.bias, -0.1, 0.1)
+        nn.init.uniform_(self.lin_l.bias, -0.1, 0.1)
+        nn.init.uniform_(self.lin_r.bias, -0.1, 0.1)
+
+    def forward(self, x: Tensor, edge_index: Tensor, edge_attr: Optional[Tensor] = None) -> Tensor:
+        n, H, C = x.shape[0], self.heads, self.head_channels
+        # every self loop of the input is replaced by exactly one per node; duplicates stay
+        keep = edge_index[0] != edge_index[1]
+        loops = torch.arange(n, dtype=edge_index.dtype)
+        src = torch.cat([edge_index[0][keep], loops])
+        dst = torch.cat([edge_index[1][keep], loops])
+        xl = self.lin_l(x).view(n, H, C)
+        xr = self.lin_r(x).view(n, H, C)
+        z = xl[src] + xr[dst]
+        if self.edge_dim is not None:
+            ea = edge_attr.reshape(-1, self.edge_dim)[keep]
+            cnt = _in_degree(edge_index[:, keep], n).clamp(min=1.0).view(-1, 1)
+            ea = torch.cat([ea, _scatter_sum(ea, edge_index[1][keep], n) / cnt])
+            z = z + self.lin_edge(ea).view(-1, H, C)
+        e = (torch.nn.functional.leaky_relu(z, self.negative_slope) * self.att).sum(-1)
+        p = (e - _scatter_minmax(e, dst, n, "amax")[dst]).exp()
+        alpha = p / _scatter_sum(p, dst, n)[dst]
+        msg = (xl[src] * alpha.unsqueeze(-1)).reshape(-1, H * C)
+        return _scatter_sum(msg, dst, n) + self.bias
+
+
 class _SAGEConv(nn.Module):
     def __init__(self, in_channels: int, out_channels: int):
         super().__init__()
@@ -310,6 +358,46 @@ class GATConv_GNNB(nn.Module):
         return self.conv(x, edge_index, edge_attr)
 
 
+class GATv2Conv_GNNB(nn.Module):
+    """Graph attention v2 (PyG ``GATv2Conv``, inference, ``share_weights=False``): per head,
+    xl = x W_l^T + b_l, xr = x W_r^T + b_r, logits e_uv = <att, LeakyReLU(xl_u + xr_v)> over the
+    in-edges of v plus one self loop, y_v = sum softmax_v(e) xl_u + bias, heads concatenated.
+    ``out_channels`` is the concatenated width and must be a multiple of ``heads``.  Pass ``heads``
+    with ``functools.partial``.
+
+    ``edge_dim`` (a positive int, also passed with ``functools.partial``) adds ``lin_edge`` (no
+    bias) inside the nonlinearity: LeakyReLU(xl_u + xr_v + e_uv W_e^T), where the self loop's e_vv
+    is the mean of v's other in-edge attributes.  The model's ``graph_input_edge_dim`` must then
+    equal it."""
+
+    def __init__(self, in_channels: int, out_channels: int, heads: int = 1,
+                 negative_slope: float = 0.2, edge_dim: Optional[int] = None, p_in: int = 1,
+                 p_out: int = 1):
+        super().__init__()
+        if not isinstance(heads, int) or isinstance(heads, bool) or heads < 1:
+            raise ValueError(f"heads must be a positive int, got {heads!r}")
+        if edge_dim is not None and (not isinstance(edge_dim, int) or isinstance(edge_dim, bool)
+                                     or edge_dim < 1):
+            raise ValueError(f"edge_dim must be None or a positive int, got {edge_dim!r}")
+        if out_channels % heads != 0:
+            raise ValueError(f"out_channels ({out_channels}) must be a multiple of heads ({heads})")
+        if not math.isfinite(negative_slope):
+            raise ValueError(f"negative_slope must be finite, got {negative_slope!r}")
+        self.in_channels = in_channels
+        self.out_channels = out_channels
+        self.heads = heads
+        self.negative_slope = float(negative_slope)
+        self.edge_dim = edge_dim
+        self.p_in = p_in
+        self.p_out = p_out
+        self.conv = _GATv2Conv(in_channels, out_channels, heads, self.negative_slope, edge_dim)
+
+    def forward(self, x: Tensor, edge_index: Tensor, edge_attr: Optional[Tensor] = None) -> Tensor:
+        if self.edge_dim is not None and edge_attr is None:
+            raise ValueError("a GATv2Conv_GNNB with edge_dim needs edge_attr")
+        return self.conv(x, edge_index, edge_attr)
+
+
 class PNAConv_GNNB(nn.Module):
     """models.py:209-240"""
 
@@ -452,10 +540,11 @@ class MLP(nn.Module):
 
 
 SUPPORTED_GNN_CONVS = [GCNConv_GNNB, GINConv_GNNB, PNAConv_GNNB, SAGEConv_GNNB, GINEConv_GNNB,
-                       GATConv_GNNB]
+                       GATConv_GNNB, GATv2Conv_GNNB]
 
+# 6 is not assigned (GNNB_CONV_GATV2 = 7 in include/gnnb_b200.h)
 CONV_TYPE_IDS = {"GCNConv_GNNB": 0, "GINConv_GNNB": 1, "SAGEConv_GNNB": 2, "PNAConv_GNNB": 3,
-                 "GINEConv_GNNB": 4, "GATConv_GNNB": 5}
+                 "GINEConv_GNNB": 4, "GATConv_GNNB": 5, "GATv2Conv_GNNB": 7}
 ACTIVATION_IDS = {None: 0, "ReLU": 1, "GELU": 2, "Sigmoid": 3, "Tanh": 4}
 POOL_IDS = {"add": 0, "mean": 1, "max": 2}
 
@@ -480,9 +569,10 @@ class GNNModel(nn.Module):
         if conv_cls not in SUPPORTED_GNN_CONVS:
             raise ValueError(f"gnn_conv must be one of {SUPPORTED_GNN_CONVS}")
         self._conv_cls = conv_cls
-        # GAT takes edge features only when its partial carries edge_dim
+        # GAT and GATv2 take edge features only when their partial carries edge_dim
         self._conv_kwargs = dict(getattr(gnn_conv, "keywords", None) or {})
-        gat_edge_dim = (self._conv_kwargs.get("edge_dim") if conv_cls is GATConv_GNNB else None)
+        gat_edge_dim = (self._conv_kwargs.get("edge_dim")
+                        if conv_cls in (GATConv_GNNB, GATv2Conv_GNNB) else None)
         self.uses_edge_features = conv_cls is GINEConv_GNNB or gat_edge_dim is not None
         conv_kwargs = {}
         if conv_cls is GINEConv_GNNB:
@@ -495,8 +585,9 @@ class GNNModel(nn.Module):
             e = graph_input_edge_dim
             for v in (gat_edge_dim, e):
                 if not isinstance(v, int) or isinstance(v, bool) or v < 1 or v != gat_edge_dim:
-                    raise ValueError(f"GATConv_GNNB with edge_dim={gat_edge_dim!r} needs a positive "
-                                     f"int edge_dim and graph_input_edge_dim equal to it, got {e!r}")
+                    raise ValueError(f"{conv_cls.__name__} with edge_dim={gat_edge_dim!r} needs a "
+                                     "positive int edge_dim and graph_input_edge_dim equal to it, "
+                                     f"got {e!r}")
         self.gnn_activation = gnn_activation
         if self.gnn_activation not in SUPPORTED_ACTIVATIONS:
             raise ValueError(f"gnn_activation must be one of {SUPPORTED_ACTIVATIONS}")
@@ -638,7 +729,7 @@ class GNNModel(nn.Module):
         )
         if self.uses_edge_features:
             d["edge_dim"] = int(self.graph_input_edge_dim)
-        if conv_name == "GATConv_GNNB":
+        if conv_name in ("GATConv_GNNB", "GATv2Conv_GNNB"):
             kw = self._conv_kwargs   # a model without layers has no conv to ask
             d["gat_heads"] = int(conv0.heads if conv0 is not None else kw.get("heads", 1))
             d["gat_negative_slope"] = float(conv0.negative_slope if conv0 is not None
