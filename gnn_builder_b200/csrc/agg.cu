@@ -5,7 +5,7 @@
 // Kernel (2) of the design: a (sub-)warp per destination row, lanes across the feature dimension
 // with float4 (16 B) gathers of each neighbor row, so one neighbor row of F=128 floats is one
 // fully coalesced 512 B warp request; neighbor loop unrolled x4 so four independent gathers are
-// in flight per lane.  Rows are bucketed by in-degree: rows above `heavy_threshold` are skipped
+// in flight per lane.  Rows are bucketed by in-degree: rows above `heavy.threshold` are skipped
 // here and handled by the chunked heavy-row kernels below (a warp per 128-neighbor chunk, chunk
 // sums added in a fixed order: deterministic).
 //
@@ -13,6 +13,8 @@
 // N*(4F self + 4F_out write + 8 [offset, degree]).  Neighbors are visited in table order, so in
 // STRICT mode (no FMA contraction, reference scaling formula) sums round exactly like the
 // reference's sum_incremental accumulators.
+#include <type_traits>
+
 #include "kernels.h"
 
 namespace gnnb {
@@ -46,6 +48,31 @@ struct Vec<4> {
         *reinterpret_cast<float4 *>(p) = make_float4(v[0], v[1], v[2], v[3]);
     }
 };
+
+inline bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
+// f(std::integral_constant<int, LPR>) for a row kernel's runtime lanes per row (1, 2, 4, 8, 16, else
+// 32): every launcher instantiates its kernel for all six
+template <typename F>
+decltype(auto) with_lpr(int lpr, F &&f)
+{
+    switch (lpr) {
+    case 1: return f(std::integral_constant<int, 1>{});
+    case 2: return f(std::integral_constant<int, 2>{});
+    case 4: return f(std::integral_constant<int, 4>{});
+    case 8: return f(std::integral_constant<int, 8>{});
+    case 16: return f(std::integral_constant<int, 16>{});
+    default: return f(std::integral_constant<int, 32>{});
+    }
+}
+
+// grid of a row kernel: 256-thread CTAs of 8 * (32 / lpr) rows, at most `cap` of them (the kernels
+// grid-stride beyond; the default is 8 resident CTAs per SM x 4 waves)
+inline int row_grid(int n, int lpr, int64_t cap = (int64_t)kNumSMs * 8 * 4)
+{
+    const int64_t g = ceil_div64(n, 8 * (32 / lpr));
+    return (int)(g < cap ? g : cap);
+}
 
 // L2 eviction-priority policies for the gathers of a large graph (hub_bit mode): rows of hub
 // sources are kept (evict_last), everything else streams through (evict_first).
@@ -216,7 +243,7 @@ __global__ void __launch_bounds__(256) agg_rows_kernel(const AggArgs a)
         if (v >= a.n) continue;
         const int deg_v = __ldg(a.in_deg + v);
         const int len_v = (!STRICT && a.counts != nullptr) ? __ldg(a.counts + v) : deg_v;
-        if (a.n_heavy > 0 && len_v > a.heavy_threshold) continue;  // CTA-per-row kernel does these
+        if (a.heavy.n > 0 && len_v > a.heavy.threshold) continue;  // CTA-per-row kernel does these
         const int off = __ldg(a.offsets + v);
         const float dinv_v = (MODE == AGG_GCN && !STRICT) ? __ldg(a.dinv + v + a.row_base) : 0.0f;
         for (int c = lg * VEC; c < a.F; c += LPR * VEC) {
@@ -248,16 +275,16 @@ __global__ void __launch_bounds__(256) agg_heavy_chunk_kernel(const AggArgs a)
     const int warps_per_block = blockDim.x >> 5;
     const int warp_global = blockIdx.x * warps_per_block + (threadIdx.x >> 5);
     const int warp_stride = gridDim.x * warps_per_block;
-    for (int chunk = warp_global; chunk < a.heavy_chunks; chunk += warp_stride) {
-        const int h = __ldg(a.heavy_chunk_row + chunk);
-        const int v = __ldg(a.heavy_rows + h);
-        const int j = chunk - __ldg(a.heavy_chunk_base + h);
+    for (int chunk = warp_global; chunk < a.heavy.chunks; chunk += warp_stride) {
+        const int h = __ldg(a.heavy.chunk_row + chunk);
+        const int v = __ldg(a.heavy.rows + h);
+        const int j = chunk - __ldg(a.heavy.chunk_base + h);
         const int deg_v = __ldg(a.in_deg + v);
         const int len_v = a.counts != nullptr ? __ldg(a.counts + v) : deg_v;
         const int off = __ldg(a.offsets + v);
         const float dinv_v = (MODE == AGG_GCN) ? __ldg(a.dinv + v + a.row_base) : 0.0f;
         const int k0 = j * kHeavyChunk, k1 = min(len_v, k0 + kHeavyChunk);
-        float *dst = a.heavy_partial + (size_t)chunk * a.F;
+        float *dst = a.heavy.partial + (size_t)chunk * a.F;
         for (int c = lane * VEC; c < a.F; c += 32 * VEC) {
             Vec<VEC> acc;
 #pragma unroll
@@ -277,12 +304,12 @@ __global__ void __launch_bounds__(256) agg_heavy_combine_kernel(const AggArgs a)
 {
     extern __shared__ float ranges[];   // [8][F]
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    for (int h = blockIdx.x; h < a.n_heavy; h += gridDim.x) {
-        const int v = __ldg(a.heavy_rows + h);
+    for (int h = blockIdx.x; h < a.heavy.n; h += gridDim.x) {
+        const int v = __ldg(a.heavy.rows + h);
         const int deg_v = __ldg(a.in_deg + v);
         const int len_v = a.counts != nullptr ? __ldg(a.counts + v) : deg_v;
         const int nch = (len_v + kHeavyChunk - 1) / kHeavyChunk;
-        const float *src = a.heavy_partial + (size_t)__ldg(a.heavy_chunk_base + h) * a.F;
+        const float *src = a.heavy.partial + (size_t)__ldg(a.heavy.chunk_base + h) * a.F;
         const float dinv_v = (MODE == AGG_GCN) ? __ldg(a.dinv + v + a.row_base) : 0.0f;
         const int per = (nch + 7) / 8;
         const int j0 = min(nch, warp * per), j1 = min(nch, j0 + per);
@@ -344,24 +371,11 @@ int launch_mode(const AggArgs &a, int grid, cudaStream_t s)
     return GNNB_OK;
 }
 
-template <int VEC, bool STRICT>
-int launch_lpr(const AggArgs &a, int lpr, int grid, cudaStream_t s)
-{
-    switch (lpr) {
-    case 1: return launch_mode<VEC, 1, STRICT>(a, grid, s);
-    case 2: return launch_mode<VEC, 2, STRICT>(a, grid, s);
-    case 4: return launch_mode<VEC, 4, STRICT>(a, grid, s);
-    case 8: return launch_mode<VEC, 8, STRICT>(a, grid, s);
-    case 16: return launch_mode<VEC, 16, STRICT>(a, grid, s);
-    default: return launch_mode<VEC, 32, STRICT>(a, grid, s);
-    }
-}
-
 template <int VEC, int MODE>
 void launch_heavy_mode(const AggArgs &a, cudaStream_t s)
 {
     const int cap = a.short_ctas ? (1 << 30) : kNumSMs * 8;   // 8 resident CTAs per SM, grid-stride beyond
-    const int g1 = min((a.heavy_chunks + 7) / 8, cap), g2 = min(a.n_heavy, cap);
+    const int g1 = min((a.heavy.chunks + 7) / 8, cap), g2 = min(a.heavy.n, cap);
     agg_heavy_chunk_kernel<VEC, MODE><<<g1, 256, 0, s>>>(a);
     agg_heavy_combine_kernel<VEC, MODE><<<g2, 256, sizeof(float) * 8 * (size_t)a.F, s>>>(a);
 }
@@ -379,7 +393,14 @@ int launch_heavy(const AggArgs &a, cudaStream_t s)
     return GNNB_OK;
 }
 
-inline bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+// the heavy-row block of an aggregation whose bucketing is on (heavy.n > 0)
+int check_heavy(const HeavyArgs &h)
+{
+    GNNB_REQUIRE(h.rows != nullptr && h.partial != nullptr && h.chunks > 0 && h.chunk_base != nullptr &&
+                     h.chunk_row != nullptr,
+                 "heavy row list / partial buffer missing");
+    return GNNB_OK;
+}
 
 }  // namespace
 
@@ -391,7 +412,7 @@ int launch_agg(const AggArgs &a_in, bool strict, cudaStream_t s, int *launches)
     if (strict) {
         GNNB_REQUIRE(a.counts == nullptr && !a.accumulate && !a.no_finish && !a.hub_bit,
                      "split-CSR / hub-hint aggregation is FAST-mode only");
-        a.n_heavy = 0;
+        a.heavy.n = 0;
     }
     if (a.mode == AGG_GCN && !strict)
         GNNB_REQUIRE(a.dinv != nullptr, "gcn aggregation needs the dinv table in fast mode");
@@ -400,23 +421,16 @@ int launch_agg(const AggArgs &a_in, bool strict, cudaStream_t s, int *launches)
     const int vec = v4 ? 4 : 1;
     int lpr = 1;
     while (lpr < 32 && lpr * vec < a.F) lpr *= 2;
-    const int rows_per_block = 8 * (32 / lpr);
-    int64_t grid64 = ceil_div64(a.n, rows_per_block);
-    const int64_t cap = a.short_ctas ? (int64_t)1 << 30
-                                     : (int64_t)kNumSMs * 8 * 4;  // 8 resident CTAs/SM x 4 waves, grid-stride
-    int grid = (int)(grid64 < cap ? grid64 : cap);
-    int rc;
-    if (vec == 4)
-        rc = strict ? launch_lpr<4, true>(a, lpr, grid, s) : launch_lpr<4, false>(a, lpr, grid, s);
-    else
-        rc = strict ? launch_lpr<1, true>(a, lpr, grid, s) : launch_lpr<1, false>(a, lpr, grid, s);
-    GNNB_TRY(rc);
+    const int grid = a.short_ctas ? row_grid(a.n, lpr, (int64_t)1 << 30) : row_grid(a.n, lpr);
+    GNNB_TRY(with_lpr(lpr, [&](auto L) {
+        if (vec == 4)
+            return strict ? launch_mode<4, L, true>(a, grid, s) : launch_mode<4, L, false>(a, grid, s);
+        return strict ? launch_mode<1, L, true>(a, grid, s) : launch_mode<1, L, false>(a, grid, s);
+    }));
     GNNB_CUDA(cudaGetLastError());
     if (launches) ++*launches;
-    if (a.n_heavy > 0) {
-        GNNB_REQUIRE(a.heavy_rows != nullptr && a.heavy_partial != nullptr && a.heavy_chunks > 0 &&
-                         a.heavy_chunk_base != nullptr && a.heavy_chunk_row != nullptr,
-                     "heavy row list / partial buffer missing");
+    if (a.heavy.n > 0) {
+        GNNB_TRY(check_heavy(a.heavy));
         GNNB_TRY(vec == 4 ? launch_heavy<4>(a, s) : launch_heavy<1>(a, s));
         GNNB_CUDA(cudaGetLastError());
         if (launches) *launches += 2;
@@ -504,20 +518,6 @@ __global__ void __launch_bounds__(256) pna_agg_kernel(const PnaAggArgs a)
     }
 }
 
-template <int VEC>
-int launch_pna_lpr(const PnaAggArgs &a, int lpr, int grid, cudaStream_t s)
-{
-    switch (lpr) {
-    case 1: pna_agg_kernel<VEC, 1><<<grid, 256, 0, s>>>(a); break;
-    case 2: pna_agg_kernel<VEC, 2><<<grid, 256, 0, s>>>(a); break;
-    case 4: pna_agg_kernel<VEC, 4><<<grid, 256, 0, s>>>(a); break;
-    case 8: pna_agg_kernel<VEC, 8><<<grid, 256, 0, s>>>(a); break;
-    case 16: pna_agg_kernel<VEC, 16><<<grid, 256, 0, s>>>(a); break;
-    default: pna_agg_kernel<VEC, 32><<<grid, 256, 0, s>>>(a); break;
-    }
-    return GNNB_OK;
-}
-
 }  // namespace
 
 int launch_pna_agg(const PnaAggArgs &a, cudaStream_t s, int *launches)
@@ -527,11 +527,11 @@ int launch_pna_agg(const PnaAggArgs &a, cudaStream_t s, int *launches)
     const int vec = v4 ? 4 : 1;
     int lpr = 1;
     while (lpr < 32 && lpr * vec < a.F) lpr *= 2;
-    const int rows_per_block = 8 * (32 / lpr);
-    int64_t grid64 = ceil_div64(a.n, rows_per_block);
-    const int64_t cap = (int64_t)kNumSMs * 8 * 4;
-    const int grid = (int)(grid64 < cap ? grid64 : cap);
-    GNNB_TRY(vec == 4 ? launch_pna_lpr<4>(a, lpr, grid, s) : launch_pna_lpr<1>(a, lpr, grid, s));
+    const int grid = row_grid(a.n, lpr);
+    with_lpr(lpr, [&](auto L) {
+        if (vec == 4) pna_agg_kernel<4, L><<<grid, 256, 0, s>>>(a);
+        else pna_agg_kernel<1, L><<<grid, 256, 0, s>>>(a);
+    });
     GNNB_CUDA(cudaGetLastError());
     if (launches) ++*launches;
     return GNNB_OK;
@@ -640,19 +640,6 @@ __global__ void __launch_bounds__(256) pna_halo_stats_kernel(const PnaHaloArgs a
     }
 }
 
-template <int VEC>
-void launch_pna_halo_lpr(const PnaHaloArgs &a, int lpr, int grid, cudaStream_t s)
-{
-    switch (lpr) {
-    case 1: pna_halo_stats_kernel<VEC, 1><<<grid, 256, 0, s>>>(a); break;
-    case 2: pna_halo_stats_kernel<VEC, 2><<<grid, 256, 0, s>>>(a); break;
-    case 4: pna_halo_stats_kernel<VEC, 4><<<grid, 256, 0, s>>>(a); break;
-    case 8: pna_halo_stats_kernel<VEC, 8><<<grid, 256, 0, s>>>(a); break;
-    case 16: pna_halo_stats_kernel<VEC, 16><<<grid, 256, 0, s>>>(a); break;
-    default: pna_halo_stats_kernel<VEC, 32><<<grid, 256, 0, s>>>(a); break;
-    }
-}
-
 }  // namespace
 
 int launch_pna_halo_stats(const PnaHaloArgs &a, cudaStream_t s, int *launches)
@@ -664,14 +651,11 @@ int launch_pna_halo_stats(const PnaHaloArgs &a, cudaStream_t s, int *launches)
     const int vec = v4 ? 4 : 1;
     int lpr = 1;
     while (lpr < 32 && lpr * vec < a.F) lpr *= 2;
-    const int rows_per_block = 8 * (32 / lpr);
-    int64_t grid64 = ceil_div64(a.n, rows_per_block);
-    const int64_t cap = (int64_t)kNumSMs * 8 * 4;
-    const int grid = (int)(grid64 < cap ? grid64 : cap);
-    if (vec == 4)
-        launch_pna_halo_lpr<4>(a, lpr, grid, s);
-    else
-        launch_pna_halo_lpr<1>(a, lpr, grid, s);
+    const int grid = row_grid(a.n, lpr);
+    with_lpr(lpr, [&](auto L) {
+        if (vec == 4) pna_halo_stats_kernel<4, L><<<grid, 256, 0, s>>>(a);
+        else pna_halo_stats_kernel<1, L><<<grid, 256, 0, s>>>(a);
+    });
     GNNB_CUDA(cudaGetLastError());
     if (launches) ++*launches;
     return GNNB_OK;
@@ -725,20 +709,6 @@ __global__ void __launch_bounds__(256) gine_agg_kernel(const GineAggArgs a)
     }
 }
 
-template <int VEC>
-int launch_gine_lpr(const GineAggArgs &a, int lpr, int grid, cudaStream_t s)
-{
-    switch (lpr) {
-    case 1: gine_agg_kernel<VEC, 1><<<grid, 256, 0, s>>>(a); break;
-    case 2: gine_agg_kernel<VEC, 2><<<grid, 256, 0, s>>>(a); break;
-    case 4: gine_agg_kernel<VEC, 4><<<grid, 256, 0, s>>>(a); break;
-    case 8: gine_agg_kernel<VEC, 8><<<grid, 256, 0, s>>>(a); break;
-    case 16: gine_agg_kernel<VEC, 16><<<grid, 256, 0, s>>>(a); break;
-    default: gine_agg_kernel<VEC, 32><<<grid, 256, 0, s>>>(a); break;
-    }
-    return GNNB_OK;
-}
-
 }  // namespace
 
 int launch_gine_agg(const GineAggArgs &a, cudaStream_t s, int *launches)
@@ -749,11 +719,11 @@ int launch_gine_agg(const GineAggArgs &a, cudaStream_t s, int *launches)
     const int vec = v4 ? 4 : 1;
     int lpr = 1;
     while (lpr < 32 && lpr * vec < a.F) lpr *= 2;
-    const int rows_per_block = 8 * (32 / lpr);
-    int64_t grid64 = ceil_div64(a.n, rows_per_block);
-    const int64_t cap = (int64_t)kNumSMs * 8 * 4;
-    const int grid = (int)(grid64 < cap ? grid64 : cap);
-    GNNB_TRY(vec == 4 ? launch_gine_lpr<4>(a, lpr, grid, s) : launch_gine_lpr<1>(a, lpr, grid, s));
+    const int grid = row_grid(a.n, lpr);
+    with_lpr(lpr, [&](auto L) {
+        if (vec == 4) gine_agg_kernel<4, L><<<grid, 256, 0, s>>>(a);
+        else gine_agg_kernel<1, L><<<grid, 256, 0, s>>>(a);
+    });
     GNNB_CUDA(cudaGetLastError());
     if (launches) ++*launches;
     return GNNB_OK;
@@ -848,15 +818,8 @@ __global__ void __launch_bounds__(256) gine_agg_proj_kernel(const GineProjAggArg
 template <int VEC, bool SMEM>
 int launch_gine_proj_lpr(const GineProjAggArgs &a, int lpr, int grid, size_t smem, cudaStream_t s)
 {
-    void (*k)(const GineProjAggArgs);
-    switch (lpr) {
-    case 1: k = gine_agg_proj_kernel<VEC, 1, SMEM>; break;
-    case 2: k = gine_agg_proj_kernel<VEC, 2, SMEM>; break;
-    case 4: k = gine_agg_proj_kernel<VEC, 4, SMEM>; break;
-    case 8: k = gine_agg_proj_kernel<VEC, 8, SMEM>; break;
-    case 16: k = gine_agg_proj_kernel<VEC, 16, SMEM>; break;
-    default: k = gine_agg_proj_kernel<VEC, 32, SMEM>; break;
-    }
+    void (*k)(const GineProjAggArgs) =
+        with_lpr(lpr, [](auto L) { return gine_agg_proj_kernel<VEC, L, SMEM>; });
     if (smem > 48 * 1024) GNNB_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     k<<<grid, 256, smem, s>>>(a);
     return GNNB_OK;
@@ -888,10 +851,7 @@ int launch_gine_agg_proj(const GineProjAggArgs &a, cudaStream_t s, int *launches
     const int vec = v4 ? 4 : 1;
     int lpr = 1;
     while (lpr < 32 && lpr * vec < a.F) lpr *= 2;
-    const int rows_per_block = 8 * (32 / lpr);
-    int64_t grid64 = ceil_div64(a.n, rows_per_block);
-    const int64_t cap = (int64_t)kNumSMs * 8 * 4;
-    const int grid = (int)(grid64 < cap ? grid64 : cap);
+    const int grid = row_grid(a.n, lpr);
     // W_e^T + b_e in shared memory when they fit (edge_dim 64 at F = 512: 130 KB); wider layers
     // read them through the read-only cache
     const size_t smem = sizeof(float) * ((size_t)a.edge_dim * a.ldw + a.F);
@@ -941,7 +901,9 @@ int launch_permute_edge_rows(const float *src, int dim, const int32_t *idx, int 
 // and stores its per-head (m, s) and its accumulator (relative to its own m) in the partial scratch.
 // One CTA per row then merges the chunks -- 8 warps over contiguous chunk ranges, then the self term
 // and the 8 range results in warp order -- a fixed order, so the result does not depend on
-// scheduling.  Algorithmic bytes per layer: E (4 + 4H + 4HC) + N (8 + 4H + 4HC [+ 4HC skip]).
+// scheduling.  GATv2 shares the online softmax, the epilogue, the partial store, both combine steps
+// and the heavy launch defined here (the attn_* functions, over AttnAggArgs).  Algorithmic bytes per
+// layer: E (4 + 4H + 4HC) + N (8 + 4H + 4HC [+ 4HC skip]).
 //
 // Edge attention (GATConv with edge_dim; the EDGE instantiations): the logit of slot k adds the edge
 // term elog[k][hd] and the self term self_elog[v][hd], both computed once per run by
@@ -951,43 +913,142 @@ namespace {
 
 __device__ __forceinline__ float leaky_relu(float x, float slope) { return x > 0.0f ? x : x * slope; }
 
-template <int VEC>
+// One lane's online softmax over NJ groups of VEC columns of one head (GAT: NJ = 1)
+template <int VEC, int NJ = 1>
 struct OnlineSoftmax {
     float m, s;
-    Vec<VEC> acc;
+    Vec<VEC> acc[NJ];
     __device__ __forceinline__ void reset()
     {
         m = -INFINITY;
         s = 0.0f;
 #pragma unroll
-        for (int i = 0; i < VEC; i++) acc.v[i] = 0.0f;
+        for (int j = 0; j < NJ; j++)
+#pragma unroll
+            for (int i = 0; i < VEC; i++) acc[j].v[i] = 0.0f;
     }
-    // adds a part with max m2, sum s2 and accumulator acc2 (one edge: e, 1, h_u); an empty part
+    // adds a part with max m2, sum s2 and accumulator acc2[NJ] (one edge: e, 1, h_u); an empty part
     // (m2 = -inf, from a chunk of self loops only) changes nothing
-    __device__ __forceinline__ void merge(float m2, float s2, const Vec<VEC> &acc2)
+    __device__ __forceinline__ void merge(float m2, float s2, const Vec<VEC> *acc2)
     {
         if (m2 == -INFINITY) return;
         const float mn = fmaxf(m, m2);
         const float r = expf(m - mn), p = expf(m2 - mn);
         s = fmaf(s, r, s2 * p);
 #pragma unroll
-        for (int i = 0; i < VEC; i++) acc.v[i] = fmaf(acc.v[i], r, acc2.v[i] * p);
+        for (int j = 0; j < NJ; j++)
+#pragma unroll
+            for (int i = 0; i < VEC; i++) acc[j].v[i] = fmaf(acc[j].v[i], r, acc2[j].v[i] * p);
         m = mn;
     }
 };
+
+// the columns of head hd a lane holds: col[j] .. col[j] + VEC for the groups j with valid[j]
+template <int NJ>
+struct AttnCols {
+    int hd;
+    int col[NJ];
+    bool valid[NJ];
+};
+
+// the epilogue of one VEC-column group: out[v][c..] = act(acc / s + bias (+ skip))
+template <int VEC>
+__device__ __forceinline__ void attn_finish(const AttnAggArgs &a, int v, int c, const Vec<VEC> &acc, float s)
+{
+    Vec<VEC> b, sk, y;
+    b.load(a.bias + c);
+    if (a.skip != nullptr) sk.load(a.skip + (size_t)v * a.ldskip + c);
+#pragma unroll
+    for (int i = 0; i < VEC; i++) {
+        float t = acc.v[i] / s + b.v[i];
+        if (a.skip != nullptr) t += sk.v[i];
+        y.v[i] = act_apply_compact(a.act, t);
+    }
+    y.store(a.out + (size_t)v * a.ldo + c);
+}
+
+// a partial [acc H*C | max H | sum H] (a chunk's in global memory, a range's in shared memory) for the
+// lane's columns; head_lane: the one lane of the head that writes (max, sum)
+template <int VEC, int NJ>
+__device__ __forceinline__ void attn_store_partial(const AttnAggArgs &a, float *dst, const AttnCols<NJ> &cl,
+                                                   bool head_lane, const OnlineSoftmax<VEC, NJ> &st)
+{
+    const int HC = a.H * a.C;
+#pragma unroll
+    for (int j = 0; j < NJ; j++)
+        if (cl.valid[j]) st.acc[j].store(dst + cl.col[j]);
+    if (head_lane) {
+        dst[HC + cl.hd] = st.m;
+        dst[HC + a.H + cl.hd] = st.s;
+    }
+}
+
+// Combine step 1, one CTA per heavy row h: each of the 8 warps merges a contiguous range of the row's
+// chunk partials, column by column, into ranges[warp] ([8][ldp], laid out as the partials).  Returns
+// the row.
+template <int VEC>
+__device__ __forceinline__ int attn_combine_chunks(const AttnAggArgs &a, int h, float *ranges)
+{
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int HC = a.H * a.C;
+    const int v = __ldg(a.heavy.rows + h);
+    const int deg = __ldg(a.in_deg + v);
+    const int nch = (deg + kHeavyChunk - 1) / kHeavyChunk;
+    const float *src = a.heavy.partial + (size_t)__ldg(a.heavy.chunk_base + h) * a.ldp;
+    const int per = (nch + 7) / 8;
+    const int j0 = min(nch, warp * per), j1 = min(nch, j0 + per);
+    float *mine = ranges + warp * a.ldp;
+    for (int c = lane * VEC; c < HC; c += 32 * VEC) {
+        const int hd = c / a.C;
+        OnlineSoftmax<VEC> st;
+        st.reset();
+        for (int j = j0; j < j1; j++) {
+            const float *p = src + (size_t)j * a.ldp;
+            Vec<VEC> t;
+            t.load_rw(p + c);
+            st.merge(p[HC + hd], p[HC + a.H + hd], &t);
+        }
+        attn_store_partial<VEC, 1>(a, mine, {hd, {c}, {true}}, c % a.C == 0, st);
+    }
+    return v;
+}
+
+// Combine step 2: merges the 8 range results, in warp order, into st (which holds the self term) for
+// the lane's columns; hd is the head whose (max, sum) are read (clamped for idle GATv2 groups)
+template <int VEC, int NJ>
+__device__ __forceinline__ void attn_merge_ranges(const AttnAggArgs &a, const float *ranges,
+                                                  const AttnCols<NJ> &cl, int hd, OnlineSoftmax<VEC, NJ> &st)
+{
+    const int HC = a.H * a.C;
+#pragma unroll 1
+    for (int w = 0; w < 8; w++) {
+        const float *r = ranges + w * a.ldp;
+        Vec<VEC> t[NJ];
+#pragma unroll
+        for (int j = 0; j < NJ; j++) {
+            if (cl.valid[j]) {
+                t[j].load_rw(r + cl.col[j]);
+            } else {
+#pragma unroll
+                for (int i = 0; i < VEC; i++) t[j].v[i] = 0.0f;
+            }
+        }
+        st.merge(r[HC + hd], r[HC + a.H + hd], t);
+    }
+}
 
 // the self term of row v for the lane's columns [c, c + VEC) of head hd; returns a_dst[v][hd]
 template <int VEC, bool EDGE>
 __device__ __forceinline__ float gat_self(const GatAggArgs &a, int v, int c, int hd, OnlineSoftmax<VEC> &st)
 {
     const int HC = a.H * a.C;
-    const float *row = a.hg + (size_t)v * a.ldg;
+    const float *row = a.g + (size_t)v * a.ldg;
     const float adst = __ldg(row + HC + a.H + hd);
     float e = __ldg(row + HC + hd) + adst;
     if (EDGE) e += __ldg(a.self_elog + (size_t)v * a.ldl + hd);
     st.m = leaky_relu(e, a.slope);
     st.s = 1.0f;
-    st.acc.load(row + c);
+    st.acc[0].load(row + c);
     return adst;
 }
 
@@ -1006,7 +1067,7 @@ __device__ __forceinline__ void gat_gather(const GatAggArgs &a, int v, int off, 
         for (int j = 0; j < 4; j++) u[j] = __ldg(a.nbr + off + k + j);
 #pragma unroll
         for (int j = 0; j < 4; j++) {
-            const float *row = a.hg + (size_t)u[j] * a.ldg;
+            const float *row = a.g + (size_t)u[j] * a.ldg;
             as[j] = __ldg(row + HC + hd);
             if (EDGE) el[j] = __ldg(a.elog + (size_t)(off + k + j) * a.ldl + hd);
             x[j].load(row + c);
@@ -1015,34 +1076,19 @@ __device__ __forceinline__ void gat_gather(const GatAggArgs &a, int v, int off, 
         for (int j = 0; j < 4; j++) {
             float e = as[j] + adst;
             if (EDGE) e += el[j];
-            if (u[j] != v) st.merge(leaky_relu(e, a.slope), 1.0f, x[j]);
+            if (u[j] != v) st.merge(leaky_relu(e, a.slope), 1.0f, &x[j]);
         }
     }
     for (; k < k1; k++) {
         const int u = __ldg(a.nbr + off + k);
         if (u == v) continue;
-        const float *row = a.hg + (size_t)u * a.ldg;
+        const float *row = a.g + (size_t)u * a.ldg;
         Vec<VEC> x;
         x.load(row + c);
         float e = __ldg(row + HC + hd) + adst;
         if (EDGE) e += __ldg(a.elog + (size_t)(off + k) * a.ldl + hd);
-        st.merge(leaky_relu(e, a.slope), 1.0f, x);
+        st.merge(leaky_relu(e, a.slope), 1.0f, &x);
     }
-}
-
-template <int VEC>
-__device__ __forceinline__ void gat_finish(const GatAggArgs &a, int v, int c, const OnlineSoftmax<VEC> &st)
-{
-    Vec<VEC> b, sk, y;
-    b.load(a.bias + c);
-    if (a.skip != nullptr) sk.load(a.skip + (size_t)v * a.ldskip + c);
-#pragma unroll
-    for (int i = 0; i < VEC; i++) {
-        float t = st.acc.v[i] / st.s + b.v[i];
-        if (a.skip != nullptr) t += sk.v[i];
-        y.v[i] = act_apply_compact(a.act, t);
-    }
-    y.store(a.out + (size_t)v * a.ldo + c);
 }
 
 template <int VEC, int LPR, bool EDGE>
@@ -1059,14 +1105,14 @@ __global__ void __launch_bounds__(256) gat_agg_kernel(const GatAggArgs a)
         const int v = (int)row0 + sub;
         if (v >= a.n) continue;
         const int deg = __ldg(a.in_deg + v);
-        if (a.n_heavy > 0 && deg > a.heavy_threshold) continue;  // the heavy-row kernels do these
+        if (a.heavy.n > 0 && deg > a.heavy.threshold) continue;  // the heavy-row kernels do these
         const int off = __ldg(a.offsets + v);
         for (int c = lg * VEC; c < HC; c += LPR * VEC) {
             const int hd = c / a.C;
             OnlineSoftmax<VEC> st;
             const float adst = gat_self<VEC, EDGE>(a, v, c, hd, st);
             gat_gather<VEC, EDGE>(a, v, off, 0, deg, c, hd, adst, st);
-            gat_finish(a, v, c, st);
+            attn_finish(a, v, c, st.acc[0], st.s);
         }
     }
 }
@@ -1079,25 +1125,21 @@ __global__ void __launch_bounds__(256) gat_heavy_chunk_kernel(const GatAggArgs a
     const int warp_global = blockIdx.x * warps_per_block + (threadIdx.x >> 5);
     const int warp_stride = gridDim.x * warps_per_block;
     const int HC = a.H * a.C;
-    for (int chunk = warp_global; chunk < a.heavy_chunks; chunk += warp_stride) {
-        const int h = __ldg(a.heavy_chunk_row + chunk);
-        const int v = __ldg(a.heavy_rows + h);
-        const int j = chunk - __ldg(a.heavy_chunk_base + h);
+    for (int chunk = warp_global; chunk < a.heavy.chunks; chunk += warp_stride) {
+        const int h = __ldg(a.heavy.chunk_row + chunk);
+        const int v = __ldg(a.heavy.rows + h);
+        const int j = chunk - __ldg(a.heavy.chunk_base + h);
         const int deg = __ldg(a.in_deg + v);
         const int off = __ldg(a.offsets + v);
         const int k0 = j * kHeavyChunk, k1 = min(deg, k0 + kHeavyChunk);
-        const float *rowv = a.hg + (size_t)v * a.ldg;
-        float *dst = a.heavy_partial + (size_t)chunk * a.ldp;
+        const float *rowv = a.g + (size_t)v * a.ldg;
+        float *dst = a.heavy.partial + (size_t)chunk * a.ldp;
         for (int c = lane * VEC; c < HC; c += 32 * VEC) {
             const int hd = c / a.C;
             OnlineSoftmax<VEC> st;
             st.reset();
             gat_gather<VEC, EDGE>(a, v, off, k0, k1, c, hd, __ldg(rowv + HC + a.H + hd), st);
-            st.acc.store(dst + c);
-            if (c % a.C == 0) {   // one lane per head
-                dst[HC + hd] = st.m;
-                dst[HC + a.H + hd] = st.s;
-            }
+            attn_store_partial<VEC, 1>(a, dst, {hd, {c}, {true}}, c % a.C == 0, st);
         }
     }
 }
@@ -1109,44 +1151,16 @@ __device__ __forceinline__ void gat_heavy_combine(const GatAggArgs &a)
     float *const ranges = reinterpret_cast<float *>(gat_smem4);   // [8][ldp], laid out as the partials
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int HC = a.H * a.C;
-    for (int h = blockIdx.x; h < a.n_heavy; h += gridDim.x) {
-        const int v = __ldg(a.heavy_rows + h);
-        const int deg = __ldg(a.in_deg + v);
-        const int nch = (deg + kHeavyChunk - 1) / kHeavyChunk;
-        const float *src = a.heavy_partial + (size_t)__ldg(a.heavy_chunk_base + h) * a.ldp;
-        const int per = (nch + 7) / 8;
-        const int j0 = min(nch, warp * per), j1 = min(nch, j0 + per);
-        float *mine = ranges + warp * a.ldp;
-        for (int c = lane * VEC; c < HC; c += 32 * VEC) {
-            const int hd = c / a.C;
-            OnlineSoftmax<VEC> st;
-            st.reset();
-            for (int j = j0; j < j1; j++) {
-                const float *p = src + (size_t)j * a.ldp;
-                Vec<VEC> t;
-                t.load_rw(p + c);
-                st.merge(p[HC + hd], p[HC + a.H + hd], t);
-            }
-            st.acc.store(mine + c);
-            if (c % a.C == 0) {
-                mine[HC + hd] = st.m;
-                mine[HC + a.H + hd] = st.s;
-            }
-        }
+    for (int h = blockIdx.x; h < a.heavy.n; h += gridDim.x) {
+        const int v = attn_combine_chunks<VEC>(a, h, ranges);
         __syncthreads();
         if (warp == 0) {
             for (int c = lane * VEC; c < HC; c += 32 * VEC) {
                 const int hd = c / a.C;
                 OnlineSoftmax<VEC> st;
                 gat_self<VEC, EDGE>(a, v, c, hd, st);
-#pragma unroll 1
-                for (int w = 0; w < 8; w++) {
-                    const float *r = ranges + w * a.ldp;
-                    Vec<VEC> t;
-                    t.load_rw(r + c);
-                    st.merge(r[HC + hd], r[HC + a.H + hd], t);
-                }
-                gat_finish(a, v, c, st);
+                attn_merge_ranges<VEC, 1>(a, ranges, {hd, {c}, {true}}, hd, st);
+                attn_finish(a, v, c, st.acc[0], st.s);
             }
         }
         __syncthreads();
@@ -1167,32 +1181,57 @@ __global__ void __maxnreg__(64) gat_heavy_combine_edge_kernel(const GatAggArgs a
     gat_heavy_combine<VEC, true>(a);
 }
 
-template <int VEC, bool EDGE>
-void launch_gat_lpr(const GatAggArgs &a, int lpr, int grid, cudaStream_t s)
+// the heavy rows of an attention aggregation: the chunk kernel, a warp per chunk, then the combine
+// kernel, a CTA per row with the [8][ldp] range table in shared memory; extra: the kernels' further
+// arguments
+template <typename Args, typename... Extra>
+int launch_attn_heavy(void (*chunk)(Args, Extra...), void (*combine)(Args, Extra...), const Args &a,
+                      cudaStream_t s, int *launches, Extra... extra)
 {
-    switch (lpr) {
-    case 1: gat_agg_kernel<VEC, 1, EDGE><<<grid, 256, 0, s>>>(a); break;
-    case 2: gat_agg_kernel<VEC, 2, EDGE><<<grid, 256, 0, s>>>(a); break;
-    case 4: gat_agg_kernel<VEC, 4, EDGE><<<grid, 256, 0, s>>>(a); break;
-    case 8: gat_agg_kernel<VEC, 8, EDGE><<<grid, 256, 0, s>>>(a); break;
-    case 16: gat_agg_kernel<VEC, 16, EDGE><<<grid, 256, 0, s>>>(a); break;
-    default: gat_agg_kernel<VEC, 32, EDGE><<<grid, 256, 0, s>>>(a); break;
+    const int cap = kNumSMs * 8;   // 8 resident CTAs per SM, grid-stride beyond
+    const int g1 = min((a.heavy.chunks + 7) / 8, cap), g2 = min(a.heavy.n, cap);
+    chunk<<<g1, 256, 0, s>>>(a, extra...);
+    const size_t smem = sizeof(float) * 8 * (size_t)a.ldp;
+    if (smem > 48 * 1024)
+        GNNB_CUDA(cudaFuncSetAttribute(combine, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    combine<<<g2, 256, smem, s>>>(a, extra...);
+    GNNB_CUDA(cudaGetLastError());
+    if (launches) *launches += 2;
+    return GNNB_OK;
+}
+
+// the arguments GAT and GATv2 share (what = the conv's name for the messages)
+int check_attn_args(const AttnAggArgs &a, const char *what)
+{
+    const int HC = a.H * a.C;
+    GNNB_REQUIRE(a.H >= 1 && a.C >= 1 && a.ldo >= HC && a.bias != nullptr &&
+                     (a.skip == nullptr || a.ldskip >= HC),
+                 std::string(what) + " aggregation: bad arguments");
+    if (a.heavy.n > 0) {
+        GNNB_TRY(check_heavy(a.heavy));
+        GNNB_REQUIRE(a.ldp >= HC + 2 * a.H && a.ldp % 4 == 0,
+                     std::string(what) + " heavy rows: bad partial stride");
     }
+    return GNNB_OK;
+}
+
+// float4 lanes: C % 4 == 0, and g, output, bias and skip 16-byte aligned with strides of whole float4s
+bool attn_v4(const AttnAggArgs &a)
+{
+    return (a.C % 4 == 0) && (a.ldg % 4 == 0) && aligned16(a.g) && (a.ldo % 4 == 0) && aligned16(a.out) &&
+           aligned16(a.bias) && (a.skip == nullptr || ((a.ldskip % 4 == 0) && aligned16(a.skip)));
 }
 
 template <int VEC, bool EDGE>
-int launch_gat_heavy(const GatAggArgs &a, cudaStream_t s)
+int launch_gat_variant(const GatAggArgs &a, int lpr, cudaStream_t s, int *launches)
 {
-    const int cap = kNumSMs * 8;   // 8 resident CTAs per SM, grid-stride beyond
-    const int g1 = min((a.heavy_chunks + 7) / 8, cap), g2 = min(a.n_heavy, cap);
-    gat_heavy_chunk_kernel<VEC, EDGE><<<g1, 256, 0, s>>>(a);
-    const size_t smem = sizeof(float) * 8 * (size_t)a.ldp;
-    void (*combine)(const GatAggArgs) =
-        EDGE ? gat_heavy_combine_edge_kernel<VEC> : gat_heavy_combine_kernel<VEC>;
-    if (smem > 48 * 1024)
-        GNNB_CUDA(cudaFuncSetAttribute(combine, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    combine<<<g2, 256, smem, s>>>(a);
-    return GNNB_OK;
+    const int grid = row_grid(a.n, lpr);
+    with_lpr(lpr, [&](auto L) { gat_agg_kernel<VEC, L, EDGE><<<grid, 256, 0, s>>>(a); });
+    GNNB_CUDA(cudaGetLastError());
+    if (launches) ++*launches;
+    if (a.heavy.n == 0) return GNNB_OK;
+    auto combine = EDGE ? gat_heavy_combine_edge_kernel<VEC> : gat_heavy_combine_kernel<VEC>;
+    return launch_attn_heavy(gat_heavy_chunk_kernel<VEC, EDGE>, combine, a, s, launches);
 }
 
 }  // namespace
@@ -1200,39 +1239,19 @@ int launch_gat_heavy(const GatAggArgs &a, cudaStream_t s)
 int launch_gat_agg(const GatAggArgs &a, cudaStream_t s, int *launches)
 {
     if (a.n <= 0) return GNNB_OK;
-    const int HC = a.H * a.C;
-    GNNB_REQUIRE(a.H >= 1 && a.C >= 1 && a.ldg >= HC + 2 * a.H && a.ldo >= HC && a.bias != nullptr &&
-                     (a.skip == nullptr || a.ldskip >= HC),
-                 "gat aggregation: bad arguments");
-    const bool v4 = (a.C % 4 == 0) && (a.ldg % 4 == 0) && (a.ldo % 4 == 0) && aligned16(a.hg) &&
-                    aligned16(a.out) && aligned16(a.bias) &&
-                    (a.skip == nullptr || ((a.ldskip % 4 == 0) && aligned16(a.skip)));
-    const int vec = v4 ? 4 : 1;
-    int lpr = 1;
-    while (lpr < 32 && lpr * vec < HC) lpr *= 2;
-    const int rows_per_block = 8 * (32 / lpr);
-    int64_t grid64 = ceil_div64(a.n, rows_per_block);
-    const int64_t cap = (int64_t)kNumSMs * 8 * 4;
-    const int grid = (int)(grid64 < cap ? grid64 : cap);
+    GNNB_TRY(check_attn_args(a, "gat"));
+    GNNB_REQUIRE(a.ldg >= a.H * a.C + 2 * a.H, "gat aggregation: bad arguments");
     const bool edge = a.elog != nullptr;
     if (edge) GNNB_REQUIRE(a.self_elog != nullptr && a.ldl >= a.H, "gat aggregation: bad edge logits");
+    const bool v4 = attn_v4(a);
+    const int vec = v4 ? 4 : 1;
+    int lpr = 1;
+    while (lpr < 32 && lpr * vec < a.H * a.C) lpr *= 2;
     if (vec == 4)
-        edge ? launch_gat_lpr<4, true>(a, lpr, grid, s) : launch_gat_lpr<4, false>(a, lpr, grid, s);
-    else
-        edge ? launch_gat_lpr<1, true>(a, lpr, grid, s) : launch_gat_lpr<1, false>(a, lpr, grid, s);
-    GNNB_CUDA(cudaGetLastError());
-    if (launches) ++*launches;
-    if (a.n_heavy > 0) {
-        GNNB_REQUIRE(a.heavy_rows != nullptr && a.heavy_partial != nullptr && a.heavy_chunks > 0 &&
-                         a.heavy_chunk_base != nullptr && a.heavy_chunk_row != nullptr &&
-                         a.ldp >= HC + 2 * a.H && a.ldp % 4 == 0,
-                     "gat heavy rows: row list / partial buffer missing");
-        GNNB_TRY(vec == 4 ? (edge ? launch_gat_heavy<4, true>(a, s) : launch_gat_heavy<4, false>(a, s))
-                          : (edge ? launch_gat_heavy<1, true>(a, s) : launch_gat_heavy<1, false>(a, s)));
-        GNNB_CUDA(cudaGetLastError());
-        if (launches) *launches += 2;
-    }
-    return GNNB_OK;
+        return edge ? launch_gat_variant<4, true>(a, lpr, s, launches)
+                    : launch_gat_variant<4, false>(a, lpr, s, launches);
+    return edge ? launch_gat_variant<1, true>(a, lpr, s, launches)
+                : launch_gat_variant<1, false>(a, lpr, s, launches);
 }
 
 // Edge logits of every layer and head, once per run (kernels.h).  LPR lanes per destination row; the
@@ -1310,18 +1329,8 @@ int launch_gat_edge_logits(const GatEdgeLogitsArgs &a, int avg_deg, cudaStream_t
     const size_t smem_w = sizeof(float) * (size_t)a.LH * a.edge_dim;
     const bool w_smem = smem_w <= 48 * 1024;
     const size_t smem = w_smem ? smem_w : 0;
-    const int rows_per_block = 8 * (32 / lpr);
-    const int64_t grid64 = ceil_div64(a.n, rows_per_block);
-    const int64_t cap = (int64_t)kNumSMs * 8;
-    const int grid = (int)(grid64 < cap ? grid64 : cap);
-    switch (lpr) {
-    case 1: gat_edge_logits_kernel<1><<<grid, 256, smem, s>>>(a, w_smem); break;
-    case 2: gat_edge_logits_kernel<2><<<grid, 256, smem, s>>>(a, w_smem); break;
-    case 4: gat_edge_logits_kernel<4><<<grid, 256, smem, s>>>(a, w_smem); break;
-    case 8: gat_edge_logits_kernel<8><<<grid, 256, smem, s>>>(a, w_smem); break;
-    case 16: gat_edge_logits_kernel<16><<<grid, 256, smem, s>>>(a, w_smem); break;
-    default: gat_edge_logits_kernel<32><<<grid, 256, smem, s>>>(a, w_smem); break;
-    }
+    const int grid = row_grid(a.n, lpr, (int64_t)kNumSMs * 8);
+    with_lpr(lpr, [&](auto L) { gat_edge_logits_kernel<L><<<grid, 256, smem, s>>>(a, w_smem); });
     GNNB_CUDA(cudaGetLastError());
     if (launches) ++*launches;
     return GNNB_OK;
@@ -1343,65 +1352,32 @@ int launch_gat_edge_logits(const GatEdgeLogitsArgs &a, int avg_deg, cudaStream_t
 // groups of a pass past the last head, contribute 0 but run the same shuffles: every shuffle's mask
 // is the row's sub-warp, whose lanes all reach it (rows of one warp differ in degree).
 //
-// The online softmax, the self term first and the skipping of entries equal to v are GAT's.  With
-// edge features each edge's projection is computed where it is consumed from ef_sorted[slot] and
-// W_e^T (staged in shared memory when it fits), never materialised.  Heavy rows are GAT's chunk /
-// fixed-order combine scheme.  The kernels declare one resident CTA per SM as their minimum: ptxas's
-// own register choice under __launch_bounds__(256) spilled them.  Algorithmic bytes per layer:
-// E (4 + 4HC [+ 4 lde]) + N (8 + 8HC + 4HC [+ 4HC skip] [+ 4 lde]).
+// The online softmax (OnlineSoftmax with NJ groups), the self term first and the skipping of entries
+// equal to v are GAT's.  With edge features each edge's projection is computed where it is consumed
+// from ef_sorted[slot] and W_e^T (staged in shared memory when it fits), never materialised.  Heavy
+// rows are GAT's chunk / fixed-order combine scheme (attn_store_partial, attn_combine_chunks,
+// attn_merge_ranges, launch_attn_heavy).  The kernels declare one resident CTA per SM as their
+// minimum: ptxas's own register choice under __launch_bounds__(256) spilled them.  Algorithmic bytes
+// per layer: E (4 + 4HC [+ 4 lde]) + N (8 + 8HC + 4HC [+ 4HC skip] [+ 4 lde]).
 namespace {
 
+// one lane's share of one head: its columns (AttnCols), and xr_v and att for them
 template <int VEC, int NJ>
-struct Gatv2State {
-    float m, s;
-    float acc[NJ][VEC];
-    __device__ __forceinline__ void reset()
-    {
-        m = -INFINITY;
-        s = 0.0f;
-#pragma unroll
-        for (int j = 0; j < NJ; j++)
-#pragma unroll
-            for (int i = 0; i < VEC; i++) acc[j][i] = 0.0f;
-    }
-    // OnlineSoftmax::merge over the lane's NJ column groups
-    __device__ __forceinline__ void merge(float m2, float s2, const float (&acc2)[NJ][VEC])
-    {
-        if (m2 == -INFINITY) return;
-        const float mn = fmaxf(m, m2);
-        const float r = expf(m - mn), p = expf(m2 - mn);
-        s = fmaf(s, r, s2 * p);
-#pragma unroll
-        for (int j = 0; j < NJ; j++)
-#pragma unroll
-            for (int i = 0; i < VEC; i++) acc[j][i] = fmaf(acc[j][i], r, acc2[j][i] * p);
-        m = mn;
-    }
-};
-
-// one lane's share of one head: columns col[j] .. col[j] + VEC of the head (valid[j]), xr_v and att
-template <int VEC, int NJ>
-struct Gatv2Lane {
-    int hd;
-    int col[NJ];
-    bool valid[NJ];
-    float xr[NJ][VEC], att[NJ][VEC];
+struct Gatv2Lane : AttnCols<NJ> {
+    Vec<VEC> xr[NJ], att[NJ];
 };
 
 template <int VEC, int NJ>
-__device__ __forceinline__ void gatv2_load(const float *row, const Gatv2Lane<VEC, NJ> &ln,
-                                           float (&x)[NJ][VEC])
+__device__ __forceinline__ void gatv2_load(const float *row, const AttnCols<NJ> &cl, Vec<VEC> (&x)[NJ])
 {
 #pragma unroll
     for (int j = 0; j < NJ; j++) {
-        Vec<VEC> t;
-        if (ln.valid[j]) t.load(row + ln.col[j]);
-        else {
+        if (cl.valid[j]) {
+            x[j].load(row + cl.col[j]);
+        } else {
 #pragma unroll
-            for (int i = 0; i < VEC; i++) t.v[i] = 0.0f;
+            for (int i = 0; i < VEC; i++) x[j].v[i] = 0.0f;
         }
-#pragma unroll
-        for (int i = 0; i < VEC; i++) x[j][i] = t.v[i];
     }
 }
 
@@ -1419,10 +1395,10 @@ __device__ __forceinline__ Gatv2Lane<VEC, NJ> gatv2_lane(const Gatv2AggArgs &a, 
         ln.col[j] = hd * a.C + cl;
     }
     const int HC = a.H * a.C;
-    Gatv2Lane<VEC, NJ> sh = ln;   // the same columns, shifted to xr
+    AttnCols<NJ> sh = ln;   // the same columns, shifted to xr
 #pragma unroll
     for (int j = 0; j < NJ; j++) sh.col[j] += HC;
-    gatv2_load<VEC, NJ>(a.xlr + (size_t)v * a.ldg, sh, ln.xr);
+    gatv2_load<VEC, NJ>(a.g + (size_t)v * a.ldg, sh, ln.xr);
     gatv2_load<VEC, NJ>(a.att, ln, ln.att);
     return ln;
 }
@@ -1430,7 +1406,7 @@ __device__ __forceinline__ Gatv2Lane<VEC, NJ> gatv2_lane(const Gatv2AggArgs &a, 
 // z += ef W_e^T for the lane's columns: ef one row of lde floats (edge_dim used), We [edge_dim][ldw]
 template <int VEC, int NJ>
 __device__ __forceinline__ void gatv2_edge_proj(const Gatv2AggArgs &a, const float *We, const float *ef,
-                                                const Gatv2Lane<VEC, NJ> &ln, float (&z)[NJ][VEC])
+                                                const Gatv2Lane<VEC, NJ> &ln, Vec<VEC> (&z)[NJ])
 {
     for (int j0 = 0; j0 < a.edge_dim; j0 += 4) {
         const float4 e4 = __ldg(reinterpret_cast<const float4 *>(ef + j0));
@@ -1443,7 +1419,7 @@ __device__ __forceinline__ void gatv2_edge_proj(const Gatv2AggArgs &a, const flo
                 for (int j = 0; j < NJ; j++) {
                     if (!ln.valid[j]) continue;
 #pragma unroll
-                    for (int i = 0; i < VEC; i++) z[j][i] = fmaf(wr[ln.col[j] + i], ej, z[j][i]);
+                    for (int i = 0; i < VEC; i++) z[j].v[i] = fmaf(wr[ln.col[j] + i], ej, z[j].v[i]);
                 }
             }
         }
@@ -1453,14 +1429,14 @@ __device__ __forceinline__ void gatv2_edge_proj(const Gatv2AggArgs &a, const flo
 // the lane's partial dot product <att, LeakyReLU(xl + xr + ep)> (columns past C hold att = 0)
 template <int VEC, int NJ>
 __device__ __forceinline__ float gatv2_partial(const Gatv2AggArgs &a, const Gatv2Lane<VEC, NJ> &ln,
-                                               const float (&xl)[NJ][VEC], const float (&ep)[NJ][VEC])
+                                               const Vec<VEC> (&xl)[NJ], const Vec<VEC> (&ep)[NJ])
 {
     float part = 0.0f;
 #pragma unroll
     for (int j = 0; j < NJ; j++)
 #pragma unroll
         for (int i = 0; i < VEC; i++)
-            part = fmaf(ln.att[j][i], leaky_relu(xl[j][i] + ln.xr[j][i] + ep[j][i], a.slope), part);
+            part = fmaf(ln.att[j].v[i], leaky_relu(xl[j].v[i] + ln.xr[j].v[i] + ep[j].v[i], a.slope), part);
     return part;
 }
 
@@ -1470,25 +1446,27 @@ __device__ __forceinline__ float gatv2_head_sum(float part, unsigned mask, int G
     return part;
 }
 
+template <int VEC, int NJ>
+__device__ __forceinline__ void gatv2_zero(Vec<VEC> (&x)[NJ])
+{
+#pragma unroll
+    for (int j = 0; j < NJ; j++)
+#pragma unroll
+        for (int i = 0; i < VEC; i++) x[j].v[i] = 0.0f;
+}
+
 // the self term of row v: logit from xl_v + xr_v (+ self_attr_v W_e^T), weight 1, message xl_v
 template <int VEC, int NJ, bool EDGE>
 __device__ __forceinline__ void gatv2_self(const Gatv2AggArgs &a, const float *We, int v,
                                            const Gatv2Lane<VEC, NJ> &ln, unsigned mask, int G,
-                                           Gatv2State<VEC, NJ> &st)
+                                           OnlineSoftmax<VEC, NJ> &st)
 {
-    float xl[NJ][VEC], ep[NJ][VEC];
-    gatv2_load<VEC, NJ>(a.xlr + (size_t)v * a.ldg, ln, xl);
-#pragma unroll
-    for (int j = 0; j < NJ; j++)
-#pragma unroll
-        for (int i = 0; i < VEC; i++) ep[j][i] = 0.0f;
+    Vec<VEC> ep[NJ];
+    gatv2_load<VEC, NJ>(a.g + (size_t)v * a.ldg, ln, st.acc);
+    gatv2_zero<VEC, NJ>(ep);
     if (EDGE) gatv2_edge_proj<VEC, NJ>(a, We, a.self_attr + (size_t)v * a.lde, ln, ep);
-    st.m = gatv2_head_sum(gatv2_partial<VEC, NJ>(a, ln, xl, ep), mask, G);
+    st.m = gatv2_head_sum(gatv2_partial<VEC, NJ>(a, ln, st.acc, ep), mask, G);
     st.s = 1.0f;
-#pragma unroll
-    for (int j = 0; j < NJ; j++)
-#pragma unroll
-        for (int i = 0; i < VEC; i++) st.acc[j][i] = xl[j][i];
 }
 
 // neighbor slots [k0, k1) of row v (entries equal to v skipped, uniformly over the sub-warp), U
@@ -1496,24 +1474,22 @@ __device__ __forceinline__ void gatv2_self(const Gatv2AggArgs &a, const float *W
 template <int VEC, int NJ, bool EDGE>
 __device__ __forceinline__ void gatv2_gather(const Gatv2AggArgs &a, const float *We, int v, int off,
                                              int k0, int k1, const Gatv2Lane<VEC, NJ> &ln,
-                                             unsigned mask, int G, Gatv2State<VEC, NJ> &st)
+                                             unsigned mask, int G, OnlineSoftmax<VEC, NJ> &st)
 {
     constexpr int U = NJ == 1 ? 4 : 2;
     int k = k0;
 #pragma unroll 1
     for (; k + U <= k1; k += U) {
         int u[U];
-        float xl[U][NJ][VEC], ep[U][NJ][VEC], e[U];
+        Vec<VEC> xl[U][NJ], ep[U][NJ];
+        float e[U];
 #pragma unroll
         for (int q = 0; q < U; q++) u[q] = __ldg(a.nbr + off + k + q);
 #pragma unroll
-        for (int q = 0; q < U; q++) gatv2_load<VEC, NJ>(a.xlr + (size_t)u[q] * a.ldg, ln, xl[q]);
+        for (int q = 0; q < U; q++) gatv2_load<VEC, NJ>(a.g + (size_t)u[q] * a.ldg, ln, xl[q]);
 #pragma unroll
         for (int q = 0; q < U; q++) {
-#pragma unroll
-            for (int j = 0; j < NJ; j++)
-#pragma unroll
-                for (int i = 0; i < VEC; i++) ep[q][j][i] = 0.0f;
+            gatv2_zero<VEC, NJ>(ep[q]);
             if (EDGE) gatv2_edge_proj<VEC, NJ>(a, We, a.ef_sorted + (size_t)(off + k + q) * a.lde, ln, ep[q]);
             e[q] = gatv2_partial<VEC, NJ>(a, ln, xl[q], ep[q]);
         }
@@ -1528,36 +1504,22 @@ __device__ __forceinline__ void gatv2_gather(const Gatv2AggArgs &a, const float 
     for (; k < k1; k++) {
         const int u = __ldg(a.nbr + off + k);
         if (u == v) continue;
-        float xl[NJ][VEC], ep[NJ][VEC];
-        gatv2_load<VEC, NJ>(a.xlr + (size_t)u * a.ldg, ln, xl);
-#pragma unroll
-        for (int j = 0; j < NJ; j++)
-#pragma unroll
-            for (int i = 0; i < VEC; i++) ep[j][i] = 0.0f;
+        Vec<VEC> xl[NJ], ep[NJ];
+        gatv2_load<VEC, NJ>(a.g + (size_t)u * a.ldg, ln, xl);
+        gatv2_zero<VEC, NJ>(ep);
         if (EDGE) gatv2_edge_proj<VEC, NJ>(a, We, a.ef_sorted + (size_t)(off + k) * a.lde, ln, ep);
         st.merge(gatv2_head_sum(gatv2_partial<VEC, NJ>(a, ln, xl, ep), mask, G), 1.0f, xl);
     }
 }
 
+// the epilogue of the lane's valid column groups (none in an idle group)
 template <int VEC, int NJ>
 __device__ __forceinline__ void gatv2_finish(const Gatv2AggArgs &a, int v, const Gatv2Lane<VEC, NJ> &ln,
-                                             const Gatv2State<VEC, NJ> &st)
+                                             const OnlineSoftmax<VEC, NJ> &st)
 {
 #pragma unroll
-    for (int j = 0; j < NJ; j++) {
-        if (!ln.valid[j]) continue;
-        const int c = ln.col[j];
-        Vec<VEC> b, sk, y;
-        b.load(a.bias + c);
-        if (a.skip != nullptr) sk.load(a.skip + (size_t)v * a.ldskip + c);
-#pragma unroll
-        for (int i = 0; i < VEC; i++) {
-            float t = st.acc[j][i] / st.s + b.v[i];
-            if (a.skip != nullptr) t += sk.v[i];
-            y.v[i] = act_apply_compact(a.act, t);
-        }
-        y.store(a.out + (size_t)v * a.ldo + c);
-    }
+    for (int j = 0; j < NJ; j++)
+        if (ln.valid[j]) attn_finish(a, v, ln.col[j], st.acc[j], st.s);
 }
 
 // W_e^T staged in shared memory (w_smem) or read in place
@@ -1590,14 +1552,14 @@ __global__ void __launch_bounds__(256, 1) gatv2_agg_kernel(const Gatv2AggArgs a,
         const int v = (int)row0 + sub;
         if (v >= a.n) continue;
         const int deg = __ldg(a.in_deg + v);
-        if (a.n_heavy > 0 && deg > a.heavy_threshold) continue;  // the heavy-row kernels do these
+        if (a.heavy.n > 0 && deg > a.heavy.threshold) continue;  // the heavy-row kernels do these
         const int off = __ldg(a.offsets + v);
         for (int h0 = 0; h0 < a.H; h0 += heads_per_pass) {
             const Gatv2Lane<VEC, NJ> ln = gatv2_lane<VEC, NJ>(a, v, h0 + grp, hl, G);
-            Gatv2State<VEC, NJ> st;
+            OnlineSoftmax<VEC, NJ> st;
             gatv2_self<VEC, NJ, EDGE>(a, We, v, ln, mask, G, st);
             gatv2_gather<VEC, NJ, EDGE>(a, We, v, off, 0, deg, ln, mask, G, st);
-            if (ln.hd < a.H) gatv2_finish<VEC, NJ>(a, v, ln, st);
+            gatv2_finish<VEC, NJ>(a, v, ln, st);
         }
     }
 }
@@ -1612,90 +1574,42 @@ __global__ void __launch_bounds__(256, 1) gatv2_heavy_chunk_kernel(const Gatv2Ag
     const int warps_per_block = blockDim.x >> 5;
     const int warp_global = blockIdx.x * warps_per_block + (threadIdx.x >> 5);
     const int warp_stride = gridDim.x * warps_per_block;
-    const int HC = a.H * a.C;
-    for (int chunk = warp_global; chunk < a.heavy_chunks; chunk += warp_stride) {
-        const int h = __ldg(a.heavy_chunk_row + chunk);
-        const int v = __ldg(a.heavy_rows + h);
-        const int j = chunk - __ldg(a.heavy_chunk_base + h);
+    for (int chunk = warp_global; chunk < a.heavy.chunks; chunk += warp_stride) {
+        const int h = __ldg(a.heavy.chunk_row + chunk);
+        const int v = __ldg(a.heavy.rows + h);
+        const int j = chunk - __ldg(a.heavy.chunk_base + h);
         const int deg = __ldg(a.in_deg + v);
         const int off = __ldg(a.offsets + v);
         const int k0 = j * kHeavyChunk, k1 = min(deg, k0 + kHeavyChunk);
-        float *dst = a.heavy_partial + (size_t)chunk * a.ldp;
+        float *dst = a.heavy.partial + (size_t)chunk * a.ldp;
         for (int h0 = 0; h0 < a.H; h0 += heads_per_pass) {
             const Gatv2Lane<VEC, NJ> ln = gatv2_lane<VEC, NJ>(a, v, h0 + grp, hl, G);
-            Gatv2State<VEC, NJ> st;
+            OnlineSoftmax<VEC, NJ> st;
             st.reset();
             gatv2_gather<VEC, NJ, EDGE>(a, a.We_t, v, off, k0, k1, ln, 0xffffffffu, G, st);
-#pragma unroll
-            for (int q = 0; q < NJ; q++) {
-                if (!ln.valid[q]) continue;
-#pragma unroll
-                for (int i = 0; i < VEC; i++) dst[ln.col[q] + i] = st.acc[q][i];
-            }
-            if (hl == 0 && ln.hd < a.H) {   // one lane per head
-                dst[HC + ln.hd] = st.m;
-                dst[HC + a.H + ln.hd] = st.s;
-            }
+            attn_store_partial<VEC, NJ>(a, dst, ln, hl == 0 && ln.hd < a.H, st);
         }
     }
 }
 
-// one CTA per heavy row: 8 warps merge contiguous chunk ranges column by column, then warp 0 starts
-// from the self term and merges the 8 range results in warp order (a fixed order)
+// one CTA per heavy row: combine steps 1 and 2 (GAT's), warp 0 starting from the self term
 template <int VEC, int NJ, bool EDGE>
 __global__ void __launch_bounds__(256, 1) gatv2_heavy_combine_kernel(const Gatv2AggArgs a, int G)
 {
     extern __shared__ float4 gatv2_comb_smem4[];
     float *const ranges = reinterpret_cast<float *>(gatv2_comb_smem4);   // [8][ldp], as the partials
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int HC = a.H * a.C;
     const int grp = lane / G, hl = lane % G, heads_per_pass = 32 / G;
-    for (int h = blockIdx.x; h < a.n_heavy; h += gridDim.x) {
-        const int v = __ldg(a.heavy_rows + h);
-        const int deg = __ldg(a.in_deg + v);
-        const int nch = (deg + kHeavyChunk - 1) / kHeavyChunk;
-        const float *src = a.heavy_partial + (size_t)__ldg(a.heavy_chunk_base + h) * a.ldp;
-        const int per = (nch + 7) / 8;
-        const int j0 = min(nch, warp * per), j1 = min(nch, j0 + per);
-        float *mine = ranges + warp * a.ldp;
-        for (int c = lane * VEC; c < HC; c += 32 * VEC) {
-            const int hd = c / a.C;
-            Gatv2State<VEC, 1> st;
-            st.reset();
-            for (int j = j0; j < j1; j++) {
-                const float *p = src + (size_t)j * a.ldp;
-                Vec<VEC> t;
-                t.load_rw(p + c);
-                float t2[1][VEC];
-#pragma unroll
-                for (int i = 0; i < VEC; i++) t2[0][i] = t.v[i];
-                st.merge(p[HC + hd], p[HC + a.H + hd], t2);
-            }
-#pragma unroll
-            for (int i = 0; i < VEC; i++) mine[c + i] = st.acc[0][i];
-            if (c % a.C == 0) {
-                mine[HC + hd] = st.m;
-                mine[HC + a.H + hd] = st.s;
-            }
-        }
+    for (int h = blockIdx.x; h < a.heavy.n; h += gridDim.x) {
+        const int v = attn_combine_chunks<VEC>(a, h, ranges);
         __syncthreads();
         if (warp == 0) {
             for (int h0 = 0; h0 < a.H; h0 += heads_per_pass) {
                 const Gatv2Lane<VEC, NJ> ln = gatv2_lane<VEC, NJ>(a, v, h0 + grp, hl, G);
-                Gatv2State<VEC, NJ> st;
+                OnlineSoftmax<VEC, NJ> st;
                 gatv2_self<VEC, NJ, EDGE>(a, a.We_t, v, ln, 0xffffffffu, G, st);
-                const int hd = ln.hd < a.H ? ln.hd : 0;
-#pragma unroll 1
-                for (int w = 0; w < 8; w++) {
-                    const float *r = ranges + w * a.ldp;
-                    float t[NJ][VEC];
-#pragma unroll
-                    for (int q = 0; q < NJ; q++)
-#pragma unroll
-                        for (int i = 0; i < VEC; i++) t[q][i] = ln.valid[q] ? r[ln.col[q] + i] : 0.0f;
-                    st.merge(r[HC + hd], r[HC + a.H + hd], t);
-                }
-                if (ln.hd < a.H) gatv2_finish<VEC, NJ>(a, v, ln, st);
+                attn_merge_ranges<VEC, NJ>(a, ranges, ln, ln.hd < a.H ? ln.hd : 0, st);
+                gatv2_finish<VEC, NJ>(a, v, ln, st);
             }
         }
         __syncthreads();
@@ -1703,27 +1617,16 @@ __global__ void __launch_bounds__(256, 1) gatv2_heavy_combine_kernel(const Gatv2
 }
 
 template <int VEC, int NJ, bool EDGE>
-int launch_gatv2_variant(const Gatv2AggArgs &a, int lpr, int G, int grid, size_t smem, cudaStream_t s,
-                         int *launches)
+int launch_gatv2_variant(const Gatv2AggArgs &a, int lpr, int G, size_t smem, cudaStream_t s, int *launches)
 {
     auto k = gatv2_agg_kernel<VEC, NJ, EDGE>;
     if (smem > 48 * 1024) GNNB_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k<<<grid, 256, smem, s>>>(a, lpr, G, smem > 0);
+    k<<<row_grid(a.n, lpr), 256, smem, s>>>(a, lpr, G, smem > 0);
     GNNB_CUDA(cudaGetLastError());
     if (launches) ++*launches;
-    if (a.n_heavy > 0) {
-        const int cap = kNumSMs * 8;   // 8 resident CTAs per SM, grid-stride beyond
-        const int g1 = min((a.heavy_chunks + 7) / 8, cap), g2 = min(a.n_heavy, cap);
-        gatv2_heavy_chunk_kernel<VEC, NJ, EDGE><<<g1, 256, 0, s>>>(a, G);
-        const size_t csmem = sizeof(float) * 8 * (size_t)a.ldp;
-        auto combine = gatv2_heavy_combine_kernel<VEC, NJ, EDGE>;
-        if (csmem > 48 * 1024)
-            GNNB_CUDA(cudaFuncSetAttribute(combine, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)csmem));
-        combine<<<g2, 256, csmem, s>>>(a, G);
-        GNNB_CUDA(cudaGetLastError());
-        if (launches) *launches += 2;
-    }
-    return GNNB_OK;
+    if (a.heavy.n == 0) return GNNB_OK;
+    return launch_attn_heavy(gatv2_heavy_chunk_kernel<VEC, NJ, EDGE>,
+                             gatv2_heavy_combine_kernel<VEC, NJ, EDGE>, a, s, launches, G);
 }
 
 __global__ void gatv2_self_attr_kernel(const float *__restrict__ ef, int lde, int edge_dim,
@@ -1756,19 +1659,15 @@ int launch_gatv2_agg(const Gatv2AggArgs &a, cudaStream_t s, int *launches)
 {
     if (a.n <= 0) return GNNB_OK;
     const int HC = a.H * a.C;
-    GNNB_REQUIRE(a.H >= 1 && a.C >= 1 && a.ldg >= 2 * HC && a.ldo >= HC && a.bias != nullptr &&
-                     a.att != nullptr && (a.skip == nullptr || a.ldskip >= HC),
-                 "gatv2 aggregation: bad arguments");
+    GNNB_TRY(check_attn_args(a, "gatv2"));
+    GNNB_REQUIRE(a.ldg >= 2 * HC && a.att != nullptr, "gatv2 aggregation: bad arguments");
     const bool edge = a.ef_sorted != nullptr;
     if (edge)
         GNNB_REQUIRE(a.self_attr != nullptr && a.We_t != nullptr && a.edge_dim >= 1 &&
                          a.edge_dim <= kGineMaxEdgeDim && a.lde % 4 == 0 && a.lde >= a.edge_dim &&
                          a.ldw % 4 == 0 && a.ldw >= HC && aligned16(a.ef_sorted) && aligned16(a.self_attr),
                      "gatv2 aggregation: bad edge features");
-    const bool v4 = (a.C % 4 == 0) && (a.ldg % 4 == 0) && (a.ldo % 4 == 0) && aligned16(a.xlr) &&
-                    aligned16(a.out) && aligned16(a.bias) && aligned16(a.att) &&
-                    (a.skip == nullptr || ((a.ldskip % 4 == 0) && aligned16(a.skip))) &&
-                    (!edge || aligned16(a.We_t));
+    const bool v4 = attn_v4(a) && aligned16(a.att) && (!edge || aligned16(a.We_t));
     const int vec = v4 ? 4 : 1;
     const int cg = (a.C + vec - 1) / vec;   // VEC-column groups per head
     int G = 1;
@@ -1780,30 +1679,21 @@ int launch_gatv2_agg(const Gatv2AggArgs &a, cudaStream_t s, int *launches)
                               std::to_string(kGatv2MaxHeadWidth1) + ")");
     int lpr = G;
     while (lpr < 32 && lpr < G * a.H) lpr *= 2;
-    const int rows_per_block = 8 * (32 / lpr);
-    const int64_t grid64 = ceil_div64(a.n, rows_per_block);
-    const int64_t cap = (int64_t)kNumSMs * 8 * 4;
-    const int grid = (int)(grid64 < cap ? grid64 : cap);
     // W_e^T in shared memory when it fits (edge_dim 64 at H*C = 256: 64 KB), as the GINE aggregation
     const size_t w_bytes = edge ? sizeof(float) * (size_t)a.edge_dim * a.ldw : 0;
     const size_t smem = w_bytes <= 200 * 1024 ? w_bytes : 0;
-    if (a.n_heavy > 0)
-        GNNB_REQUIRE(a.heavy_rows != nullptr && a.heavy_partial != nullptr && a.heavy_chunks > 0 &&
-                         a.heavy_chunk_base != nullptr && a.heavy_chunk_row != nullptr &&
-                         a.ldp >= HC + 2 * a.H && a.ldp % 4 == 0,
-                     "gatv2 heavy rows: row list / partial buffer missing");
     if (vec == 4) {
         if (nj == 1)
-            return edge ? launch_gatv2_variant<4, 1, true>(a, lpr, G, grid, smem, s, launches)
-                        : launch_gatv2_variant<4, 1, false>(a, lpr, G, grid, 0, s, launches);
-        return edge ? launch_gatv2_variant<4, 2, true>(a, lpr, G, grid, smem, s, launches)
-                    : launch_gatv2_variant<4, 2, false>(a, lpr, G, grid, 0, s, launches);
+            return edge ? launch_gatv2_variant<4, 1, true>(a, lpr, G, smem, s, launches)
+                        : launch_gatv2_variant<4, 1, false>(a, lpr, G, 0, s, launches);
+        return edge ? launch_gatv2_variant<4, 2, true>(a, lpr, G, smem, s, launches)
+                    : launch_gatv2_variant<4, 2, false>(a, lpr, G, 0, s, launches);
     }
     if (nj == 1)
-        return edge ? launch_gatv2_variant<1, 1, true>(a, lpr, G, grid, smem, s, launches)
-                    : launch_gatv2_variant<1, 1, false>(a, lpr, G, grid, 0, s, launches);
-    return edge ? launch_gatv2_variant<1, 2, true>(a, lpr, G, grid, smem, s, launches)
-                : launch_gatv2_variant<1, 2, false>(a, lpr, G, grid, 0, s, launches);
+        return edge ? launch_gatv2_variant<1, 1, true>(a, lpr, G, smem, s, launches)
+                    : launch_gatv2_variant<1, 1, false>(a, lpr, G, 0, s, launches);
+    return edge ? launch_gatv2_variant<1, 2, true>(a, lpr, G, smem, s, launches)
+                : launch_gatv2_variant<1, 2, false>(a, lpr, G, 0, s, launches);
 }
 
 int launch_gatv2_self_attr(const float *ef_sorted, int lde, int edge_dim, const int32_t *offsets,

@@ -92,6 +92,23 @@ inline size_t hub_l2_budget()
 int compute_dinv(const int32_t *in_deg, float *dinv, int n, cudaStream_t s, int *launches);
 
 // ---------------------------------------------------------------- aggregation (agg.cu)
+// The heavy rows of one aggregation (degree bucketing): rows longer than `threshold` are left to the
+// chunked heavy-row kernels; n == 0 (the zero-initialised block) turns the bucketing off.
+struct HeavyArgs {
+    const int32_t *rows;   // [n] row ids
+    int n;
+    int threshold;
+    float *partial;        // [chunks][...] per-chunk partials, laid out by the aggregation
+    const int32_t *chunk_base, *chunk_row;   // HeavyList::chunk_base / chunk_row
+    int chunks;
+    void set(const HeavyList &hl, float *p)
+    {
+        rows = hl.rows.as<int32_t>(); n = hl.n_heavy;
+        chunk_base = hl.chunk_base.as<int32_t>(); chunk_row = hl.chunk_row.as<int32_t>();
+        chunks = hl.n_chunks; partial = p;
+    }
+};
+
 enum AggMode { AGG_GCN = 0, AGG_GIN = 1, AGG_MEAN = 2, AGG_SUM = 3, AGG_LG = 4 };
 
 struct AggArgs {
@@ -105,18 +122,7 @@ struct AggArgs {
     const float *dinv;     // AGG_GCN fast mode only
     int n;
     float eps;             // AGG_GIN
-    const int32_t *heavy_rows;  // optional list of rows handled by the chunked heavy-row kernels
-    int n_heavy;
-    int heavy_threshold;
-    float *heavy_partial;  // [heavy_chunks][F] chunk sums of the heavy rows
-    const int32_t *heavy_chunk_base, *heavy_chunk_row;
-    int heavy_chunks;
-    void set_heavy(const HeavyList &hl, float *partial)
-    {
-        heavy_rows = hl.rows.as<int32_t>(); n_heavy = hl.n_heavy;
-        heavy_chunk_base = hl.chunk_base.as<int32_t>(); heavy_chunk_row = hl.chunk_row.as<int32_t>();
-        heavy_chunks = hl.n_chunks; heavy_partial = partial;
-    }
+    HeavyArgs heavy;       // partial: [chunks][F] chunk sums
     int row_base;          // row-partitioned graphs: global id of local row 0 (x / dinv are global,
                            // offsets / in_deg / out are local); 0 otherwise
     // ---- FAST-mode extensions (all 0 / null by default)
@@ -171,17 +177,14 @@ int launch_gine_agg_proj(const GineProjAggArgs &a, cudaStream_t s, int *launches
 int launch_permute_edge_rows(const float *src, int dim, const int32_t *idx, int e, float *dst,
                              int ldd, cudaStream_t s, int *launches);
 
-// GAT attention aggregation (PyG GATConv, concat heads, inference).  hg is the output of the layer's
-// one GEMM: per row h (H*C columns, head-major), then a_src [H] and a_dst [H].  Per destination v and
-// head: e_uv = LeakyReLU(a_src[u] + a_dst[v]) over the in-neighbours u != v plus one self term,
-// y_v = act(sum softmax_v(e) h_u + bias (+ skip_v)), written to out.  One gather pass with an online
-// softmax (running max, rescaled sum and accumulator).  Rows longer than heavy_threshold (when a
-// heavy list is given) are cut into kHeavyChunk-neighbour chunks whose (max, sum, accumulator)
-// partials are merged per row in a fixed order.
-struct GatAggArgs {
-    const float *hg;       // [n][ldg]
-    int ldg, H, C;
-    float slope;
+// What the GAT and GATv2 aggregations share: the layer's GEMM output, the attention shape, the
+// epilogue y_v = act(sum softmax_v(e) m_u + bias (+ skip_v)) written to out, the CSR and the heavy
+// rows, whose partials are [heavy.chunks][ldp]: accumulator (H*C), then max [H], sum [H].
+struct AttnAggArgs {
+    const float *g;        // [n][ldg]: GAT [h | a_src | a_dst], GATv2 [xl | xr]
+    int ldg;
+    int H, C;
+    float slope;           // LeakyReLU negative slope
     const float *bias;     // [H*C]
     const float *skip;     // [n][ldskip] or null
     int ldskip;
@@ -190,24 +193,23 @@ struct GatAggArgs {
     int ldo;
     const int32_t *offsets, *nbr, *in_deg;
     int n;
-    const int32_t *heavy_rows;
-    int n_heavy;
-    int heavy_threshold;
-    float *heavy_partial;  // [heavy_chunks][ldp]: accumulator (H*C), then max [H], sum [H]
-    int ldp;               // round_up(H*C + 2H, 4)
-    const int32_t *heavy_chunk_base, *heavy_chunk_row;
-    int heavy_chunks;
+    HeavyArgs heavy;
+    int ldp;               // >= H*C + 2H, multiple of 4
+};
+
+// GAT attention aggregation (PyG GATConv, concat heads, inference).  g is the output of the layer's
+// one GEMM: per row h (H*C columns, head-major), then a_src [H] and a_dst [H].  Per destination v and
+// head: e_uv = LeakyReLU(a_src[u] + a_dst[v]) over the in-neighbours u != v plus one self term,
+// y_v = act(sum softmax_v(e) h_u + bias (+ skip_v)), written to out.  One gather pass with an online
+// softmax (running max, rescaled sum and accumulator).  Rows longer than heavy.threshold (when a
+// heavy list is given) are cut into kHeavyChunk-neighbour chunks whose (max, sum, accumulator)
+// partials are merged per row in a fixed order.
+struct GatAggArgs : AttnAggArgs {
     // edge attention (GATConv with edge_dim), else null: the logits of launch_gat_edge_logits
     // advanced to this layer's H columns; the neighbor logit adds elog[slot][hd], the self term
     // self_elog[v][hd]
     const float *elog, *self_elog;   // [slots][ldl], [n][ldl]
     int ldl;
-    void set_heavy(const HeavyList &hl, float *partial)
-    {
-        heavy_rows = hl.rows.as<int32_t>(); n_heavy = hl.n_heavy;
-        heavy_chunk_base = hl.chunk_base.as<int32_t>(); heavy_chunk_row = hl.chunk_row.as<int32_t>();
-        heavy_chunks = hl.n_chunks; heavy_partial = partial;
-    }
 };
 int launch_gat_agg(const GatAggArgs &a, cudaStream_t s, int *launches);
 
@@ -229,28 +231,17 @@ struct GatEdgeLogitsArgs {
 };
 int launch_gat_edge_logits(const GatEdgeLogitsArgs &a, int avg_deg, cudaStream_t s, int *launches);
 
-// GATv2 attention aggregation (PyG GATv2Conv, concat heads, inference).  xlr holds the layer's two
+// GATv2 attention aggregation (PyG GATv2Conv, concat heads, inference).  g holds the layer's two
 // GEMM outputs per row: xl = x W_l^T + b_l in columns [0, H*C), xr = x W_r^T + b_r in [H*C, 2 H*C).
 // Per destination v and head h, over the in-neighbours u != v plus one self term (u = v):
 // z = xl_u + xr_v (+ e_uv W_e^T), e_uvh = sum_c att_hc LeakyReLU(z_hc), y_v = act(sum softmax_v(e)
 // xl_u + bias (+ skip_v)).  The logit is a dot product over each head's lanes, computed per edge; the
-// online softmax and the heavy-row partials [acc H*C | max H | sum H] are GAT's.
+// online softmax, the epilogue and the heavy-row scheme are GAT's (AttnAggArgs).
 // a head's columns are spread over at most 32 lanes, each holding at most two VEC-column groups
 constexpr int kGatv2MaxHeadWidth = 256;   // C % 4 == 0 (float4 lanes)
 constexpr int kGatv2MaxHeadWidth1 = 64;   // other C (scalar lanes)
-struct Gatv2AggArgs {
-    const float *xlr;      // [n][ldg]
-    int ldg, H, C;
-    float slope;
+struct Gatv2AggArgs : AttnAggArgs {
     const float *att;      // [H*C]
-    const float *bias;     // [H*C]
-    const float *skip;     // [n][ldskip] or null
-    int ldskip;
-    int act;
-    float *out;            // [n][ldo]
-    int ldo;
-    const int32_t *offsets, *nbr, *in_deg;
-    int n;
     // edge features (edge_dim > 0), else ef_sorted null: the edge term of slot k is
     // ef_sorted[k] W_e^T, the self term's self_attr[v] W_e^T
     const float *ef_sorted;  // [slots][lde], neighbor-slot order
@@ -258,19 +249,6 @@ struct Gatv2AggArgs {
     int lde, edge_dim;
     const float *We_t;       // [edge_dim][ldw] (ldw multiple of 4, zero padded)
     int ldw;
-    const int32_t *heavy_rows;
-    int n_heavy;
-    int heavy_threshold;
-    float *heavy_partial;  // [heavy_chunks][ldp]: accumulator (H*C), then max [H], sum [H]
-    int ldp;               // >= H*C + 2H, multiple of 4
-    const int32_t *heavy_chunk_base, *heavy_chunk_row;
-    int heavy_chunks;
-    void set_heavy(const HeavyList &hl, float *partial)
-    {
-        heavy_rows = hl.rows.as<int32_t>(); n_heavy = hl.n_heavy;
-        heavy_chunk_base = hl.chunk_base.as<int32_t>(); heavy_chunk_row = hl.chunk_row.as<int32_t>();
-        heavy_chunks = hl.n_chunks; heavy_partial = partial;
-    }
 };
 int launch_gatv2_agg(const Gatv2AggArgs &a, cudaStream_t s, int *launches);
 // self_attr[v][0..lde) = the mean of ef_sorted[k] over the slots k of row v whose source is not v, in

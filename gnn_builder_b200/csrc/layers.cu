@@ -613,7 +613,7 @@ int halo_agg_part(const AggArgs &a, const int32_t *off, const int32_t *cnt, cons
     } else {
         b.in_deg = cnt + row_begin;
     }
-    b.set_heavy(hc.list, g_part.ws.heavy_partial.as<float>());
+    b.heavy.set(hc.list, g_part.ws.heavy_partial.as<float>());
     b.accumulate = accumulate ? 1 : 0; b.no_finish = finish ? 0 : 1;
     return launch_agg(b, false, s, nullptr);
 }
@@ -781,8 +781,8 @@ extern "C" int gnnb_gcn_conv_partition(int n_local, int row_begin, int n_total, 
     a.mode = AGG_GCN; a.x = x_full; a.ldx = emb_in; a.F = emb_in; a.out = g_part.agg.as<float>();
     a.ldo = lda; a.offsets = offsets_local; a.nbr = neighbor_table_global; a.in_deg = in_degree_local;
     a.dinv = dinv_full; a.n = n_local; a.row_base = row_begin;
-    a.heavy_threshold = heavy_threshold();
-    a.set_heavy(g_part.whole.list, g_part.ws.heavy_partial.as<float>());
+    a.heavy.threshold = heavy_threshold();
+    a.heavy.set(g_part.whole.list, g_part.ws.heavy_partial.as<float>());
     GNNB_TRY(launch_agg(a, false, s, nullptr));
     GemmArgs g = simple_gemm(a.out, lda, emb_in, dw.wt.as<float>(), dw.ldw, bias, y_local, emb_out,
                              n_local, emb_out, act);
@@ -959,7 +959,7 @@ extern "C" int gnnb_gcn_conv_halo(int n_local, int n_ext, const float *x_ext, fl
     a.out = g_part.agg.as<float>() + (size_t)row_begin * lda;
     a.ldo = lda; a.dinv = dinv_ext; a.n = row_count;
     a.row_base = row_begin;      // owned row v is ext row v: self row and dinv are indexed v + row_base
-    a.heavy_threshold = heavy_threshold(); a.hub_bit = hub_bit ? 1 : 0;
+    a.heavy.threshold = heavy_threshold(); a.hub_bit = hub_bit ? 1 : 0;
     // block mode (opt-in): the halo pack of the previous row block runs beside these kernels
     a.short_ctas = row_count < n_local ? 1 : 0;
     if (phase & 1)
@@ -1002,7 +1002,7 @@ extern "C" int gnnb_gin_conv_halo(int n_local, int n_ext, const float *x_ext, fl
     AggArgs a{};
     a.mode = AGG_GIN; a.x = x_ext; a.ldx = emb_in; a.F = emb_in; a.out = g_part.agg.as<float>();
     a.ldo = lda; a.n = n_local; a.eps = gin_eps;   // (1 + eps) x_v with ext row v = owned row v
-    a.heavy_threshold = heavy_threshold(); a.hub_bit = hub_bit ? 1 : 0;
+    a.heavy.threshold = heavy_threshold(); a.hub_bit = hub_bit ? 1 : 0;
     if (phase & 1)
         GNNB_TRY(halo_agg_part(a, own_offsets, own_counts, own_nbr, nullptr, false, !has_halo, 0,
                                n_local, s));
@@ -1049,7 +1049,7 @@ extern "C" int gnnb_sage_conv_halo(int n_local, int n_ext, const float *x_ext, f
     AggArgs a{};
     a.mode = AGG_MEAN; a.x = x_ext; a.ldx = emb_in; a.F = emb_in; a.out = g_part.agg.as<float>();
     a.ldo = lda; a.n = n_local;
-    a.heavy_threshold = heavy_threshold(); a.hub_bit = hub_bit ? 1 : 0;
+    a.heavy.threshold = heavy_threshold(); a.hub_bit = hub_bit ? 1 : 0;
     // the parts' lengths walk the edges, the full in-degree divides (in-degree 0 gives 0, lib:2180-2207)
     if (phase & 1)
         GNNB_TRY(halo_agg_part(a, own_offsets, own_counts, own_nbr, in_degree_local, false, !has_halo,

@@ -750,8 +750,8 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
         a.x = cur; a.ldx = cur_ld; a.F = fi; a.out = m->agg.as<float>(); a.ldo = round_up(fi, 4);
         a.offsets = offsets; a.nbr = nbr; a.in_deg = in_deg; a.dinv = dinv; a.n = T;
         a.eps = d.gin_eps;
-        a.heavy_threshold = heavy_thr;
-        a.set_heavy(m->heavy, m->tws.heavy_partial.as<float>());
+        a.heavy.threshold = heavy_thr;
+        a.heavy.set(m->heavy, m->tws.heavy_partial.as<float>());
         a.hub_bit = hub_bit;
         switch (d.conv_type) {
         case GNNB_CONV_GCN: {
@@ -817,51 +817,46 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
             { ProfScope ps(m->prof, PROF_GEMM, s); GNNB_TRY(launch_gemm(g2, false, s, launches)); }   // lib:2150
             break;
         }
-        case GNNB_CONV_GAT: {
-            // one GEMM: [h | a_src | a_dst] = x.[W | w_src | w_dst]^T, no bias; then the attention
-            // aggregation, whose epilogue applies bias, skip and activation and writes the layer
-            const int H = d.gat_heads, ldg = round_up(fo + 2 * H, 4);
-            float *hg = m->hid.as<float>();
-            GemmArgs g = gemm_args(cur, cur_ld, L.a, hg, ldg, T, GNNB_ACT_IDENTITY);
-            { ProfScope ps(m->prof, PROF_GEMM, s); GNNB_TRY(launch_gemm(g, strict, s, launches)); }
-            GatAggArgs ga{};
-            ga.hg = hg; ga.ldg = ldg; ga.H = H; ga.C = fo / H; ga.slope = d.gat_negative_slope;
-            ga.bias = L.b.bias; ga.skip = skip; ga.ldskip = cur_ld; ga.act = d.gnn_act;
-            ga.out = dst; ga.ldo = ld_out;
-            ga.offsets = offsets; ga.nbr = nbr; ga.in_deg = in_deg; ga.n = T;
-            ga.heavy_threshold = heavy_thr;
-            ga.set_heavy(m->heavy, m->tws.heavy_partial.as<float>());
-            ga.ldp = ldg;
-            if (gat_edges) {
-                ga.elog = m->elog.as<float>() + (size_t)k * H;
-                ga.self_elog = m->self_elog.as<float>() + (size_t)k * H;
-                ga.ldl = LH;
-            }
-            { ProfScope ps(m->prof, PROF_AGG, s); GNNB_TRY(launch_gat_agg(ga, s, launches)); }
-            break;
-        }
+        case GNNB_CONV_GAT:
         case GNNB_CONV_GATV2: {
-            // two GEMMs, xl = x.W_l^T + b_l and xr = x.W_r^T + b_r, side by side in one buffer (one GEMM
-            // of N = 2 H*C would not fit the tensor-core GEMM at H*C = 128); then the attention
-            // aggregation, whose epilogue applies bias, skip and activation and writes the layer
-            const int H = d.gat_heads, ldg = round_up(2 * fo, 4);
-            float *xlr = m->hid.as<float>();
-            GemmArgs gl = gemm_args(cur, cur_ld, L.a, xlr, ldg, T, GNNB_ACT_IDENTITY);
-            GemmArgs gr = gemm_args(cur, cur_ld, L.b, xlr + fo, ldg, T, GNNB_ACT_IDENTITY);
+            // the attention aggregation's epilogue applies bias, skip and activation and writes the
+            // layer; heavy-row partials [acc H*C | max H | sum H]
+            const int H = d.gat_heads;
+            AttnAggArgs at{};
+            at.H = H; at.C = fo / H; at.slope = d.gat_negative_slope;
+            at.skip = skip; at.ldskip = cur_ld; at.act = d.gnn_act; at.out = dst; at.ldo = ld_out;
+            at.offsets = offsets; at.nbr = nbr; at.in_deg = in_deg; at.n = T;
+            at.heavy.threshold = heavy_thr;
+            at.heavy.set(m->heavy, m->tws.heavy_partial.as<float>());
+            at.ldp = round_up(fo + 2 * H, 4);
+            float *hid = m->hid.as<float>();
+            at.g = hid;
+            if (gat) {
+                // one GEMM: [h | a_src | a_dst] = x.[W | w_src | w_dst]^T, no bias
+                GatAggArgs ga{at};
+                ga.bias = L.b.bias; ga.ldg = at.ldp;
+                GemmArgs g = gemm_args(cur, cur_ld, L.a, hid, ga.ldg, T, GNNB_ACT_IDENTITY);
+                { ProfScope ps(m->prof, PROF_GEMM, s); GNNB_TRY(launch_gemm(g, strict, s, launches)); }
+                if (gat_edges) {
+                    ga.elog = m->elog.as<float>() + (size_t)k * H;
+                    ga.self_elog = m->self_elog.as<float>() + (size_t)k * H;
+                    ga.ldl = LH;
+                }
+                { ProfScope ps(m->prof, PROF_AGG, s); GNNB_TRY(launch_gat_agg(ga, s, launches)); }
+                break;
+            }
+            // two GEMMs, xl = x.W_l^T + b_l and xr = x.W_r^T + b_r, side by side in one buffer (one
+            // GEMM of N = 2 H*C would not fit the tensor-core GEMM at H*C = 128)
+            Gatv2AggArgs ga{at};
+            ga.bias = L.d.bias; ga.ldg = round_up(2 * fo, 4); ga.att = L.c.bias;
+            GemmArgs gl = gemm_args(cur, cur_ld, L.a, hid, ga.ldg, T, GNNB_ACT_IDENTITY);
+            GemmArgs gr = gemm_args(cur, cur_ld, L.b, hid + fo, ga.ldg, T, GNNB_ACT_IDENTITY);
             { ProfScope ps(m->prof, PROF_GEMM, s); GNNB_TRY(launch_gemm(gl, strict, s, launches)); }
             { ProfScope ps(m->prof, PROF_GEMM, s); GNNB_TRY(launch_gemm(gr, strict, s, launches)); }
-            Gatv2AggArgs ga{};
-            ga.xlr = xlr; ga.ldg = ldg; ga.H = H; ga.C = fo / H; ga.slope = d.gat_negative_slope;
-            ga.att = L.c.bias; ga.bias = L.d.bias; ga.skip = skip; ga.ldskip = cur_ld; ga.act = d.gnn_act;
-            ga.out = dst; ga.ldo = ld_out;
-            ga.offsets = offsets; ga.nbr = nbr; ga.in_deg = in_deg; ga.n = T;
             if (gatv2_edges) {
                 ga.ef_sorted = m->ef_sorted.as<float>(); ga.self_attr = m->self_attr.as<float>();
                 ga.lde = lde; ga.edge_dim = d.edge_dim; ga.We_t = L.e.Wt; ga.ldw = L.e.ldw;
             }
-            ga.heavy_threshold = heavy_thr;
-            ga.set_heavy(m->heavy, m->tws.heavy_partial.as<float>());
-            ga.ldp = round_up(fo + 2 * H, 4);
             { ProfScope ps(m->prof, PROF_AGG, s); GNNB_TRY(launch_gatv2_agg(ga, s, launches)); }
             break;
         }
