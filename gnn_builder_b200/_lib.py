@@ -54,7 +54,8 @@ EXPORTS = [
     "gnnb_pool_partial",
     "gnnb_halo_pack", "gnnb_halo_pack_ranges", "gnnb_halo_signal", "gnnb_halo_wait", "gnnb_ipc_alloc", "gnnb_ipc_open",
     "gnnb_ipc_close", "gnnb_ipc_free", "gnnb_mark_hub_sources", "gnnb_gcn_conv_halo",
-    "gnnb_gin_conv_halo", "gnnb_sage_conv_halo", "gnnb_pna_conv_halo",
+    "gnnb_gin_conv_halo", "gnnb_sage_conv_halo", "gnnb_pna_conv_halo", "gnnb_gat_conv_halo",
+    "gnnb_gatv2_conv_halo",
 ]
 # include/gnnb_b200_debug.h: tcgen05 probes in libgnnb_b200_debug.so (tests / tools only)
 DEBUG_LIB_PATH = PKG / "libgnnb_b200_debug.so"
@@ -144,6 +145,10 @@ def load(build_if_missing: bool = True) -> C.CDLL:
                                         ci, ci, ci, ci, vp]
     lib.gnnb_pna_conv_halo.argtypes = [ci, ci, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp,
                                        vp, vp, cf, vp, ci, ci, ci, ci, vp]
+    lib.gnnb_gat_conv_halo.argtypes = [ci, ci, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, ci, cf, vp, ci,
+                                       ci, ci, ci, vp]
+    lib.gnnb_gatv2_conv_halo.argtypes = [ci, ci, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, ci, cf,
+                                         vp, ci, ci, ci, ci, vp]
     lib.gnnb_partition_tables.argtypes = [vp, ci, ci, ci, vp, vp, vp, vp]
     lib.gnnb_degree_inv_sqrt.argtypes = [vp, vp, ci, vp]
     lib.gnnb_pool_partial.argtypes = [vp, C.c_int64, ci, vp, vp]

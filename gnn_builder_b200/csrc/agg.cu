@@ -1381,8 +1381,10 @@ __device__ __forceinline__ void gatv2_load(const float *row, const AttnCols<NJ> 
     }
 }
 
-// head hd (>= H: an idle group), lane hl of its G lanes
-template <int VEC, int NJ>
+// head hd (>= H: an idle group), lane hl of its G lanes.  XR: xr has a pointer and stride of its own
+// (the row partition); else it sits in columns [H*C, 2 H*C) of g (the model handle), addressed
+// from g's row so that those kernels keep their register budget
+template <int VEC, int NJ, bool XR>
 __device__ __forceinline__ Gatv2Lane<VEC, NJ> gatv2_lane(const Gatv2AggArgs &a, int v, int hd, int hl,
                                                          int G)
 {
@@ -1394,11 +1396,15 @@ __device__ __forceinline__ Gatv2Lane<VEC, NJ> gatv2_lane(const Gatv2AggArgs &a, 
         ln.valid[j] = hd < a.H && cl < a.C;
         ln.col[j] = hd * a.C + cl;
     }
-    const int HC = a.H * a.C;
-    AttnCols<NJ> sh = ln;   // the same columns, shifted to xr
+    if (XR) {
+        gatv2_load<VEC, NJ>(a.xr + (size_t)v * a.ldxr, ln, ln.xr);
+    } else {
+        const int HC = a.H * a.C;
+        AttnCols<NJ> sh = ln;   // the same columns, shifted to xr
 #pragma unroll
-    for (int j = 0; j < NJ; j++) sh.col[j] += HC;
-    gatv2_load<VEC, NJ>(a.g + (size_t)v * a.ldg, sh, ln.xr);
+        for (int j = 0; j < NJ; j++) sh.col[j] += HC;
+        gatv2_load<VEC, NJ>(a.g + (size_t)v * a.ldg, sh, ln.xr);
+    }
     gatv2_load<VEC, NJ>(a.att, ln, ln.att);
     return ln;
 }
@@ -1535,7 +1541,7 @@ __device__ __forceinline__ const float *gatv2_stage_we(const Gatv2AggArgs &a, bo
 }
 
 // lpr lanes per destination row (a power of two, a multiple of G); G lanes per head
-template <int VEC, int NJ, bool EDGE>
+template <int VEC, int NJ, bool EDGE, bool XR>
 __global__ void __launch_bounds__(256, 1) gatv2_agg_kernel(const Gatv2AggArgs a, int lpr, int G, bool w_smem)
 {
     const float *We = EDGE ? gatv2_stage_we(a, w_smem) : nullptr;
@@ -1555,7 +1561,7 @@ __global__ void __launch_bounds__(256, 1) gatv2_agg_kernel(const Gatv2AggArgs a,
         if (a.heavy.n > 0 && deg > a.heavy.threshold) continue;  // the heavy-row kernels do these
         const int off = __ldg(a.offsets + v);
         for (int h0 = 0; h0 < a.H; h0 += heads_per_pass) {
-            const Gatv2Lane<VEC, NJ> ln = gatv2_lane<VEC, NJ>(a, v, h0 + grp, hl, G);
+            const Gatv2Lane<VEC, NJ> ln = gatv2_lane<VEC, NJ, XR>(a, v, h0 + grp, hl, G);
             OnlineSoftmax<VEC, NJ> st;
             gatv2_self<VEC, NJ, EDGE>(a, We, v, ln, mask, G, st);
             gatv2_gather<VEC, NJ, EDGE>(a, We, v, off, 0, deg, ln, mask, G, st);
@@ -1566,7 +1572,7 @@ __global__ void __launch_bounds__(256, 1) gatv2_agg_kernel(const Gatv2AggArgs a,
 
 // one warp per kHeavyChunk-neighbor chunk of a heavy row: the chunk's per-head (m, s) and its
 // accumulator, as GAT's chunk kernel
-template <int VEC, int NJ, bool EDGE>
+template <int VEC, int NJ, bool EDGE, bool XR>
 __global__ void __launch_bounds__(256, 1) gatv2_heavy_chunk_kernel(const Gatv2AggArgs a, int G)
 {
     const int lane = threadIdx.x & 31;
@@ -1583,7 +1589,7 @@ __global__ void __launch_bounds__(256, 1) gatv2_heavy_chunk_kernel(const Gatv2Ag
         const int k0 = j * kHeavyChunk, k1 = min(deg, k0 + kHeavyChunk);
         float *dst = a.heavy.partial + (size_t)chunk * a.ldp;
         for (int h0 = 0; h0 < a.H; h0 += heads_per_pass) {
-            const Gatv2Lane<VEC, NJ> ln = gatv2_lane<VEC, NJ>(a, v, h0 + grp, hl, G);
+            const Gatv2Lane<VEC, NJ> ln = gatv2_lane<VEC, NJ, XR>(a, v, h0 + grp, hl, G);
             OnlineSoftmax<VEC, NJ> st;
             st.reset();
             gatv2_gather<VEC, NJ, EDGE>(a, a.We_t, v, off, k0, k1, ln, 0xffffffffu, G, st);
@@ -1593,7 +1599,7 @@ __global__ void __launch_bounds__(256, 1) gatv2_heavy_chunk_kernel(const Gatv2Ag
 }
 
 // one CTA per heavy row: combine steps 1 and 2 (GAT's), warp 0 starting from the self term
-template <int VEC, int NJ, bool EDGE>
+template <int VEC, int NJ, bool EDGE, bool XR>
 __global__ void __launch_bounds__(256, 1) gatv2_heavy_combine_kernel(const Gatv2AggArgs a, int G)
 {
     extern __shared__ float4 gatv2_comb_smem4[];
@@ -1605,7 +1611,7 @@ __global__ void __launch_bounds__(256, 1) gatv2_heavy_combine_kernel(const Gatv2
         __syncthreads();
         if (warp == 0) {
             for (int h0 = 0; h0 < a.H; h0 += heads_per_pass) {
-                const Gatv2Lane<VEC, NJ> ln = gatv2_lane<VEC, NJ>(a, v, h0 + grp, hl, G);
+                const Gatv2Lane<VEC, NJ> ln = gatv2_lane<VEC, NJ, XR>(a, v, h0 + grp, hl, G);
                 OnlineSoftmax<VEC, NJ> st;
                 gatv2_self<VEC, NJ, EDGE>(a, a.We_t, v, ln, 0xffffffffu, G, st);
                 attn_merge_ranges<VEC, NJ>(a, ranges, ln, ln.hd < a.H ? ln.hd : 0, st);
@@ -1616,17 +1622,17 @@ __global__ void __launch_bounds__(256, 1) gatv2_heavy_combine_kernel(const Gatv2
     }
 }
 
-template <int VEC, int NJ, bool EDGE>
+template <int VEC, int NJ, bool EDGE, bool XR = false>
 int launch_gatv2_variant(const Gatv2AggArgs &a, int lpr, int G, size_t smem, cudaStream_t s, int *launches)
 {
-    auto k = gatv2_agg_kernel<VEC, NJ, EDGE>;
+    auto k = gatv2_agg_kernel<VEC, NJ, EDGE, XR>;
     if (smem > 48 * 1024) GNNB_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     k<<<row_grid(a.n, lpr), 256, smem, s>>>(a, lpr, G, smem > 0);
     GNNB_CUDA(cudaGetLastError());
     if (launches) ++*launches;
     if (a.heavy.n == 0) return GNNB_OK;
-    return launch_attn_heavy(gatv2_heavy_chunk_kernel<VEC, NJ, EDGE>,
-                             gatv2_heavy_combine_kernel<VEC, NJ, EDGE>, a, s, launches, G);
+    return launch_attn_heavy(gatv2_heavy_chunk_kernel<VEC, NJ, EDGE, XR>,
+                             gatv2_heavy_combine_kernel<VEC, NJ, EDGE, XR>, a, s, launches, G);
 }
 
 __global__ void gatv2_self_attr_kernel(const float *__restrict__ ef, int lde, int edge_dim,
@@ -1655,19 +1661,28 @@ __global__ void gatv2_self_attr_kernel(const float *__restrict__ ef, int lde, in
 
 }  // namespace
 
-int launch_gatv2_agg(const Gatv2AggArgs &a, cudaStream_t s, int *launches)
+int launch_gatv2_agg(const Gatv2AggArgs &args, cudaStream_t s, int *launches)
 {
-    if (a.n <= 0) return GNNB_OK;
+    if (args.n <= 0) return GNNB_OK;
+    Gatv2AggArgs a = args;
     const int HC = a.H * a.C;
     GNNB_TRY(check_attn_args(a, "gatv2"));
-    GNNB_REQUIRE(a.ldg >= 2 * HC && a.att != nullptr, "gatv2 aggregation: bad arguments");
+    const bool sep = a.xr != nullptr;   // xr through its own pointer: the XR kernels
+    if (!sep) {
+        GNNB_REQUIRE(a.ldg >= 2 * HC, "gatv2 aggregation: bad arguments");
+        a.xr = a.g + HC;
+        a.ldxr = a.ldg;
+    }
+    GNNB_REQUIRE(a.ldg >= HC && a.ldxr >= HC && a.att != nullptr, "gatv2 aggregation: bad arguments");
     const bool edge = a.ef_sorted != nullptr;
     if (edge)
         GNNB_REQUIRE(a.self_attr != nullptr && a.We_t != nullptr && a.edge_dim >= 1 &&
                          a.edge_dim <= kGineMaxEdgeDim && a.lde % 4 == 0 && a.lde >= a.edge_dim &&
                          a.ldw % 4 == 0 && a.ldw >= HC && aligned16(a.ef_sorted) && aligned16(a.self_attr),
                      "gatv2 aggregation: bad edge features");
-    const bool v4 = attn_v4(a) && aligned16(a.att) && (!edge || aligned16(a.We_t));
+    GNNB_REQUIRE(!(edge && sep), "gatv2 aggregation: a separate xr is taken without edge features only");
+    const bool v4 = attn_v4(a) && aligned16(a.att) && a.ldxr % 4 == 0 && aligned16(a.xr) &&
+                    (!edge || aligned16(a.We_t));
     const int vec = v4 ? 4 : 1;
     const int cg = (a.C + vec - 1) / vec;   // VEC-column groups per head
     int G = 1;
@@ -1685,15 +1700,19 @@ int launch_gatv2_agg(const Gatv2AggArgs &a, cudaStream_t s, int *launches)
     if (vec == 4) {
         if (nj == 1)
             return edge ? launch_gatv2_variant<4, 1, true>(a, lpr, G, smem, s, launches)
-                        : launch_gatv2_variant<4, 1, false>(a, lpr, G, 0, s, launches);
+                        : sep ? launch_gatv2_variant<4, 1, false, true>(a, lpr, G, 0, s, launches)
+              : launch_gatv2_variant<4, 1, false>(a, lpr, G, 0, s, launches);
         return edge ? launch_gatv2_variant<4, 2, true>(a, lpr, G, smem, s, launches)
-                    : launch_gatv2_variant<4, 2, false>(a, lpr, G, 0, s, launches);
+                    : sep ? launch_gatv2_variant<4, 2, false, true>(a, lpr, G, 0, s, launches)
+              : launch_gatv2_variant<4, 2, false>(a, lpr, G, 0, s, launches);
     }
     if (nj == 1)
         return edge ? launch_gatv2_variant<1, 1, true>(a, lpr, G, smem, s, launches)
-                    : launch_gatv2_variant<1, 1, false>(a, lpr, G, 0, s, launches);
+                    : sep ? launch_gatv2_variant<1, 1, false, true>(a, lpr, G, 0, s, launches)
+              : launch_gatv2_variant<1, 1, false>(a, lpr, G, 0, s, launches);
     return edge ? launch_gatv2_variant<1, 2, true>(a, lpr, G, smem, s, launches)
-                : launch_gatv2_variant<1, 2, false>(a, lpr, G, 0, s, launches);
+                : sep ? launch_gatv2_variant<1, 2, false, true>(a, lpr, G, 0, s, launches)
+              : launch_gatv2_variant<1, 2, false>(a, lpr, G, 0, s, launches);
 }
 
 int launch_gatv2_self_attr(const float *ef_sorted, int lde, int edge_dim, const int32_t *offsets,

@@ -242,6 +242,10 @@ constexpr int kGatv2MaxHeadWidth = 256;   // C % 4 == 0 (float4 lanes)
 constexpr int kGatv2MaxHeadWidth1 = 64;   // other C (scalar lanes)
 struct Gatv2AggArgs : AttnAggArgs {
     const float *att;      // [H*C]
+    // xr of row v at xr + v * ldxr; null: g + H*C with stride ldg.  The row partition passes the
+    // owned rows' xr separately, since only xl crosses ranks.
+    const float *xr;
+    int ldxr;
     // edge features (edge_dim > 0), else ef_sorted null: the edge term of slot k is
     // ef_sorted[k] W_e^T, the self term's self_attr[v] W_e^T
     const float *ef_sorted;  // [slots][lde], neighbor-slot order

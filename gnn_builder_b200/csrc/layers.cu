@@ -4,7 +4,9 @@
 // the reference; each call stages host buffers, runs the same kernels the model path uses on
 // the default stream, and returns when the results are back.
 #include <algorithm>
+#include <cmath>
 #include <cstring>
+#include <string>
 #include <utility>
 #include <vector>
 
@@ -554,6 +556,8 @@ struct DevWeight {
 struct PartitionCache {
     TableWorkspace ws;
     DeviceBuf agg, hid, pna_b, pna_stats, pool_tmp, pool_ptr;
+    DeviceBuf gat_w;      // GAT: [W | w_src | w_dst], folded on every call
+    DeviceBuf gatv2_xr;   // GATv2: xr of the owned rows, from phase 1 to phase 2
     DevWeight w[5];       // the weights of the layer being computed
     int64_t pool_n = -1;
     HeavyCache whole;     // gnnb_gcn_conv_partition (one CSR)
@@ -1140,4 +1144,157 @@ extern "C" int gnnb_pna_conv_halo(int n_local, int n_ext, const float *x_local, 
     g2.img1 = wf.img.as<float>();
     GNNB_TRY(launch_gemm(g2, false, s, nullptr));
     return GNNB_OK;
+}
+
+// ---- the attention convs on the rank's CSR in ext indices ------------------------------------
+// An attention layer has nothing to aggregate before the GEMM output of its halo rows arrives, so
+// these take the rank's whole per-row CSR (neighbor entries = ext indices) rather than the split
+// one.  Owned row v is ext row v, so the unchanged aggregation kernels read the self term at g[v]
+// and skip the entries equal to v (input self loops); halo entries are >= n_local.
+namespace gnnb {
+// Wg [H*C + 2H][fi] = [W | w_src | w_dst], w_src,h[k] = sum_c W[h*C + c][k] att_src[h*C + c] (w_dst
+// alike): summed in double in ascending c with separately rounded products and sums, rounded once,
+// which is the model handle's fold (model.cu), so both give the same GEMM weights
+__global__ void gat_fold_weight_kernel(const float *__restrict__ W, const float *__restrict__ att_src,
+                                       const float *__restrict__ att_dst, float *__restrict__ Wg, int H,
+                                       int C, int fi)
+{
+    const int HC = H * C;
+    const int64_t total = (int64_t)(HC + 2 * H) * fi;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total;
+         i += (int64_t)gridDim.x * blockDim.x) {
+        const int r = (int)(i / fi), k = (int)(i % fi);
+        if (r < HC) {
+            Wg[i] = W[i];
+            continue;
+        }
+        const int q = r - HC, h = q % H;
+        const float *att = (q < H ? att_src : att_dst) + h * C;
+        double acc = 0.0;
+        for (int c = 0; c < C; c++)
+            acc = __dadd_rn(acc, __dmul_rn((double)W[(size_t)(h * C + c) * fi + k], (double)att[c]));
+        Wg[i] = __double2float_rn(acc);
+    }
+}
+}  // namespace gnnb
+
+namespace {
+
+// argument checks of the attention halo layers (before any device work)
+int check_attn_halo_args(const char *conv, int heads, float slope, int emb_in, int emb_out,
+                         const float *skip_local, bool gatv2)
+{
+    const std::string name(conv);
+    GNNB_REQUIRE(heads >= 1 && heads <= GNNB_GAT_MAX_HEADS,
+                 name + " heads must be 1.." + std::to_string(GNNB_GAT_MAX_HEADS));
+    GNNB_REQUIRE(emb_out % heads == 0, name + ": emb_out must be a multiple of heads");
+    GNNB_REQUIRE(std::isfinite(slope), name + " negative_slope must be finite");
+    const int C = emb_out / heads;
+    GNNB_REQUIRE(!gatv2 || C <= (C % 4 == 0 ? kGatv2MaxHeadWidth : kGatv2MaxHeadWidth1),
+                 "GATv2: a head's width (layer width / gat_heads) must be at most " +
+                     std::to_string(kGatv2MaxHeadWidth) + " when a multiple of 4, else at most " +
+                     std::to_string(kGatv2MaxHeadWidth1) + ", got " + std::to_string(C));
+    GNNB_REQUIRE(skip_local == nullptr || emb_in == emb_out, "a skip connection needs emb_in == emb_out");
+    return GNNB_OK;
+}
+
+// the attention arguments both convs share: the rank's CSR, the epilogue and the heavy rows (every
+// row above heavy_threshold(), partials [ldp] wide)
+int attn_halo_common(AttnAggArgs &at, int n_local, const int32_t *offsets_local,
+                     const int32_t *in_degree_local, const int32_t *nbr_ext, int heads, float slope,
+                     const float *bias, const float *skip_local, int emb_in, int emb_out, int act,
+                     float *y_local, cudaStream_t s)
+{
+    at.H = heads; at.C = emb_out / heads; at.slope = slope;
+    at.bias = bias; at.skip = skip_local; at.ldskip = emb_in; at.act = act;
+    at.out = y_local; at.ldo = emb_out;
+    at.offsets = offsets_local; at.nbr = nbr_ext; at.in_deg = in_degree_local; at.n = n_local;
+    at.ldp = round_up(emb_out + 2 * heads, 4);
+    HeavyCache &hc = part_cache(in_degree_local, n_local);
+    GNNB_TRY(heavy_rows_of(hc, in_degree_local, n_local, s));
+    GNNB_TRY(heavy_setup(g_part.ws, hc.list.n_chunks, at.ldp));
+    at.heavy.threshold = heavy_threshold();
+    at.heavy.set(hc.list, g_part.ws.heavy_partial.as<float>());
+    return GNNB_OK;
+}
+}  // namespace
+
+extern "C" int gnnb_gat_conv_halo(int n_local, int n_ext, const float *x_local, float *g_ext,
+                                  float *y_local, const int32_t *offsets_local,
+                                  const int32_t *in_degree_local, const int32_t *nbr_ext,
+                                  const float *att_src, const float *att_dst, const float *bias,
+                                  const float *lin_weight, int heads, float negative_slope,
+                                  const float *skip_local, int emb_in, int emb_out, int act, int phase,
+                                  void *stream)
+{
+    GNNB_TRY(check_halo_args(n_local, n_ext, emb_in, emb_out, act, phase));
+    GNNB_TRY(check_attn_halo_args("GAT", heads, negative_slope, emb_in, emb_out, skip_local, false));
+    if (n_local == 0) return GNNB_OK;
+    GNNB_REQUIRE(is_device_pointer(x_local) && is_device_pointer(g_ext) && is_device_pointer(y_local) &&
+                     is_device_pointer(offsets_local) && is_device_pointer(in_degree_local),
+                 "gnnb_gat_conv_halo takes device pointers");
+    cudaStream_t s = (cudaStream_t)stream;
+    const int N = emb_out + 2 * heads, ldg = round_up(N, 4);
+    if (phase & 1) {
+        // [h | a_src | a_dst] of the owned rows = x.[W | w_src | w_dst]^T: what the peers gather
+        GNNB_TRY(g_part.gat_w.ensure(sizeof(float) * (size_t)N * emb_in));
+        float *Wg = g_part.gat_w.as<float>();
+        const int64_t total = (int64_t)N * emb_in;
+        gat_fold_weight_kernel<<<(int)std::min<int64_t>((total + 255) / 256, 4096), 256, 0, s>>>(
+            lin_weight, att_src, att_dst, Wg, heads, emb_out / heads, emb_in);
+        GNNB_CUDA(cudaGetLastError());
+        DevWeight &dw = g_part.w[0];
+        GNNB_TRY(dev_weight(dw, Wg, N, emb_in, 0, s));
+        GemmArgs g = simple_gemm(x_local, emb_in, emb_in, dw.wt.as<float>(), dw.ldw, nullptr, g_ext, ldg,
+                                 n_local, N, GNNB_ACT_IDENTITY);
+        g.img1 = dw.img.as<float>();
+        GNNB_TRY(launch_gemm(g, false, s, nullptr));
+    }
+    if (!(phase & 2)) return GNNB_OK;
+    GatAggArgs ga{};
+    GNNB_TRY(attn_halo_common(ga, n_local, offsets_local, in_degree_local, nbr_ext, heads, negative_slope,
+                              bias, skip_local, emb_in, emb_out, act, y_local, s));
+    ga.g = g_ext; ga.ldg = ldg;
+    return launch_gat_agg(ga, s, nullptr);
+}
+
+extern "C" int gnnb_gatv2_conv_halo(int n_local, int n_ext, const float *x_local, float *xl_ext,
+                                    float *y_local, const int32_t *offsets_local,
+                                    const int32_t *in_degree_local, const int32_t *nbr_ext,
+                                    const float *att, const float *bias, const float *lin_l_weight,
+                                    const float *lin_l_bias, const float *lin_r_weight,
+                                    const float *lin_r_bias, int heads, float negative_slope,
+                                    const float *skip_local, int emb_in, int emb_out, int act, int phase,
+                                    void *stream)
+{
+    GNNB_TRY(check_halo_args(n_local, n_ext, emb_in, emb_out, act, phase));
+    GNNB_TRY(check_attn_halo_args("GATv2", heads, negative_slope, emb_in, emb_out, skip_local, true));
+    if (n_local == 0) return GNNB_OK;
+    GNNB_REQUIRE(is_device_pointer(x_local) && is_device_pointer(xl_ext) && is_device_pointer(y_local) &&
+                     is_device_pointer(offsets_local) && is_device_pointer(in_degree_local),
+                 "gnnb_gatv2_conv_halo takes device pointers");
+    cudaStream_t s = (cudaStream_t)stream;
+    const int ldl = round_up(emb_out, 4);
+    GNNB_TRY(g_part.gatv2_xr.ensure(sizeof(float) * (size_t)n_local * ldl));
+    float *xr = g_part.gatv2_xr.as<float>();
+    if (phase & 1) {
+        // xl of the owned rows goes to the peers, xr stays here
+        DevWeight &wl = g_part.w[0], &wr = g_part.w[1];
+        GNNB_TRY(dev_weight(wl, lin_l_weight, emb_out, emb_in, 0, s));
+        GNNB_TRY(dev_weight(wr, lin_r_weight, emb_out, emb_in, 0, s));
+        GemmArgs gl = simple_gemm(x_local, emb_in, emb_in, wl.wt.as<float>(), wl.ldw, lin_l_bias, xl_ext, ldl,
+                                  n_local, emb_out, GNNB_ACT_IDENTITY);
+        gl.img1 = wl.img.as<float>();
+        GNNB_TRY(launch_gemm(gl, false, s, nullptr));
+        GemmArgs gr = simple_gemm(x_local, emb_in, emb_in, wr.wt.as<float>(), wr.ldw, lin_r_bias, xr, ldl,
+                                  n_local, emb_out, GNNB_ACT_IDENTITY);
+        gr.img1 = wr.img.as<float>();
+        GNNB_TRY(launch_gemm(gr, false, s, nullptr));
+    }
+    if (!(phase & 2)) return GNNB_OK;
+    Gatv2AggArgs ga{};
+    GNNB_TRY(attn_halo_common(ga, n_local, offsets_local, in_degree_local, nbr_ext, heads, negative_slope,
+                              bias, skip_local, emb_in, emb_out, act, y_local, s));
+    ga.g = xl_ext; ga.ldg = ldl; ga.xr = xr; ga.ldxr = ldl; ga.att = att;
+    return launch_gatv2_agg(ga, s, nullptr);
 }

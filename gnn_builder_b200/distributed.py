@@ -6,7 +6,8 @@ Two ways the hot path shards (SURVEY 8e):
   balanced by node count; every rank runs its shard through its own ``Engine``; there is NO
   data-path collective (``run_sharded`` optionally gathers the per-graph outputs at the end).
 * **one large graph** (BASELINE config 5 is GCN; GIN, SAGE and PNA run the same way, PNA
-  exchanging its pre-transformed rows instead of the input): 1D partition by destination row.  Rank g owns
+  exchanging its pre-transformed rows instead of the input; GAT and GATv2 run in
+  ``LargeGraphAttentionModel`` and exchange their layer GEMM's output): 1D partition by destination row.  Rank g owns
   rows ``[g*n/W, (g+1)*n/W)``, their CSR slice (in-edges) and the matching feature rows, plus a
   **halo**: ONE copy of every remote row its in-edges reference (on the 2M-node power-law graph
   that is 84 % / 65 % / 45 % of the remote rows at W = 2 / 4 / 8).  Sources are renumbered into
@@ -104,9 +105,13 @@ class HaloPlan:
     split by where the source lives (offsets / counts per owned row, neighbor entries = ext
     indices), each part in the stable neighbor order of lib:1086-1124.  ``send_idx`` /
     ``send_counts``: the owned rows every peer needs, in that peer's halo order.
+    ``keep_ext_csr``: also keep ``nbr_ext``, the rank's whole CSR (the order of ``nbr_global``)
+    with every entry mapped to its ext index, which the attention convs aggregate over
+    (4 bytes per local edge, so only they ask for it).
     Works on torch tensors of any device (the gloo tests run it on CPU)."""
 
-    def __init__(self, ind_local, nbr_global, rank: int, part: RowPartition, dist=None):
+    def __init__(self, ind_local, nbr_global, rank: int, part: RowPartition, dist=None,
+                 keep_ext_csr: bool = False):
         import torch
 
         W, n_local = part.world, part.n_local
@@ -120,6 +125,7 @@ class HaloPlan:
         self.n_local, self.n_halo = n_local, int(self.halo_ids.numel())
         self.n_ext = n_local + self.n_halo
         ext = torch.where(is_halo, n_local + torch.searchsorted(self.halo_ids, nbr), nbr - r0)
+        self.nbr_ext = ext.to(torch.int32).contiguous() if keep_ext_csr else None
         own = ~is_halo
         # one contiguous table [owned-source part | halo-source part] (hub marking runs over both)
         self.nbr_all = torch.cat([ext[own], ext[is_halo]]).to(torch.int32).contiguous()
@@ -295,6 +301,22 @@ class CudaBackend:
             self._p(bpost), self._p(Wlin), self._p(blin), float(delta), self._p(skip), emb_in,
             emb_out, act, phase, self._stream()))
 
+    def gat_layer_halo(self, x_local, g_ext, y_local, plan: HaloPlan, offsets, in_deg, att_src,
+                       att_dst, bias, W, heads, slope, skip, act, phase, emb_in, emb_out):
+        self._lib.check(self.lib.gnnb_gat_conv_halo(
+            plan.n_local, plan.n_ext, self._p(x_local), self._p(g_ext), self._p(y_local),
+            self._p(offsets), self._p(in_deg), self._p(plan.nbr_ext), self._p(att_src),
+            self._p(att_dst), self._p(bias), self._p(W), int(heads), float(slope), self._p(skip),
+            emb_in, emb_out, act, phase, self._stream()))
+
+    def gatv2_layer_halo(self, x_local, xl_ext, y_local, plan: HaloPlan, offsets, in_deg, att, bias,
+                         Wl, bl, Wr, br, heads, slope, skip, act, phase, emb_in, emb_out):
+        self._lib.check(self.lib.gnnb_gatv2_conv_halo(
+            plan.n_local, plan.n_ext, self._p(x_local), self._p(xl_ext), self._p(y_local),
+            self._p(offsets), self._p(in_deg), self._p(plan.nbr_ext), self._p(att), self._p(bias),
+            self._p(Wl), self._p(bl), self._p(Wr), self._p(br), int(heads), float(slope),
+            self._p(skip), emb_in, emb_out, act, phase, self._stream()))
+
     def halo_pack(self, x_own, F: int, plan: HaloPlan, dst_ptrs, max_ctas: int = 0):
         """dst_ptrs: one raw device address per peer (0 where nothing is sent)"""
         W = len(dst_ptrs)
@@ -387,7 +409,12 @@ _LAYER_PARAMS = {
     "sage": ("conv_lin_l_weight", "conv_lin_l_bias", "conv_lin_r_weight"),
     "pna": ("conv_pre_nns_0_0_weight", "conv_pre_nns_0_0_bias", "conv_post_nns_0_0_weight",
             "conv_post_nns_0_0_bias", "conv_lin_weight", "conv_lin_bias"),
+    "gat": ("conv_att_src", "conv_att_dst", "conv_bias", "conv_lin_weight"),
+    "gatv2": ("conv_att", "conv_bias", "conv_lin_l_weight", "conv_lin_l_bias", "conv_lin_r_weight",
+              "conv_lin_r_bias"),
 }
+
+_CONV_NAMES = {0: "GCN", 1: "GIN", 2: "SAGE", 3: "PNA", 4: "GINE", 5: "GAT", 7: "GATv2"}
 
 
 class LargeGraphModel:
@@ -400,14 +427,23 @@ class LargeGraphModel:
     through CUDA-IPC mappings; flag hand-off on the device), "nccl" (pack + all_to_all_single) or
     "auto" (p2p when every rank can map its peers, else nccl)."""
 
+    # conv_type -> conv this class runs
+    CONVS = {0: "gcn", 1: "gin", 2: "sage", 3: "pna"}
+    REFUSAL = ("LargeGraphModel runs GCN, GIN, SAGE and PNA models; GAT and GATv2 models run "
+               "row-partitioned in LargeGraphAttentionModel")
+    # whether the halo plan keeps the rank's whole CSR in ext indices (HaloPlan.nbr_ext)
+    EXT_CSR = False
+
     def __init__(self, model, n_total: int, rank: int, world: int, dist=None, backend=None,
                  transport: str = "auto", hub_l2_mb: Optional[int] = None):
         d = model.describe()
-        if d["conv_type"] not in (0, 1, 2, 3):
-            raise NotImplementedError("row-partitioned inference runs GCN, GIN, SAGE and PNA models "
-                                      "(GINE has no edge-feature halo exchange, GAT and GATv2 no "
-                                      "split-CSR attention kernel)")
-        self.conv = ("gcn", "gin", "sage", "pna")[d["conv_type"]]
+        name = _CONV_NAMES.get(d["conv_type"], f"conv_type {d['conv_type']}")
+        if d["conv_type"] == 4 or d.get("edge_dim"):
+            raise NotImplementedError(f"{name} models with edge features cannot run row-partitioned: "
+                                      "edge features have no halo exchange")
+        if d["conv_type"] not in self.CONVS:
+            raise NotImplementedError(f"{name}: {self.REFUSAL}")
+        self.conv = self.CONVS[d["conv_type"]]
         self.model, self.desc = model, d
         self.part = RowPartition(n_total, world)
         self.rank, self.world, self.dist = rank, world, dist
@@ -454,7 +490,7 @@ class LargeGraphModel:
         r0, _ = self.part.rows(self.rank)
         n_local = self.part.n_local
         self.tables = B.partition_tables(B.to_device(coo_local.astype(np.int32)), r0, n_local)
-        ind_local, _, nbr_global = self.tables
+        ind_local, self.offsets_local, nbr_global = self.tables
         self.in_deg = ind_local
         if self.conv == "gcn":   # GCN normalises by the in-degree of both endpoints: all-gather it
             if W > 1:
@@ -463,10 +499,10 @@ class LargeGraphModel:
                 ind_full = ind_local
             dinv_full = B.dinv(ind_full)
         self.plan = plan = HaloPlan(ind_local, nbr_global, self.rank, self.part,
-                                    self.dist if W > 1 else None)
+                                    self.dist if W > 1 else None, keep_ext_csr=self.EXT_CSR)
         if self.conv == "gcn":
             self.dinv_ext = dinv_full[plan.ext_ids(self.rank)].contiguous()
-        fmax = max(self.dims)
+        fmax = self._buf_width()
         # (PNA gathers A rows through its own statistics kernel, which takes no cache hints)
         if self.conv != "pna" and self.hub_l2_mb > 0 and hasattr(B, "mark_hubs") and \
                 plan.n_ext * fmax * 4 > (96 << 20):
@@ -586,6 +622,10 @@ class LargeGraphModel:
         """ext buffer that holds the INPUT of conv layer k (and receives its halo): the layer-0
         input has a buffer of its own, so a forward never overwrites it; the others alternate"""
         return 2 if k == 0 else (k & 1)
+
+    def _buf_width(self) -> int:
+        """floats per row of every ext buffer and of the NCCL send buffer"""
+        return max(self.dims)
 
     def _n_bufs(self) -> int:
         """three layer-input buffers; PNA adds two for the exchanged A rows (layer parity: a peer
@@ -748,6 +788,75 @@ class LargeGraphGCN(LargeGraphModel):
             raise NotImplementedError("LargeGraphGCN runs GCN models; LargeGraphModel runs every conv")
         super().__init__(model, n_total, rank, world, dist=dist, backend=backend,
                          transport=transport, hub_l2_mb=hub_l2_mb)
+
+
+class LargeGraphAttentionModel(LargeGraphModel):
+    """GNNModel with GAT or GATv2 convs (no edge features) over one large row-partitioned graph.
+
+    An attention layer gathers, per source row, what its GEMM produced for that row, so the
+    exchange carries the GEMM output rather than the layer input, and no GEMM runs on a halo row:
+    per layer, the owned rows' GEMM output (GAT: [h | a_src | a_dst], ``round_up(H*C + 2H, 4)``
+    floats a row; GATv2: xl, ``round_up(H*C, 4)``) is computed, pushed to the peers, and the
+    attention softmax runs once it has arrived.  Nothing can be aggregated before that, so the
+    aggregation walks the rank's whole CSR in ext indices (``HaloPlan.nbr_ext``) rather than the
+    split one, and the exchange is not overlapped with compute.  Transports as LargeGraphModel;
+    ``hub_l2_mb`` is ignored (the attention kernels take no cache hints)."""
+
+    CONVS = {5: "gat", 7: "gatv2"}
+    REFUSAL = ("LargeGraphAttentionModel runs GAT and GATv2 models; GCN, GIN, SAGE and PNA models "
+               "run row-partitioned in LargeGraphModel")
+    EXT_CSR = True
+
+    def __init__(self, model, n_total: int, rank: int, world: int, dist=None, backend=None,
+                 transport: str = "auto", hub_l2_mb: Optional[int] = None):
+        super().__init__(model, n_total, rank, world, dist=dist, backend=backend,
+                         transport=transport, hub_l2_mb=0)
+        self.heads = self.desc["gat_heads"]
+        self.slope = self.desc["gat_negative_slope"]
+
+    def _xwidth(self, k: int) -> int:
+        """floats per exchanged row of layer k: GAT [h | a_src | a_dst], GATv2 xl"""
+        fo = self.dims[k + 1]
+        return (fo + (2 * self.heads if self.conv == "gat" else 0) + 3) // 4 * 4
+
+    def _buf_width(self) -> int:
+        return max(self.dims + [self._xwidth(k) for k in range(len(self.dims) - 1)])
+
+    def _n_bufs(self) -> int:
+        """three layer-feature buffers and two for the exchanged GEMM output, alternating by layer
+        parity: a fast peer may push layer k+1's rows while this rank still reads layer k's"""
+        return 5
+
+    def _xbuf(self, k: int) -> int:
+        return 3 + (k & 1)
+
+    def _autotune(self, F: int):
+        super()._autotune(self._xwidth(0))
+
+    def setup(self, coo_local: np.ndarray):
+        super().setup(coo_local)
+        self.stats["exchanged_floats_per_halo_row"] = [self._xwidth(k)
+                                                       for k in range(self.desc["num_layers"])]
+        return self
+
+    def _conv_layer(self, k: int, x_ext, y_local, skip):
+        """layer k: the owned rows' GEMM output, the exchange, then the attention aggregation"""
+        B, d, plan = self.backend, self.desc, self.plan
+        fi, fo, xw = self.dims[k], self.dims[k + 1], self._xwidth(k)
+        layer = B.gat_layer_halo if self.conv == "gat" else B.gatv2_layer_halo
+        g_ext = self.ext[self._xbuf(k)][: plan.n_ext * xw]
+
+        def call(phase):
+            layer(x_ext[: plan.n_local * fi], g_ext, y_local, plan, self.offsets_local, self.in_deg,
+                  *self.layers[k], self.heads, self.slope, skip, d["gnn_act"], phase, fi, fo)
+
+        if self.world == 1:
+            call(3)
+        else:   # (every rank takes part in the exchange, even with an empty halo)
+            call(1)
+            self._exchange(k, xw)
+            self._arrived()
+            call(2)
 
 
 def _cat(ts):

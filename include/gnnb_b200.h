@@ -382,6 +382,38 @@ int gnnb_pna_conv_halo(int n_local, int n_ext, const float *x_local, float *a_ex
                        const float *final_lin_weight, const float *final_lin_bias,
                        float pna_avg_degree_log, const float *skip_local, int emb_in, int emb_out,
                        int act, int phase, void *stream);
+/* The attention convs (PyG GATConv / GATv2Conv, concat heads, no edge features), FAST math.  An
+ * attention layer gathers what its GEMM produced for each source, so what crosses ranks is that
+ * GEMM output, and no GEMM runs on a halo row.  The CSR is the rank's own, whole
+ * (offsets_local / in_degree_local as from gnnb_partition_tables, which are the FULL in-degrees),
+ * with every neighbor entry mapped to its ext index (nbr_ext, same order).  phase 1 computes the
+ * GEMM output of the owned rows into rows [0, n_local) of the ext buffer (the caller then sends
+ * them, e.g. with gnnb_halo_pack at the width below, into the peers' halo regions); phase 2, once
+ * rows [n_local, n_ext) have arrived, runs the attention softmax and the epilogue,
+ * y_local[n_local][emb_out] = act(sum_u alpha_vu m_u + bias (+ skip_local)); phase 3 both.
+ * Input self loops are replaced by one per node as PyG does; rows above the heavy-row threshold
+ * are cut into chunks.  x_local[n_local][emb_in] are the owned input rows.  emb_out = heads * C,
+ * heads 1..GNNB_GAT_MAX_HEADS.  Weights in PyG's layout, device pointers.
+ *
+ * GAT: g_ext [n_ext][ld_g], ld_g = round_up(emb_out + 2 heads, 4), rows [h | a_src | a_dst].  The
+ * per-head vectors w_src,h = W_h^T att_src,h (w_dst alike) are folded into the GEMM weight on every
+ * phase-1 call, in double and rounded once as the model handle does. */
+int gnnb_gat_conv_halo(int n_local, int n_ext, const float *x_local, float *g_ext, float *y_local,
+                       const int32_t *offsets_local, const int32_t *in_degree_local,
+                       const int32_t *nbr_ext, const float *att_src, const float *att_dst,
+                       const float *bias, const float *lin_weight, int heads, float negative_slope,
+                       const float *skip_local, int emb_in, int emb_out, int act, int phase,
+                       void *stream);
+/* GATv2: xl_ext [n_ext][ld_l], ld_l = round_up(emb_out, 4), holds xl = x.W_l^T + b_l; xr = x.W_r^T +
+ * b_r of the owned rows stays in library scratch from phase 1 to phase 2 (one layer in flight per
+ * thread).  A head's width C must be at most 256 when a multiple of 4, else at most 64. */
+int gnnb_gatv2_conv_halo(int n_local, int n_ext, const float *x_local, float *xl_ext, float *y_local,
+                         const int32_t *offsets_local, const int32_t *in_degree_local,
+                         const int32_t *nbr_ext, const float *att, const float *bias,
+                         const float *lin_l_weight, const float *lin_l_bias,
+                         const float *lin_r_weight, const float *lin_r_bias, int heads,
+                         float negative_slope, const float *skip_local, int emb_in, int emb_out,
+                         int act, int phase, void *stream);
 
 #ifdef __cplusplus
 }
