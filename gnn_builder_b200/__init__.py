@@ -13,7 +13,7 @@ from .engine import (MATH_FAST, MATH_STRICT, PATH_AUTO, PATH_FUSED, PATH_LAYERWI
                      Engine)
 from .models import (MLP, GATConv_GNNB, GATv2Conv_GNNB, GCNConv_GNNB, GINConv_GNNB,  # noqa: F401
                      GINEConv_GNNB, GlobalPooling, GNNModel, PNAConv_GNNB, SAGEConv_GNNB,
-                     build_model)
+                     TransformerConv_GNNB, build_model)
 from .utils import (compute_average_degree, compute_average_nodes_and_edges,  # noqa: F401
                     compute_in_deg_histogram, compute_max_nodes_and_edges,
                     compute_median_degree, compute_median_nodes_and_edges)

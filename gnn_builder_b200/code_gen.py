@@ -217,6 +217,11 @@ extern "C" void {self.name}_top(
                 f"{what}: the reference has no GATv2 kernel and its <name>_top no attention-head "
                 "arguments, so a GATv2Conv_GNNB model cannot be rendered; run it through Engine "
                 "instead")
+        if self.model is not None and self.model.describe()["conv_type"] == 8:
+            raise NotImplementedError(
+                f"{what}: the reference has no TransformerConv kernel and its <name>_top no "
+                "attention-head arguments, so a TransformerConv_GNNB model cannot be rendered; run "
+                "it through Engine instead")
         if getattr(self.model, "uses_edge_features", False):
             raise NotImplementedError(
                 f"{what}: the reference's <name>_top signature has no edge-feature argument, so a "

@@ -1200,7 +1200,7 @@ int launch_attn_heavy(void (*chunk)(Args, Extra...), void (*combine)(Args, Extra
     return GNNB_OK;
 }
 
-// the arguments GAT and GATv2 share (what = the conv's name for the messages)
+// the arguments the attention aggregations share (what = the conv's name for the messages)
 int check_attn_args(const AttnAggArgs &a, const char *what)
 {
     const int HC = a.H * a.C;
@@ -1381,6 +1381,19 @@ __device__ __forceinline__ void gatv2_load(const float *row, const AttnCols<NJ> 
     }
 }
 
+// the columns of head hd (>= H: an idle group) that lane hl of its G lanes holds
+template <int VEC, int NJ>
+__device__ __forceinline__ void attn_lane_cols(const AttnAggArgs &a, int hd, int hl, int G, AttnCols<NJ> &cl)
+{
+    cl.hd = hd;
+#pragma unroll
+    for (int j = 0; j < NJ; j++) {
+        const int c = (hl + j * G) * VEC;
+        cl.valid[j] = hd < a.H && c < a.C;
+        cl.col[j] = hd * a.C + c;
+    }
+}
+
 // head hd (>= H: an idle group), lane hl of its G lanes.  XR: xr has a pointer and stride of its own
 // (the row partition); else it sits in columns [H*C, 2 H*C) of g (the model handle), addressed
 // from g's row so that those kernels keep their register budget
@@ -1389,13 +1402,7 @@ __device__ __forceinline__ Gatv2Lane<VEC, NJ> gatv2_lane(const Gatv2AggArgs &a, 
                                                          int G)
 {
     Gatv2Lane<VEC, NJ> ln;
-    ln.hd = hd;
-#pragma unroll
-    for (int j = 0; j < NJ; j++) {
-        const int cl = (hl + j * G) * VEC;
-        ln.valid[j] = hd < a.H && cl < a.C;
-        ln.col[j] = hd * a.C + cl;
-    }
+    attn_lane_cols<VEC, NJ>(a, hd, hl, G, ln);
     if (XR) {
         gatv2_load<VEC, NJ>(a.xr + (size_t)v * a.ldxr, ln, ln.xr);
     } else {
@@ -1409,10 +1416,11 @@ __device__ __forceinline__ Gatv2Lane<VEC, NJ> gatv2_lane(const Gatv2AggArgs &a, 
     return ln;
 }
 
-// z += ef W_e^T for the lane's columns: ef one row of lde floats (edge_dim used), We [edge_dim][ldw]
-template <int VEC, int NJ>
-__device__ __forceinline__ void gatv2_edge_proj(const Gatv2AggArgs &a, const float *We, const float *ef,
-                                                const Gatv2Lane<VEC, NJ> &ln, Vec<VEC> (&z)[NJ])
+// z += ef W_e^T for the lane's columns: ef one row of lde floats (edge_dim used), We [edge_dim][ldw].
+// Args: Gatv2AggArgs or TransformerAggArgs (edge_dim, ldw)
+template <int VEC, int NJ, typename Args>
+__device__ __forceinline__ void gatv2_edge_proj(const Args &a, const float *We, const float *ef,
+                                                const AttnCols<NJ> &ln, Vec<VEC> (&z)[NJ])
 {
     for (int j0 = 0; j0 < a.edge_dim; j0 += 4) {
         const float4 e4 = __ldg(reinterpret_cast<const float4 *>(ef + j0));
@@ -1528,8 +1536,9 @@ __device__ __forceinline__ void gatv2_finish(const Gatv2AggArgs &a, int v, const
         if (ln.valid[j]) attn_finish(a, v, ln.col[j], st.acc[j], st.s);
 }
 
-// W_e^T staged in shared memory (w_smem) or read in place
-__device__ __forceinline__ const float *gatv2_stage_we(const Gatv2AggArgs &a, bool w_smem)
+// W_e^T staged in shared memory (w_smem) or read in place; Args as gatv2_edge_proj
+template <typename Args>
+__device__ __forceinline__ const float *gatv2_stage_we(const Args &a, bool w_smem)
 {
     extern __shared__ float4 gatv2_smem4[];
     if (!w_smem) return a.We_t;
@@ -1727,6 +1736,261 @@ int launch_gatv2_self_attr(const float *ef_sorted, int lde, int edge_dim, const 
     GNNB_CUDA(cudaGetLastError());
     if (launches) ++*launches;
     return GNNB_OK;
+}
+
+// ----------------------------------------------------------------------------- TransformerConv
+//
+// PyG TransformerConv (concat heads, root_weight, no beta, inference).  The layer's GEMMs wrote
+// [k | v] per row into g and q (scaled by 1/sqrt(C) at finalize) into its own rows; the root term
+// r = x W_skip^T (+ the model's residual) comes in as the epilogue's skip and b_skip as its bias.
+// The logit e_uvh = <q_v, k_u (+ ê_uv)>_h is a dot product over the head's lanes, formed per edge as
+// GATv2's: each lane holds q_v for its columns in registers and the head's lanes add their partials
+// with the xor butterfly, so every lane of a head holds the same logit bits.  With edge features
+// ê_uv = ef_sorted[slot] W_e^T is computed once per slot (gatv2_edge_proj) and added to both k_u and
+// the message v_u.  Lane layout, masks and the W_e^T staging are GATv2's.
+//
+// There is no self term: every neighbor entry, the input's self loops and duplicates included, is an
+// ordinary edge, and the online softmax starts from reset().  A row with no in-edges ends with s = 0
+// and acc = 0; its epilogue divides by 1 instead, so y_v = act(b_skip + r_v).  Heavy rows are GAT's
+// chunk / fixed-order combine scheme, warp 0 of the combine also starting from reset().  Algorithmic
+// bytes per layer: E (4 + 8HC [+ 4 lde]) + N (8 + 4HC q + 4HC r + 4HC out).
+namespace {
+
+// one lane's share of one head: its columns (AttnCols) and q_v for them
+template <int VEC, int NJ>
+struct TransformerLane : AttnCols<NJ> {
+    Vec<VEC> q[NJ];
+};
+
+template <int VEC, int NJ>
+__device__ __forceinline__ TransformerLane<VEC, NJ> transformer_lane(const TransformerAggArgs &a, int v, int hd,
+                                                                     int hl, int G)
+{
+    TransformerLane<VEC, NJ> ln;
+    attn_lane_cols<VEC, NJ>(a, hd, hl, G, ln);
+    gatv2_load<VEC, NJ>(a.q + (size_t)v * a.ldq, ln, ln.q);
+    return ln;
+}
+
+// the lane's partial dot product <q_v, k> (columns past C hold q = 0)
+template <int VEC, int NJ>
+__device__ __forceinline__ float transformer_partial(const TransformerLane<VEC, NJ> &ln, const Vec<VEC> (&k)[NJ])
+{
+    float part = 0.0f;
+#pragma unroll
+    for (int j = 0; j < NJ; j++)
+#pragma unroll
+        for (int i = 0; i < VEC; i++) part = fmaf(ln.q[j].v[i], k[j].v[i], part);
+    return part;
+}
+
+// k_u and v_u of one slot for the lane's columns, both plus ê = ef_sorted[slot] W_e^T with EDGE
+template <int VEC, int NJ, bool EDGE>
+__device__ __forceinline__ void transformer_load(const TransformerAggArgs &a, const float *We, int u, int slot,
+                                                 const AttnCols<NJ> &cl, Vec<VEC> (&k)[NJ], Vec<VEC> (&val)[NJ])
+{
+    const float *row = a.g + (size_t)u * a.ldg;
+    gatv2_load<VEC, NJ>(row, cl, k);
+    gatv2_load<VEC, NJ>(row + a.H * a.C, cl, val);
+    if (EDGE) {
+        Vec<VEC> ep[NJ];
+        gatv2_zero<VEC, NJ>(ep);
+        gatv2_edge_proj<VEC, NJ>(a, We, a.ef_sorted + (size_t)slot * a.lde, cl, ep);
+#pragma unroll
+        for (int j = 0; j < NJ; j++)
+#pragma unroll
+            for (int i = 0; i < VEC; i++) {
+                k[j].v[i] += ep[j].v[i];
+                val[j].v[i] += ep[j].v[i];
+            }
+    }
+}
+
+// neighbor slots [k0, k1) of a row (none skipped), U gathers in flight
+template <int VEC, int NJ, bool EDGE>
+__device__ __forceinline__ void transformer_gather(const TransformerAggArgs &a, const float *We, int off, int k0,
+                                                   int k1, const TransformerLane<VEC, NJ> &ln, unsigned mask,
+                                                   int G, OnlineSoftmax<VEC, NJ> &st)
+{
+    constexpr int U = NJ == 1 ? 4 : 2;
+    int k = k0;
+#pragma unroll 1
+    for (; k + U <= k1; k += U) {
+        int u[U];
+        Vec<VEC> kk[U][NJ], val[U][NJ];
+        float e[U];
+#pragma unroll
+        for (int q = 0; q < U; q++) u[q] = __ldg(a.nbr + off + k + q);
+#pragma unroll
+        for (int q = 0; q < U; q++) {
+            transformer_load<VEC, NJ, EDGE>(a, We, u[q], off + k + q, ln, kk[q], val[q]);
+            e[q] = transformer_partial<VEC, NJ>(ln, kk[q]);
+        }
+        for (int o = G >> 1; o > 0; o >>= 1)
+#pragma unroll
+            for (int q = 0; q < U; q++) e[q] += __shfl_xor_sync(mask, e[q], o);
+#pragma unroll
+        for (int q = 0; q < U; q++) st.merge(e[q], 1.0f, val[q]);
+    }
+#pragma unroll 1
+    for (; k < k1; k++) {
+        Vec<VEC> kk[NJ], val[NJ];
+        transformer_load<VEC, NJ, EDGE>(a, We, __ldg(a.nbr + off + k), off + k, ln, kk, val);
+        st.merge(gatv2_head_sum(transformer_partial<VEC, NJ>(ln, kk), mask, G), 1.0f, val);
+    }
+}
+
+// the epilogue of the lane's valid column groups; a row without in-edges (s = 0, acc = 0) divides by 1
+template <int VEC, int NJ>
+__device__ __forceinline__ void transformer_finish(const TransformerAggArgs &a, int v, const AttnCols<NJ> &cl,
+                                                   const OnlineSoftmax<VEC, NJ> &st)
+{
+    const float s = st.s == 0.0f ? 1.0f : st.s;
+#pragma unroll
+    for (int j = 0; j < NJ; j++)
+        if (cl.valid[j]) attn_finish(a, v, cl.col[j], st.acc[j], s);
+}
+
+// lpr lanes per destination row (a power of two, a multiple of G); G lanes per head
+template <int VEC, int NJ, bool EDGE>
+__global__ void __launch_bounds__(256, 1) transformer_agg_kernel(const TransformerAggArgs a, int lpr, int G,
+                                                                 bool w_smem)
+{
+    const float *We = EDGE ? gatv2_stage_we(a, w_smem) : nullptr;
+    const int rows_per_warp = 32 / lpr;
+    const int lane = threadIdx.x & 31;
+    const int lg = lane % lpr, sub = lane / lpr;
+    const unsigned mask = lpr == 32 ? 0xffffffffu : ((1u << lpr) - 1u) << (sub * lpr);
+    const int grp = lg / G, hl = lg % G, heads_per_pass = lpr / G;
+    const int warps_per_block = blockDim.x >> 5;
+    const int64_t warp_global = (int64_t)blockIdx.x * warps_per_block + (threadIdx.x >> 5);
+    const int64_t warp_stride = (int64_t)gridDim.x * warps_per_block;
+    for (int64_t row0 = warp_global * rows_per_warp; row0 < a.n; row0 += warp_stride * rows_per_warp) {
+        // everything below is uniform over the row's sub-warp, so all its lanes reach every shuffle
+        const int v = (int)row0 + sub;
+        if (v >= a.n) continue;
+        const int deg = __ldg(a.in_deg + v);
+        if (a.heavy.n > 0 && deg > a.heavy.threshold) continue;  // the heavy-row kernels do these
+        const int off = __ldg(a.offsets + v);
+        for (int h0 = 0; h0 < a.H; h0 += heads_per_pass) {
+            const TransformerLane<VEC, NJ> ln = transformer_lane<VEC, NJ>(a, v, h0 + grp, hl, G);
+            OnlineSoftmax<VEC, NJ> st;
+            st.reset();
+            transformer_gather<VEC, NJ, EDGE>(a, We, off, 0, deg, ln, mask, G, st);
+            transformer_finish<VEC, NJ>(a, v, ln, st);
+        }
+    }
+}
+
+// one warp per kHeavyChunk-neighbor chunk of a heavy row: the chunk's per-head (m, s) and accumulator
+template <int VEC, int NJ, bool EDGE>
+__global__ void __launch_bounds__(256, 1) transformer_heavy_chunk_kernel(const TransformerAggArgs a, int G)
+{
+    const int lane = threadIdx.x & 31;
+    const int grp = lane / G, hl = lane % G, heads_per_pass = 32 / G;
+    const int warps_per_block = blockDim.x >> 5;
+    const int warp_global = blockIdx.x * warps_per_block + (threadIdx.x >> 5);
+    const int warp_stride = gridDim.x * warps_per_block;
+    for (int chunk = warp_global; chunk < a.heavy.chunks; chunk += warp_stride) {
+        const int h = __ldg(a.heavy.chunk_row + chunk);
+        const int v = __ldg(a.heavy.rows + h);
+        const int j = chunk - __ldg(a.heavy.chunk_base + h);
+        const int deg = __ldg(a.in_deg + v);
+        const int off = __ldg(a.offsets + v);
+        const int k0 = j * kHeavyChunk, k1 = min(deg, k0 + kHeavyChunk);
+        float *dst = a.heavy.partial + (size_t)chunk * a.ldp;
+        for (int h0 = 0; h0 < a.H; h0 += heads_per_pass) {
+            const TransformerLane<VEC, NJ> ln = transformer_lane<VEC, NJ>(a, v, h0 + grp, hl, G);
+            OnlineSoftmax<VEC, NJ> st;
+            st.reset();
+            transformer_gather<VEC, NJ, EDGE>(a, a.We_t, off, k0, k1, ln, 0xffffffffu, G, st);
+            attn_store_partial<VEC, NJ>(a, dst, ln, hl == 0 && ln.hd < a.H, st);
+        }
+    }
+}
+
+// one CTA per heavy row: combine steps 1 and 2, warp 0 starting from reset() (there is no self term)
+template <int VEC, int NJ>
+__global__ void __launch_bounds__(256, 1) transformer_heavy_combine_kernel(const TransformerAggArgs a, int G)
+{
+    extern __shared__ float4 transformer_comb_smem4[];
+    float *const ranges = reinterpret_cast<float *>(transformer_comb_smem4);   // [8][ldp], as the partials
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int grp = lane / G, hl = lane % G, heads_per_pass = 32 / G;
+    for (int h = blockIdx.x; h < a.heavy.n; h += gridDim.x) {
+        const int v = attn_combine_chunks<VEC>(a, h, ranges);
+        __syncthreads();
+        if (warp == 0) {
+            for (int h0 = 0; h0 < a.H; h0 += heads_per_pass) {
+                AttnCols<NJ> cl;
+                attn_lane_cols<VEC, NJ>(a, h0 + grp, hl, G, cl);
+                OnlineSoftmax<VEC, NJ> st;
+                st.reset();
+                attn_merge_ranges<VEC, NJ>(a, ranges, cl, cl.hd < a.H ? cl.hd : 0, st);
+                transformer_finish<VEC, NJ>(a, v, cl, st);
+            }
+        }
+        __syncthreads();
+    }
+}
+
+template <int VEC, int NJ, bool EDGE>
+int launch_transformer_variant(const TransformerAggArgs &a, int lpr, int G, size_t smem, cudaStream_t s,
+                               int *launches)
+{
+    auto k = transformer_agg_kernel<VEC, NJ, EDGE>;
+    if (smem > 48 * 1024) GNNB_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k<<<row_grid(a.n, lpr), 256, smem, s>>>(a, lpr, G, smem > 0);
+    GNNB_CUDA(cudaGetLastError());
+    if (launches) ++*launches;
+    if (a.heavy.n == 0) return GNNB_OK;
+    return launch_attn_heavy(transformer_heavy_chunk_kernel<VEC, NJ, EDGE>,
+                             transformer_heavy_combine_kernel<VEC, NJ>, a, s, launches, G);
+}
+
+template <int VEC, int NJ>
+int launch_transformer_nj(const TransformerAggArgs &a, bool edge, int lpr, int G, size_t smem, cudaStream_t s,
+                          int *launches)
+{
+    return edge ? launch_transformer_variant<VEC, NJ, true>(a, lpr, G, smem, s, launches)
+                : launch_transformer_variant<VEC, NJ, false>(a, lpr, G, 0, s, launches);
+}
+
+}  // namespace
+
+int launch_transformer_agg(const TransformerAggArgs &a, cudaStream_t s, int *launches)
+{
+    if (a.n <= 0) return GNNB_OK;
+    const int HC = a.H * a.C;
+    GNNB_TRY(check_attn_args(a, "transformer"));
+    GNNB_REQUIRE(a.g != nullptr && a.ldg >= 2 * HC && a.q != nullptr && a.ldq >= HC,
+                 "transformer aggregation: bad arguments");
+    const bool edge = a.ef_sorted != nullptr;
+    if (edge)
+        GNNB_REQUIRE(a.We_t != nullptr && a.edge_dim >= 1 && a.edge_dim <= kGineMaxEdgeDim &&
+                         a.lde % 4 == 0 && a.lde >= a.edge_dim && a.ldw % 4 == 0 && a.ldw >= HC &&
+                         aligned16(a.ef_sorted),
+                     "transformer aggregation: bad edge features");
+    const bool v4 = attn_v4(a) && a.ldq % 4 == 0 && aligned16(a.q) && (!edge || aligned16(a.We_t));
+    const int vec = v4 ? 4 : 1;
+    const int cg = (a.C + vec - 1) / vec;   // VEC-column groups per head
+    int G = 1;
+    while (G < 32 && G < cg) G *= 2;
+    const int nj = (cg + G - 1) / G;
+    GNNB_REQUIRE(nj <= 2, "transformer aggregation: head width C = " + std::to_string(a.C) +
+                              " exceeds the lanes of a warp (at most " +
+                              std::to_string(kGatv2MaxHeadWidth) + " with C % 4 == 0, else " +
+                              std::to_string(kGatv2MaxHeadWidth1) + ")");
+    int lpr = G;
+    while (lpr < 32 && lpr < G * a.H) lpr *= 2;
+    // W_e^T in shared memory when it fits, as GATv2
+    const size_t w_bytes = edge ? sizeof(float) * (size_t)a.edge_dim * a.ldw : 0;
+    const size_t smem = w_bytes <= 200 * 1024 ? w_bytes : 0;
+    if (vec == 4)
+        return nj == 1 ? launch_transformer_nj<4, 1>(a, edge, lpr, G, smem, s, launches)
+                       : launch_transformer_nj<4, 2>(a, edge, lpr, G, smem, s, launches);
+    return nj == 1 ? launch_transformer_nj<1, 1>(a, edge, lpr, G, smem, s, launches)
+                   : launch_transformer_nj<1, 2>(a, edge, lpr, G, smem, s, launches);
 }
 
 }  // namespace gnnb

@@ -177,11 +177,11 @@ int launch_gine_agg_proj(const GineProjAggArgs &a, cudaStream_t s, int *launches
 int launch_permute_edge_rows(const float *src, int dim, const int32_t *idx, int e, float *dst,
                              int ldd, cudaStream_t s, int *launches);
 
-// What the GAT and GATv2 aggregations share: the layer's GEMM output, the attention shape, the
-// epilogue y_v = act(sum softmax_v(e) m_u + bias (+ skip_v)) written to out, the CSR and the heavy
-// rows, whose partials are [heavy.chunks][ldp]: accumulator (H*C), then max [H], sum [H].
+// What the GAT, GATv2 and TransformerConv aggregations share: the layer's GEMM output, the attention
+// shape, the epilogue y_v = act(sum softmax_v(e) m_u + bias (+ skip_v)) written to out, the CSR and
+// the heavy rows, whose partials are [heavy.chunks][ldp]: accumulator (H*C), then max [H], sum [H].
 struct AttnAggArgs {
-    const float *g;        // [n][ldg]: GAT [h | a_src | a_dst], GATv2 [xl | xr]
+    const float *g;        // [n][ldg]: GAT [h | a_src | a_dst], GATv2 [xl | xr], TransformerConv [k | v]
     int ldg;
     int H, C;
     float slope;           // LeakyReLU negative slope
@@ -260,6 +260,25 @@ int launch_gatv2_agg(const Gatv2AggArgs &a, cudaStream_t s, int *launches);
 int launch_gatv2_self_attr(const float *ef_sorted, int lde, int edge_dim, const int32_t *offsets,
                            const int32_t *nbr, const int32_t *in_deg, int n, float *self_attr,
                            cudaStream_t s, int *launches);
+
+// TransformerConv attention aggregation (PyG TransformerConv, concat heads, root_weight, inference).
+// g holds the source-side GEMM outputs per row: k = x W_k^T + b_k in columns [0, H*C), v = x W_v^T +
+// b_v in [H*C, 2 H*C); q holds q = x W_q^T + b_q, already scaled by 1/sqrt(C).  Per destination v and
+// head h, over every in-edge u -> v (self loops and duplicates included, no self term):
+// ê = e_uv W_e^T (edge features only, else 0), e_uvh = <q_v, k_u + ê>_h, y_v = act(sum softmax_v(e)
+// (v_u + ê) + bias (+ skip_v)); a row without in-edges gets act(bias (+ skip_v)).  The model handle
+// passes bias = b_skip and skip = x W_skip^T (+ the model's residual).  GATv2's lane layout, head
+// width limits and edge projection; GAT's online softmax, epilogue and heavy-row scheme.
+struct TransformerAggArgs : AttnAggArgs {
+    const float *q;          // [n][ldq]
+    int ldq;
+    // edge features (edge_dim > 0), else ef_sorted null: the edge term of slot k is ef_sorted[k] W_e^T
+    const float *ef_sorted;  // [slots][lde], neighbor-slot order
+    int lde, edge_dim;
+    const float *We_t;       // [edge_dim][ldw] (ldw multiple of 4, zero padded)
+    int ldw;
+};
+int launch_transformer_agg(const TransformerAggArgs &a, cudaStream_t s, int *launches);
 
 struct PnaAggArgs {
     const float *ab;       // [n][2F]: cols [0,F) = x.W_nbr^T, cols [F,2F) = x.W_self^T + b_pre

@@ -134,6 +134,15 @@ void enumerate_params(gnnb_model *m)
             add_param(m, base + "_conv_lin_r_bias", {fo});
             if (m->has_edge_features()) add_param(m, base + "_conv_lin_edge_weight", {fo, d.edge_dim});
             break;
+        case GNNB_CONV_TRANSFORMER:   // PyG TransformerConv: lin_key, lin_query, lin_value, lin_edge, lin_skip
+            for (const char *lin : {"_conv_lin_key", "_conv_lin_query", "_conv_lin_value"}) {
+                add_param(m, base + lin + "_weight", {fo, fi});
+                add_param(m, base + lin + "_bias", {fo});
+            }
+            if (m->has_edge_features()) add_param(m, base + "_conv_lin_edge_weight", {fo, d.edge_dim});
+            add_param(m, base + "_conv_lin_skip_weight", {fo, fi});
+            add_param(m, base + "_conv_lin_skip_bias", {fo});
+            break;
         }
     }
 }
@@ -237,8 +246,9 @@ extern "C" int gnnb_model_create(const gnnb_model_desc *desc, int device, gnnb_m
     gnnb_model_desc d{};
     std::memcpy(&d, desc, offsetof(gnnb_model_desc, edge_dim));
     GNNB_REQUIRE((d.conv_type >= GNNB_CONV_GCN && d.conv_type <= GNNB_CONV_GAT) ||
-                     d.conv_type == GNNB_CONV_GATV2,
-                 "conv_type must be GCN, GIN, SAGE, PNA, GINE, GAT or GATv2 (0..5 or 7)");
+                     d.conv_type == GNNB_CONV_GATV2 || d.conv_type == GNNB_CONV_TRANSFORMER,
+                 "conv_type must be GCN, GIN, SAGE, PNA, GINE, GAT, GATv2 or TransformerConv (0..5, 7 "
+                 "or 8)");
     if (d.conv_type == GNNB_CONV_GINE) {
         d.edge_dim = desc->edge_dim;
         GNNB_REQUIRE(d.edge_dim >= 1 && d.edge_dim <= kGineMaxEdgeDim,
@@ -246,15 +256,19 @@ extern "C" int gnnb_model_create(const gnnb_model_desc *desc, int device, gnnb_m
     }
     GNNB_REQUIRE(d.num_layers >= 0 && d.num_layers <= 64, "num_layers out of range");
     GNNB_REQUIRE(d.in_dim > 0 && d.hidden_dim > 0 && d.out_dim > 0, "dimensions must be positive");
-    if (d.conv_type == GNNB_CONV_GAT || d.conv_type == GNNB_CONV_GATV2) {
-        // the GAT fields follow edge_dim; only GAT and GATv2 callers set them
-        const std::string conv = d.conv_type == GNNB_CONV_GAT ? "GAT" : "GATv2";
+    const bool transformer = d.conv_type == GNNB_CONV_TRANSFORMER;
+    if (d.conv_type == GNNB_CONV_GAT || d.conv_type == GNNB_CONV_GATV2 || transformer) {
+        // the GAT fields follow edge_dim; only GAT, GATv2 and TransformerConv callers set them, and
+        // TransformerConv has no slope to read
+        const std::string conv = d.conv_type == GNNB_CONV_GAT     ? "GAT"
+                                 : d.conv_type == GNNB_CONV_GATV2 ? "GATv2"
+                                                                  : "TransformerConv";
         d.edge_dim = desc->edge_dim;
         GNNB_REQUIRE(d.edge_dim >= 0 && d.edge_dim <= kGineMaxEdgeDim,
                      conv + " edge_dim must be 0 (no edge features) or 1.." +
                          std::to_string(kGineMaxEdgeDim));
         d.gat_heads = desc->gat_heads;
-        d.gat_negative_slope = desc->gat_negative_slope;
+        if (!transformer) d.gat_negative_slope = desc->gat_negative_slope;
         GNNB_REQUIRE(d.gat_heads >= 1 && d.gat_heads <= GNNB_GAT_MAX_HEADS,
                      conv + " gat_heads must be 1.." + std::to_string(GNNB_GAT_MAX_HEADS));
         GNNB_REQUIRE(std::isfinite(d.gat_negative_slope), conv + " gat_negative_slope must be finite");
@@ -264,11 +278,11 @@ extern "C" int gnnb_model_create(const gnnb_model_desc *desc, int device, gnnb_m
                          conv + ": every layer's output width (hidden_dim, out_dim) must be a multiple "
                          "of gat_heads, got width " + std::to_string(fo) + " with " +
                              std::to_string(d.gat_heads) + " heads");
-            // GATv2 spreads a head's columns over at most one warp (agg.cu)
+            // GATv2 and TransformerConv spread a head's columns over at most one warp (agg.cu)
             const int C = fo / d.gat_heads;
             GNNB_REQUIRE(d.conv_type == GNNB_CONV_GAT ||
                              C <= (C % 4 == 0 ? kGatv2MaxHeadWidth : kGatv2MaxHeadWidth1),
-                         "GATv2: a head's width (layer width / gat_heads) must be at most " +
+                         conv + ": a head's width (layer width / gat_heads) must be at most " +
                              std::to_string(kGatv2MaxHeadWidth) + " when a multiple of 4, else at "
                              "most " + std::to_string(kGatv2MaxHeadWidth1) + ", got " +
                              std::to_string(C));
@@ -506,6 +520,25 @@ extern "C" int gnnb_model_finalize(gnnb_model_t *m)
             idx += m->has_edge_features() ? 7 : 6;
             break;
         }
+        case GNNB_CONV_TRANSFORMER: {
+            // [key w, b, query w, b, value w, b (, lin_edge_weight), skip w, b]: a = lin_key,
+            // b = lin_value, c = lin_query scaled by 1/sqrt(C) (in double, rounded once: exact when
+            // C is a power of 4), d = lin_skip, e = W_e^T (no bias)
+            const bool edges = m->has_edge_features();
+            const double scale = 1.0 / std::sqrt((double)(fo / d.gat_heads));
+            std::vector<float> Wq(param(m, idx + 2), param(m, idx + 2) + (size_t)fo * fi);
+            std::vector<float> bq(param(m, idx + 3), param(m, idx + 3) + fo);
+            for (float &w : Wq) w = (float)((double)w * scale);
+            for (float &b : bq) b = (float)((double)b * scale);
+            L.a = pack_linear(pk, param(m, idx), param(m, idx + 1), fo, fi);
+            L.b = pack_linear(pk, param(m, idx + 4), param(m, idx + 5), fo, fi);
+            L.c = pack_linear(pk, Wq.data(), bq.data(), fo, fi);
+            const size_t is = idx + (edges ? 7 : 6);
+            L.d = pack_linear(pk, param(m, is), param(m, is + 1), fo, fi);
+            if (edges) L.e = pack_linear(pk, param(m, idx + 6), nullptr, fo, d.edge_dim);
+            idx = is + 2;
+            break;
+        }
         }
         layer_p.push_back(L);
     }
@@ -546,8 +579,8 @@ extern "C" int gnnb_model_finalize(gnnb_model_t *m)
     }
     fused_release(m);
     fused_tc_release(m);
-    // neither fused kernel takes GINE, GAT or GATv2 (they leave m->fused / m->fused_tc null): those
-    // run layerwise
+    // neither fused kernel takes GINE, GAT, GATv2 or TransformerConv (they leave m->fused /
+    // m->fused_tc null): those run layerwise
     GNNB_TRY(fused_prepare(m));
     GNNB_TRY(fused_tc_prepare(m));
     m->finalized = true;
@@ -647,17 +680,21 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
     const bool gat_edges = gat && m->has_edge_features();
     const bool gatv2 = d.conv_type == GNNB_CONV_GATV2;
     const bool gatv2_edges = gatv2 && m->has_edge_features();
+    const bool transformer = d.conv_type == GNNB_CONV_TRANSFORMER;
+    const bool transformer_edges = transformer && m->has_edge_features();
+    const bool attn = gat || gatv2 || transformer;
     const int LH = gat_edges ? d.num_layers * d.gat_heads : 0;   // edge logit columns per slot / row
-    // GINE has no heavy-row bucketing or hub hints, as PNA; GAT and GATv2 are bucketed but take no
-    // hub hints
+    // GINE has no heavy-row bucketing or hub hints, as PNA; the attention convs are bucketed but take
+    // no hub hints
     const bool bucketed = d.conv_type != GNNB_CONV_PNA && !gine;
-    const bool hub_hints = bucketed && !gat && !gatv2;
+    const bool hub_hints = bucketed && !attn;
     const int lde = round_up(std::max(d.edge_dim, 1), 4);
     // GAT: the layer GEMM's output rows [h | a_src | a_dst], and the heavy-row partials, are
     // H*C + 2H floats wide
-    const int ld_gat = gat || gatv2 ? round_up(std::max(d.hidden_dim, d.out_dim) + 2 * d.gat_heads, 4) : 0;
-    // GATv2: the layer GEMMs' output rows [xl | xr], 2 H*C floats wide
-    const int ld_xlr = gatv2 ? round_up(2 * std::max(d.hidden_dim, d.out_dim), 4) : 0;
+    const int ld_gat = attn ? round_up(std::max(d.hidden_dim, d.out_dim) + 2 * d.gat_heads, 4) : 0;
+    // GATv2: the layer GEMMs' output rows [xl | xr], 2 H*C floats wide; TransformerConv: [k | v] and
+    // [q | r] as wide
+    const int ld_xlr = gatv2 || transformer ? round_up(2 * std::max(d.hidden_dim, d.out_dim), 4) : 0;
     if (d.num_layers > 0) {
         ProfScope ps(m->prof, PROF_TABLES, s);
         // the out-degree table (lib:1051-1083) is only read by the optional hub-row hints
@@ -675,7 +712,7 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
                               want_out_deg ? m->out_deg.as<int32_t>() : nullptr, offsets, nbr, eidx,
                               m->tws, s, launches, m->edge_flag.as<int>()));
         // edge features in neighbor-slot order, once per run; every layer reads them in order
-        if (gine || gatv2_edges) {
+        if (gine || gatv2_edges || transformer_edges) {
             GNNB_TRY(m->ef_sorted.ensure(sizeof(float) * (size_t)En * lde));
             GNNB_TRY(launch_permute_edge_rows(ef, d.edge_dim, eidx, E, m->ef_sorted.as<float>(), lde, s,
                                               launches));
@@ -709,7 +746,7 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
     m->last_hub_rows = 0;
     if (!strict && d.num_layers > 0 && bucketed && n_graphs > 0 && T64 / n_graphs > 50000) {
         GNNB_TRY(find_heavy_rows(in_deg, T, heavy_thr, m->tws, m->heavy, s, launches));
-        GNNB_TRY(heavy_setup(m->tws, m->heavy.n_chunks, gat || gatv2 ? ld_gat : maxf));
+        GNNB_TRY(heavy_setup(m->tws, m->heavy.n_chunks, attn ? ld_gat : maxf));
         // a feature matrix larger than L2: keep the rows of the most-referenced sources resident
         // (the out-degree table, lib:1051-1083, is what ranks them)
         const size_t row_bytes = sizeof(float) * (size_t)std::max(d.in_dim, d.hidden_dim);
@@ -728,12 +765,13 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
 
     GNNB_TRY(m->feat[0].ensure(sizeof(float) * (size_t)Tn * ldf));
     GNNB_TRY(m->feat[1].ensure(sizeof(float) * (size_t)Tn * ldf));
-    // GAT and GATv2 aggregate into dst
-    if (!gat && !gatv2) GNNB_TRY(m->agg.ensure(sizeof(float) * (size_t)Tn * ldf));
+    // the attention convs aggregate into dst; TransformerConv keeps [q | r] in agg
+    if (!attn) GNNB_TRY(m->agg.ensure(sizeof(float) * (size_t)Tn * ldf));
+    if (transformer) GNNB_TRY(m->agg.ensure(sizeof(float) * (size_t)Tn * ld_xlr));
     if (d.conv_type == GNNB_CONV_GIN || d.conv_type == GNNB_CONV_PNA || gine)
         GNNB_TRY(m->hid.ensure(sizeof(float) * (size_t)Tn * ldf));
     if (gat) GNNB_TRY(m->hid.ensure(sizeof(float) * (size_t)Tn * ld_gat));
-    if (gatv2) GNNB_TRY(m->hid.ensure(sizeof(float) * (size_t)Tn * ld_xlr));
+    if (gatv2 || transformer) GNNB_TRY(m->hid.ensure(sizeof(float) * (size_t)Tn * ld_xlr));
     if (d.conv_type == GNNB_CONV_PNA)
         GNNB_TRY(m->wide.ensure(sizeof(float) * (size_t)Tn * 14 * (size_t)ldf));
 
@@ -818,7 +856,8 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
             break;
         }
         case GNNB_CONV_GAT:
-        case GNNB_CONV_GATV2: {
+        case GNNB_CONV_GATV2:
+        case GNNB_CONV_TRANSFORMER: {
             // the attention aggregation's epilogue applies bias, skip and activation and writes the
             // layer; heavy-row partials [acc H*C | max H | sum H]
             const int H = d.gat_heads;
@@ -831,6 +870,31 @@ static int run_layerwise(gnnb_model *m, const float *x, const int32_t *coo, cons
             at.ldp = round_up(fo + 2 * H, 4);
             float *hid = m->hid.as<float>();
             at.g = hid;
+            if (transformer) {
+                // four GEMMs: [k | v] = x.[W_k | W_v]^T + [b_k | b_v] into hid, and [q | r] into agg:
+                // q = x.W_q^T + b_q (1/sqrt(C) folded in), r = x.W_skip^T (+ the model's skip) without
+                // b_skip.  The epilogue adds b_skip as its bias and r as its skip.
+                const int ld2 = round_up(2 * fo, 4);
+                float *qr = m->agg.as<float>();
+                TransformerAggArgs ta{at};
+                ta.g = hid; ta.ldg = ld2; ta.q = qr; ta.ldq = ld2;
+                ta.bias = L.d.bias; ta.skip = qr + fo; ta.ldskip = ld2;
+                GemmArgs gk = gemm_args(cur, cur_ld, L.a, hid, ld2, T, GNNB_ACT_IDENTITY);
+                GemmArgs gv = gemm_args(cur, cur_ld, L.b, hid + fo, ld2, T, GNNB_ACT_IDENTITY);
+                GemmArgs gq = gemm_args(cur, cur_ld, L.c, qr, ld2, T, GNNB_ACT_IDENTITY);
+                GemmArgs gs = gemm_args(cur, cur_ld, L.d, qr + fo, ld2, T, GNNB_ACT_IDENTITY, skip, cur_ld);
+                gs.bias = nullptr;
+                for (const GemmArgs *g : {&gk, &gv, &gq, &gs}) {
+                    ProfScope ps(m->prof, PROF_GEMM, s);
+                    GNNB_TRY(launch_gemm(*g, strict, s, launches));
+                }
+                if (transformer_edges) {
+                    ta.ef_sorted = m->ef_sorted.as<float>();
+                    ta.lde = lde; ta.edge_dim = d.edge_dim; ta.We_t = L.e.Wt; ta.ldw = L.e.ldw;
+                }
+                { ProfScope ps(m->prof, PROF_AGG, s); GNNB_TRY(launch_transformer_agg(ta, s, launches)); }
+                break;
+            }
             if (gat) {
                 // one GEMM: [h | a_src | a_dst] = x.[W | w_src | w_dst]^T, no bias
                 GatAggArgs ga{at};
@@ -948,6 +1012,11 @@ static int choose_path(gnnb_model_t *m, int max_n, int max_e, int *path, int *ke
                       "models run on the layerwise path");
             return GNNB_ERR_INVALID;
         }
+        if (m->d.conv_type == GNNB_CONV_TRANSFORMER) {
+            set_error("fused path requested but the fused kernels have no TransformerConv attention; "
+                      "TransformerConv models run on the layerwise path");
+            return GNNB_ERR_INVALID;
+        }
         if (!can_tc && !can_fma) {
             set_error("fused path requested but unsupported for this model/batch (graph larger than "
                       "a CTA tile, strict math, or unsupported dims)");
@@ -984,23 +1053,24 @@ static int fused_any_status(gnnb_model_t *m, int *status)
     return m->last_kernel == 3 ? fused_tc_status(m, status) : fused_status(m, status);
 }
 
-// a handle with edge features (GINE, GAT with edge_dim) takes them through the *_edges entry
-// points, every other handle runs through the plain ones
+// a handle with edge features (GINE, or GAT, GATv2 or TransformerConv with edge_dim) takes them
+// through the *_edges entry points, every other handle runs through the plain ones
 static int check_edges_entry(gnnb_model_t *m, bool edges_entry)
 {
     GNNB_TRY(check_ready(m));
     const bool edges = m->has_edge_features();
     if (edges && !edges_entry) {
-        set_error(std::string(m->d.conv_type == GNNB_CONV_GAT     ? "a GAT model with edge_dim"
-                              : m->d.conv_type == GNNB_CONV_GATV2 ? "a GATv2 model with edge_dim"
-                                                                  : "a GINE model") +
+        set_error(std::string(m->d.conv_type == GNNB_CONV_GAT           ? "a GAT model with edge_dim"
+                              : m->d.conv_type == GNNB_CONV_GATV2       ? "a GATv2 model with edge_dim"
+                              : m->d.conv_type == GNNB_CONV_TRANSFORMER ? "a TransformerConv model with edge_dim"
+                                                                        : "a GINE model") +
                   " needs its edge features: run it with gnnb_model_run_batch_edges or "
                   "gnnb_model_run_batch_edges_async");
         return GNNB_ERR_INVALID;
     }
     if (!edges && edges_entry) {
-        set_error("the *_edges entry points run GINE models and GAT and GATv2 models with edge_dim "
-                  "only; this model has no edge features");
+        set_error("the *_edges entry points run GINE models and GAT, GATv2 and TransformerConv models "
+                  "with edge_dim only; this model has no edge features");
         return GNNB_ERR_INVALID;
     }
     return GNNB_OK;

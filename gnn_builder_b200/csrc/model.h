@@ -35,6 +35,9 @@ struct LayerPack {
 // GATv2: a = lin_l and b = lin_r (weights and biases, two GEMMs into one [T][round_up(2 H*C, 4)]
 // buffer); c carries att [H*C] and d the conv bias [H*C] as vectors; e = lin_edge's W_e^T
 // [edge_dim][ldw] without a bias (edge_dim > 0 only), applied per edge by the aggregation.
+// TransformerConv: a = lin_key and b = lin_value (two GEMMs into [k | v], one [T][round_up(2 H*C, 4)]
+// buffer), c = lin_query with 1/sqrt(C) folded into its weight and bias, d = lin_skip (its GEMM runs
+// without the bias; the aggregation epilogue adds d.bias), e = lin_edge's W_e^T as for GATv2.
 
 // fused-kernel plans (fused.cu, fused_tc.cu)
 struct FusedPlan;
@@ -108,7 +111,8 @@ struct gnnb_model {
     // layerwise workspaces
     gnnb::DeviceBuf in_deg, out_deg, offsets, nbr, nbr_hub, dinv, feat[2], agg, hid, wide, pooled,
         hbuf[2], pool_tmp, ptr_tmp;
-    gnnb::DeviceBuf edge_index, ef_sorted;   // GINE, GATv2: edge id and edge features per neighbor slot
+    // GINE, GATv2, TransformerConv: edge id and edge features per neighbor slot
+    gnnb::DeviceBuf edge_index, ef_sorted;
     gnnb::DeviceBuf self_attr;   // GATv2 with edge_dim: each row's self-loop attribute [n][lde]
     // GAT with edge_dim: the edge logits of every layer and head per neighbor slot and per row
     // (gat_edge_logits_kernel), and the folded edge weights [L*H][edge_dim] inside `weights`
@@ -128,7 +132,8 @@ struct gnnb_model {
     int64_t last_emb_rows = 0;
 
     int emb_dim() const { return d.num_layers == 0 ? d.in_dim : d.out_dim; }
-    // GINE, and GAT and GATv2 with edge_dim: edge features come through the *_edges entry points
+    // GINE, and GAT, GATv2 and TransformerConv with edge_dim: edge features come through the *_edges
+    // entry points
     bool has_edge_features() const { return d.edge_dim > 0; }
     void layer_dims(int layer, int *fi, int *fo) const
     {

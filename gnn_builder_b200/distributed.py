@@ -414,7 +414,8 @@ _LAYER_PARAMS = {
               "conv_lin_r_bias"),
 }
 
-_CONV_NAMES = {0: "GCN", 1: "GIN", 2: "SAGE", 3: "PNA", 4: "GINE", 5: "GAT", 7: "GATv2"}
+_CONV_NAMES = {0: "GCN", 1: "GIN", 2: "SAGE", 3: "PNA", 4: "GINE", 5: "GAT", 7: "GATv2",
+               8: "TransformerConv"}
 
 
 class LargeGraphModel:

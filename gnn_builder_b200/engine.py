@@ -48,9 +48,10 @@ class Engine:
         self.desc = dict(desc)
         self.out_dim = int(desc["mlp_out"])
         self.in_dim = int(desc["in_dim"])
-        # GINE models, and GAT and GATv2 models with edge_dim, take edge features and run through
-        # the *_edges entry points
-        self.edge_dim = int(desc.get("edge_dim", 0)) if int(desc["conv_type"]) in (4, 5, 7) else 0
+        # GINE models, and GAT, GATv2 and TransformerConv models with edge_dim, take edge features
+        # and run through the *_edges entry points
+        self.edge_dim = (int(desc.get("edge_dim", 0)) if int(desc["conv_type"]) in (4, 5, 7, 8)
+                         else 0)
         self._h = C.c_void_p()
         self._pinned = {}
         s = _desc_struct(desc, max_nodes, max_edges)

@@ -192,6 +192,44 @@ class _GATv2Conv(nn.Module):
         return _scatter_sum(msg, dst, n) + self.bias
 
 
+class _TransformerConv(nn.Module):
+    """PyG TransformerConv with an int ``in_channels``, concatenated heads, ``beta=False`` and
+    ``root_weight=True``, for inference.  Parameters in PyG's order: ``lin_key``, ``lin_query``,
+    ``lin_value`` (weight [H*C][in] and bias each), with ``edge_dim`` ``lin_edge.weight``
+    [H*C][edge_dim] (no bias), then ``lin_skip`` (weight and bias).  No self loops are added: the
+    input's self loops and duplicate edges are ordinary edges, and a node without in-edges gets
+    ``lin_skip(x)`` alone."""
+
+    def __init__(self, in_channels: int, out_channels: int, heads: int,
+                 edge_dim: Optional[int] = None):
+        super().__init__()
+        self.heads = heads
+        self.head_channels = out_channels // heads
+        self.edge_dim = edge_dim
+        self.lin_key = nn.Linear(in_channels, out_channels, bias=True)
+        self.lin_query = nn.Linear(in_channels, out_channels, bias=True)
+        self.lin_value = nn.Linear(in_channels, out_channels, bias=True)
+        if edge_dim is not None:
+            self.lin_edge = nn.Linear(edge_dim, out_channels, bias=False)
+        self.lin_skip = nn.Linear(in_channels, out_channels, bias=True)
+
+    def forward(self, x: Tensor, edge_index: Tensor, edge_attr: Optional[Tensor] = None) -> Tensor:
+        n, H, C = x.shape[0], self.heads, self.head_channels
+        src, dst = edge_index[0], edge_index[1]
+        q = self.lin_query(x).view(n, H, C)
+        k = self.lin_key(x)[src].view(-1, H, C)
+        v = self.lin_value(x)[src].view(-1, H, C)
+        if self.edge_dim is not None:
+            e = self.lin_edge(edge_attr.reshape(-1, self.edge_dim)).view(-1, H, C)
+            k = k + e
+            v = v + e
+        logit = (q[dst] * k).sum(-1) / math.sqrt(C)
+        p = (logit - _scatter_minmax(logit, dst, n, "amax")[dst]).exp()
+        alpha = p / _scatter_sum(p, dst, n)[dst]
+        msg = (v * alpha.unsqueeze(-1)).reshape(-1, H * C)
+        return _scatter_sum(msg, dst, n) + self.lin_skip(x)
+
+
 class _SAGEConv(nn.Module):
     def __init__(self, in_channels: int, out_channels: int):
         super().__init__()
@@ -398,6 +436,54 @@ class GATv2Conv_GNNB(nn.Module):
         return self.conv(x, edge_index, edge_attr)
 
 
+class TransformerConv_GNNB(nn.Module):
+    """Graph transformer attention (PyG ``TransformerConv``, inference): per head,
+    q = x W_q^T + b_q, k = x W_k^T + b_k, v = x W_v^T + b_v, logits a_uv = <q_v, k_u> / sqrt(C) over
+    the in-edges of v, y_v = sum softmax_v(a) v_u + x_v W_skip^T + b_skip, heads concatenated.  No
+    self loops are added; a node without in-edges gets x_v W_skip^T + b_skip.  ``out_channels`` is
+    the concatenated width and must be a multiple of ``heads``.  Pass ``heads`` with
+    ``functools.partial``.
+
+    ``edge_dim`` (a positive int, also passed with ``functools.partial``) adds ``lin_edge`` (no
+    bias): e_uv W_e^T is added to both k_u and v_u.  The model's ``graph_input_edge_dim`` must then
+    equal it.  PyG's ``concat=False``, ``beta=True``, ``root_weight=False``, ``bias=False``,
+    ``dropout`` and bipartite ``in_channels`` are not supported."""
+
+    def __init__(self, in_channels: int, out_channels: int, heads: int = 1,
+                 edge_dim: Optional[int] = None, concat: bool = True, beta: bool = False,
+                 dropout: float = 0.0, bias: bool = True, root_weight: bool = True, p_in: int = 1,
+                 p_out: int = 1):
+        super().__init__()
+        if not isinstance(in_channels, int) or isinstance(in_channels, bool):
+            raise ValueError(f"in_channels must be an int (bipartite inputs are not supported), "
+                             f"got {in_channels!r}")
+        if not isinstance(heads, int) or isinstance(heads, bool) or heads < 1:
+            raise ValueError(f"heads must be a positive int, got {heads!r}")
+        if edge_dim is not None and (not isinstance(edge_dim, int) or isinstance(edge_dim, bool)
+                                     or edge_dim < 1):
+            raise ValueError(f"edge_dim must be None or a positive int, got {edge_dim!r}")
+        if out_channels % heads != 0:
+            raise ValueError(f"out_channels ({out_channels}) must be a multiple of heads ({heads})")
+        for name, value, default in (("concat", concat, True), ("beta", beta, False),
+                                     ("bias", bias, True), ("root_weight", root_weight, True)):
+            if value is not default:
+                raise ValueError(f"TransformerConv_GNNB supports only {name}={default}, got {value!r}")
+        if dropout != 0.0:
+            raise ValueError(f"TransformerConv_GNNB runs inference without dropout, got {dropout!r}")
+        self.in_channels = in_channels
+        self.out_channels = out_channels
+        self.heads = heads
+        self.edge_dim = edge_dim
+        self.p_in = p_in
+        self.p_out = p_out
+        self.conv = _TransformerConv(in_channels, out_channels, heads, edge_dim)
+
+    def forward(self, x: Tensor, edge_index: Tensor, edge_attr: Optional[Tensor] = None) -> Tensor:
+        if self.edge_dim is not None and edge_attr is None:
+            raise ValueError("a TransformerConv_GNNB with edge_dim needs edge_attr")
+        return self.conv(x, edge_index, edge_attr)
+
+
 class PNAConv_GNNB(nn.Module):
     """models.py:209-240"""
 
@@ -540,11 +626,14 @@ class MLP(nn.Module):
 
 
 SUPPORTED_GNN_CONVS = [GCNConv_GNNB, GINConv_GNNB, PNAConv_GNNB, SAGEConv_GNNB, GINEConv_GNNB,
-                       GATConv_GNNB, GATv2Conv_GNNB]
+                       GATConv_GNNB, GATv2Conv_GNNB, TransformerConv_GNNB]
 
-# 6 is not assigned (GNNB_CONV_GATV2 = 7 in include/gnnb_b200.h)
+# 6 is not assigned (GNNB_CONV_GATV2 = 7, GNNB_CONV_TRANSFORMER = 8 in include/gnnb_b200.h)
 CONV_TYPE_IDS = {"GCNConv_GNNB": 0, "GINConv_GNNB": 1, "SAGEConv_GNNB": 2, "PNAConv_GNNB": 3,
-                 "GINEConv_GNNB": 4, "GATConv_GNNB": 5, "GATv2Conv_GNNB": 7}
+                 "GINEConv_GNNB": 4, "GATConv_GNNB": 5, "GATv2Conv_GNNB": 7,
+                 "TransformerConv_GNNB": 8}
+# the attention convs: heads, and edge features only when their partial carries edge_dim
+_ATTENTION_CONVS = ("GATConv_GNNB", "GATv2Conv_GNNB", "TransformerConv_GNNB")
 ACTIVATION_IDS = {None: 0, "ReLU": 1, "GELU": 2, "Sigmoid": 3, "Tanh": 4}
 POOL_IDS = {"add": 0, "mean": 1, "max": 2}
 
@@ -569,10 +658,10 @@ class GNNModel(nn.Module):
         if conv_cls not in SUPPORTED_GNN_CONVS:
             raise ValueError(f"gnn_conv must be one of {SUPPORTED_GNN_CONVS}")
         self._conv_cls = conv_cls
-        # GAT and GATv2 take edge features only when their partial carries edge_dim
+        # the attention convs take edge features only when their partial carries edge_dim
         self._conv_kwargs = dict(getattr(gnn_conv, "keywords", None) or {})
         gat_edge_dim = (self._conv_kwargs.get("edge_dim")
-                        if conv_cls in (GATConv_GNNB, GATv2Conv_GNNB) else None)
+                        if conv_cls.__name__ in _ATTENTION_CONVS else None)
         self.uses_edge_features = conv_cls is GINEConv_GNNB or gat_edge_dim is not None
         conv_kwargs = {}
         if conv_cls is GINEConv_GNNB:
@@ -729,9 +818,10 @@ class GNNModel(nn.Module):
         )
         if self.uses_edge_features:
             d["edge_dim"] = int(self.graph_input_edge_dim)
-        if conv_name in ("GATConv_GNNB", "GATv2Conv_GNNB"):
+        if conv_name in _ATTENTION_CONVS:
             kw = self._conv_kwargs   # a model without layers has no conv to ask
             d["gat_heads"] = int(conv0.heads if conv0 is not None else kw.get("heads", 1))
+        if conv_name in ("GATConv_GNNB", "GATv2Conv_GNNB"):   # TransformerConv has no slope
             d["gat_negative_slope"] = float(conv0.negative_slope if conv0 is not None
                                             else kw.get("negative_slope", 0.2))
         return d

@@ -57,13 +57,20 @@ enum {
  * edge_dim > 0 the self loop's attribute is the mean of the node's other in-edge attributes.
  * Each head's width C must be at most 256 when C is a multiple of 4, else at most 64.  The value 6
  * is not assigned. */
+/* TransformerConv (PyG TransformerConv for inference: concat heads, root_weight, no beta, no self
+ * loops added) reads edge_dim and gat_heads as GAT does, not gat_negative_slope, and follows GAT's
+ * entry-point, path and math rules.  Per head, e_uv = <q_v, k_u (+ e_uv W_e^T)> / sqrt(C) over the
+ * in-edges of v (input self loops and duplicate edges count as ordinary edges),
+ * y_v = sum softmax_v(e) (v_u (+ e_uv W_e^T)) + x_v W_skip^T + b_skip; a node without in-edges gets
+ * x_v W_skip^T + b_skip.  Parameters in PyG's order: lin_key, lin_query, lin_value (weight and bias
+ * each), lin_edge.weight (edge_dim > 0), lin_skip.  Head widths as GATv2. */
 enum {
     GNNB_CONV_GCN = 0, GNNB_CONV_GIN = 1, GNNB_CONV_SAGE = 2, GNNB_CONV_PNA = 3, GNNB_CONV_GINE = 4,
-    GNNB_CONV_GAT = 5, GNNB_CONV_GATV2 = 7
+    GNNB_CONV_GAT = 5, GNNB_CONV_GATV2 = 7, GNNB_CONV_TRANSFORMER = 8
 };
-/* edge feature widths a GINE, edge-attention GAT or GATv2 model handle accepts */
+/* edge feature widths a GINE, edge-attention GAT, GATv2 or TransformerConv model handle accepts */
 #define GNNB_GINE_MAX_EDGE_DIM 64
-/* attention head counts a GAT or GATv2 model handle accepts */
+/* attention head counts a GAT, GATv2 or TransformerConv model handle accepts */
 #define GNNB_GAT_MAX_HEADS 16
 enum { GNNB_POOL_ADD = 0, GNNB_POOL_MEAN = 1, GNNB_POOL_MAX = 2 };
 
@@ -104,12 +111,13 @@ typedef struct gnnb_model_desc {
     int32_t edge_dim;       /* GINE: edge feature width, 1..GNNB_GINE_MAX_EDGE_DIM.  GAT: 0 for no
                                edge features, else 1..GNNB_GINE_MAX_EDGE_DIM (edge attention), so
                                C callers of GAT must set it to 0 for plain GAT (zero-initialising
-                               the struct does).  GATv2: as GAT.  Read only when conv_type is
-                               GNNB_CONV_GINE, GNNB_CONV_GAT or GNNB_CONV_GATV2, so a caller built
-                               against a header without it keeps working for the other convs. */
-    int32_t gat_heads;      /* GAT and GATv2 only: heads H, 1..GNNB_GAT_MAX_HEADS; every layer's
-                               output width must be a multiple of H (C = width / H channels per
-                               head) */
+                               the struct does).  GATv2 and TransformerConv: as GAT.  Read only
+                               when conv_type is GNNB_CONV_GINE, GNNB_CONV_GAT, GNNB_CONV_GATV2 or
+                               GNNB_CONV_TRANSFORMER, so a caller built against a header without it
+                               keeps working for the other convs. */
+    int32_t gat_heads;      /* GAT, GATv2 and TransformerConv only: heads H, 1..GNNB_GAT_MAX_HEADS;
+                               every layer's output width must be a multiple of H (C = width / H
+                               channels per head) */
     float gat_negative_slope;  /* GAT and GATv2 only: LeakyReLU slope of the attention logits (PyG:
                                   0.2).  Both fields are read only when conv_type is GNNB_CONV_GAT
                                   or GNNB_CONV_GATV2. */
@@ -164,9 +172,9 @@ int gnnb_model_run_batch(gnnb_model_t *m, const float *x, const int32_t *edge_li
 int gnnb_model_run_batch_async(gnnb_model_t *m, const float *x, const int32_t *edge_list,
                                const int64_t *node_ptr, const int64_t *edge_ptr, int n_graphs,
                                int64_t total_nodes, int64_t total_edges, float *out, void *stream);
-/* GINE models, and GAT and GATv2 models with edge_dim > 0: the same contracts as gnnb_model_run_batch /
- * gnnb_model_run_batch_async, plus edge_attr float [edge_ptr[G]][edge_dim] in the memory space of
- * the other buffers, row i the features of COO edge i (one row per stored direction).  Such a handle
+/* GINE models, and GAT, GATv2 and TransformerConv models with edge_dim > 0: the same contracts as
+ * gnnb_model_run_batch / gnnb_model_run_batch_async, plus edge_attr float [edge_ptr[G]][edge_dim] in
+ * the memory space of the other buffers, row i the features of COO edge i (one row per stored direction).  Such a handle
  * must be run through these two; a handle without edge features is rejected by them
  * (GNNB_ERR_INVALID), and so is a null edge_attr with edges present. */
 int gnnb_model_run_batch_edges(gnnb_model_t *m, const float *x, const int32_t *edge_list,
